@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: ``change_basis`` (four-index transform + one-body) in FP64.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One *step* = one ``change_basis(C)`` pass over one synthetic basis set.  The workload follows BASELINE.json:
 
@@ -27,6 +27,11 @@ through the public API from HOST arrays (H2D of the step's inputs and D2H of its
 ``cpu_baseline`` = the numpy oracle (the reference's own call sequence) on the box's host cores.
 
 ``--impl reference`` times that CPU path alone, all host threads.
+
+``--dump-outputs DIR`` (one GPU) writes what the headline leg's caller holds after its last timed step as float64
+``.npy`` files: ``h`` and ``s`` whole, ``u`` as a fixed seeded sample of its elements (``u_sample``) with their flat
+indices (``u_sample_index``).  The inputs are seeded, so two builds run with the same arguments can be compared
+file for file.
 """
 
 import argparse
@@ -58,7 +63,14 @@ def parse_args():
     ap.add_argument("--legs", default="", help="comma list restricting the sharded legs (development): c5,c4,weak")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the headline leg's outputs after its last timed step to DIR/<name>.npy (one GPU only)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs is implemented for the one-GPU workload of --impl ours")
+    return args
 
 
 def transform_flops(n, m=None, kappa=1):
@@ -243,6 +255,30 @@ def workload_name_single(n):
     return f"configs[1]: synthetic real FP64 BasisSet l={n}, random orthonormal C, change_basis on 1xB200"
 
 
+DUMP_U_SAMPLE = 1 << 21  # at most 2^21 elements of u (16 MB of values + 16 MB of indices; u is 2.1 GB at n = 128)
+
+
+def dump_outputs(directory, basis):
+    """``--dump-outputs``: ``h``, ``s`` and a fixed seeded sample of ``u`` (all of it when small enough) as float64."""
+    import numpy as np
+    import torch
+
+    u = basis.u.reshape(-1)
+    if u.numel() <= DUMP_U_SAMPLE:
+        index = np.arange(u.numel())
+    else:
+        index = np.unique(np.random.default_rng(0).integers(0, u.numel(), DUMP_U_SAMPLE))
+    arrays = {
+        "h": basis.h.cpu().numpy(),
+        "s": basis.s.cpu().numpy(),
+        "u_sample": u[torch.from_numpy(index).to(u.device)].cpu().numpy(),
+        "u_sample_index": index,
+    }
+    os.makedirs(directory, exist_ok=True)
+    for name, array in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(array, dtype=np.float64))
+
+
 # ------------------------------------------------------------------------------------------------
 # clocks
 # ------------------------------------------------------------------------------------------------
@@ -397,6 +433,8 @@ def run_single(args, torch, lib):
         ops.EXPLOIT_SYMMETRY = True
     ms_per_step = ms / args.steps
     value = flops / (ms_per_step * 1e-3) * 1e-12
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, basis)
 
     # ---- leg 1b: the default API path (exact symmetry of u detected on the device, mirror tiles skipped) ----
     basis = fresh_basis()
@@ -465,7 +503,7 @@ def run_single(args, torch, lib):
             d2h = sum(a.nbytes for a in (host_basis.h, host_basis.s, host_basis.u))
             return seconds, d2h
 
-        e2e_steps = min(args.steps, 10)
+        e2e_steps = args.steps
         pinned_in = {k: pinned(v) for k, v in inputs.items()}
         h2d = sum(a.nbytes for a in pinned_in.values())
         e2e_s, d2h = e2e_loop(pinned_in, e2e_steps)
@@ -737,7 +775,7 @@ def run_sharded_leg(spec, args, ctx, torch, dist, lib, peak_tflops, with_e2e):
         host_slab = torch.empty((max(sp1 - sp0, 0), l, l, l), dtype=torch.float64, pin_memory=True)
         host_slab.copy_(slab["u"])
         host_f = torch.empty((n, n), dtype=dtype, pin_memory=True)
-        e2e_steps = min(args.steps, 10)
+        e2e_steps = args.steps
         out = {}
 
         def e2e_step():
