@@ -99,17 +99,28 @@ ANTISYMMETRIC_LAST_PAIR = 1  # u[p,q,r,s] = -u[p,q,s,r]
 PARTICLE_EXCHANGE = 2        # u[p,q,r,s] =  u[q,p,s,r]
 
 
+def _mark_written(t):
+    """A kernel of this library has written into ``t``, a tensor the caller supplied: bump torch's in-place version
+    counter (shared by ``t``, its base and every other view of it) so that what the library remembers about the old
+    contents -- the symmetry tag, the imaginary-part cache -- is void, exactly as after an in-place torch op."""
+    torch.autograd.graph.increment_version(t)
+    return t
+
+
 def _tag_symmetry(t, kind):
     """Remember on the tensor object that the library itself has just made ``t`` EXACTLY (anti-)symmetric (mirror
     fill, fused anti-symmetrisation).  The tag carries torch's in-place version counter: any later in-place
-    modification through torch bumps ``t._version`` and voids it, and a new tensor (copy, host round trip, the
-    ``u`` setter of a host array) never has it -- then the device-side test runs again."""
+    modification through torch or through this library (``_mark_written``) bumps ``t._version`` and voids it, and a
+    new tensor (copy, host round trip, the ``u`` setter of a host array) never has it -- then the device-side test
+    runs again."""
     t._qs_symmetry = (int(kind), t._version)
     return t
 
 
 def proven_symmetry(t):
-    """The symmetry kind the library has proven for this very tensor object, or 0."""
+    """The symmetry kind the library has proven for this very tensor object, or 0.  Writes that bypass torch's
+    version counter are not seen: ``t.data``, DLPack or ``__cuda_array_interface__`` consumers writing into the
+    memory of ``t`` leave a stale proof behind."""
     tag = getattr(t, "_qs_symmetry", None)
     return tag[0] if tag is not None and tag[1] == t._version else 0
 
@@ -217,7 +228,7 @@ def quarter_transform(A, X, K, lda, image, m_dtype, W, out, x_inner, sx0, sx1, w
         "qs_quarter_transform", _ptr(A), _code(A), X, K, lda, _ptr(image), _DTYPES[m_dtype], W, _ptr(out), x_inner,
         sx0, sx1, w_inner, sw0, sw1, _stream(),
     )
-    return out
+    return _mark_written(out)
 
 
 def add_spin_two_body(u, anti_symmetrize=False, out_dtype=None, planes=None, out=None, first_spatial_plane=0):
@@ -239,6 +250,8 @@ def add_spin_two_body(u, anti_symmetrize=False, out_dtype=None, planes=None, out
         )
     if out is None:
         out = torch.empty((p1 - p0, 2 * l, 2 * l, 2 * l), dtype=out_dtype, device=u.device)
+    else:
+        _mark_written(out)
     # the kernel addresses spatial plane p at base + p * l^3: hand it the (virtual) base of the whole tensor
     base = ctypes.c_void_p(u.data_ptr() - first_spatial_plane * l**3 * u.element_size())
     _native.call(
@@ -289,6 +302,7 @@ def _fock(name, h, u, n_occ, f):
             raise RuntimeError("f must be a contiguous CUDA tensor to be filled in place")
         if f.shape != h.shape or f.dtype != h.dtype:
             raise ValueError("f must have the shape and dtype of h")
+        _mark_written(f)
     _native.call(name, _ptr(h), _code(h), _ptr(u), _code(u), n, int(n_occ), _ptr(f), 0, n, _stream())
     return f
 
@@ -400,6 +414,8 @@ def fock_gathered(h, direct, exchange, n_occ, scale_direct, scale_exchange, f=No
     n = h.shape[0]
     if f is None:
         f = torch.empty_like(h)
+    else:
+        _mark_written(f)
     _native.call(
         "qs_fock_gathered", _ptr(h), _code(h), _ptr(direct), _ptr(exchange), _code(direct), n, int(n_occ),
         float(scale_direct), float(scale_exchange), _ptr(f), _stream(),
@@ -480,6 +496,8 @@ def scale_add(x, alpha, y=None, beta=0.0, out=None):
         out = torch.empty_like(x)
     elif out.dtype != x.dtype or out.shape != x.shape or not out.is_contiguous():
         raise ValueError("out must be a contiguous tensor of the result's shape and dtype")
+    else:
+        _mark_written(out)
     _native.call(
         "qs_scale_add", _ptr(x), _ptr(y), _code(x), x.numel(), alpha.real, alpha.imag, beta.real, beta.imag,
         _ptr(out), _stream(),

@@ -406,12 +406,28 @@ class ShardedTwoBody:
         self._buffers = buffers  # {rank: [buffer of every rank]}
         self.spare = spare
         self.block, self.offsets = block_partition(n, ctx.world)
-        # True once the library itself has made the tensor EXACTLY anti-symmetric in its last pair (fused spin
-        # doubling, cyclic mirror fill): the transform then skips the device-side test (a full read of u, a host
-        # synchronisation and an all-reduce per call).  Writing through ``local()`` voids it: set it to False.
         self.proven_antisymmetric = False
         # who currently owns a buffer set: a transform that recycles the set invalidates that handle
         _owners(ctx)[id(buffers)] = weakref.ref(self)
+
+    def _slab_versions(self):
+        # as_tensor() is cached per buffer, so every local() view shares its tensor's version counter
+        return tuple(self._buffers[r][r].as_tensor()._version for r in self.ctx.local_ranks)
+
+    @property
+    def proven_antisymmetric(self):
+        """True once the library itself has made the slabs of THIS process EXACTLY anti-symmetric in their last pair
+        (fused spin doubling, cyclic mirror fill): the transform then skips the device-side read of them.  Setting it
+        stamps the version counters of the local slabs; any write through torch into ``local()`` (or through an
+        ``ops`` entry point with ``out=local()``) bumps a counter and voids the proof, reads keep it.  Writes that
+        bypass torch (raw pointers) are not seen.  The proof is local: with one process per rank, a write on some ranks
+        voids it on those ranks only, so the transform combines the ranks' answers in one all-reduce
+        (``is_antisymmetric_last_pair(trust_proof=True)``) and every rank takes the same schedule."""
+        return self._proof is not None and self._buffers is not None and self._proof == self._slab_versions()
+
+    @proven_antisymmetric.setter
+    def proven_antisymmetric(self, value):
+        self._proof = self._slab_versions() if value else None
 
     @property
     def buffers(self):
@@ -692,8 +708,11 @@ class _RankTransform:
         # region of this source in destination j: behind the regions of the sources before it
         dests = [(recv[j], a0 * self.r_count(j) * m * P) for j in range(self.ctx.world)]
         if pairs_only and MASK_FIRST_EXCHANGE and not self.tile_start:
+            # the tiles sent here must cover the pairs of the (cached) tables steps 3 and 4 read
+            self.prepare_pairs()
+            assert self.rows_paired == self.pairs_padded(), "cached pair tables of another T2 dtype"
             eng.quarter_scatter_pairs(self.scratch, m * A * n, n, P, self.img2, self.c_dtype, m, dests, n, A, 1, P,
-                                      A * P, m * A * P, A * n, self.pairs_padded())
+                                      A * P, m * A * P, A * n, self.rows_paired)
             return
         eng.quarter_scatter(self.scratch, m * A * n, n, P, self.img2, self.c_dtype, m, dests, n, A, 1, P, A * P,
                             0, m * A * P, deal=1, cyclic=True, tile_start=self.tile_start)
@@ -756,9 +775,10 @@ class _RankTransform:
         import numpy
 
         m, R, P, W = self.m, self.R, self.P, self.ctx.world
-        # shape-dependent only: built and uploaded once per (rank, n, m, world, P), then reused by every transform
+        # built and uploaded once per (rank, n, m, world, P, dtype of T2), then reused by every transform; the dtype
+        # decides whether the lists are padded to aligned couples (pairs_padded)
         cache = self.ctx.__dict__.setdefault("_pair_tables", {})
-        key = (self.rank, self.n, m, W, P, self.cyclic)
+        key = (self.rank, self.n, m, W, P, self.cyclic, self.t_dtype)
         if key in cache:
             (self.npairs, self.step3_tables, self.rs_of_pair, self.rs_of_pair_dev, self.rows_paired) = cache[key]
             return
@@ -836,14 +856,18 @@ def _slice(buf, offset, numel):
     return buf.slice(offset, numel)
 
 
-def is_antisymmetric_last_pair(u):
+def is_antisymmetric_last_pair(u, trust_proof=False):
     """Exact, collective test of ``u[p,q,r,s] == -u[p,q,s,r]`` on a ``ShardedTwoBody``: every rank tests its own
-    planes on the device (``qs_is_antisymmetric_last_pair``), the flags are combined with a one-element all-reduce."""
+    planes on the device (``qs_is_antisymmetric_last_pair``), the flags are combined with a one-element all-reduce.
+    ``trust_proof``: a process whose slabs carry the library's proof (``proven_antisymmetric``) skips the read of its
+    planes but still takes part in the all-reduce, so every rank returns the same answer after the same collectives."""
     ctx = u.ctx
-    ok = True
-    for r in ctx.local_ranks:
-        p0, p1 = u.planes(r)
-        ok = ok and ctx.engine.is_antisymmetric(u.buffers[r][r], u.n, p1 - p0)
+    ok = trust_proof and u.proven_antisymmetric
+    if not ok:
+        ok = True
+        for r in ctx.local_ranks:
+            p0, p1 = u.planes(r)
+            ok = ok and ctx.engine.is_antisymmetric(u.buffers[r][r], u.n, p1 - p0)
     if isinstance(ctx, ProcessContext) and ctx.world > 1:
         flag = torch.tensor([1.0 if ok else 0.0], dtype=torch.float32, device="cuda" if ctx.on_cuda else "cpu")
         ctx.dist.all_reduce(flag, op=ctx.dist.ReduceOp.MIN, group=ctx.group)
@@ -869,7 +893,7 @@ def transform_two_body_sharded(u, C, C_tilde=None, symmetry=None):
         raise ValueError(f"C has {n} rows but u has {u.n} orbitals")
     if symmetry is None:
         symmetry = 1 if (EXPLOIT_SYMMETRY and ctx.exchange == "peer" and min(n, m) >= SYMMETRY_MIN_N
-                         and (u.proven_antisymmetric or is_antisymmetric_last_pair(u))) else 0
+                         and is_antisymmetric_last_pair(u, trust_proof=True)) else 0
     if symmetry and ctx.exchange != "peer":
         raise ValueError("the symmetry-aware sharded transform needs the peer exchange")
     work = {r: _RankTransform(ctx, r, n, m, u.dtype, C.dtype) for r in ctx.local_ranks}
