@@ -13,7 +13,7 @@
 //     32 x (8*NT) accumulator tile each in registers) issue mma.sync m8n8k4 f64 (SASS DMMA.8x8x4; measured
 //     16 clk issue interval per sub-partition, 26 clk latency) on alternate tiles, each fed by its own TMA
 //     producer warp over its own full/empty mbarrier stage ring; the producer warp group donates registers
-//     (setmaxnreg 24 / 240); tile starts are ordered so one group's epilogue overlaps the other's main loop
+//     (setmaxnreg 40 / 232); tile starts are ordered so one group's epilogue overlaps the other's main loop
 //     (details above quarter_gemm_kernel);
 //   * the epilogue writes the new index as the slowest axis (or any 2-level strided address).
 #include <stdlib.h>
@@ -40,12 +40,24 @@ constexpr int kGroupWarps = 4;  // one warp per SM sub-partition
 constexpr int kMmaWarps = kGroups * kGroupWarps;
 constexpr int kThreads = (kMmaWarps + 4) * 32;  // + the producer warp group (register donor, one lane issues TMA)
 // Register split (setmaxnreg, whole warp groups): the kernel launches with 168 registers per thread
-// (65536 / 384); the producer group shrinks to 24 and each MMA group grows to 240 (2 x 128 x 240 + 128 x 24 = 384 x 168).
-constexpr int kRegsProducer = 24;
-constexpr int kRegsMma = 240;
+// (65536 / 384); the producer group shrinks to 40 and each MMA group grows to 232 (2 x 128 x 232 + 128 x 40 <= 384 x 168).
+// At 24 the producer's tile loop spills to local memory; 232 still holds every NT = 8 instantiation without spills.
+constexpr int kRegsProducer = 40;
+constexpr int kRegsMma = 232;
 constexpr int kATileBytes = kBlockX * kChunkK * 8;  // 16 KiB
 
 constexpr int kMaxDest = 16;    // destination buffers of a scattering store (ranks of one NVSwitch domain)
+
+// Unsigned division by a launch constant d >= 1 of numerators below 2^31 as a multiply and a shift: with
+// l = ceil(log2 d), shift = 31 + l and mul = ceil(2^shift / d) < 2^32, the error e = mul d - 2^shift < d makes
+// x e < 2^31 2^l = 2^shift, so (x mul) >> shift == x / d exactly (make_divisor on the host).
+struct Divisor {
+    uint32_t mul, shift;
+};
+
+__device__ __forceinline__ uint32_t divide(uint32_t x, Divisor d) {
+    return (uint32_t)(((unsigned long long)x * d.mul) >> d.shift);
+}
 
 struct QuarterParams {
     const double* image;      // [tiles_w][nchunks][2][NT][32][2] doubles (this launch's tile group)
@@ -64,6 +76,7 @@ struct QuarterParams {
     // store address = (w/w_inner)*sw1 + (w%w_inner)*sw0 + x2*sx2 + x1*sx1 + x0*sx0 with
     // x = (x2 * x_mid + x1) * x_inner + x0, in OUTPUT ELEMENTS (w = w' for real output, w'/2 for complex)
     uint32_t x_inner, x_mid, w_inner;
+    Divisor x_inner_div, tiles_w_div;
     long long sx0, sx1, sx2, sw0, sw1;
     int vec2;                 // real output: row pairs (x, x + 1), x even, are adjacent and 16-byte aligned
     int bulk;                 // staged asynchronous epilogue (BULK kernels): consecutive rows of a block are adjacent
@@ -112,6 +125,30 @@ __device__ __forceinline__ uint32_t tile_at(const QuarterParams& p, uint32_t k, 
 #define QS_FULL_WAIT(bar, par) mbar_wait(bar, par)
 #endif
 
+#ifdef QS_DBG_PHASE_CLOCKS
+// Development switch (tools/qgemm_bench.cu): every MMA warp of quarter_gemm_kernel stamps clock64() at tile start, at
+// the start of the main loop (after the ordered-start wait), at the end of the main loop and at the end of the
+// epilogue (which includes the wait for the next tile's first chunk and its fragment loads), and adds the three phase
+// lengths to histograms of kPhaseBinClk-clock bins.  Not part of a default build.
+constexpr int kPhaseBins = 256, kPhaseBinClk = 256;
+__device__ unsigned long long g_phase_hist[3][kPhaseBins];
+__device__ unsigned long long g_phase_sum[3];
+__device__ unsigned long long g_phase_count;
+__device__ __forceinline__ void phase_record(int lane, const long long (&t)[4]) {
+    if (lane != 0) return;
+    for (int ph = 0; ph < 3; ++ph) {
+        const unsigned long long d = (unsigned long long)(t[ph + 1] - t[ph]);
+        const unsigned long long bin = d / kPhaseBinClk;
+        atomicAdd(&g_phase_hist[ph][bin < kPhaseBins ? bin : kPhaseBins - 1], 1ull);
+        atomicAdd(&g_phase_sum[ph], d);
+    }
+    atomicAdd(&g_phase_count, 1ull);
+}
+#define QS_PHASE_STAMP(i) (phase_t[i] = clock64())
+#else
+#define QS_PHASE_STAMP(i) ((void)0)
+#endif
+
 // Row ownership inside a warp's 32 x 8NT tile: MMA row g of m-tile mt is tile row
 //     row_base(g) + (mt & 1) + 16 * (mt >> 1),      row_base = {0, 4, 2, 6, 8, 12, 10, 14}[g].
 // (a) the two row groups of a quarter-warp (g = 2q, 2q + 1) differ in bit 2, so the TMA-swizzled LDS.128 fragment
@@ -156,9 +193,19 @@ struct RingConfig {
 // contiguous in the output (256 bytes for a real, 512 bytes for a complex column) to the copy engine with
 // cp.async.bulk shared -> global.  The warp goes on to its next tile while the copies drain: the stores -- over
 // NVLink in the scattering launches -- no longer hold the tensor pipe through the depth of the store queue.
-template <int NT, bool COMPLEX_OUT, bool BULK>
+// ROTATED: the local rotated store of the dense transforms (one destination, no dealing, no row tables, x_mid
+// unused, sx0 = 1, 16-byte row pairs for real output), element (x, w) at w sw1 + (x / x_inner) sx1 + x % x_inner.  It
+// carries none of the other addressing modes, so the kernel the headline transform runs is small and keeps no
+// per-launch branches in its epilogue.
+// Cross-tile pipelining: after its main loop a warp waits for the first chunk of its NEXT tile and loads that chunk's
+// first A and B fragments (registers that are dead in the epilogue) before it stores the current tile, so its DMMA
+// stream restarts right behind the stores.
+enum Epilogue { kEpiStrided = 0, kEpiBulk = 1, kEpiRotated = 2 };
+
+template <int NT, bool COMPLEX_OUT, int EPI>
 __global__ void __launch_bounds__(kThreads, 1)
 quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ QuarterParams p) {
+    constexpr bool BULK = EPI == kEpiBulk;
     using Ring = RingConfig<NT, BULK>;
     constexpr int kBTileBytes = Ring::kBTileBytes;
     constexpr int kStageBytes = Ring::kStageBytes;
@@ -201,8 +248,9 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             uint32_t j = 0;
             for (uint32_t i = pg; i < my_tiles; i += kGroups) {
                 const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x, total_tiles);
-                const uint32_t tw = tile % (uint32_t)p.tiles_w;
-                const int px0 = (int)((tile / (uint32_t)p.tiles_w) * kBlockX);
+                const uint32_t tx = divide(tile, p.tiles_w_div);
+                const uint32_t tw = tile - tx * (uint32_t)p.tiles_w;
+                const int px0 = (int)(tx * kBlockX);
                 const double* img = p.image + (size_t)tw * p.nchunks * (kBTileBytes / 8);
                 for (int c = 0; c < p.nchunks; ++c, ++j) {
                     const uint32_t s = j % kStages;
@@ -264,7 +312,23 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 #endif
 
     uint32_t bulk_pass = 0;  // BULK: staging passes done so far (selects the buffer, bounds the pending copy groups)
+#ifdef QS_DBG_PHASE_CLOCKS
+    long long phase_t[4];
+#endif
+    // The group's tiles take consecutive chunks of its ring: chunk j sits in stage s = j % kStages, phase parity
+    // par = (j / kStages) & 1.  a0 and b hold the first fragments of the chunk about to start.
+    uint32_t s = 0, par = 0;
+    uint32_t stage = ring;
+    double2 a0[4], a1[4], b[NT];
+    auto load_first = [&]() {
+        QS_FULL_WAIT(bar_full + 8 * s, par);
+        load_a(a0, stage, 0);
+#pragma unroll
+        for (int nt = 0; nt < NT; ++nt) b[nt] = load_b(stage, 0, nt);
+    };
+    if ((uint32_t)group < my_tiles) load_first();
     for (uint32_t i = group; i < my_tiles; i += kGroups) {
+        QS_PHASE_STAMP(0);
         const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x, total_tiles);
 
         double acc[4][NT][2];
@@ -302,16 +366,6 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             }
         };
 
-        // chunk j of this group's ring: stage s, phase parity par
-        const uint32_t j = (i >> 1) * (uint32_t)p.nchunks;
-        uint32_t s = j % kStages, par = (j / kStages) & 1;
-        uint32_t stage = ring + s * kStageBytes;
-        double2 a0[4], a1[4], b[NT];
-        QS_FULL_WAIT(bar_full + 8 * s, par);
-        load_a(a0, stage, 0);
-#pragma unroll
-        for (int nt = 0; nt < NT; ++nt) b[nt] = load_b(stage, 0, nt);
-
         // ordered start: the other group has passed the signal point (midpoint) of the main loop of tile i - 1
         const uint32_t k = i >> 1;
         if (i > 0) mbar_wait(bar_order + 8 * group, (group == 0 ? k - 1 : k) & 1);
@@ -322,6 +376,7 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 #else
         const int signal_chunk = (p.nchunks - 1) >> 1;
 #endif
+        QS_PHASE_STAMP(1);
 
         bool tail = false;  // b[NT - 1] of the half about to start is still to be fetched
         for (int c = 0; c + 1 < p.nchunks; ++c) {
@@ -361,6 +416,14 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             mbar_arrive(bar_empty + 8 * s);
             if (signal_chunk == p.nchunks - 1) mbar_arrive(bar_order + 8 * (group ^ 1));
         }
+        QS_PHASE_STAMP(2);
+        // the next tile's first chunk follows in the ring; its fragments load while this tile is stored
+        if (++s == (uint32_t)kStages) {
+            s = 0;
+            par ^= 1;
+        }
+        stage = ring + s * kStageBytes;
+        if (i + kGroups < my_tiles) load_first();
 
         // ===== epilogue: rotated / strided / scattering store straight from the accumulators =====
 #ifdef QS_DBG_NOSTORE
@@ -371,11 +434,16 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 #pragma unroll
                 for (int nt = 0; nt < NT; ++nt) sum += acc[mt][nt][0] + acc[mt][nt][1];
             if (sum == 1.2345e-300) p.out[0] = sum;
+#ifdef QS_DBG_PHASE_CLOCKS
+            QS_PHASE_STAMP(3);
+            phase_record(lane, phase_t);
+#endif
             continue;
         }
 #endif
-        const uint32_t tile_w = tile % (uint32_t)p.tiles_w;
-        const uint32_t x0 = (tile / (uint32_t)p.tiles_w) * kBlockX;
+        const uint32_t tile_x = divide(tile, p.tiles_w_div);
+        const uint32_t tile_w = tile - tile_x * (uint32_t)p.tiles_w;
+        const uint32_t x0 = tile_x * kBlockX;
         const uint32_t wbase = p.w_first + tile_w * (8 * NT);
         const bool plain_w = p.w_inner == 1 && p.ndest == 0;  // plain rotated store: column address = w * sw1
         if constexpr (BULK) {
@@ -388,7 +456,7 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             // are adjacent in the output (sx0 = 1): one run per block
             const uint32_t xw0 = x0 + 32 * wg;
             const uint32_t nrow = xw0 < p.X ? (p.X - xw0 < 32u ? p.X - xw0 : 32u) : 0u;
-            const uint32_t xq0 = xw0 / p.x_inner;
+            const uint32_t xq0 = divide(xw0, p.x_inner_div);
             const uint32_t xr0 = xw0 - xq0 * p.x_inner;
             const uint32_t nruns = nrow ? (xr0 + nrow + p.x_inner - 1) / p.x_inner : 0u;
             const uint32_t items = CPP * nruns;              // (column, run) pairs per pass
@@ -459,6 +527,45 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                 asm volatile("cp.async.bulk.commit_group;" ::: "memory");
             }
             bulk_pass += PASSES;
+        } else if constexpr (EPI == kEpiRotated) {
+            // rows x = xt + (mt & 1) + 16 (mt >> 1) of this thread; for real output the row pairs (xt, xt + 1) and
+            // (xt + 16, xt + 17) share a block (xt and x_inner are even) and leave as one 16-byte store each
+            const uint32_t xt = x0 + 32 * wg + rbase;
+            constexpr int NX = COMPLEX_OUT ? 4 : 2;
+            long long xoff[NX];
+            bool xok[NX];
+#pragma unroll
+            for (int r = 0; r < NX; ++r) {
+                const uint32_t x = COMPLEX_OUT ? xt + (r & 1) + 16 * (r >> 1) : xt + 16 * r;
+                const uint32_t xq = divide(x, p.x_inner_div);
+                xok[r] = x < p.X;
+                xoff[r] = (long long)xq * p.sx1 + (long long)(x - xq * p.x_inner);
+            }
+#pragma unroll
+            for (int nt = 0; nt < NT; ++nt) {
+                const uint32_t wp = wbase + 8 * nt + 2 * t;  // real column of acc[..][nt][0]; wp + 1 for [1]
+                if (COMPLEX_OUT) {
+                    if (wp < p.Wp) {
+                        double* col = p.out + 2 * ((long long)(wp >> 1) * p.sw1);
+#pragma unroll
+                        for (int mt = 0; mt < 4; ++mt)
+                            if (xok[mt])
+                                *reinterpret_cast<double2*>(col + 2 * xoff[mt]) = make_double2(acc[mt][nt][0], acc[mt][nt][1]);
+                    }
+                } else {
+#pragma unroll
+                    for (int e = 0; e < 2; ++e) {
+                        if (wp + e < p.Wp) {
+                            double* col = p.out + (long long)(wp + e) * p.sw1;
+#pragma unroll
+                            for (int r = 0; r < 2; ++r)
+                                if (xok[r])
+                                    *reinterpret_cast<double2*>(col + xoff[r]) =
+                                        make_double2(acc[2 * r][nt][e], acc[2 * r + 1][nt][e]);
+                        }
+                    }
+                }
+            }
         } else {
         long long xoff[4];
         bool xok[4];
@@ -466,7 +573,7 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         for (int mt = 0; mt < 4; ++mt) {
             const uint32_t x = x0 + 32 * wg + rbase + (mt & 1) + 16 * (mt >> 1);
             xok[mt] = x < p.X;
-            const uint32_t xq = x / p.x_inner;
+            const uint32_t xq = divide(x, p.x_inner_div);
             const uint32_t xr = x - xq * p.x_inner;
             long long off = (p.xr_table && xok[mt]) ? p.xr_table[xr] : (long long)xr * p.sx0;
             if (p.x_mid != 0xFFFFFFFFu) {
@@ -528,6 +635,10 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             }
         }
         }  // register-store epilogue
+#ifdef QS_DBG_PHASE_CLOCKS
+        QS_PHASE_STAMP(3);
+        phase_record(lane, phase_t);
+#endif
     }
     // the staging buffers must outlive the copies that read them; completion also orders the stores before the exit
     if constexpr (BULK) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
@@ -598,8 +709,9 @@ quarter_gemm_split_kernel(const __grid_constant__ CUtensorMap map_a, const __gri
             uint32_t j = 0;
             for (uint32_t i = pg; i < my_tiles; i += kGroups) {
                 const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x, total_tiles);
-                const uint32_t tw = tile % (uint32_t)p.tiles_w;
-                const int px0 = (int)((tile / (uint32_t)p.tiles_w) * kBlockX);
+                const uint32_t tx = divide(tile, p.tiles_w_div);
+                const uint32_t tw = tile - tx * (uint32_t)p.tiles_w;
+                const int px0 = (int)(tx * kBlockX);
                 const double* img = p.image + (size_t)tw * p.nchunks * (kBTileBytes / 8);
                 for (int c = 0; c < p.nchunks; ++c, ++j) {
                     const uint32_t s = j % kStages;
@@ -709,15 +821,16 @@ quarter_gemm_split_kernel(const __grid_constant__ CUtensorMap map_a, const __gri
         }
 
         // ===== epilogue: complex128 (re, im) pairs, rotated / strided / scattering store =====
-        const uint32_t tile_w = tile % (uint32_t)p.tiles_w;
-        const uint32_t x0 = (tile / (uint32_t)p.tiles_w) * kBlockX;
+        const uint32_t tile_x = divide(tile, p.tiles_w_div);
+        const uint32_t tile_w = tile - tile_x * (uint32_t)p.tiles_w;
+        const uint32_t x0 = tile_x * kBlockX;
         long long xoff[4];
         bool xok[4];
 #pragma unroll
         for (int mt = 0; mt < 4; ++mt) {
             const uint32_t x = x0 + 32 * wg + rbase + (mt & 1) + 16 * (mt >> 1);
             xok[mt] = x < p.X;
-            const uint32_t xq = x / p.x_inner;
+            const uint32_t xq = divide(x, p.x_inner_div);
             const uint32_t xr = x - xq * p.x_inner;
             long long off = (p.xr_table && xok[mt]) ? p.xr_table[xr] : (long long)xr * p.sx0;
             if (p.x_mid != 0xFFFFFFFFu) {
@@ -923,35 +1036,35 @@ EncodeTiledFn get_encode_fn() {
     return fn;
 }
 
-template <int NT, bool CO, bool BULK>
+template <int NT, bool CO, int EPI>
 int launch_variant(const CUtensorMap& map, const QuarterParams& p, cudaStream_t st) {
-    constexpr int smem = RingConfig<NT, BULK>::kSmemBytes;
+    constexpr int smem = RingConfig<NT, EPI == kEpiBulk>::kSmemBytes;
     static_assert(smem <= 227 * 1024, "shared memory budget of one CTA per SM");
     static bool configured[kMaxDevices] = {false};  // the attribute belongs to the device's context
     const int dev = qs_current_device();
     if (!configured[dev]) {
-        QS_CUDA(cudaFuncSetAttribute(quarter_gemm_kernel<NT, CO, BULK>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        QS_CUDA(cudaFuncSetAttribute(quarter_gemm_kernel<NT, CO, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         configured[dev] = true;
     }
     const int64_t total = p.tile_list ? (int64_t)p.n_listed : (int64_t)p.tiles_x * p.tiles_w;
     const int64_t resident = qs_sm_count();  // one persistent CTA per SM
     const int64_t grid = total < resident ? total : resident;
-    quarter_gemm_kernel<NT, CO, BULK><<<(unsigned)grid, kThreads, smem, st>>>(map, p);
+    quarter_gemm_kernel<NT, CO, EPI><<<(unsigned)grid, kThreads, smem, st>>>(map, p);
     QS_LAUNCH_CHECK();
     return QS_OK;
 }
 
-template <bool CO, bool BULK>
+template <bool CO, int EPI>
 int launch_nt(int NT, const CUtensorMap& map, const QuarterParams& p, cudaStream_t st) {
     switch (NT) {
-        case 1: return launch_variant<1, CO, BULK>(map, p, st);
-        case 2: return launch_variant<2, CO, BULK>(map, p, st);
-        case 3: return launch_variant<3, CO, BULK>(map, p, st);
-        case 4: return launch_variant<4, CO, BULK>(map, p, st);
-        case 5: return launch_variant<5, CO, BULK>(map, p, st);
-        case 6: return launch_variant<6, CO, BULK>(map, p, st);
-        case 7: return launch_variant<7, CO, BULK>(map, p, st);
-        case 8: return launch_variant<8, CO, BULK>(map, p, st);
+        case 1: return launch_variant<1, CO, EPI>(map, p, st);
+        case 2: return launch_variant<2, CO, EPI>(map, p, st);
+        case 3: return launch_variant<3, CO, EPI>(map, p, st);
+        case 4: return launch_variant<4, CO, EPI>(map, p, st);
+        case 5: return launch_variant<5, CO, EPI>(map, p, st);
+        case 6: return launch_variant<6, CO, EPI>(map, p, st);
+        case 7: return launch_variant<7, CO, EPI>(map, p, st);
+        case 8: return launch_variant<8, CO, EPI>(map, p, st);
     }
     qs_set_error("internal: NT=%d out of range", NT);
     return QS_ERR_INVALID;
@@ -972,6 +1085,23 @@ int launch_split_variant(const CUtensorMap& map, const QuarterParams& p, cudaStr
     quarter_gemm_split_kernel<NTC><<<(unsigned)grid, kThreads, smem, st>>>(map, p);
     QS_LAUNCH_CHECK();
     return QS_OK;
+}
+
+template <bool CO>
+int launch_epilogue(int epi, int NT, const CUtensorMap& map, const QuarterParams& p, cudaStream_t st) {
+    switch (epi) {
+        case kEpiStrided: return launch_nt<CO, kEpiStrided>(NT, map, p, st);
+        case kEpiBulk: return launch_nt<CO, kEpiBulk>(NT, map, p, st);
+        default: return launch_nt<CO, kEpiRotated>(NT, map, p, st);
+    }
+}
+
+// Divisor of d (1 <= d < 2^32) for numerators below 2^31 (see Divisor).
+Divisor make_divisor(uint64_t d) {
+    uint32_t l = 0;
+    while ((1ull << l) < d) ++l;
+    const uint32_t shift = 31 + l;
+    return {(uint32_t)(((1ull << shift) + d - 1) / d), shift};
 }
 
 int launch_split(int NTC, const CUtensorMap& map, const QuarterParams& p, cudaStream_t st) {
@@ -1021,6 +1151,24 @@ extern "C" int qs_set_bulk_epilogue_mode(int mode) {
     if (mode >= 0 && mode <= 2) g_bulk_mode = mode;
     return previous;
 }
+
+#ifdef QS_DBG_PHASE_CLOCKS
+// Copies out the phase histograms (3 x kPhaseBins), the summed phase lengths (3) and the number of warp tiles recorded
+// since the last reset; `reset` zeroes them afterwards.
+extern "C" int qs_dbg_phase_clocks(unsigned long long* hist, unsigned long long* sum, unsigned long long* count,
+                                   int reset) {
+    if (hist) QS_CUDA(cudaMemcpyFromSymbol(hist, g_phase_hist, sizeof(g_phase_hist)));
+    if (sum) QS_CUDA(cudaMemcpyFromSymbol(sum, g_phase_sum, sizeof(g_phase_sum)));
+    if (count) QS_CUDA(cudaMemcpyFromSymbol(count, g_phase_count, sizeof(g_phase_count)));
+    if (reset) {
+        static const unsigned long long zeros[3 * kPhaseBins] = {};
+        QS_CUDA(cudaMemcpyToSymbol(g_phase_hist, zeros, sizeof(g_phase_hist)));
+        QS_CUDA(cudaMemcpyToSymbol(g_phase_sum, zeros, sizeof(g_phase_sum)));
+        QS_CUDA(cudaMemcpyToSymbol(g_phase_count, zeros, sizeof(g_phase_count)));
+    }
+    return QS_OK;
+}
+#endif
 
 extern "C" int qs_coeff_image_bytes(int64_t K, int64_t W, int a_dtype, int m_dtype, int64_t* bytes) {
     QS_REQUIRE(K > 0 && W > 0 && bytes, "qs_coeff_image_bytes: bad arguments");
@@ -1313,6 +1461,11 @@ int quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda
                (n_dest > 0 || sw1 % 2 == 0) && (reinterpret_cast<uintptr_t>(out) & 15) == 0 && (!xq_table || xq_even);
         for (int64_t d = 0; d < n_dest; ++d) bulk = bulk && (reinterpret_cast<uintptr_t>(out_table[d]) & 15) == 0;
     }
+    // The rotated epilogue: one local destination, undealt columns, no row tables, the two-level row split with
+    // adjacent rows, and 16-byte row pairs for real output.
+    const bool rotated = n_dest == 0 && w_deal == 1 && !xq_table && !xr_table && x_mid == 0xFFFFFFFFLL && w_inner == 1 &&
+                         sx0 == 1 && (out_complex || vec2);
+    const int epi = bulk ? kEpiBulk : rotated ? kEpiRotated : kEpiStrided;
 
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     // symmetry mask: per tile group, the ascending list of wanted linear tile ids, staged into list_ws
@@ -1364,6 +1517,8 @@ int quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda
         p.last_halves = tl.last_halves;
         p.tiles_w = gr.tiles_w;
         p.x_inner = (uint32_t)x_inner;
+        p.x_inner_div = make_divisor((uint64_t)x_inner);
+        p.tiles_w_div = make_divisor((uint64_t)gr.tiles_w);
         p.x_mid = (uint32_t)x_mid;
         p.w_inner = (uint32_t)w_inner;
         p.sx0 = sx0;
@@ -1384,8 +1539,8 @@ int quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda
         QS_REQUIRE((int64_t)p.tiles_x * p.tiles_w < (1LL << 31), "qs_quarter_transform: too many tiles");
         p.bulk = bulk;
         const int rc = tl.split      ? launch_split(gr.NT, map, p, st)
-                       : out_complex ? (bulk ? launch_nt<true, true>(gr.NT, map, p, st) : launch_nt<true, false>(gr.NT, map, p, st))
-                                     : (bulk ? launch_nt<false, true>(gr.NT, map, p, st) : launch_nt<false, false>(gr.NT, map, p, st));
+                       : out_complex ? launch_epilogue<true>(epi, gr.NT, map, p, st)
+                                     : launch_epilogue<false>(epi, gr.NT, map, p, st);
         if (rc) return rc;
     }
     qs_timing_end(span, stream);

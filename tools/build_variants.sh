@@ -8,6 +8,8 @@ FLAGS="-gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo"
 build() { name=$1; shift; nvcc $FLAGS "$@" -o tools/variants/$name $SRC & }
 build base
 build nostore -DQS_DBG_NOSTORE
+build phase -DQS_DBG_PHASE_CLOCKS
+build phase_nostore -DQS_DBG_PHASE_CLOCKS -DQS_DBG_NOSTORE
 build noload -DQS_DBG_NOLOAD
 build noload_nostore -DQS_DBG_NOLOAD -DQS_DBG_NOSTORE
 build nolds -DQS_DBG_NOLDS -DQS_DBG_NOSTORE

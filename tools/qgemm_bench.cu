@@ -10,6 +10,13 @@
 
 #include "../include/qsb200.h"
 
+#ifdef QS_DBG_PHASE_CLOCKS
+// exported by quarter_gemm.cu in a -DQS_DBG_PHASE_CLOCKS build only
+extern "C" int qs_dbg_phase_clocks(unsigned long long* hist, unsigned long long* sum, unsigned long long* count,
+                                   int reset);
+constexpr int kPhaseBins = 256, kPhaseBinClk = 256;
+#endif
+
 #define CK(x)                                                                        \
     do {                                                                             \
         cudaError_t e = (x);                                                         \
@@ -58,6 +65,9 @@ int main(int argc, char** argv) {
         for (int i = 0; i < 3; ++i) QK(qs_quarter_transform(A, QS_F64, X, K, K, image, QS_F64, W, out, X, 1, 0, 1, 0, X, 0));
         CK(cudaDeviceSynchronize());
         const int reps = 10;
+#ifdef QS_DBG_PHASE_CLOCKS
+        QK(qs_dbg_phase_clocks(nullptr, nullptr, nullptr, 1));
+#endif
         CK(cudaEventRecord(e0));
         for (int i = 0; i < reps; ++i) QK(qs_quarter_transform(A, QS_F64, X, K, K, image, QS_F64, W, out, X, 1, 0, 1, 0, X, 0));
         CK(cudaEventRecord(e1));
@@ -66,6 +76,26 @@ int main(int argc, char** argv) {
         CK(cudaEventElapsedTime(&ms, e0, e1));
         ms /= reps;
         printf("{\"variant\":\"%s\",\"n\":%d,\"ms\":%.4f,\"tflops\":%.2f}\n", tag, n, ms, 2.0 * X * K * W / ms * 1e-9);
+#ifdef QS_DBG_PHASE_CLOCKS
+        {   // per warp tile: clocks from tile start to main loop (waits), main loop, epilogue; histogram bins as
+            // {"first clock of the bin": warp tiles}
+            std::vector<unsigned long long> hist(3 * kPhaseBins);
+            unsigned long long sum[3], count = 0;
+            QK(qs_dbg_phase_clocks(hist.data(), sum, &count, 0));
+            const char* names[3] = {"start_wait", "main_loop", "epilogue"};
+            for (int ph = 0; ph < 3; ++ph) {
+                printf("{\"variant\":\"%s\",\"n\":%d,\"phase\":\"%s\",\"warp_tiles\":%llu,\"mean_clk\":%.1f,\"hist\":{",
+                       tag, n, names[ph], count, count ? (double)sum[ph] / count : 0.0);
+                bool first = true;
+                for (int b = 0; b < kPhaseBins; ++b)
+                    if (hist[ph * kPhaseBins + b]) {
+                        printf("%s\"%d\":%llu", first ? "" : ",", b * kPhaseBinClk, hist[ph * kPhaseBins + b]);
+                        first = false;
+                    }
+                printf("}}\n");
+            }
+        }
+#endif
         cudaFree(A); cudaFree(out); cudaFree(M); cudaFree(image);
     }
     return 0;
