@@ -282,6 +282,19 @@ int qs_fock_general_cols(const void* h, int h_dtype, const void* u_cols, int u_d
 int qs_fock_gathered(const void* h, int h_dtype, const void* direct, const void* exchange,
                      int u_dtype, int64_t n, int64_t n_occ, double scale_direct,
                      double scale_exchange, void* f, void* stream);
+/* Fock matrix from a general density matrix rho (n, n), the O(n^4) step of a Hartree-Fock iteration:
+ *   f[p,q] = h[p,q] + scale_direct   * sum_{r,s} u[p,r,q,s] rho[s,r]
+ *                   + scale_exchange * sum_{r,s} u[p,r,s,q] rho[s,r]          for p in [p_begin, p_end)
+ * `u` points at plane p_begin: the (p_end - p_begin, n, n, n) slab u[p_begin:p_end]; h, rho, f are whole (n, n)
+ * matrices and rows of f outside [p_begin, p_end) are not touched.  h, u, rho may each be F64 or C128; f_dtype
+ * must be C128 when any of them is.  Every element of u is read once.  Deterministic (no atomics): per-(plane,
+ * r-chunk) partial rows go to the workspace (qs_fock_density_workspace_bytes) and are summed in a fixed order; the
+ * chunking depends on n only, so a row is bit-identical whatever plane range it is computed in. */
+int qs_fock_density_workspace_bytes(int64_t n, int64_t p_begin, int64_t p_end, int u_dtype, int rho_dtype,
+                                    int64_t* bytes);
+int qs_fock_density(const void* h, int h_dtype, const void* u, int u_dtype, const void* rho, int rho_dtype,
+                    int64_t n, double scale_direct, double scale_exchange, void* f, int f_dtype,
+                    int64_t p_begin, int64_t p_end, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * ODQD grid Coulomb build  u_abcd = sum_pq C_pa C_qb C_pc C_qd alpha/sqrt((x_p-x_q)^2 + a^2)

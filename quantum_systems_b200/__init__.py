@@ -18,6 +18,7 @@ from .random_basis import RandomBasisSet
 from .odqd import ODHO, ODQD
 from .sinc_dvr import ODSincDVR
 from . import time_evolution_operators  # noqa: F401
+from . import hartree_fock  # noqa: F401
 from . import two_dim_ho  # noqa: F401
 from .two_dim_ho import (
     get_coulomb_elements,
@@ -41,5 +42,6 @@ __all__ = [
     "TwoDimSmoothDoubleWell",
     "TwoDimHarmonicOscB",
     "get_coulomb_elements",
+    "hartree_fock",
     "xp",
 ]

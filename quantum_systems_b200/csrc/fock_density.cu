@@ -1,0 +1,272 @@
+// Fock matrix from a general density matrix (the O(n^4) step of a Hartree-Fock iteration):
+//
+//   f[p,q] = h[p,q] + a_d sum_{r,s} u[p,r,q,s] rho[s,r] + a_x sum_{r,s} u[p,r,s,q] rho[s,r],   p in [p_begin, p_end)
+//
+// For fixed (p, r) the block B = u[p,r,:,:] is contiguous (rows q, columns s).  The direct term of row q is the dot
+// product B[q,:] . rho[:,r]; the exchange term of column q is the weighted column sum sum_s rho[s,r] B[s,q].  Both
+// come from the same coalesced 16-byte loads of B, so every element of u is read from HBM once.
+//
+// Pass 1: one CTA per (plane p, chunk of r).  A warp owns the rows q = warp, warp + 8, ...; its lanes sweep the
+// columns of a row in 16-byte pieces.  The direct partial of row q accumulates in the lane over the r of the chunk
+// and is reduced with a warp butterfly once per (q, column block); the exchange partials of the lane's columns stay
+// in registers over all rows and r, and the 8 warps are summed through shared memory in warp order.  The chunk's
+// partial row a_d D + a_x X goes to the caller's workspace.
+// Pass 2: f[p,q] = h[p,q] + sum over chunks in chunk order.
+//
+// No floating-point atomics.  The chunking depends on n only (fd_chunk), never on the plane range, so a row computed
+// on a shard is bit-identical to the same row computed on the whole tensor.
+#include "common.cuh"
+
+namespace {
+
+constexpr int kFdThreads = 256;
+constexpr int kFdWarps = kFdThreads / 32;
+constexpr int kFdTiles = 4;  // 16-byte column pieces a lane holds per column block
+
+// r per CTA: about 1024 / n rows of r, between 1 and 16 -- enough CTAs for a few planes, few partial rows.
+inline int64_t fd_chunk(int64_t n) {
+    int64_t c = 1024 / n;
+    return c < 1 ? 1 : (c > 16 ? 16 : c);
+}
+
+struct cplx {
+    double x, y;
+};
+
+template <bool C>
+struct Val;
+template <>
+struct Val<false> {
+    using T = double;
+};
+template <>
+struct Val<true> {
+    using T = cplx;
+};
+
+__device__ __forceinline__ double mul(double a, double b) { return a * b; }
+__device__ __forceinline__ cplx mul(cplx a, double b) { return {a.x * b, a.y * b}; }
+__device__ __forceinline__ cplx mul(double a, cplx b) { return {a * b.x, a * b.y}; }
+__device__ __forceinline__ cplx mul(cplx a, cplx b) { return {a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x}; }
+__device__ __forceinline__ double add(double a, double b) { return a + b; }
+__device__ __forceinline__ cplx add(cplx a, cplx b) { return {a.x + b.x, a.y + b.y}; }
+__device__ __forceinline__ void zero(double& a) { a = 0.0; }
+__device__ __forceinline__ void zero(cplx& a) { a = {0.0, 0.0}; }
+
+__device__ __forceinline__ double warp_sum(double v) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+    return v;
+}
+__device__ __forceinline__ cplx warp_sum(cplx v) { return {warp_sum(v.x), warp_sum(v.y)}; }
+
+// V elements of u per lane piece: 2 for real u with an even row (one 16-byte load), else 1 (8 or 16 bytes).
+template <bool UC, int V>
+struct Piece {
+    typename Val<UC>::T e[V];
+};
+
+template <bool UC, int V>
+__device__ __forceinline__ Piece<UC, V> load_piece(const double* __restrict__ p) {
+    Piece<UC, V> r;
+    if constexpr (UC) {
+        const double2 v = __ldg(reinterpret_cast<const double2*>(p));
+        r.e[0] = {v.x, v.y};
+    } else if constexpr (V == 2) {
+        const double2 v = __ldg(reinterpret_cast<const double2*>(p));
+        r.e[0] = v.x;
+        r.e[1] = v.y;
+    } else {
+        r.e[0] = __ldg(p);
+    }
+    return r;
+}
+
+// UC: u complex, RC: rho complex, V: elements per piece.  Accumulators are complex when either is.  Real u with
+// complex rho and 16-byte pieces holds twice the exchange accumulators: two CTAs per SM give it the registers.
+// (Unrolling the r loop of real u four times instead of two needs that register budget for every real kernel and
+// was measured slower at n = 128: 0.508 against 0.412 ms on a B200.)
+template <bool UC, bool RC, int V>
+__global__ void __launch_bounds__(kFdThreads, (!UC && RC && V == 2) ? 2 : 3)
+    fock_density_kernel(const double* __restrict__ u, const double* __restrict__ rho, int n, int chunk, int n_chunks,
+                        double a_d, double a_x, double* __restrict__ ws) {
+    using R = typename Val<RC>::T;
+    using A = typename Val<UC || RC>::T;
+    constexpr int kBlockCols = 32 * V * kFdTiles;
+
+    extern __shared__ double4 fd_smem[];
+    R* rho_s = reinterpret_cast<R*>(fd_smem);               // [chunk][n]: rho_s[rl][s] = rho[s, r0 + rl]
+    A* dacc = reinterpret_cast<A*>(rho_s + (size_t)chunk * n);  // [n] direct partials (row q owned by warp q % 8)
+    A* xcol = dacc + n;                                        // [n] exchange partials
+    A* xs = xcol + n;                                          // [kFdWarps][32 * V * kFdTiles]
+
+    const int pl = blockIdx.x / n_chunks;  // plane relative to p_begin
+    const int c_idx = blockIdx.x - pl * n_chunks;
+    const int r0 = c_idx * chunk;
+    const int rc = min(chunk, n - r0);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+
+    for (int i = threadIdx.x; i < rc * n; i += kFdThreads) {
+        const int s = i / rc, rl = i - s * rc;
+        rho_s[(size_t)rl * n + s] = reinterpret_cast<const R*>(rho)[(size_t)s * n + r0 + rl];
+    }
+    for (int q = threadIdx.x; q < n; q += kFdThreads) zero(dacc[q]);
+    __syncthreads();
+
+    const size_t n2 = (size_t)n * n;
+    const double* plane = u + (size_t)pl * n * n2 * (UC ? 2 : 1);
+    for (int cb = 0; cb < n; cb += kBlockCols) {
+        A x[kFdTiles][V];
+#pragma unroll
+        for (int k = 0; k < kFdTiles; ++k)
+#pragma unroll
+            for (int v = 0; v < V; ++v) zero(x[k][v]);
+        for (int q = warp; q < n; q += kFdWarps) {
+            A d;
+            zero(d);
+#pragma unroll 2
+            for (int rl = 0; rl < rc; ++rl) {
+                const R rq = rho_s[(size_t)rl * n + q];
+                const double* row = plane + ((size_t)(r0 + rl) * n2 + (size_t)q * n) * (UC ? 2 : 1);
+                Piece<UC, V> pc[kFdTiles];
+#pragma unroll
+                for (int k = 0; k < kFdTiles; ++k) {
+                    const int c = cb + (k * 32 + lane) * V;
+                    if (c < n) pc[k] = load_piece<UC, V>(row + (size_t)c * (UC ? 2 : 1));
+                }
+#pragma unroll
+                for (int k = 0; k < kFdTiles; ++k) {
+                    const int c = cb + (k * 32 + lane) * V;
+                    if (c < n) {
+#pragma unroll
+                        for (int v = 0; v < V; ++v) {
+                            d = add(d, mul(pc[k].e[v], rho_s[(size_t)rl * n + c + v]));
+                            x[k][v] = add(x[k][v], mul(rq, pc[k].e[v]));
+                        }
+                    }
+                }
+            }
+            d = warp_sum(d);
+            if (lane == 0) dacc[q] = add(dacc[q], d);
+        }
+#pragma unroll
+        for (int k = 0; k < kFdTiles; ++k)
+#pragma unroll
+            for (int v = 0; v < V; ++v) xs[warp * kBlockCols + (k * 32 + lane) * V + v] = x[k][v];
+        __syncthreads();
+        for (int j = threadIdx.x; j < kBlockCols && cb + j < n; j += kFdThreads) {
+            A t = xs[j];
+            for (int w = 1; w < kFdWarps; ++w) t = add(t, xs[w * kBlockCols + j]);
+            xcol[cb + j] = t;
+        }
+        __syncthreads();
+    }
+    A* out = reinterpret_cast<A*>(ws) + ((size_t)pl * n_chunks + c_idx) * n;
+    for (int q = threadIdx.x; q < n; q += kFdThreads) out[q] = add(mul(dacc[q], a_d), mul(xcol[q], a_x));
+}
+
+// f[p,q] = h[p,q] + sum_c ws[p][c][q] in chunk order.
+__global__ void fock_density_sum_kernel(const double* __restrict__ h, bool h_c, const double* __restrict__ ws,
+                                        bool ws_c, double* __restrict__ f, bool f_c, int n, int n_chunks,
+                                        long long p_begin, long long rows) {
+    const long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (e >= rows * n) return;
+    const long long pl = e / n, q = e - pl * n;
+    const long long o = (p_begin + pl) * n + q;
+    double re = h_c ? h[2 * o] : h[o];
+    double im = h_c ? h[2 * o + 1] : 0.0;
+    for (int c = 0; c < n_chunks; ++c) {
+        const long long w = (pl * n_chunks + c) * n + q;
+        if (ws_c) {
+            re += ws[2 * w];
+            im += ws[2 * w + 1];
+        } else {
+            re += ws[w];
+        }
+    }
+    if (f_c) {
+        f[2 * o] = re;
+        f[2 * o + 1] = im;
+    } else {
+        f[o] = re;
+    }
+}
+
+size_t fd_smem_bytes(int64_t n, int u_dtype, int rho_dtype) {
+    const bool acc_c = u_dtype == QS_C128 || rho_dtype == QS_C128;
+    const int v = (u_dtype == QS_F64 && n % 2 == 0) ? 2 : 1;
+    const size_t a = acc_c ? 16 : 8;
+    return (size_t)fd_chunk(n) * n * (rho_dtype == QS_C128 ? 16 : 8) + 2 * (size_t)n * a +
+           (size_t)kFdWarps * 32 * v * kFdTiles * a;
+}
+
+template <bool UC, bool RC, int V>
+int launch_pass1(const void* u, const void* rho, int n, int chunk, int n_chunks, double a_d, double a_x, void* ws,
+                 long long rows, size_t smem, cudaStream_t st) {
+    auto kern = fock_density_kernel<UC, RC, V>;
+    QS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<(unsigned)(rows * n_chunks), kFdThreads, smem, st>>>(static_cast<const double*>(u),
+                                                                 static_cast<const double*>(rho), n, chunk, n_chunks,
+                                                                 a_d, a_x, static_cast<double*>(ws));
+    QS_LAUNCH_CHECK();
+    return QS_OK;
+}
+
+}  // namespace
+
+extern "C" int qs_fock_density_workspace_bytes(int64_t n, int64_t p_begin, int64_t p_end, int u_dtype, int rho_dtype,
+                                               int64_t* bytes) {
+    QS_REQUIRE(bytes && n >= 1 && 0 <= p_begin && p_begin <= p_end && p_end <= n,
+               "qs_fock_density_workspace_bytes: bad arguments");
+    QS_REQUIRE((u_dtype == QS_F64 || u_dtype == QS_C128) && (rho_dtype == QS_F64 || rho_dtype == QS_C128),
+               "qs_fock_density_workspace_bytes: bad dtype");
+    const int64_t acc = (u_dtype == QS_C128 || rho_dtype == QS_C128) ? 16 : 8;
+    *bytes = (p_end - p_begin) * qs_ceil_div(n, fd_chunk(n)) * n * acc;
+    return QS_OK;
+}
+
+extern "C" int qs_fock_density(const void* h, int h_dtype, const void* u, int u_dtype, const void* rho, int rho_dtype,
+                               int64_t n, double scale_direct, double scale_exchange, void* f, int f_dtype,
+                               int64_t p_begin, int64_t p_end, void* workspace, int64_t workspace_bytes,
+                               void* stream) {
+    QS_REQUIRE(h && rho && f && n >= 1 && n <= (1 << 20), "qs_fock_density: bad arguments");
+    QS_REQUIRE(0 <= p_begin && p_begin <= p_end && p_end <= n, "qs_fock_density: bad row range");
+    for (int d : {h_dtype, u_dtype, rho_dtype, f_dtype})
+        QS_REQUIRE(d == QS_F64 || d == QS_C128, "qs_fock_density: bad dtype");
+    QS_REQUIRE(!(f_dtype == QS_F64 && (h_dtype == QS_C128 || u_dtype == QS_C128 || rho_dtype == QS_C128)),
+               "qs_fock_density: complex u cannot be accumulated into a real Fock matrix");
+    if (p_begin == p_end) return QS_OK;
+    int64_t need = 0;
+    qs_fock_density_workspace_bytes(n, p_begin, p_end, u_dtype, rho_dtype, &need);
+    QS_REQUIRE(u && workspace && workspace_bytes >= need, "qs_fock_density: workspace too small (%lld < %lld bytes)",
+               (long long)workspace_bytes, (long long)need);
+    const int N = (int)n;
+    const int chunk = (int)fd_chunk(n);
+    const int n_chunks = (int)qs_ceil_div(n, chunk);
+    const long long rows = p_end - p_begin;
+    QS_REQUIRE(rows * n_chunks < (1LL << 31), "qs_fock_density: too many planes for one launch");
+    const size_t smem = fd_smem_bytes(n, u_dtype, rho_dtype);
+    QS_REQUIRE(smem <= 227 * 1024, "qs_fock_density: n = %lld needs %zu bytes of shared memory", (long long)n, smem);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    // 16-byte loads of a real row need an even row length and a 16-byte aligned plane
+    const bool vec = u_dtype == QS_F64 && n % 2 == 0 && (reinterpret_cast<uintptr_t>(u) & 15) == 0;
+    int status;
+    if (u_dtype == QS_C128)
+        status = rho_dtype == QS_C128
+                     ? launch_pass1<true, true, 1>(u, rho, N, chunk, n_chunks, scale_direct, scale_exchange, workspace, rows, smem, st)
+                     : launch_pass1<true, false, 1>(u, rho, N, chunk, n_chunks, scale_direct, scale_exchange, workspace, rows, smem, st);
+    else if (rho_dtype == QS_C128)
+        status = vec ? launch_pass1<false, true, 2>(u, rho, N, chunk, n_chunks, scale_direct, scale_exchange, workspace, rows, smem, st)
+                     : launch_pass1<false, true, 1>(u, rho, N, chunk, n_chunks, scale_direct, scale_exchange, workspace, rows, smem, st);
+    else
+        status = vec ? launch_pass1<false, false, 2>(u, rho, N, chunk, n_chunks, scale_direct, scale_exchange, workspace, rows, smem, st)
+                     : launch_pass1<false, false, 1>(u, rho, N, chunk, n_chunks, scale_direct, scale_exchange, workspace, rows, smem, st);
+    if (status != QS_OK) return status;
+    const long long total = rows * n;
+    fock_density_sum_kernel<<<(unsigned)qs_ceil_div(total, 256), 256, 0, st>>>(
+        static_cast<const double*>(h), h_dtype == QS_C128, static_cast<const double*>(workspace),
+        u_dtype == QS_C128 || rho_dtype == QS_C128, static_cast<double*>(f), f_dtype == QS_C128, N, n_chunks, p_begin,
+        rows);
+    QS_LAUNCH_CHECK();
+    return QS_OK;
+}

@@ -317,6 +317,44 @@ def fock_spatial(h, u, n_occ, f=None):
     return _fock("qs_fock_spatial", h, u, n_occ, f)
 
 
+def fock_from_density(h, u, rho, scale_direct, scale_exchange, f=None, planes=None):
+    """``f[p,q] = h[p,q] + a_d sum_rs u[p,r,q,s] rho[s,r] + a_x sum_rs u[p,r,s,q] rho[s,r]`` for a general density
+    matrix ``rho`` (``qs_fock_density``): one read of ``u``, deterministic.  ``(1, 0)`` with an anti-symmetrised
+    ``u`` is the GHF Fock matrix, ``(1, -1/2)`` with ``rho = 2 C_o C_o^dagger`` the RHF one.  ``planes=(p0, p1)``:
+    ``u`` is the leading-index shard ``(p1 - p0, n, n, n)`` and only rows ``[p0, p1)`` of ``f`` are written (a new
+    ``f`` is zero elsewhere).  ``f`` is complex128 when any input is; a given ``f`` is filled in place."""
+    h = _device_tensor(h, "h")
+    u = _device_tensor(u, "u")
+    rho = _device_tensor(rho, "rho")
+    n = h.shape[0]
+    p0, p1 = (0, n) if planes is None else (int(planes[0]), int(planes[1]))
+    if not 0 <= p0 <= p1 <= n:
+        raise ValueError(f"planes {planes} out of range for n = {n}")
+    if tuple(h.shape) != (n, n) or tuple(rho.shape) != (n, n) or tuple(u.shape) != (p1 - p0, n, n, n):
+        raise ValueError(
+            f"h and rho must be (n,n) and u (planes,n,n,n), got {tuple(h.shape)}, {tuple(rho.shape)}, {tuple(u.shape)}"
+        )
+    if f is None:
+        alloc = torch.empty if (p0, p1) == (0, n) else torch.zeros
+        f = alloc((n, n), dtype=_result_dtype(h, u, rho), device=h.device)
+    else:
+        if not (isinstance(f, torch.Tensor) and f.is_cuda and f.is_contiguous()):
+            raise RuntimeError("f must be a contiguous CUDA tensor to be filled in place")
+        if tuple(f.shape) != (n, n):
+            raise ValueError(f"f must be {(n, n)}, got {tuple(f.shape)}")
+        _code(f)
+        _mark_written(f)
+    nbytes = ctypes.c_int64(0)
+    _native.call("qs_fock_density_workspace_bytes", n, p0, p1, _code(u), _code(rho), ctypes.byref(nbytes))
+    owner, ws = _workspace(nbytes.value, h.device)
+    _native.call(
+        "qs_fock_density", _ptr(h), _code(h), _ptr(u), _code(u), _ptr(rho), _code(rho), n, float(scale_direct),
+        float(scale_exchange), _ptr(f), _code(f), p0, p1, ws, nbytes.value, _stream(),
+    )
+    owner.record_stream(torch.cuda.current_stream())
+    return f
+
+
 def odqd_coulomb(C, inner_grid, alpha, a, planes=None):
     """Grid Coulomb elements ``u_abcd`` of the 1-D quantum dot (reference one_dim_qd.py:275-280).
     ``C``: (G', l) eigenvectors on the interior grid; ``inner_grid``: (G',).  ``planes=(a0, a1)`` builds only the

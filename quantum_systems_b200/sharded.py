@@ -1136,14 +1136,38 @@ class ShardedBasisSet:
                     "qs_fock_general", ops._ptr(h), ops._code(h), ctypes.c_void_p(u.buffers[r][r].at(0)),
                     _CODES[u.dtype], n, int(n_occ), ops._ptr(f), p0, p1, ops._stream(),
                 )
-        if isinstance(ctx, ProcessContext) and ctx.world > 1:
-            block, offsets = u.block, u.offsets
-            padded = torch.zeros((ctx.world, block, n), dtype=f.dtype, device=f.device)
-            p0, p1 = u.planes(ctx.rank)
-            padded[ctx.rank, : p1 - p0] = f[p0:p1]
-            flat = torch.view_as_real(padded) if padded.is_complex() else padded
-            ctx.dist.all_reduce(flat, group=ctx.group)  # disjoint rows: sum == gather
-            for r in range(ctx.world):
-                q0, q1 = offsets[r], offsets[r + 1]
-                f[q0:q1] = padded[r, : q1 - q0]
-        return f
+        return _gather_rows(ctx, u, f)
+
+    def fock_from_density(self, h, rho, scale_direct, scale_exchange, f=None):
+        """``f[p,q] = h[p,q] + a_d sum_rs u[p,r,q,s] rho[s,r] + a_x sum_rs u[p,r,s,q] rho[s,r]``
+        (``ops.fock_from_density``): every rank computes the rows p it owns from its own planes, then the rows are
+        all-gathered (n^2 elements).  ``h`` and ``rho`` are replicated.  A row is bit-identical to the same row of
+        the single-tensor kernel."""
+        from . import _arrays, ops
+
+        ctx, u = self.ctx, self.u
+        h, rho = _arrays.to_device(h), _arrays.to_device(rho)
+        if f is None:
+            f = torch.zeros((u.n, u.n), dtype=ops._result_dtype(h, rho, u.local(ctx.local_ranks[0])), device=h.device)
+        for r in ctx.local_ranks:
+            p0, p1 = u.planes(r)
+            if p1 > p0:
+                ops.fock_from_density(h, u.local(r), rho, scale_direct, scale_exchange, f=f, planes=(p0, p1))
+        return _gather_rows(ctx, u, f)
+
+
+def _gather_rows(ctx, u, f):
+    """Every rank has written the rows of ``f`` that belong to its planes of ``u``; afterwards every rank holds all
+    rows.  One process per rank: an all-reduce of the disjoint rows (n^2 elements).  Emulated: nothing to do."""
+    if isinstance(ctx, ProcessContext) and ctx.world > 1:
+        n = u.n
+        block, offsets = u.block, u.offsets
+        padded = torch.zeros((ctx.world, block, n), dtype=f.dtype, device=f.device)
+        p0, p1 = u.planes(ctx.rank)
+        padded[ctx.rank, : p1 - p0] = f[p0:p1]
+        flat = torch.view_as_real(padded) if padded.is_complex() else padded
+        ctx.dist.all_reduce(flat, group=ctx.group)  # disjoint rows: sum == gather
+        for r in range(ctx.world):
+            q0, q1 = offsets[r], offsets[r + 1]
+            f[q0:q1] = padded[r, : q1 - q0]
+    return f
