@@ -123,11 +123,7 @@ int qs_quarter_transform(const void* A, int a_dtype, int64_t X, int64_t K, int64
  * writes rows that INTERLEAVE with the other ranks' rows.  That matters: eight ranks that each fill one of eight
  * ADJACENT chunks of a block in a destination's memory at the same time see position-dependent NVLink throughput
  * (the ranks writing the outermost chunks are 30 % slower at n = 192 on 8 B200s -- the slow ranks follow the chunk
- * position, not the physical GPU; profiles/r02h_*, r02i_*).
- *
- * Rotated tile order.  `tile_start` (a fraction of the launch's tiles in units of 1/65536, 0 = natural order) makes
- * the CTAs start their walk over the tiles there and wrap around: ranks given different fractions are never in the
- * same block of a destination at the same time. */
+ * position, not the physical GPU; profiles/r02h_*, r02i_*). */
 int qs_scatter_deal(int64_t W, int64_t* w_deal);
 int qs_build_coeff_image_dealt(const void* m, int m_dtype, int64_t m_sk, int64_t m_sw, int m_conj,
                                int64_t K, int64_t W, int a_dtype, int64_t w_deal, void* image,
@@ -137,7 +133,7 @@ int qs_quarter_transform_scatter(const void* A, int a_dtype, int64_t X, int64_t 
                                  void* const* host_out_table, int64_t n_dest, int64_t x_inner,
                                  int64_t x_mid, int64_t sx0, int64_t sx1, int64_t sx2,
                                  int64_t w_inner, int64_t sw0, int64_t w_deal, int w_cyclic,
-                                 int64_t tile_start, void* stream);
+                                 void* stream);
 
 /* The scattering store of the anti-symmetric schedule's first exchange: cyclic destinations (column r goes to
  * host_out_table[r % n_dest], column r / n_dest there, stride sw0), restricted to the CTA tiles that hold a pair
@@ -206,8 +202,7 @@ int qs_quarter_transform_scatter_rows(const void* A, int a_dtype, int64_t X, int
                                       const void* image, int m_dtype, int64_t W,
                                       void* const* host_out_table, int64_t n_dest, int64_t x_inner,
                                       int64_t sx1, const int64_t* xr_table, int64_t w_inner,
-                                      int64_t sw0, int64_t w_deal, int64_t tile_start, int rows_paired,
-                                      void* stream);
+                                      int64_t sw0, int64_t w_deal, int rows_paired, void* stream);
 
 /* Copy `rows` rows of n elements into rows of `pitch` >= n elements, zero-filling the tail (real
  * tensors with odd n need an even pitch before they can be described to TMA). */

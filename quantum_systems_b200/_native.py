@@ -33,7 +33,7 @@ SIGNATURES = {
     "qs_quarter_transform": [_ptr, _int, _i64, _i64, _i64, _ptr, _int, _i64, _ptr, _i64, _i64, _i64, _i64, _i64, _i64, _ptr],
     "qs_scatter_deal": [_i64, ctypes.POINTER(_i64)],
     "qs_build_coeff_image_dealt": [_ptr, _int, _i64, _i64, _int, _i64, _i64, _int, _i64, _ptr, _ptr],
-    "qs_quarter_transform_scatter": [_ptr, _int, _i64, _i64, _i64, _ptr, _int, _i64, ctypes.POINTER(_ptr), _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _int, _i64, _ptr],
+    "qs_quarter_transform_scatter": [_ptr, _int, _i64, _i64, _i64, _ptr, _int, _i64, ctypes.POINTER(_ptr), _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _int, _ptr],
     "qs_quarter_transform_scatter_pairs": [_ptr, _int, _i64, _i64, _i64, _ptr, _int, _i64, ctypes.POINTER(_ptr), _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _int, _ptr, _i64, _ptr],
     "qs_transform_two_body_diagonal_workspace_bytes": [_i64, _i64, _int, _int, _int, ctypes.POINTER(_i64)],
     "qs_transform_two_body_diagonal": [_ptr, _int, _ptr, _ptr, _int, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr],
@@ -43,7 +43,7 @@ SIGNATURES = {
     "qs_quarter_plan_tiles": [_i64, _i64, _i64, _int, _int, _i64, _int, _int, _i64, _i64, _i64, _i64, _ptr, _ptr, _i64, ctypes.POINTER(_i64)],
     "qs_quarter_tile_list_bytes": [_i64, _i64, _i64, _int, _int, ctypes.POINTER(_i64)],
     "qs_quarter_transform_rows": [_ptr, _int, _i64, _i64, _i64, _ptr, _int, _i64, _ptr, _i64, _i64, _ptr, _ptr, _i64, _i64, _i64, _ptr, _i64, _ptr],
-    "qs_quarter_transform_scatter_rows": [_ptr, _int, _i64, _i64, _i64, _ptr, _int, _i64, ctypes.POINTER(_ptr), _i64, _i64, _i64, _ptr, _i64, _i64, _i64, _i64, _int, _ptr],
+    "qs_quarter_transform_scatter_rows": [_ptr, _int, _i64, _i64, _i64, _ptr, _int, _i64, ctypes.POINTER(_ptr), _i64, _i64, _i64, _ptr, _i64, _i64, _i64, _int, _ptr],
     "qs_pad_rows": [_ptr, _ptr, _i64, _i64, _i64, _int, _ptr],
     "qs_ipc_handle_bytes": [],
     "qs_ipc_alloc": [_i64, ctypes.POINTER(_ptr), _ptr],

@@ -91,10 +91,6 @@ struct QuarterParams {
     // destinations by themselves, and a rank that owns the cyclic columns writes rows INTERLEAVED with the other
     // ranks' rows later on, never one of W adjacent chunks of a block (see sharded.py, "where the tiles land").
     int w_cyclic;
-    // Rotated tile order (scattering store): the CTAs walk the tiles starting at tile_start (mod the number of
-    // tiles).  Ranks that start at different places do not write into the same block of a destination at the same
-    // time.
-    uint32_t tile_start;
     // Optional tile list (symmetry-aware transforms): when non-null the launch visits only the n_listed linear
     // tile ids (row_tile * tiles_w + col_tile, ascending) stored there instead of all tiles_x * tiles_w tiles.
     const uint32_t* tile_list;
@@ -110,12 +106,8 @@ __device__ __forceinline__ uint32_t dealt_column(uint32_t w, uint32_t mul, uint3
     return mul == 1 ? w : (uint32_t)(((unsigned long long)w * mul) % mod);
 }
 
-// The k-th tile of this launch: through the optional list, in the optionally rotated order.
-__device__ __forceinline__ uint32_t tile_at(const QuarterParams& p, uint32_t k, uint32_t total) {
-    if (p.tile_start) {
-        k += p.tile_start;
-        if (k >= total) k -= total;
-    }
+// The k-th tile of this launch: through the optional list.
+__device__ __forceinline__ uint32_t tile_at(const QuarterParams& p, uint32_t k) {
     return p.tile_list ? p.tile_list[k] : k;
 }
 
@@ -247,7 +239,7 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             const uint32_t bar_empty = bar_full + 8 * kStages;
             uint32_t j = 0;
             for (uint32_t i = pg; i < my_tiles; i += kGroups) {
-                const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x, total_tiles);
+                const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x);
                 const uint32_t tx = divide(tile, p.tiles_w_div);
                 const uint32_t tw = tile - tx * (uint32_t)p.tiles_w;
                 const int px0 = (int)(tx * kBlockX);
@@ -329,7 +321,7 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
     if ((uint32_t)group < my_tiles) load_first();
     for (uint32_t i = group; i < my_tiles; i += kGroups) {
         QS_PHASE_STAMP(0);
-        const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x, total_tiles);
+        const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x);
 
         double acc[4][NT][2];
 #pragma unroll
@@ -708,7 +700,7 @@ quarter_gemm_split_kernel(const __grid_constant__ CUtensorMap map_a, const __gri
             const uint32_t bar_empty = bar_full + 8 * kStages;
             uint32_t j = 0;
             for (uint32_t i = pg; i < my_tiles; i += kGroups) {
-                const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x, total_tiles);
+                const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x);
                 const uint32_t tx = divide(tile, p.tiles_w_div);
                 const uint32_t tw = tile - tx * (uint32_t)p.tiles_w;
                 const int px0 = (int)(tx * kBlockX);
@@ -752,7 +744,7 @@ quarter_gemm_split_kernel(const __grid_constant__ CUtensorMap map_a, const __gri
     };
 
     for (uint32_t i = group; i < my_tiles; i += kGroups) {
-        const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x, total_tiles);
+        const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x);
 
         double re[4][NTC][2], im[4][NTC][2];
 #pragma unroll
@@ -965,8 +957,6 @@ __global__ void build_image_kernel(ImageParams q, double* __restrict__ image) {
 // The W' real columns are cut into 8-wide MMA column tiles; those are dealt to CTA tiles of NT <= 8
 // column tiles each, in at most two groups whose NT differ by one (e.g. W' = 400 -> 6 x NT=7 + 1 x NT=8),
 // so no CTA tile carries more than 7 padding columns.  Each group is one persistent launch.
-// Development switch (QS_DISABLE_SPLIT=1): lower complex A x real M through the generic 4M image instead.
-const bool g_disable_split = getenv("QS_DISABLE_SPLIT") != nullptr;
 // Which launches use the staged asynchronous epilogue (QS_BULK = off | scatter | all; default scatter).  Measured on
 // a B200 (profiles/r02d_perf_bulk_vs_register_epilogue.jsonl): for LOCAL stores the register epilogue is 1-6 %
 // faster (one more ring stage, no lane-serialised copy issue), so only the scattering launches -- whose stores
@@ -995,7 +985,7 @@ struct Tiling {
 Tiling make_tiling(int64_t K, int64_t W, int a_dtype, int m_dtype) {
     Tiling tl;
     const bool out_complex = a_dtype == QS_C128 || m_dtype == QS_C128;
-    tl.split = (a_dtype == QS_C128 && m_dtype == QS_F64 && !g_disable_split) ? 1 : 0;
+    tl.split = (a_dtype == QS_C128 && m_dtype == QS_F64) ? 1 : 0;
     tl.Kp = (int)(K * (a_dtype == QS_C128 ? 2 : 1));
     tl.Wp = (int)(tl.split ? W : W * (out_complex ? 2 : 1));  // split: complex columns, 8 per column tile
     tl.nchunks = (int)qs_ceil_div(tl.Kp, kChunkK);
@@ -1393,7 +1383,7 @@ int quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda
                    void* stream, const QsTileMask* mask = nullptr, void* list_ws = nullptr,
                    const long long* xq_table = nullptr, const long long* xr_table = nullptr,
                    const long long* host_xq_table = nullptr, int xq_even = 0, int w_cyclic = 0,
-                   int64_t tile_start = 0, int xr_paired = 0) {
+                   int xr_paired = 0) {
     QS_REQUIRE(A && image && (out || out_table), "qs_quarter_transform: null pointer");
     QS_REQUIRE(w_deal >= 1 && w_deal < (W > 1 ? W : 2) && gcd64(w_deal, W) == 1,
                "qs_quarter_transform_scatter: the dealing multiplier %lld is not coprime to W = %lld",
@@ -1530,10 +1520,6 @@ int quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda
         p.deal_mul = (uint32_t)w_deal;
         p.deal_mod = (uint32_t)W;
         p.w_cyclic = w_cyclic;
-        {   // rotation of the tile order, as a fraction of this group's tiles (tile_start is given in 1/65536)
-            const int64_t total = p.tile_list ? (int64_t)p.n_listed : (int64_t)p.tiles_x * p.tiles_w;
-            p.tile_start = (uint32_t)((total * (tile_start & 0xFFFF)) >> 16);
-        }
         p.xq_table = xq_table;
         p.xr_table = xr_table;
         QS_REQUIRE((int64_t)p.tiles_x * p.tiles_w < (1LL << 31), "qs_quarter_transform: too many tiles");
@@ -1564,7 +1550,7 @@ int qs_quarter_transform_masked(const void* A, int a_dtype, int64_t X, int64_t K
                                 const long long* xq_table, const long long* xr_table, int xq_even, int xr_paired,
                                 void* stream) {
     return quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, out, nullptr, 0, x_inner, 0xFFFFFFFFLL, sx0, sx1, 0,
-                          w_inner, sw0, sw1, 1, stream, mask, list_ws, xq_table, xr_table, nullptr, xq_even, 0, 0,
+                          w_inner, sw0, sw1, 1, stream, mask, list_ws, xq_table, xr_table, nullptr, xq_even, 0,
                           xr_paired);
 }
 
@@ -1628,13 +1614,11 @@ extern "C" int qs_quarter_transform_scatter_rows(const void* A, int a_dtype, int
                                                  const void* image, int m_dtype, int64_t W,
                                                  void* const* host_out_table, int64_t n_dest, int64_t x_inner,
                                                  int64_t sx1, const int64_t* xr_table, int64_t w_inner, int64_t sw0,
-                                                 int64_t w_deal, int64_t tile_start, int rows_paired,
-                                                 void* stream) {
+                                                 int64_t w_deal, int rows_paired, void* stream) {
     QS_REQUIRE(host_out_table && n_dest > 0 && xr_table, "qs_quarter_transform_scatter_rows: null pointer");
-    QS_REQUIRE(tile_start >= 0 && tile_start < 65536, "qs_quarter_transform_scatter_rows: tile_start is a fraction in 1/65536");
     return quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, nullptr, host_out_table, n_dest, x_inner,
                           0xFFFFFFFFLL, 0, sx1, 0, w_inner, sw0, 0, w_deal, stream, nullptr, nullptr, nullptr,
-                          reinterpret_cast<const long long*>(xr_table), nullptr, 0, 0, tile_start, rows_paired);
+                          reinterpret_cast<const long long*>(xr_table), nullptr, 0, 0, rows_paired);
 }
 
 // The scattering store restricted to the CTA tiles that hold a pair (column r, row index s) the cyclic pair rule of
@@ -1667,10 +1651,9 @@ extern "C" int qs_quarter_transform_scatter(const void* A, int a_dtype, int64_t 
                                             const void* image, int m_dtype, int64_t W, void* const* host_out_table,
                                             int64_t n_dest, int64_t x_inner, int64_t x_mid, int64_t sx0, int64_t sx1,
                                             int64_t sx2, int64_t w_inner, int64_t sw0, int64_t w_deal,
-                                            int w_cyclic, int64_t tile_start, void* stream) {
+                                            int w_cyclic, void* stream) {
     QS_REQUIRE(host_out_table && n_dest > 0, "qs_quarter_transform_scatter: empty destination table");
-    QS_REQUIRE(tile_start >= 0 && tile_start < 65536, "qs_quarter_transform_scatter: tile_start is a fraction in 1/65536");
     return quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, nullptr, host_out_table, n_dest, x_inner, x_mid, sx0,
                           sx1, sx2, w_inner, sw0, 0, w_deal, stream, nullptr, nullptr, nullptr, nullptr, nullptr, 0,
-                          w_cyclic, tile_start);
+                          w_cyclic);
 }

@@ -33,7 +33,6 @@ check the schedule under gloo without a GPU.
 """
 
 import ctypes
-import os
 import weakref
 
 import torch
@@ -56,14 +55,6 @@ def block_partition(n, world):
 SYMMETRY_MIN_N = 48
 # False: `transform_two_body_sharded(symmetry=None)` never tests for anti-symmetry and runs the four full quarter steps
 EXPLOIT_SYMMETRY = True
-# Where the scattered tiles land in the peer schedule (see _RankTransform): "source_major" = cyclic intermediate index
-# and source-major T2; "interleaved" = block partition of r and T2[r_loc][s][a][b] (the round-1 layout).
-# ROTATE_TILES: every rank starts its walk over the tiles of a scattering launch at a different place (rank / world
-# of the way through), so that the ranks are never in the same block of a destination at the same time.
-SCATTER_LAYOUT = os.environ.get("QS_SHARD_LAYOUT", "source_major")
-ROTATE_TILES = os.environ.get("QS_SHARD_ROTATE", "0") == "1"
-# False (QS_SHARD_MASK=0): the first exchange of the anti-symmetric schedule sends every tile, as in round 1.
-MASK_FIRST_EXCHANGE = os.environ.get("QS_SHARD_MASK", "1") != "0"
 
 
 def cyclic_wanted(r, s, m):
@@ -125,6 +116,18 @@ class CudaEngine:
     def _stream():
         return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 
+    @staticmethod
+    def _dest_table(dests):
+        """Host array of the destination pointers of a scattering launch."""
+        return (ctypes.c_void_p * len(dests))(*[buf.at(off) for buf, off in dests])
+
+    @staticmethod
+    def _tile_lists(X, K, W, a_dtype, m_dtype):
+        """Device workspace for the tile lists of a masked launch (``qs_quarter_tile_list_bytes``)."""
+        nbytes = ctypes.c_int64(0)
+        _native.call("qs_quarter_tile_list_bytes", X, K, W, _CODES[a_dtype], _CODES[m_dtype], ctypes.byref(nbytes))
+        return torch.empty(nbytes.value, dtype=torch.uint8, device="cuda")
+
     def asarray(self, a, dtype=None):
         from . import _arrays
 
@@ -176,27 +179,23 @@ class CudaEngine:
                      sw1):
         if X <= 0:
             return
-        nbytes = ctypes.c_int64(0)
-        _native.call("qs_quarter_tile_list_bytes", X, K, W, _CODES[A.dtype], _CODES[m_dtype], ctypes.byref(nbytes))
-        lists = torch.empty(nbytes.value, dtype=torch.uint8, device="cuda")
+        lists = self._tile_lists(X, K, W, A.dtype, m_dtype)
         _native.call(
             "qs_quarter_transform_rows", ctypes.c_void_p(A.at(0)), _CODES[A.dtype], X, K, lda,
             ctypes.c_void_p(image.data_ptr()), _CODES[m_dtype], W, ctypes.c_void_p(out.at(0)), x_inner, sx0,
             ctypes.c_void_p(host_table.ctypes.data), ctypes.c_void_p(dev_table.data_ptr()), w_inner, sw0, sw1,
-            ctypes.c_void_p(lists.data_ptr()), nbytes.value, self._stream(),
+            ctypes.c_void_p(lists.data_ptr()), lists.numel(), self._stream(),
         )
         lists.record_stream(torch.cuda.current_stream())
 
     def quarter_scatter_rows(self, A, X, K, lda, image, m_dtype, W, dests, x_inner, sx1, xr_table, w_inner, sw0,
-                             deal=1, tile_start=0, rows_paired=False):
+                             deal=1, rows_paired=False):
         if X <= 0:
             return
-        table = (ctypes.c_void_p * len(dests))(*[buf.at(off) for buf, off in dests])
         _native.call(
             "qs_quarter_transform_scatter_rows", ctypes.c_void_p(A.at(0)), _CODES[A.dtype], X, K, lda,
-            ctypes.c_void_p(image.data_ptr()), _CODES[m_dtype], W, table, len(dests), x_inner, sx1,
-            ctypes.c_void_p(xr_table.data_ptr()), w_inner, sw0, int(deal), int(tile_start), int(bool(rows_paired)),
-            self._stream(),
+            ctypes.c_void_p(image.data_ptr()), _CODES[m_dtype], W, self._dest_table(dests), len(dests), x_inner, sx1,
+            ctypes.c_void_p(xr_table.data_ptr()), w_inner, sw0, int(deal), int(bool(rows_paired)), self._stream(),
         )
 
     def quarter_scatter_pairs(self, A, X, K, lda, image, m_dtype, W, dests, x_inner, x_mid, sx0, sx1, sx2, sw0,
@@ -205,14 +204,12 @@ class CudaEngine:
         (r, s) the cyclic pair rule wants (qs_quarter_transform_scatter_pairs)."""
         if X <= 0:
             return
-        nbytes = ctypes.c_int64(0)
-        _native.call("qs_quarter_tile_list_bytes", X, K, W, _CODES[A.dtype], _CODES[m_dtype], ctypes.byref(nbytes))
-        lists = torch.empty(nbytes.value, dtype=torch.uint8, device="cuda")
-        table = (ctypes.c_void_p * len(dests))(*[buf.at(off) for buf, off in dests])
+        lists = self._tile_lists(X, K, W, A.dtype, m_dtype)
         _native.call(
             "qs_quarter_transform_scatter_pairs", ctypes.c_void_p(A.at(0)), _CODES[A.dtype], X, K, lda,
-            ctypes.c_void_p(image.data_ptr()), _CODES[m_dtype], W, table, len(dests), x_inner, max(x_mid, 1), sx0, sx1,
-            sx2, sw0, rows_per_s, int(bool(padded)), ctypes.c_void_p(lists.data_ptr()), nbytes.value, self._stream(),
+            ctypes.c_void_p(image.data_ptr()), _CODES[m_dtype], W, self._dest_table(dests), len(dests), x_inner,
+            max(x_mid, 1), sx0, sx1, sx2, sw0, rows_per_s, int(bool(padded)), ctypes.c_void_p(lists.data_ptr()),
+            lists.numel(), self._stream(),
         )
         lists.record_stream(torch.cuda.current_stream())
 
@@ -245,14 +242,13 @@ class CudaEngine:
         return out
 
     def quarter_scatter(self, A, X, K, lda, image, m_dtype, W, dests, x_inner, x_mid, sx0, sx1, sx2, w_inner, sw0,
-                        deal=1, cyclic=False, tile_start=0):
+                        deal=1, cyclic=False):
         if X <= 0:
             return
-        table = (ctypes.c_void_p * len(dests))(*[buf.at(off) for buf, off in dests])
         _native.call(
             "qs_quarter_transform_scatter", ctypes.c_void_p(A.at(0)), _CODES[A.dtype], X, K, lda,
-            ctypes.c_void_p(image.data_ptr()), _CODES[m_dtype], W, table, len(dests), x_inner, max(x_mid, 1), sx0, sx1,
-            sx2, max(w_inner, 1), sw0, int(deal), int(bool(cyclic)), int(tile_start), self._stream(),
+            ctypes.c_void_p(image.data_ptr()), _CODES[m_dtype], W, self._dest_table(dests), len(dests), x_inner,
+            max(x_mid, 1), sx0, sx1, sx2, max(w_inner, 1), sw0, int(deal), int(bool(cyclic)), self._stream(),
         )
 
 
@@ -469,20 +465,7 @@ class ShardedTwoBody:
 
     def gather(self):
         """The full tensor on every rank (small n only: tests, inspection)."""
-        ctx = self.ctx
-        if isinstance(ctx, EmulatedContext):
-            return torch.cat([self.local(r) for r in range(ctx.world)], dim=0)
-        local = self.local()
-        n = self.n
-        padded = torch.zeros((self.block, n, n, n), dtype=local.dtype, device=local.device)
-        padded[: local.shape[0]] = local
-        parts = [torch.empty_like(padded) for _ in range(ctx.world)]  # equal sizes: short trailing blocks are padded
-        if padded.is_complex():
-            ctx.dist.all_gather([torch.view_as_real(p) for p in parts], torch.view_as_real(padded), group=ctx.group)
-        else:
-            ctx.dist.all_gather(parts, padded, group=ctx.group)
-        parts = [parts[r][: self.offsets[r + 1] - self.offsets[r]] for r in range(ctx.world)]
-        return torch.cat(parts, dim=0)
+        return self.extract()
 
 
     # -------------------------------------------------------------- consumers (SURVEY.md section 8f-3)
@@ -510,7 +493,7 @@ class ShardedTwoBody:
         piece = pieces[ctx.rank]
         padded = torch.zeros((self.block,) + tuple(piece.shape[1:]), dtype=piece.dtype, device=piece.device)
         padded[: piece.shape[0]] = piece
-        parts = [torch.empty_like(padded) for _ in range(ctx.world)]
+        parts = [torch.empty_like(padded) for _ in range(ctx.world)]  # equal sizes: short trailing blocks are padded
         if padded.is_complex():
             ctx.dist.all_gather([torch.view_as_real(p) for p in parts], torch.view_as_real(padded), group=ctx.group)
         else:
@@ -521,23 +504,29 @@ class ShardedTwoBody:
             rows.append(parts[r][: max(min(a1, p1) - max(a0, p0), 0)])
         return torch.cat(rows, dim=0)
 
-    def axpby_(self, alpha, other=None, beta=0.0):
-        """In place ``u <- alpha u + beta other`` on every shard (``other`` sharded alike); no communication.
-        ``u_t = f(t) u`` of an adiabatic switching is ``axpby_(f(t))`` on a copy."""
+    def _scale_add(self, alpha, other, beta, dest=None):
+        """``dest <- alpha u + beta other`` on every local shard (``qs_scale_add``), ``dest`` a new tensor (own
+        buffers, no spare) if None; no communication."""
         if other is not None and (other.n != self.n or other.dtype != self.dtype):
             raise ValueError("operands must share extent and dtype")
         alpha, beta = complex(alpha), complex(beta)
         if self.dtype != torch.complex128 and (alpha.imag != 0 or beta.imag != 0):
             raise TypeError("complex factor on a real sharded tensor")
+        if dest is None:
+            dest = ShardedTwoBody.empty(self.ctx, self.n, self.dtype, with_spare=False)
         for r in self.ctx.local_ranks:
             p0, p1 = self.planes(r)
             count = (p1 - p0) * self.n**3
             if count:
-                mine = self.buffers[r][r]
-                self.ctx.engine.scale_add(mine, other.buffers[r][r] if other is not None else None, count, alpha, beta,
-                                          mine)
-        self.proven_antisymmetric = self.proven_antisymmetric and (other is None or other.proven_antisymmetric)
-        return self
+                self.ctx.engine.scale_add(self.buffers[r][r], other.buffers[r][r] if other is not None else None,
+                                          count, alpha, beta, dest.buffers[r][r])
+        dest.proven_antisymmetric = self.proven_antisymmetric and (other is None or other.proven_antisymmetric)
+        return dest
+
+    def axpby_(self, alpha, other=None, beta=0.0):
+        """In place ``u <- alpha u + beta other`` on every shard (``other`` sharded alike); no communication.
+        ``u_t = f(t) u`` of an adiabatic switching is ``axpby_(f(t))`` on a copy."""
+        return self._scale_add(alpha, other, beta, self)
 
     def successor(self):
         """A handle over this tensor's SPARE buffers whose own spare is this tensor's memory, for a caller that is
@@ -552,33 +541,13 @@ class ShardedTwoBody:
     def scaled(self, alpha, other=None, beta=0.0):
         """A NEW sharded tensor ``alpha u + beta other`` in one pass per shard (``qs_scale_add``), no
         communication: ``u_t = u_0 + f(t) u`` of reference system.py:203-215 / operator.py:182-196."""
-        if other is not None and (other.n != self.n or other.dtype != self.dtype):
-            raise ValueError("operands must share extent and dtype")
-        alpha, beta = complex(alpha), complex(beta)
-        if self.dtype != torch.complex128 and (alpha.imag != 0 or beta.imag != 0):
-            raise TypeError("complex factor on a real sharded tensor")
-        new = ShardedTwoBody.empty(self.ctx, self.n, self.dtype, with_spare=False)
-        for r in self.ctx.local_ranks:
-            p0, p1 = self.planes(r)
-            count = (p1 - p0) * self.n**3
-            if count:
-                self.ctx.engine.scale_add(self.buffers[r][r], other.buffers[r][r] if other is not None else None,
-                                          count, alpha, beta, new.buffers[r][r])
+        new = self._scale_add(alpha, other, beta)
         self.ctx.barrier()
-        new.proven_antisymmetric = self.proven_antisymmetric and (other is None or other.proven_antisymmetric)
         return new
 
     def copy(self):
         """A new sharded tensor (own buffers, no spare) with the same contents."""
-        new = ShardedTwoBody.empty(self.ctx, self.n, self.dtype, with_spare=False)
-        for r in self.ctx.local_ranks:
-            p0, p1 = self.planes(r)
-            count = (p1 - p0) * self.n**3
-            if count:
-                self.ctx.engine.scale_add(self.buffers[r][r], None, count, 1.0, 0.0, new.buffers[r][r])
-        self.ctx.barrier()
-        new.proven_antisymmetric = self.proven_antisymmetric
-        return new
+        return self.scaled(1.0)
 
     def occupied_traces(self, h, n_occ):
         """``(tr h[o,o], sum_ij u[i,j,i,j], sum_ij u[i,j,j,i])`` as Python complex numbers: every rank reduces
@@ -624,8 +593,6 @@ class _RankTransform:
         self.a_block, self.a_off = block_partition(n, ctx.world)  # partition of the old leading index
         self.r_block, self.r_off = block_partition(m, ctx.world)  # partition of the new leading index p (and of r
         #                                                           in the collective schedule)
-        self.cyclic = ctx.exchange == "peer" and SCATTER_LAYOUT == "source_major"  # r dealt cyclically
-        self.tile_start = (rank * 65536) // ctx.world if (ROTATE_TILES and ctx.exchange == "peer") else 0
         self.Pu = padded_pitch(n, u_dtype)
         self.P = padded_pitch(n, self.t_dtype)
         self.A = self.a_off[rank + 1] - self.a_off[rank]
@@ -634,18 +601,10 @@ class _RankTransform:
         self.even_sources = all(self.a_off[j + 1] - self.a_off[j] == self.A for j in range(ctx.world))
 
     def r_count(self, rank):
-        """Number of intermediate indices r that `rank` owns."""
-        if self.cyclic:
+        """Number of intermediate indices r that `rank` owns (peer: dealt cyclically, collective: a block)."""
+        if self.ctx.exchange == "peer":
             return len(range(rank, self.m, self.ctx.world))
         return self.r_off[rank + 1] - self.r_off[rank]
-
-    def r_values(self):
-        """The intermediate indices r of this rank, in the order of its local index r_loc."""
-        import numpy
-
-        if self.cyclic:
-            return numpy.arange(self.rank, self.m, self.ctx.world, dtype=numpy.int64)
-        return self.r_off[self.rank] + numpy.arange(self.R, dtype=numpy.int64)
 
     # sizes (elements of t_dtype unless noted)
     def recv_numel(self, rank):
@@ -669,9 +628,6 @@ class _RankTransform:
         # its output columns over all destinations (uniform NVLink traffic): its image holds the columns of C~ in
         # dealt order.  The first exchange sends cyclic columns and needs no dealing.
         self.deal = eng.scatter_deal(m) if self.ctx.exchange == "peer" and self.ctx.world > 1 else 1
-        self.img2_scatter = self.img2
-        if self.deal > 1 and not self.cyclic:  # block partition of r: the first exchange deals its columns too
-            self.img2_scatter = eng.image(C, n, m, self.t_dtype, m, 1, deal=self.deal)
         if self.deal > 1:
             if C_tilde is not None:
                 self.img4_scatter = eng.image(C_tilde, n, m, self.t_dtype, 1, n, deal=self.deal)
@@ -699,15 +655,9 @@ class _RankTransform:
         and this rank's tiles fill ONE contiguous region of every destination.  ``pairs_only`` (anti-symmetric u):
         only the tiles that hold a pair (r, s) which steps 3 and 4 will use are computed and sent."""
         eng, n, m, A, P = self.engine, self.n, self.m, self.A, self.P
-        a0 = self.a_off[self.rank]
-        if not self.cyclic:  # interleaved layout: [r_loc][s][a][b], this rank's planes between the others'
-            dests = [(recv[j], a0 * P) for j in range(self.ctx.world)]
-            eng.quarter_scatter(self.scratch, m * A * n, n, P, self.img2_scatter, self.c_dtype, m, dests, n, A, 1, P,
-                                n * P, self.r_block, m * n * P, deal=self.deal, tile_start=self.tile_start)
-            return
         # region of this source in destination j: behind the regions of the sources before it
-        dests = [(recv[j], a0 * self.r_count(j) * m * P) for j in range(self.ctx.world)]
-        if pairs_only and MASK_FIRST_EXCHANGE and not self.tile_start:
+        dests = [(recv[j], self.a_off[self.rank] * self.r_count(j) * m * P) for j in range(self.ctx.world)]
+        if pairs_only:
             # the tiles sent here must cover the pairs of the (cached) tables steps 3 and 4 read
             self.prepare_pairs()
             assert self.rows_paired == self.pairs_padded(), "cached pair tables of another T2 dtype"
@@ -715,7 +665,7 @@ class _RankTransform:
                                       A * P, m * A * P, A * n, self.rows_paired)
             return
         eng.quarter_scatter(self.scratch, m * A * n, n, P, self.img2, self.c_dtype, m, dests, n, A, 1, P, A * P,
-                            0, m * A * P, deal=1, cyclic=True, tile_start=self.tile_start)
+                            0, m * A * P, deal=1, cyclic=True)
 
     def step2_local(self, send):
         """Collective schedule: T2[r, s, a_loc, b] written locally, blocks of r contiguous per destination."""
@@ -729,9 +679,7 @@ class _RankTransform:
         eng, n, m, R, P = self.engine, self.n, self.m, self.R, self.P
         if R == 0:
             return
-        if not self.cyclic:  # interleaved layout: rows (r_loc, s, a) in place
-            eng.quarter(recv_local, R * m * n, n, P, self.img3, self.c_dtype, m, self.scratch, 0, n, 1, P, 1, 0, R * m * P)
-        elif self.even_sources:
+        if self.even_sources:
             eng.quarter_scatter(recv_local, R * m * n, n, P, self.img3, self.c_dtype, m, [(self.scratch, 0)], self.A,
                                 R * m, 1, P, self.A, m, R * m * P, deal=1)
         else:
@@ -756,14 +704,9 @@ class _RankTransform:
         [p_loc][q][r][s]: the result is sharded on its leading index again.  r = rank + W r_loc: this rank's rows
         of every (r, s) block interleave with the other ranks' rows."""
         eng, n, m, R, P, W = self.engine, self.n, self.m, self.R, self.P, self.ctx.world
-        if not self.cyclic:  # block partition of r: this rank's rows are one chunk of every (r, s) block
-            dests = [(out[j], self.r_off[self.rank] * m) for j in range(W)]
-            eng.quarter_scatter(self.scratch, m * R * m, n, P, self.img4_scatter, self.c_dtype, m, dests, m, R, 1, m,
-                                m * m, self.r_block, m**3, deal=self.deal, tile_start=self.tile_start)
-            return
         dests = [(out[j], self.rank * m) for j in range(W)]
         eng.quarter_scatter(self.scratch, m * R * m, n, P, self.img4_scatter, self.c_dtype, m, dests, m, R, 1, W * m,
-                            m * m, self.r_block, m**3, deal=self.deal, tile_start=self.tile_start)
+                            m * m, self.r_block, m**3, deal=self.deal)
 
     # ---- anti-symmetric u: steps 3 and 4 on half of the (r, s) pairs (cyclic rule), packed by pair -------------
     def pairs_padded(self):
@@ -778,11 +721,11 @@ class _RankTransform:
         # built and uploaded once per (rank, n, m, world, P, dtype of T2), then reused by every transform; the dtype
         # decides whether the lists are padded to aligned couples (pairs_padded)
         cache = self.ctx.__dict__.setdefault("_pair_tables", {})
-        key = (self.rank, self.n, m, W, P, self.cyclic, self.t_dtype)
+        key = (self.rank, self.n, m, W, P, self.t_dtype)
         if key in cache:
             (self.npairs, self.step3_tables, self.rs_of_pair, self.rs_of_pair_dev, self.rows_paired) = cache[key]
             return
-        r = self.r_values()[:, None]
+        r = numpy.arange(self.rank, m, W, dtype=numpy.int64)[:, None]  # the owned r (cyclic), in r_loc order
         sI = numpy.arange(m, dtype=numpy.int64)[None, :]
         wanted = cyclic_wanted(r, sI, m)
         # Real tensors with an even extent: complete every aligned couple (s even, s + 1) that holds a wanted partner.
@@ -800,10 +743,7 @@ class _RankTransform:
         # step 3 reads the source-major T2: rows (src, r_loc, s, a_loc) -> T3p[q, pair(r_loc, s), a_off[src] + a_loc]
         self.step3_tables = []
         if self.npairs:
-            if not self.cyclic:  # interleaved layout: rows (r_loc, s, a), blocks of n rows
-                table = numpy.ascontiguousarray(slot.reshape(-1))
-                self.step3_tables = [("interleaved", table, self.engine.index_table(table))]
-            elif self.even_sources:
+            if self.even_sources:
                 per_source = [slot.reshape(-1) + numpy.where(slot.reshape(-1) >= 0, self.a_off[src], 0)
                               for src in range(W)]
                 table = numpy.ascontiguousarray(numpy.concatenate(per_source))
@@ -821,10 +761,7 @@ class _RankTransform:
         if self.npairs == 0:
             return
         for src, host_table, dev_table in self.step3_tables:
-            if src == "interleaved":
-                eng.quarter_rows(recv_local, R * m * n, n, P, self.img3, self.c_dtype, m, self.scratch, n, 1,
-                                 host_table, dev_table, 1, 0, self.npairs * P)
-            elif src is None:  # all sources in one launch: blocks of A rows, table over (src, r_loc, s)
+            if src is None:  # all sources in one launch: blocks of A rows, table over (src, r_loc, s)
                 eng.quarter_rows(recv_local, R * m * n, n, P, self.img3, self.c_dtype, m, self.scratch, self.A, 1,
                                  host_table, dev_table, 1, 0, self.npairs * P)
             else:
@@ -841,7 +778,7 @@ class _RankTransform:
         dests = [(out[j], 0) for j in range(self.ctx.world)]
         eng.quarter_scatter_rows(self.scratch, m * self.npairs, n, P, self.img4_scatter, self.c_dtype, m, dests,
                                  self.npairs, m * m, self.rs_of_pair_dev, self.r_block, m**3, deal=self.deal,
-                                 tile_start=self.tile_start, rows_paired=self.rows_paired)
+                                 rows_paired=self.rows_paired)
 
     def step4_local(self, out_local):
         """Collective schedule: u'[p, q, r_loc, s] dense on this rank (sharded on the third index)."""
@@ -1016,26 +953,13 @@ class ShardedBasisSet:
         """Spin-double a replicated spatial basis into a sharded spin-orbital one: every rank writes its
         own planes P = 2p + sigma of the (2l)^4 tensor with the fused add_spin + anti-symmetrise (+ cast)
         kernel -- no communication (SURVEY.md section 8e)."""
-        from . import _arrays, ops
+        from . import _arrays
 
         u_dev = _arrays.to_device(u_spatial)
-        l = u_dev.shape[0]
-        n = 2 * l
         if u_dev.is_complex():
             out_dtype = torch.complex128
-        u = into if into is not None else ShardedTwoBody.empty(ctx, n, out_dtype)
-        if u.n != n or u.dtype != out_dtype:
-            raise ValueError("`into` must be a ShardedTwoBody of extent 2 l and the requested dtype")
-        for r in ctx.local_ranks:
-            p0, p1 = u.planes(r)
-            if p1 > p0:
-                ops.add_spin_two_body(u_dev, anti_symmetrize=anti_symmetrize, out_dtype=out_dtype, planes=(p0, p1),
-                                      out=u.local(r))
-        ctx.barrier()
-        u.proven_antisymmetric = bool(anti_symmetrize)  # the fused pass writes a - b and b - a: exact negatives
-        h2 = ops.add_spin_one_body(_arrays.to_device(h), out_dtype=out_dtype)
-        s2 = ops.add_spin_one_body(_arrays.to_device(s), out_dtype=out_dtype)
-        return cls(ctx, n, h2, s2, u, includes_spin=True, anti_symmetrized_u=bool(anti_symmetrize))
+        return cls.from_spatial_planes(ctx, h, s, u_dev.shape[0], lambda p0, p1: u_dev[p0:p1],
+                                       anti_symmetrize=anti_symmetrize, out_dtype=out_dtype, into=into)
 
     @classmethod
     def from_spatial_planes(cls, ctx, h, s, l, spatial_planes, anti_symmetrize=True, out_dtype=torch.complex128,

@@ -72,7 +72,7 @@ class NumpyEngine:
         out.flat()[out_offset + ax[:, None] + aw[None, :]] = res
 
     def quarter_scatter(self, A, X, K, lda, image, m_dtype, W, dests, x_inner, x_mid, sx0, sx1, sx2, w_inner, sw0,
-                        deal=1, cyclic=False, tile_start=0):
+                        deal=1, cyclic=False):
         if X <= 0:
             return
         res = self._product(A, X, K, lda, image)
@@ -187,7 +187,7 @@ class NumpyEngine:
         out.flat()[ax[:, None] + aw[None, :]] = res[keep]
 
     def quarter_scatter_rows(self, A, X, K, lda, image, m_dtype, W, dests, x_inner, sx1, xr_table, w_inner, sw0, deal=1,
-                             tile_start=0, rows_paired=False):
+                             rows_paired=False):
         if X <= 0:
             return
         res = self._product(A, X, K, lda, image)

@@ -32,6 +32,13 @@ def test_header_and_binding_agree(library):
     names = declared_functions()
     assert len(names) >= 20
     assert sorted(_native.SIGNATURES) == names
+    # a stale argtypes list is not caught at compile time: ctypes would pass the arguments shifted
+    text = re.sub(r"/\*.*?\*/", "", open(HEADER).read(), flags=re.S)
+    prototypes = dict(re.findall(r"\b(qs_[a-z0-9_]+)\s*\(([^()]*)\)\s*;", text))
+    assert sorted(prototypes) == names
+    for name, params in prototypes.items():
+        count = 0 if params.strip() in ("", "void") else params.count(",") + 1
+        assert count == len(_native.SIGNATURES[name]), f"{name}: {count} parameters in the header"
 
 
 def test_every_declared_symbol_is_exported(library):

@@ -46,7 +46,6 @@ def main():
             del u
         del base
     # complex u with REAL coefficients: the split (2M) quarter GEMM; 16 n^5 real flops are necessary
-    # (QS_DISABLE_SPLIT=1 in the environment lowers it through the generic 4M image for comparison)
     for n in (40, 96, 128):
         u = torch.randn((n,) * 4, dtype=torch.complex128, device="cuda")
         C = torch.linalg.qr(torch.randn((n, n), dtype=torch.float64, device="cuda"))[0].contiguous()
@@ -54,8 +53,7 @@ def main():
             ms = timed(lambda: ops.transform_two_body(u, coeff))
             print(json.dumps({"op": "transform_two_body", "n": n, "u": "complex128", "C": label, "ms": round(ms, 3),
                               "tflops_2M": round(16.0 * n**5 / ms * 1e-9, 2),
-                              "frac_of_dmma_peak_2M": round(16.0 * n**5 / ms * 1e-9 / peak, 3),
-                              "split_disabled": bool(os.environ.get("QS_DISABLE_SPLIT"))}))
+                              "frac_of_dmma_peak_2M": round(16.0 * n**5 / ms * 1e-9 / peak, 3)}))
         del u
     for l in [64, 100]:
         u = torch.randn((l,) * 4, dtype=torch.float64, device="cuda")
