@@ -90,11 +90,33 @@ struct QsTileMask {
     int64_t dh, mh, dl, ml;  // row_hi(x) = (x / dh) % mh, row_lo(x) = (x / dl) % ml
 };
 int64_t qs_tile_list_bytes(int64_t X, int64_t K, int64_t W, int a_dtype, int m_dtype);
-int qs_quarter_transform_masked(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda, const void* image,
-                                int m_dtype, int64_t W, void* out, int64_t x_inner, int64_t sx0, int64_t sx1,
-                                int64_t w_inner, int64_t sw0, int64_t sw1, const QsTileMask* mask, void* list_ws,
-                                const long long* xq_table, const long long* xr_table, int xq_even, int xr_paired,
-                                void* stream);
+
+// Where a quarter transform stores, and which of its tiles it computes.  Output element (x, w), in output elements
+// (complex output: complex elements), with x = (x2 * x_mid + x1) * x_inner + x0:
+//     (w / w_inner) * sw1 + (w % w_inner) * sw0 + x2 * sx2 + x1 * sx1 + x0 * sx0
+// Defaults: one local destination, no middle row split, undealt columns, no tables, every tile; strides are 0.
+struct QsQuarterStore {
+    void* out = nullptr;                  // the local destination, or:
+    void* const* out_table = nullptr;     // scattering store: n_dest destinations, w / w_inner selects one (sw1 unused)
+    int64_t n_dest = 0;
+    int w_cyclic = 0;                     // scattering: column w goes to destination w % n_dest as its column w / n_dest
+    int64_t w_deal = 1;                   // column dealing: logical column j is stored as column (j * w_deal) % W
+    int64_t x_inner = 1, x_mid = 0xFFFFFFFFLL, w_inner = 1;  // x_mid 0xFFFFFFFF: x = x1 * x_inner + x0, no sx2
+    int64_t sx0 = 0, sx1 = 0, sx2 = 0, sw0 = 0, sw1 = 0;
+    // Row tables (device memory), with x = xq * x_inner + xr: row x is at xq_table[xq] + xr_table[xr] in place of
+    // xq * sx1 and xr * sx0; a negative xq_table entry drops the rows of that block.
+    const long long* xq_table = nullptr;
+    const long long* xr_table = nullptr;
+    int xq_even = 0;                      // promise: every kept xq_table entry is even
+    int xr_paired = 0;                    // promise: xr_table places rows 2k, 2k + 1 adjacently at an even offset
+    // Masked launch: only the tiles the mask, or the host copy of the block table, wants.  list_ws holds
+    // qs_tile_list_bytes() bytes of device memory.
+    const QsTileMask* mask = nullptr;
+    const long long* host_xq_table = nullptr;
+    void* list_ws = nullptr;
+};
+int qs_quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda, const void* image, int m_dtype,
+                      int64_t W, const QsQuarterStore& st, void* stream);
 
 int qs_mirror_fill(void* out, int dtype, int64_t m, int mode, void* stream);
 

@@ -27,12 +27,6 @@
 
 namespace {
 
-#ifndef QS_L2_PROMOTION
-#define QS_L2_PROMOTION CU_TENSOR_MAP_L2_PROMOTION_L2_256B
-#endif
-#ifndef QS_STAGES
-#define QS_STAGES 0             // 0 = as deep as shared memory allows (at most 8)
-#endif
 constexpr int kBlockX = 128;    // rows of A per CTA tile
 constexpr int kChunkK = 16;     // k' per pipeline stage (= one 128-byte swizzled row)
 constexpr int kGroups = 2;      // MMA warp groups that ping-pong on the tensor pipe
@@ -79,8 +73,6 @@ struct QuarterParams {
     Divisor x_inner_div, tiles_w_div;
     long long sx0, sx1, sx2, sw0, sw1;
     int vec2;                 // real output: row pairs (x, x + 1), x even, are adjacent and 16-byte aligned
-    int bulk;                 // staged asynchronous epilogue (BULK kernels): consecutive rows of a block are adjacent
-                              // in the output and every run starts 16-byte aligned (see launch conditions)
     // Column dealing (scattering store): logical output column j of the tile order is the physical column
     // (j * deal_mul) % deal_mod, so every CTA tile's columns are spread over ALL destinations and the NVLink
     // traffic of a launch is uniform in time (contiguous column ranges make every rank write to the same one or
@@ -104,6 +96,46 @@ struct QuarterParams {
 
 __device__ __forceinline__ uint32_t dealt_column(uint32_t w, uint32_t mul, uint32_t mod) {
     return mul == 1 ? w : (uint32_t)(((unsigned long long)w * mul) % mod);
+}
+
+// Store addressing of the strided, staged and split epilogues (the rotated one has its own, see quarter_gemm_kernel).
+// Base of output column wl (before dealing) for output elements of ES bytes: the dealt column w goes to destination
+// w % ndest as its column w / ndest (cyclic) or to block w / w_inner as its column w % w_inner.  `plain`
+// (w_inner == 1 and no destination table, evaluated once per tile) stores column w at w * sw1.
+template <int ES>
+__device__ __forceinline__ double* column_base(const QuarterParams& p, bool plain, uint32_t wl) {
+    const uint32_t w = dealt_column(wl, p.deal_mul, p.deal_mod);
+    if (plain) return p.out + (ES / 8) * ((long long)w * p.sw1);
+    const uint32_t wq = p.w_cyclic ? w % (uint32_t)p.ndest : w / p.w_inner;
+    const uint32_t wr = p.w_cyclic ? w / (uint32_t)p.ndest : w - wq * p.w_inner;
+    return (p.ndest ? p.outs[wq] : p.out) + (ES / 8) * ((long long)wq * p.sw1 + (long long)wr * p.sw0);
+}
+
+// Offset of row block xq (rows xq * x_inner + xr): through x_mid, the block table or sx1.  `kept` enters as "the row
+// is in range" and leaves false for a block the table drops (a row the symmetry does not need).
+__device__ __forceinline__ long long block_offset(const QuarterParams& p, uint32_t xq, bool& kept) {
+    if (p.x_mid != 0xFFFFFFFFu) {
+        const uint32_t x2 = xq / p.x_mid;
+        const uint32_t x1 = xq - x2 * p.x_mid;
+        return (long long)x2 * p.sx2 + (long long)x1 * p.sx1;
+    }
+    if (p.xq_table && kept) {
+        const long long tq = p.xq_table[xq];
+        if (tq < 0) kept = false;
+        return tq;
+    }
+    return (long long)xq * p.sx1;
+}
+
+// Offset of row x and whether anything is stored for it: the in-block part from the row table or xr * sx0, plus
+// the block's offset.
+__device__ __forceinline__ bool row_offset(const QuarterParams& p, uint32_t x, long long& off) {
+    bool kept = x < p.X;
+    const uint32_t xq = divide(x, p.x_inner_div);
+    const uint32_t xr = x - xq * p.x_inner;
+    off = (p.xr_table && kept) ? p.xr_table[xr] : (long long)xr * p.sx0;
+    off += block_offset(p, xq, kept);
+    return kept;
 }
 
 // The k-th tile of this launch: through the optional list.
@@ -152,21 +184,85 @@ __device__ __forceinline__ int row_base(int g) { return 2 * ((g >> 1) & 1) + 4 *
 constexpr int kStagingPerWarp = 2 * 4096;
 constexpr int kStagingBytes = kMmaWarps * kStagingPerWarp;  // 64 KiB
 
-// One stage ring per MMA group: as many 16 KiB + NT KiB stages as fit, at most 6 (4 at NT = 8; with the staging
-// buffers of the BULK epilogue 3 at NT >= 5, else 4).
-template <int NT, bool BULK = false>
+// One stage ring per MMA group: as many stages (an A tile and a B tile of B_TILE_BYTES) as fit, at most 6.  The
+// generic kernel's B tile is 16 k' x 8*NT w' doubles, NT KiB: 4 stages at NT = 8; with the staging buffers of the
+// BULK epilogue 3 at NT >= 5, else 4.
+template <int B_TILE_BYTES, bool BULK = false>
 struct RingConfig {
-    static constexpr int kBTileBytes = NT * 1024;  // 16 k' x 8*NT w' doubles
-    static constexpr int kStageBytes = kATileBytes + kBTileBytes;
+    static constexpr int kBTileBytes = B_TILE_BYTES;
+    // stages stay 1 KiB aligned: the 128-byte TMA swizzle of the A tile is a function of the address bits
+    static constexpr int kStageBytes = kATileBytes + (kBTileBytes + 1023) / 1024 * 1024;
     static constexpr int kGroupBudget = BULK ? (227 * 1024 - kStagingBytes - 3 * 1024) / kGroups : 110 * 1024;
     static constexpr int kFit = kGroupBudget / kStageBytes;
-    static constexpr int kStages = QS_STAGES > 0 ? QS_STAGES : (kFit < 6 ? kFit : 6);
+    static constexpr int kStages = kFit < 6 ? kFit : 6;
     static constexpr int kRingBytes = kStages * kStageBytes;
     static constexpr int kBarrierBytes = (kGroups * 2 * kStages + 2) * 8;
     // rings | barriers (padded to 128 B) | staging buffers ; + 1 KiB slack for the 1 KiB alignment of the rings
     static constexpr int kStagingOffset = kGroups * kRingBytes + (kBarrierBytes + 127) / 128 * 128;
     static constexpr int kSmemBytes = kStagingOffset + (BULK ? kStagingBytes : 0) + 1024;
 };
+
+// The CTA frame of both kernels.  The barriers sit behind the two rings: group g has full[s] at bar_base + 16 g S + 8 s,
+// empty[s] S slots further, then order[g] at bar_base + 16 G S + 8 g.  The producer warp group gives its registers
+// to the MMA groups (setmaxnreg) and one lane of warp 8 + g fills group g's ring: chunk j of the group's tiles (in
+// order) goes to stage j % S.  Returns true on the MMA warps, which then hold kRegsMma registers.
+template <class Ring>
+__device__ __forceinline__ bool cta_frame(const CUtensorMap& map_a, const QuarterParams& p, uint32_t smem_base,
+                                          uint32_t my_tiles) {
+    constexpr int kStages = Ring::kStages;
+    const uint32_t bar_base = smem_base + kGroups * Ring::kRingBytes;
+    const uint32_t bar_order = bar_base + kGroups * 2 * kStages * 8;
+    if (threadIdx.x == 0) {
+        for (int gs = 0; gs < kGroups * kStages; ++gs) {
+            const uint32_t base = bar_base + (gs / kStages) * 16 * kStages + (gs % kStages) * 8;
+            mbar_init(base, 1);
+            mbar_init(base + 8 * kStages, kGroupWarps);
+        }
+        mbar_init(bar_order, kGroupWarps);
+        mbar_init(bar_order + 8, kGroupWarps);
+        mbar_fence_init();
+        prefetch_tensormap(&map_a);
+    }
+    __syncthreads();
+
+    const int warp = threadIdx.x >> 5;
+    if (warp >= kMmaWarps) {
+        asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kRegsProducer));
+        const int pg = warp - kMmaWarps;  // producer of group pg
+        if (pg >= kGroups) return false;
+        if ((threadIdx.x & 31) == 0) {
+            const uint32_t ring = smem_base + pg * Ring::kRingBytes;
+            const uint32_t bar_full = bar_base + pg * 16 * kStages;
+            const uint32_t bar_empty = bar_full + 8 * kStages;
+            uint32_t j = 0;
+            for (uint32_t i = pg; i < my_tiles; i += kGroups) {
+                const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x);
+                const uint32_t tx = divide(tile, p.tiles_w_div);
+                const uint32_t tw = tile - tx * (uint32_t)p.tiles_w;
+                const int px0 = (int)(tx * kBlockX);
+                const double* img = p.image + (size_t)tw * p.nchunks * (Ring::kBTileBytes / 8);
+                for (int c = 0; c < p.nchunks; ++c, ++j) {
+                    const uint32_t s = j % kStages;
+                    if (j >= (uint32_t)kStages) mbar_wait(bar_empty + 8 * s, ((j / kStages) - 1) & 1);
+                    const uint32_t full = bar_full + 8 * s;
+#ifdef QS_DBG_NOLOAD
+                    mbar_arrive(full);
+                    (void)px0; (void)img; (void)ring;
+#else
+                    mbar_expect_tx(full, kATileBytes + Ring::kBTileBytes);
+                    const uint32_t dst = ring + s * Ring::kStageBytes;
+                    tma_load_2d(dst, &map_a, c * kChunkK, px0, full);
+                    bulk_load_1d(dst + kATileBytes, img + (size_t)c * (Ring::kBTileBytes / 8), Ring::kBTileBytes,
+                                 full);
+#endif
+                }
+            }
+        }
+        return false;
+    }
+    asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kRegsMma));
+    return true;
+}
 
 // One persistent CTA per SM, 12 warps:
 //   warps 0-3     MMA group 0, one warp per SM sub-partition, a 32 x 8NT accumulator tile each in registers;
@@ -198,72 +294,22 @@ template <int NT, bool COMPLEX_OUT, int EPI>
 __global__ void __launch_bounds__(kThreads, 1)
 quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ QuarterParams p) {
     constexpr bool BULK = EPI == kEpiBulk;
-    using Ring = RingConfig<NT, BULK>;
-    constexpr int kBTileBytes = Ring::kBTileBytes;
+    using Ring = RingConfig<NT * 1024, BULK>;
     constexpr int kStageBytes = Ring::kStageBytes;
     constexpr int kStages = Ring::kStages;
 
     extern __shared__ unsigned char smem_raw[];
     uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     asm volatile("" : "+r"(smem_base));  // keep it in a register: ptxas otherwise re-derives it inside the main loop
-    // barriers behind the two rings: group g has full[s] at bar_base + 16 g S + 8 s, empty[s] S slots further
-    const uint32_t bar_base = smem_base + kGroups * Ring::kRingBytes;
-    const uint32_t bar_order = bar_base + kGroups * 2 * kStages * 8;  // order[g] at +8g
+    const uint32_t bar_base = smem_base + kGroups * Ring::kRingBytes;  // barrier layout: see cta_frame
+    const uint32_t bar_order = bar_base + kGroups * 2 * kStages * 8;
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
     const uint32_t total_tiles = p.tile_list ? p.n_listed : p.tiles_x * (uint32_t)p.tiles_w;
     const uint32_t my_tiles = blockIdx.x < total_tiles ? (total_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+    if (!cta_frame<Ring>(map_a, p, smem_base, my_tiles)) return;
 
-    if (threadIdx.x == 0) {
-        for (int gs = 0; gs < kGroups * kStages; ++gs) {
-            const uint32_t base = bar_base + (gs / kStages) * 16 * kStages + (gs % kStages) * 8;
-            mbar_init(base, 1);
-            mbar_init(base + 8 * kStages, kGroupWarps);
-        }
-        mbar_init(bar_order, kGroupWarps);
-        mbar_init(bar_order + 8, kGroupWarps);
-        mbar_fence_init();
-        prefetch_tensormap(&map_a);
-    }
-    __syncthreads();
-
-    if (warp >= kMmaWarps) {
-        asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kRegsProducer));
-        const int pg = warp - kMmaWarps;  // producer of group pg
-        if (pg >= kGroups) return;
-        // ===== TMA producer of group pg: chunk j of the group's tiles (in order) goes to stage j % kStages =====
-        if (lane == 0) {
-            const uint32_t ring = smem_base + pg * Ring::kRingBytes;
-            const uint32_t bar_full = bar_base + pg * 16 * kStages;
-            const uint32_t bar_empty = bar_full + 8 * kStages;
-            uint32_t j = 0;
-            for (uint32_t i = pg; i < my_tiles; i += kGroups) {
-                const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x);
-                const uint32_t tx = divide(tile, p.tiles_w_div);
-                const uint32_t tw = tile - tx * (uint32_t)p.tiles_w;
-                const int px0 = (int)(tx * kBlockX);
-                const double* img = p.image + (size_t)tw * p.nchunks * (kBTileBytes / 8);
-                for (int c = 0; c < p.nchunks; ++c, ++j) {
-                    const uint32_t s = j % kStages;
-                    if (j >= (uint32_t)kStages) mbar_wait(bar_empty + 8 * s, ((j / kStages) - 1) & 1);
-                    const uint32_t full = bar_full + 8 * s;
-#ifdef QS_DBG_NOLOAD
-                    mbar_arrive(full);
-                    (void)px0; (void)img; (void)ring;
-#else
-                    mbar_expect_tx(full, kStageBytes);
-                    const uint32_t dst = ring + s * kStageBytes;
-                    tma_load_2d(dst, &map_a, c * kChunkK, px0, full);
-                    bulk_load_1d(dst + kATileBytes, img + (size_t)c * (kBTileBytes / 8), kBTileBytes, full);
-#endif
-                }
-            }
-        }
-        return;
-    }
-
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kRegsMma));
     // ===== MMA groups: warp wg of group `group` owns rows [32 wg, 32 wg + 32) x all 8*NT columns of its tile =====
     const int group = warp >> 2;
     const int wg = warp & 3;
@@ -361,13 +407,7 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         // ordered start: the other group has passed the signal point (midpoint) of the main loop of tile i - 1
         const uint32_t k = i >> 1;
         if (i > 0) mbar_wait(bar_order + 8 * group, (group == 0 ? k - 1 : k) & 1);
-#ifdef QS_SIGNAL_END
-        const int signal_chunk = p.nchunks - 1;
-#elif defined(QS_SIGNAL_NUM)
-        const int signal_chunk = ((p.nchunks - 1) * QS_SIGNAL_NUM) >> 3;
-#else
         const int signal_chunk = (p.nchunks - 1) >> 1;
-#endif
         QS_PHASE_STAMP(1);
 
         bool tail = false;  // b[NT - 1] of the half about to start is still to be fetched
@@ -437,7 +477,7 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         const uint32_t tile_w = tile - tile_x * (uint32_t)p.tiles_w;
         const uint32_t x0 = tile_x * kBlockX;
         const uint32_t wbase = p.w_first + tile_w * (8 * NT);
-        const bool plain_w = p.w_inner == 1 && p.ndest == 0;  // plain rotated store: column address = w * sw1
+        const bool plain_w = p.w_inner == 1 && p.ndest == 0;
         if constexpr (BULK) {
             constexpr int ES = COMPLEX_OUT ? 16 : 8;         // bytes per output element
             constexpr int CPP = COMPLEX_OUT ? 8 : 16;        // output columns per pass (16 real accumulator columns)
@@ -487,33 +527,15 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                     const uint32_t wl = (COMPLEX_OUT ? (wbase >> 1) : wbase) + (uint32_t)(CPP * pass) + c;  // output column
                     // padding columns of the last column tile, and the absent second column group of an odd NT
                     if (wl >= (COMPLEX_OUT ? (p.Wp >> 1) : p.Wp) || 2 * pass + (int)(c / (CPP / 2)) >= NT) continue;
-                    const uint32_t w = dealt_column(wl, p.deal_mul, p.deal_mod);
-                    double* colp;
-                    if (plain_w) {
-                        colp = p.out + (ES / 8) * ((long long)w * p.sw1);
-                    } else {
-                        const uint32_t wq = p.w_cyclic ? w % (uint32_t)p.ndest : w / p.w_inner;
-                        const uint32_t wr = p.w_cyclic ? w / (uint32_t)p.ndest : w - wq * p.w_inner;
-                        colp = (p.ndest ? p.outs[wq] : p.out) + (ES / 8) * ((long long)wq * p.sw1 + (long long)wr * p.sw0);
-                    }
+                    double* colp = column_base<ES>(p, plain_w, wl);
                     // run `run`: rows [rs, rs + len) of the warp's 32, block xq0 + run, first row of the block xr
                     const uint32_t rs = run ? run * p.x_inner - xr0 : 0u;
                     const uint32_t xr = run ? 0u : xr0;
                     uint32_t len = p.x_inner - xr;
                     if (len > nrow - rs) len = nrow - rs;
-                    const uint32_t xq = xq0 + run;
-                    long long off = xr;
-                    if (p.x_mid != 0xFFFFFFFFu) {
-                        const uint32_t x2 = xq / p.x_mid;
-                        const uint32_t x1 = xq - x2 * p.x_mid;
-                        off += (long long)x2 * p.sx2 + (long long)x1 * p.sx1;
-                    } else if (p.xq_table) {
-                        const long long tq = p.xq_table[xq];
-                        if (tq < 0) continue;  // rows the symmetry does not need
-                        off += tq;
-                    } else {
-                        off += (long long)xq * p.sx1;
-                    }
+                    bool kept = true;
+                    const long long off = xr + block_offset(p, xq0 + run, kept);
+                    if (!kept) continue;
                     bulk_store(colp + (ES / 8) * off, buf + c * COL_BYTES + rs * ES, len * ES);
                 }
                 asm volatile("cp.async.bulk.commit_group;" ::: "memory");
@@ -562,39 +584,13 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         long long xoff[4];
         bool xok[4];
 #pragma unroll
-        for (int mt = 0; mt < 4; ++mt) {
-            const uint32_t x = x0 + 32 * wg + rbase + (mt & 1) + 16 * (mt >> 1);
-            xok[mt] = x < p.X;
-            const uint32_t xq = divide(x, p.x_inner_div);
-            const uint32_t xr = x - xq * p.x_inner;
-            long long off = (p.xr_table && xok[mt]) ? p.xr_table[xr] : (long long)xr * p.sx0;
-            if (p.x_mid != 0xFFFFFFFFu) {
-                const uint32_t x2 = xq / p.x_mid;
-                const uint32_t x1 = xq - x2 * p.x_mid;
-                off += (long long)x2 * p.sx2 + (long long)x1 * p.sx1;
-            } else if (p.xq_table && xok[mt]) {
-                const long long tq = p.xq_table[xq];
-                if (tq < 0) xok[mt] = false;  // a row the symmetry does not need
-                off += tq;
-            } else {
-                off += (long long)xq * p.sx1;
-            }
-            xoff[mt] = off;
-        }
+        for (int mt = 0; mt < 4; ++mt) xok[mt] = row_offset(p, x0 + 32 * wg + rbase + (mt & 1) + 16 * (mt >> 1), xoff[mt]);
 #pragma unroll
         for (int nt = 0; nt < NT; ++nt) {
             const uint32_t wp = wbase + 8 * nt + 2 * t;  // real column of acc[..][nt][0]; wp + 1 for [1]
             if (COMPLEX_OUT) {
                 if (wp < p.Wp) {
-                    const uint32_t w = dealt_column(wp >> 1, p.deal_mul, p.deal_mod);
-                    double* col;
-                    if (plain_w) {
-                        col = p.out + 2 * ((long long)w * p.sw1);
-                    } else {
-                        const uint32_t wq = p.w_cyclic ? w % (uint32_t)p.ndest : w / p.w_inner;
-                        const uint32_t wr = p.w_cyclic ? w / (uint32_t)p.ndest : w - wq * p.w_inner;
-                        col = (p.ndest ? p.outs[wq] : p.out) + 2 * ((long long)wq * p.sw1 + (long long)wr * p.sw0);
-                    }
+                    double* col = column_base<16>(p, plain_w, wp >> 1);
 #pragma unroll
                     for (int mt = 0; mt < 4; ++mt)
                         if (xok[mt])
@@ -604,15 +600,7 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 #pragma unroll
                 for (int e = 0; e < 2; ++e) {
                     if (wp + e < p.Wp) {
-                        const uint32_t w = dealt_column(wp + e, p.deal_mul, p.deal_mod);
-                        double* col;
-                        if (plain_w) {
-                            col = p.out + (long long)w * p.sw1;
-                        } else {
-                            const uint32_t wq = p.w_cyclic ? w % (uint32_t)p.ndest : w / p.w_inner;
-                            const uint32_t wr = p.w_cyclic ? w / (uint32_t)p.ndest : w - wq * p.w_inner;
-                            col = (p.ndest ? p.outs[wq] : p.out) + (long long)wq * p.sw1 + (long long)wr * p.sw0;
-                        }
+                        double* col = column_base<8>(p, plain_w, wp + e);
                         if (p.vec2) {
                             // rows (mt = 0, 1) and (mt = 2, 3) are adjacent and 16-byte aligned in the output
                             if (xok[0]) *reinterpret_cast<double2*>(col + xoff[0]) = make_double2(acc[0][nt][e], acc[1][nt][e]);
@@ -648,21 +636,12 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 // setmaxnreg split); a CTA tile is 128 rows x 8 NTC complex columns (NTC <= 4).
 // ---------------------------------------------------------------------------------------------
 template <int NTC>
-struct SplitRing {
-    static constexpr int kBTileBytes = NTC * 512;  // 8 complex k x 8*NTC columns, one double each
-    // stages stay 1 KiB aligned: the 128-byte TMA swizzle of the A tile is a function of the address bits
-    static constexpr int kStageBytes = kATileBytes + ((kBTileBytes + 1023) / 1024) * 1024;
-    static constexpr int kFit = (110 * 1024) / kStageBytes;
-    static constexpr int kStages = kFit < 6 ? kFit : 6;
-    static constexpr int kRingBytes = kStages * kStageBytes;
-    static constexpr int kSmemBytes = kGroups * kRingBytes + (kGroups * 2 * kStages + 2) * 8 + 1024;
-};
+using SplitRing = RingConfig<NTC * 512>;  // B tile: 8 complex k x 8*NTC columns, one double each
 
 template <int NTC>
 __global__ void __launch_bounds__(kThreads, 1)
 quarter_gemm_split_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ QuarterParams p) {
     using Ring = SplitRing<NTC>;
-    constexpr int kBTileBytes = Ring::kBTileBytes;
     constexpr int kStageBytes = Ring::kStageBytes;
     constexpr int kStages = Ring::kStages;
 
@@ -676,50 +655,8 @@ quarter_gemm_split_kernel(const __grid_constant__ CUtensorMap map_a, const __gri
     const int lane = threadIdx.x & 31;
     const uint32_t total_tiles = p.tile_list ? p.n_listed : p.tiles_x * (uint32_t)p.tiles_w;
     const uint32_t my_tiles = blockIdx.x < total_tiles ? (total_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+    if (!cta_frame<Ring>(map_a, p, smem_base, my_tiles)) return;
 
-    if (threadIdx.x == 0) {
-        for (int gs = 0; gs < kGroups * kStages; ++gs) {
-            const uint32_t base = bar_base + (gs / kStages) * 16 * kStages + (gs % kStages) * 8;
-            mbar_init(base, 1);
-            mbar_init(base + 8 * kStages, kGroupWarps);
-        }
-        mbar_init(bar_order, kGroupWarps);
-        mbar_init(bar_order + 8, kGroupWarps);
-        mbar_fence_init();
-        prefetch_tensormap(&map_a);
-    }
-    __syncthreads();
-
-    if (warp >= kMmaWarps) {
-        asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kRegsProducer));
-        const int pg = warp - kMmaWarps;
-        if (pg >= kGroups) return;
-        if (lane == 0) {
-            const uint32_t ring = smem_base + pg * Ring::kRingBytes;
-            const uint32_t bar_full = bar_base + pg * 16 * kStages;
-            const uint32_t bar_empty = bar_full + 8 * kStages;
-            uint32_t j = 0;
-            for (uint32_t i = pg; i < my_tiles; i += kGroups) {
-                const uint32_t tile = tile_at(p, blockIdx.x + i * gridDim.x);
-                const uint32_t tx = divide(tile, p.tiles_w_div);
-                const uint32_t tw = tile - tx * (uint32_t)p.tiles_w;
-                const int px0 = (int)(tx * kBlockX);
-                const double* img = p.image + (size_t)tw * p.nchunks * (kBTileBytes / 8);
-                for (int c = 0; c < p.nchunks; ++c, ++j) {
-                    const uint32_t s = j % kStages;
-                    if (j >= (uint32_t)kStages) mbar_wait(bar_empty + 8 * s, ((j / kStages) - 1) & 1);
-                    const uint32_t full = bar_full + 8 * s;
-                    mbar_expect_tx(full, kATileBytes + kBTileBytes);
-                    const uint32_t dst = ring + s * kStageBytes;
-                    tma_load_2d(dst, &map_a, c * kChunkK, px0, full);
-                    bulk_load_1d(dst + kATileBytes, img + (size_t)c * (kBTileBytes / 8), kBTileBytes, full);
-                }
-            }
-        }
-        return;
-    }
-
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kRegsMma));
     const int group = warp >> 2;
     const int wg = warp & 3;
     const uint32_t ring = smem_base + group * Ring::kRingBytes;
@@ -819,25 +756,7 @@ quarter_gemm_split_kernel(const __grid_constant__ CUtensorMap map_a, const __gri
         long long xoff[4];
         bool xok[4];
 #pragma unroll
-        for (int mt = 0; mt < 4; ++mt) {
-            const uint32_t x = x0 + 32 * wg + rbase + (mt & 1) + 16 * (mt >> 1);
-            xok[mt] = x < p.X;
-            const uint32_t xq = divide(x, p.x_inner_div);
-            const uint32_t xr = x - xq * p.x_inner;
-            long long off = (p.xr_table && xok[mt]) ? p.xr_table[xr] : (long long)xr * p.sx0;
-            if (p.x_mid != 0xFFFFFFFFu) {
-                const uint32_t x2 = xq / p.x_mid;
-                const uint32_t x1 = xq - x2 * p.x_mid;
-                off += (long long)x2 * p.sx2 + (long long)x1 * p.sx1;
-            } else if (p.xq_table && xok[mt]) {
-                const long long tq = p.xq_table[xq];
-                if (tq < 0) xok[mt] = false;  // a row the symmetry does not need
-                off += tq;
-            } else {
-                off += (long long)xq * p.sx1;
-            }
-            xoff[mt] = off;
-        }
+        for (int mt = 0; mt < 4; ++mt) xok[mt] = row_offset(p, x0 + 32 * wg + rbase + (mt & 1) + 16 * (mt >> 1), xoff[mt]);
         const uint32_t wbase = p.w_first + tile_w * (8 * NTC);  // complex columns
         const bool plain_w = p.w_inner == 1 && p.ndest == 0;
 #pragma unroll
@@ -846,15 +765,7 @@ quarter_gemm_split_kernel(const __grid_constant__ CUtensorMap map_a, const __gri
             for (int e = 0; e < 2; ++e) {
                 const uint32_t wl = wbase + 8 * ntc + 2 * t + e;
                 if (wl >= p.Wp) continue;  // Wp = number of complex columns in this mode
-                const uint32_t w = dealt_column(wl, p.deal_mul, p.deal_mod);
-                double* col;
-                if (plain_w) {
-                    col = p.out + 2 * ((long long)w * p.sw1);
-                } else {
-                    const uint32_t wq = p.w_cyclic ? w % (uint32_t)p.ndest : w / p.w_inner;
-                    const uint32_t wr = p.w_cyclic ? w / (uint32_t)p.ndest : w - wq * p.w_inner;
-                    col = (p.ndest ? p.outs[wq] : p.out) + 2 * ((long long)wq * p.sw1 + (long long)wr * p.sw0);
-                }
+                double* col = column_base<16>(p, plain_w, wl);
 #pragma unroll
                 for (int mt = 0; mt < 4; ++mt)
                     if (xok[mt])
@@ -1026,55 +937,39 @@ EncodeTiledFn get_encode_fn() {
     return fn;
 }
 
-template <int NT, bool CO, int EPI>
+// One persistent CTA per SM (at most one per tile) of KERNEL with SMEM bytes of dynamic shared memory.
+template <auto KERNEL, int SMEM>
 int launch_variant(const CUtensorMap& map, const QuarterParams& p, cudaStream_t st) {
-    constexpr int smem = RingConfig<NT, EPI == kEpiBulk>::kSmemBytes;
-    static_assert(smem <= 227 * 1024, "shared memory budget of one CTA per SM");
+    static_assert(SMEM <= 227 * 1024, "shared memory budget of one CTA per SM");
     static bool configured[kMaxDevices] = {false};  // the attribute belongs to the device's context
     const int dev = qs_current_device();
     if (!configured[dev]) {
-        QS_CUDA(cudaFuncSetAttribute(quarter_gemm_kernel<NT, CO, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        QS_CUDA(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
         configured[dev] = true;
     }
     const int64_t total = p.tile_list ? (int64_t)p.n_listed : (int64_t)p.tiles_x * p.tiles_w;
-    const int64_t resident = qs_sm_count();  // one persistent CTA per SM
+    const int64_t resident = qs_sm_count();
     const int64_t grid = total < resident ? total : resident;
-    quarter_gemm_kernel<NT, CO, EPI><<<(unsigned)grid, kThreads, smem, st>>>(map, p);
+    KERNEL<<<(unsigned)grid, kThreads, SMEM, st>>>(map, p);
     QS_LAUNCH_CHECK();
     return QS_OK;
 }
 
 template <bool CO, int EPI>
 int launch_nt(int NT, const CUtensorMap& map, const QuarterParams& p, cudaStream_t st) {
+    constexpr bool B = EPI == kEpiBulk;
     switch (NT) {
-        case 1: return launch_variant<1, CO, EPI>(map, p, st);
-        case 2: return launch_variant<2, CO, EPI>(map, p, st);
-        case 3: return launch_variant<3, CO, EPI>(map, p, st);
-        case 4: return launch_variant<4, CO, EPI>(map, p, st);
-        case 5: return launch_variant<5, CO, EPI>(map, p, st);
-        case 6: return launch_variant<6, CO, EPI>(map, p, st);
-        case 7: return launch_variant<7, CO, EPI>(map, p, st);
-        case 8: return launch_variant<8, CO, EPI>(map, p, st);
+        case 1: return launch_variant<quarter_gemm_kernel<1, CO, EPI>, RingConfig<1 * 1024, B>::kSmemBytes>(map, p, st);
+        case 2: return launch_variant<quarter_gemm_kernel<2, CO, EPI>, RingConfig<2 * 1024, B>::kSmemBytes>(map, p, st);
+        case 3: return launch_variant<quarter_gemm_kernel<3, CO, EPI>, RingConfig<3 * 1024, B>::kSmemBytes>(map, p, st);
+        case 4: return launch_variant<quarter_gemm_kernel<4, CO, EPI>, RingConfig<4 * 1024, B>::kSmemBytes>(map, p, st);
+        case 5: return launch_variant<quarter_gemm_kernel<5, CO, EPI>, RingConfig<5 * 1024, B>::kSmemBytes>(map, p, st);
+        case 6: return launch_variant<quarter_gemm_kernel<6, CO, EPI>, RingConfig<6 * 1024, B>::kSmemBytes>(map, p, st);
+        case 7: return launch_variant<quarter_gemm_kernel<7, CO, EPI>, RingConfig<7 * 1024, B>::kSmemBytes>(map, p, st);
+        case 8: return launch_variant<quarter_gemm_kernel<8, CO, EPI>, RingConfig<8 * 1024, B>::kSmemBytes>(map, p, st);
     }
     qs_set_error("internal: NT=%d out of range", NT);
     return QS_ERR_INVALID;
-}
-
-template <int NTC>
-int launch_split_variant(const CUtensorMap& map, const QuarterParams& p, cudaStream_t st) {
-    constexpr int smem = SplitRing<NTC>::kSmemBytes;
-    static bool configured[kMaxDevices] = {false};  // the attribute belongs to the device's context
-    const int dev = qs_current_device();
-    if (!configured[dev]) {
-        QS_CUDA(cudaFuncSetAttribute(quarter_gemm_split_kernel<NTC>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        configured[dev] = true;
-    }
-    const int64_t total = p.tile_list ? (int64_t)p.n_listed : (int64_t)p.tiles_x * p.tiles_w;
-    const int64_t resident = qs_sm_count();
-    const int64_t grid = total < resident ? total : resident;
-    quarter_gemm_split_kernel<NTC><<<(unsigned)grid, kThreads, smem, st>>>(map, p);
-    QS_LAUNCH_CHECK();
-    return QS_OK;
 }
 
 template <bool CO>
@@ -1096,10 +991,10 @@ Divisor make_divisor(uint64_t d) {
 
 int launch_split(int NTC, const CUtensorMap& map, const QuarterParams& p, cudaStream_t st) {
     switch (NTC) {
-        case 1: return launch_split_variant<1>(map, p, st);
-        case 2: return launch_split_variant<2>(map, p, st);
-        case 3: return launch_split_variant<3>(map, p, st);
-        case 4: return launch_split_variant<4>(map, p, st);
+        case 1: return launch_variant<quarter_gemm_split_kernel<1>, SplitRing<1>::kSmemBytes>(map, p, st);
+        case 2: return launch_variant<quarter_gemm_split_kernel<2>, SplitRing<2>::kSmemBytes>(map, p, st);
+        case 3: return launch_variant<quarter_gemm_split_kernel<3>, SplitRing<3>::kSmemBytes>(map, p, st);
+        case 4: return launch_variant<quarter_gemm_split_kernel<4>, SplitRing<4>::kSmemBytes>(map, p, st);
     }
     qs_set_error("internal: NTC=%d out of range", NTC);
     return QS_ERR_INVALID;
@@ -1377,27 +1272,26 @@ bool planned_lists(const Tiling& tl, int a_dtype, int m_dtype, int64_t X, int64_
     return true;
 }
 
-int quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda, const void* image, int m_dtype,
-                   int64_t W, void* out, void* const* out_table, int64_t n_dest, int64_t x_inner, int64_t x_mid,
-                   int64_t sx0, int64_t sx1, int64_t sx2, int64_t w_inner, int64_t sw0, int64_t sw1, int64_t w_deal,
-                   void* stream, const QsTileMask* mask = nullptr, void* list_ws = nullptr,
-                   const long long* xq_table = nullptr, const long long* xr_table = nullptr,
-                   const long long* host_xq_table = nullptr, int xq_even = 0, int w_cyclic = 0,
-                   int xr_paired = 0) {
-    QS_REQUIRE(A && image && (out || out_table), "qs_quarter_transform: null pointer");
-    QS_REQUIRE(w_deal >= 1 && w_deal < (W > 1 ? W : 2) && gcd64(w_deal, W) == 1,
+}  // namespace
+
+// Internal (common.cuh): one quarter transform, stored as `s` describes.
+int qs_quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda, const void* image, int m_dtype,
+                      int64_t W, const QsQuarterStore& s, void* stream) {
+    QS_REQUIRE(A && image && (s.out || s.out_table), "qs_quarter_transform: null pointer");
+    QS_REQUIRE(s.w_deal >= 1 && s.w_deal < (W > 1 ? W : 2) && gcd64(s.w_deal, W) == 1,
                "qs_quarter_transform_scatter: the dealing multiplier %lld is not coprime to W = %lld",
-               (long long)w_deal, (long long)W);
+               (long long)s.w_deal, (long long)W);
     QS_REQUIRE(X > 0 && K > 0 && W > 0 && lda >= K, "qs_quarter_transform: bad extents");
     QS_REQUIRE(X < (1LL << 31) - kBlockX, "qs_quarter_transform: X=%lld exceeds 2^31", (long long)X);
-    QS_REQUIRE(x_inner > 0 && w_inner > 0 && x_inner < (1LL << 32) && w_inner < (1LL << 31) && x_mid > 0 &&
-                   x_mid < (1LL << 32),
+    QS_REQUIRE(s.x_inner > 0 && s.w_inner > 0 && s.x_inner < (1LL << 32) && s.w_inner < (1LL << 31) && s.x_mid > 0 &&
+                   s.x_mid < (1LL << 32),
                "qs_quarter_transform: bad inner extents");
+    const int64_t n_dest = s.n_dest;
     QS_REQUIRE(n_dest >= 0 && n_dest <= kMaxDest, "qs_quarter_transform_scatter: at most %d destinations", kMaxDest);
-    QS_REQUIRE(n_dest == 0 || w_cyclic || qs_ceil_div(W, w_inner) <= n_dest,
+    QS_REQUIRE(n_dest == 0 || s.w_cyclic || qs_ceil_div(W, s.w_inner) <= n_dest,
                "qs_quarter_transform_scatter: W=%lld needs more than %lld destinations of %lld", (long long)W,
-               (long long)n_dest, (long long)w_inner);
-    QS_REQUIRE(!w_cyclic || n_dest > 0, "qs_quarter_transform_scatter: cyclic columns need a destination table");
+               (long long)n_dest, (long long)s.w_inner);
+    QS_REQUIRE(!s.w_cyclic || n_dest > 0, "qs_quarter_transform_scatter: cyclic columns need a destination table");
     const Tiling tl = make_tiling(K, W, a_dtype, m_dtype);
     const bool out_complex = a_dtype == QS_C128 || m_dtype == QS_C128;
     const int64_t pitch_bytes = lda * 8 * qs_elem_doubles(a_dtype);
@@ -1406,10 +1300,10 @@ int quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda
     // A and the image are TMA / bulk-copy sources (16 bytes); the epilogue stores whole elements
     const uintptr_t out_mask = out_complex ? 15 : 7;
     QS_REQUIRE((reinterpret_cast<uintptr_t>(A) & 15) == 0 && (reinterpret_cast<uintptr_t>(image) & 15) == 0 &&
-                   (reinterpret_cast<uintptr_t>(out) & out_mask) == 0,
+                   (reinterpret_cast<uintptr_t>(s.out) & out_mask) == 0,
                "qs_quarter_transform: A and image must be 16-byte aligned, out element-aligned");
     for (int64_t d = 0; d < n_dest; ++d)
-        QS_REQUIRE(out_table[d] && (reinterpret_cast<uintptr_t>(out_table[d]) & out_mask) == 0,
+        QS_REQUIRE(s.out_table[d] && (reinterpret_cast<uintptr_t>(s.out_table[d]) & out_mask) == 0,
                    "qs_quarter_transform_scatter: destination %lld is null or misaligned", (long long)d);
 
     EncodeTiledFn encode = get_encode_fn();
@@ -1420,7 +1314,7 @@ int quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda
     const cuuint32_t box[2] = {kChunkK, kBlockX};
     const cuuint32_t estr[2] = {1, 1};
     CUresult cr = encode(&map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, const_cast<void*>(A), gdim, gstride, box, estr,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, QS_L2_PROMOTION,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (cr != CUDA_SUCCESS) {
         qs_set_error("cuTensorMapEncodeTiled failed with CUresult %d (X=%lld K'=%d pitch=%lld)", (int)cr, (long long)X,
@@ -1428,55 +1322,54 @@ int quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda
         return QS_ERR_CUDA;
     }
 
-    if (host_xq_table) {  // the caller's own table: every kept entry must be even for 16-byte aligned real runs
+    int xq_even = s.xq_even;
+    if (s.host_xq_table) {  // the caller's own table: every kept entry must be even for 16-byte aligned real runs
         xq_even = 1;
-        for (int64_t q = 0, nq = qs_ceil_div(X, x_inner); q < nq && xq_even; ++q)
-            xq_even = host_xq_table[q] < 0 || host_xq_table[q] % 2 == 0;
+        for (int64_t q = 0, nq = qs_ceil_div(X, s.x_inner); q < nq && xq_even; ++q)
+            xq_even = s.host_xq_table[q] < 0 || s.host_xq_table[q] % 2 == 0;
     }
-    // 16-byte row-pair stores of the real epilogue need adjacent, aligned rows and even strides everywhere.  With
-    // tabulated offsets that is the table's business: block offsets (xq_table) must be even, and a per-row table
-    // (xr_table) must place rows 2k and 2k + 1 next to each other at an even offset (`xr_paired`, the caller's promise).
-    const bool rows_adjacent = xr_table ? xr_paired != 0 : sx0 == 1;
-    int vec2 = !out_complex && rows_adjacent && x_inner % 2 == 0 && X % 2 == 0 && sx1 % 2 == 0 && sx2 % 2 == 0 &&
-               sw0 % 2 == 0 && (n_dest > 0 || sw1 % 2 == 0) && (reinterpret_cast<uintptr_t>(out) & 15) == 0 &&
-               (!xq_table || xq_even);
-    for (int64_t d = 0; d < n_dest; ++d) vec2 = vec2 && (reinterpret_cast<uintptr_t>(out_table[d]) & 15) == 0;
+    // Real rows leave in 16-byte pieces (row pairs of the register epilogue, runs of the staged one) when all extents,
+    // strides and bases are even and every destination is 16-byte aligned.  With tabulated offsets that is the
+    // table's business: block offsets (xq_table) must be even.
+    bool even16 = s.x_inner % 2 == 0 && X % 2 == 0 && s.sx1 % 2 == 0 && s.sx2 % 2 == 0 && s.sw0 % 2 == 0 &&
+                  (n_dest > 0 || s.sw1 % 2 == 0) && (reinterpret_cast<uintptr_t>(s.out) & 15) == 0 &&
+                  (!s.xq_table || xq_even);
+    for (int64_t d = 0; d < n_dest; ++d) even16 = even16 && (reinterpret_cast<uintptr_t>(s.out_table[d]) & 15) == 0;
+    // Row-pair stores of the real register epilogue also need rows 2k, 2k + 1 adjacent: sx0 = 1, or a per-row table
+    // (xr_table) that places them so (`xr_paired`, the caller's promise).
+    const bool rows_adjacent = s.xr_table ? s.xr_paired != 0 : s.sx0 == 1;
+    const int vec2 = !out_complex && rows_adjacent && even16;
     // Staged asynchronous epilogue: consecutive rows of a block are adjacent in the output (sx0 = 1) and every run of
-    // rows handed to cp.async.bulk starts 16-byte aligned: always for complex output (16-byte elements); for real
-    // output when all extents, strides and bases are even (the conditions of vec2), with an even row table.
-    // Rows placed one by one (xr_table) keep the register stores.
-    int bulk = (bulk_mode() == 2 || (bulk_mode() == 1 && n_dest > 1)) && sx0 == 1 && !xr_table && !tl.split;
-    if (bulk && !out_complex) {
-        bulk = x_inner % 2 == 0 && X % 2 == 0 && sx1 % 2 == 0 && sx2 % 2 == 0 && sw0 % 2 == 0 &&
-               (n_dest > 0 || sw1 % 2 == 0) && (reinterpret_cast<uintptr_t>(out) & 15) == 0 && (!xq_table || xq_even);
-        for (int64_t d = 0; d < n_dest; ++d) bulk = bulk && (reinterpret_cast<uintptr_t>(out_table[d]) & 15) == 0;
-    }
+    // rows handed to cp.async.bulk starts 16-byte aligned: always for complex output (16-byte elements), for real
+    // output under the conditions above.  Rows placed one by one (xr_table) keep the register stores.
+    const bool bulk = (bulk_mode() == 2 || (bulk_mode() == 1 && n_dest > 1)) && s.sx0 == 1 && !s.xr_table &&
+                      !tl.split && (out_complex || even16);
     // The rotated epilogue: one local destination, undealt columns, no row tables, the two-level row split with
     // adjacent rows, and 16-byte row pairs for real output.
-    const bool rotated = n_dest == 0 && w_deal == 1 && !xq_table && !xr_table && x_mid == 0xFFFFFFFFLL && w_inner == 1 &&
-                         sx0 == 1 && (out_complex || vec2);
+    const bool rotated = n_dest == 0 && s.w_deal == 1 && !s.xq_table && !s.xr_table && s.x_mid == 0xFFFFFFFFLL &&
+                         s.w_inner == 1 && s.sx0 == 1 && (out_complex || vec2);
     const int epi = bulk ? kEpiBulk : rotated ? kEpiRotated : kEpiStrided;
 
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     // symmetry mask: per tile group, the ascending list of wanted linear tile ids, staged into list_ws
     std::vector<uint32_t> lists[2];
     double wanted_fraction = 1.0;
-    QS_REQUIRE(!(xq_table || xr_table) || x_mid == 0xFFFFFFFFLL,
+    QS_REQUIRE(!(s.xq_table || s.xr_table) || s.x_mid == 0xFFFFFFFFLL,
                "qs_quarter_transform: row-offset tables need the two-level row split");
-    const bool masked = (mask && mask->kind) || host_xq_table;
+    const bool masked = (s.mask && s.mask->kind) || s.host_xq_table;
     PlannedLists cached;
     memset(&cached, 0, sizeof(cached));
     bool lists_cached = false;
     if (masked) {
-        QS_REQUIRE(list_ws && w_deal == 1, "qs_quarter_transform: a masked launch needs list space and undealt columns");
-        lists_cached = planned_lists(tl, a_dtype, m_dtype, X, x_inner, K, W, out_complex, mask, host_xq_table, &cached,
-                                     lists);
+        QS_REQUIRE(s.list_ws && s.w_deal == 1, "qs_quarter_transform: a masked launch needs list space and undealt columns");
+        lists_cached = planned_lists(tl, a_dtype, m_dtype, X, s.x_inner, K, W, out_complex, s.mask, s.host_xq_table,
+                                     &cached, lists);
         wanted_fraction = cached.fraction;
     }
     int span = -1;
     // issued flops; the split variant's Wp counts complex columns, each fed by Kp real multiply-adds per row
     qs_timing_begin(QS_FAMILY_QUARTER_GEMM, 2.0 * (double)X * tl.Kp * tl.Wp * wanted_fraction, stream, &span);
-    uint32_t* list_dev = static_cast<uint32_t*>(list_ws);
+    uint32_t* list_dev = static_cast<uint32_t*>(s.list_ws);
     for (int gi = 0; gi < tl.ngroups; ++gi) {
         const TileGroup& gr = tl.group[gi];
         QuarterParams p;
@@ -1496,9 +1389,9 @@ int quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda
             list_dev += (lists[gi].size() + 3) / 4 * 4;
         }
         p.image = static_cast<const double*>(image) + gr.image_offset;
-        p.out = static_cast<double*>(out);
+        p.out = static_cast<double*>(s.out);
         p.ndest = (int)n_dest;
-        for (int64_t d = 0; d < n_dest; ++d) p.outs[d] = static_cast<double*>(out_table[d]);
+        for (int64_t d = 0; d < n_dest; ++d) p.outs[d] = static_cast<double*>(s.out_table[d]);
         p.X = (uint32_t)X;
         p.Wp = (uint32_t)tl.Wp;
         p.w_first = (uint32_t)gr.w_first;
@@ -1506,24 +1399,23 @@ int quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda
         p.nchunks = tl.nchunks;
         p.last_halves = tl.last_halves;
         p.tiles_w = gr.tiles_w;
-        p.x_inner = (uint32_t)x_inner;
-        p.x_inner_div = make_divisor((uint64_t)x_inner);
+        p.x_inner = (uint32_t)s.x_inner;
+        p.x_inner_div = make_divisor((uint64_t)s.x_inner);
         p.tiles_w_div = make_divisor((uint64_t)gr.tiles_w);
-        p.x_mid = (uint32_t)x_mid;
-        p.w_inner = (uint32_t)w_inner;
-        p.sx0 = sx0;
-        p.sx1 = sx1;
-        p.sx2 = sx2;
-        p.sw0 = sw0;
-        p.sw1 = n_dest ? 0 : sw1;
+        p.x_mid = (uint32_t)s.x_mid;
+        p.w_inner = (uint32_t)s.w_inner;
+        p.sx0 = s.sx0;
+        p.sx1 = s.sx1;
+        p.sx2 = s.sx2;
+        p.sw0 = s.sw0;
+        p.sw1 = n_dest ? 0 : s.sw1;
         p.vec2 = vec2;
-        p.deal_mul = (uint32_t)w_deal;
+        p.deal_mul = (uint32_t)s.w_deal;
         p.deal_mod = (uint32_t)W;
-        p.w_cyclic = w_cyclic;
-        p.xq_table = xq_table;
-        p.xr_table = xr_table;
+        p.w_cyclic = s.w_cyclic;
+        p.xq_table = s.xq_table;
+        p.xr_table = s.xr_table;
         QS_REQUIRE((int64_t)p.tiles_x * p.tiles_w < (1LL << 31), "qs_quarter_transform: too many tiles");
-        p.bulk = bulk;
         const int rc = tl.split      ? launch_split(gr.NT, map, p, st)
                        : out_complex ? launch_epilogue<true>(epi, gr.NT, map, p, st)
                                      : launch_epilogue<false>(epi, gr.NT, map, p, st);
@@ -1533,25 +1425,12 @@ int quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda
     return QS_OK;
 }
 
-}  // namespace
-
-// Internal (common.cuh): a quarter transform restricted to the tiles a symmetry mask wants.  list_ws needs
-// qs_tile_list_bytes() bytes of device memory.
+// Internal (common.cuh): device memory a masked quarter transform needs for its tile lists (QsQuarterStore::list_ws).
 int64_t qs_tile_list_bytes(int64_t X, int64_t K, int64_t W, int a_dtype, int m_dtype) {
     const Tiling tl = make_tiling(K, W, a_dtype, m_dtype);
     int64_t tiles = 0;
     for (int gi = 0; gi < tl.ngroups; ++gi) tiles += qs_ceil_div(X, kBlockX) * tl.group[gi].tiles_w + 4;
     return tiles * (int64_t)sizeof(uint32_t);
-}
-
-int qs_quarter_transform_masked(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda, const void* image,
-                                int m_dtype, int64_t W, void* out, int64_t x_inner, int64_t sx0, int64_t sx1,
-                                int64_t w_inner, int64_t sw0, int64_t sw1, const QsTileMask* mask, void* list_ws,
-                                const long long* xq_table, const long long* xr_table, int xq_even, int xr_paired,
-                                void* stream) {
-    return quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, out, nullptr, 0, x_inner, 0xFFFFFFFFLL, sx0, sx1, 0,
-                          w_inner, sw0, sw1, 1, stream, mask, list_ws, xq_table, xr_table, nullptr, xq_even, 0,
-                          xr_paired);
 }
 
 // Host-only: the tiles a masked quarter transform would launch, as rows of (first row, last row, first output
@@ -1604,10 +1483,17 @@ extern "C" int qs_quarter_transform_rows(const void* A, int a_dtype, int64_t X, 
     QS_REQUIRE(host_xq_table && xq_table && list_ws, "qs_quarter_transform_rows: null pointer");
     QS_REQUIRE(X > 0 && K > 0 && W > 0 && list_ws_bytes >= qs_tile_list_bytes(X, K, W, a_dtype, m_dtype),
                "qs_quarter_transform_rows: tile-list space too small");
-    return quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, out, nullptr, 0, x_inner, 0xFFFFFFFFLL, sx0, 0, 0,
-                          w_inner, sw0, sw1, 1, stream, nullptr, list_ws,
-                          reinterpret_cast<const long long*>(xq_table), nullptr,
-                          reinterpret_cast<const long long*>(host_xq_table));
+    QsQuarterStore s;
+    s.out = out;
+    s.x_inner = x_inner;
+    s.sx0 = sx0;
+    s.xq_table = reinterpret_cast<const long long*>(xq_table);
+    s.host_xq_table = reinterpret_cast<const long long*>(host_xq_table);
+    s.w_inner = w_inner;
+    s.sw0 = sw0;
+    s.sw1 = sw1;
+    s.list_ws = list_ws;
+    return qs_quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, s, stream);
 }
 
 extern "C" int qs_quarter_transform_scatter_rows(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda,
@@ -1616,9 +1502,17 @@ extern "C" int qs_quarter_transform_scatter_rows(const void* A, int a_dtype, int
                                                  int64_t sx1, const int64_t* xr_table, int64_t w_inner, int64_t sw0,
                                                  int64_t w_deal, int rows_paired, void* stream) {
     QS_REQUIRE(host_out_table && n_dest > 0 && xr_table, "qs_quarter_transform_scatter_rows: null pointer");
-    return quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, nullptr, host_out_table, n_dest, x_inner,
-                          0xFFFFFFFFLL, 0, sx1, 0, w_inner, sw0, 0, w_deal, stream, nullptr, nullptr, nullptr,
-                          reinterpret_cast<const long long*>(xr_table), nullptr, 0, 0, rows_paired);
+    QsQuarterStore s;
+    s.out_table = host_out_table;
+    s.n_dest = n_dest;
+    s.x_inner = x_inner;
+    s.sx1 = sx1;
+    s.xr_table = reinterpret_cast<const long long*>(xr_table);
+    s.xr_paired = rows_paired;
+    s.w_inner = w_inner;
+    s.sw0 = sw0;
+    s.w_deal = w_deal;
+    return qs_quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, s, stream);
 }
 
 // The scattering store restricted to the CTA tiles that hold a pair (column r, row index s) the cyclic pair rule of
@@ -1636,15 +1530,33 @@ extern "C" int qs_quarter_transform_scatter_pairs(const void* A, int a_dtype, in
                    list_ws_bytes >= qs_tile_list_bytes(X, K, W, a_dtype, m_dtype),
                "qs_quarter_transform_scatter_pairs: bad extents or tile-list space too small");
     const QsTileMask mask = {3, padded ? 0 : 1, 1, 1, rows_per_s, W};
-    return quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, nullptr, host_out_table, n_dest, x_inner, x_mid, sx0,
-                          sx1, sx2, 1, sw0, 0, 1, stream, &mask, list_ws, nullptr, nullptr, nullptr, 0, /*w_cyclic=*/1);
+    QsQuarterStore s;
+    s.out_table = host_out_table;
+    s.n_dest = n_dest;
+    s.w_cyclic = 1;
+    s.x_inner = x_inner;
+    s.x_mid = x_mid;
+    s.sx0 = sx0;
+    s.sx1 = sx1;
+    s.sx2 = sx2;
+    s.sw0 = sw0;
+    s.mask = &mask;
+    s.list_ws = list_ws;
+    return qs_quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, s, stream);
 }
 
 extern "C" int qs_quarter_transform(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda, const void* image,
                                     int m_dtype, int64_t W, void* out, int64_t x_inner, int64_t sx0, int64_t sx1,
                                     int64_t w_inner, int64_t sw0, int64_t sw1, void* stream) {
-    return quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, out, nullptr, 0, x_inner, 0xFFFFFFFFLL, sx0, sx1, 0,
-                          w_inner, sw0, sw1, 1, stream);
+    QsQuarterStore s;
+    s.out = out;
+    s.x_inner = x_inner;
+    s.sx0 = sx0;
+    s.sx1 = sx1;
+    s.w_inner = w_inner;
+    s.sw0 = sw0;
+    s.sw1 = sw1;
+    return qs_quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, s, stream);
 }
 
 extern "C" int qs_quarter_transform_scatter(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda,
@@ -1653,7 +1565,17 @@ extern "C" int qs_quarter_transform_scatter(const void* A, int a_dtype, int64_t 
                                             int64_t sx2, int64_t w_inner, int64_t sw0, int64_t w_deal,
                                             int w_cyclic, void* stream) {
     QS_REQUIRE(host_out_table && n_dest > 0, "qs_quarter_transform_scatter: empty destination table");
-    return quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, nullptr, host_out_table, n_dest, x_inner, x_mid, sx0,
-                          sx1, sx2, w_inner, sw0, 0, w_deal, stream, nullptr, nullptr, nullptr, nullptr, nullptr, 0,
-                          w_cyclic);
+    QsQuarterStore s;
+    s.out_table = host_out_table;
+    s.n_dest = n_dest;
+    s.w_cyclic = w_cyclic;
+    s.w_deal = w_deal;
+    s.x_inner = x_inner;
+    s.x_mid = x_mid;
+    s.sx0 = sx0;
+    s.sx1 = sx1;
+    s.sx2 = sx2;
+    s.w_inner = w_inner;
+    s.sw0 = sw0;
+    return qs_quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, s, stream);
 }

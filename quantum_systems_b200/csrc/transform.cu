@@ -89,9 +89,15 @@ int rotated_quarter(const void* A, int a_dtype, int64_t X, int64_t K, int64_t ld
 int masked_rotated_quarter(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda, const void* image,
                            int m_dtype, int64_t W, void* out, int64_t lo_extent, int64_t lo_pitch,
                            const QsTileMask* mask, void* list_ws, void* stream) {
-    const int64_t plane = X / lo_extent * lo_pitch;
-    return qs_quarter_transform_masked(A, a_dtype, X, K, lda, image, m_dtype, W, out, lo_extent, 1, lo_pitch, 1, 0,
-                                       plane, mask, list_ws, nullptr, nullptr, 0, 0, stream);
+    QsQuarterStore s;
+    s.out = out;
+    s.x_inner = lo_extent;
+    s.sx0 = 1;
+    s.sx1 = lo_pitch;
+    s.sw1 = X / lo_extent * lo_pitch;
+    s.mask = mask;
+    s.list_ws = list_ws;
+    return qs_quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, s, stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -310,14 +316,25 @@ extern "C" int qs_transform_two_body_symmetric(const void* u, int u_dtype, const
     if ((rc = masked_rotated_quarter(bufA, td, M * N * N, N, P, img2, c_dtype, M, bufB, N, P, &m2, lists, stream))) return rc;
     // step 3: rows (r, s, a) -- tiles wanted iff they hold some r < s;  packed store T3p[q, pair(r, s), a]
     const QsTileMask m3 = {2, strict, M * N, M, N, M};
-    if ((rc = qs_quarter_transform_masked(bufB, td, M * M * N, N, P, img3, c_dtype, M, bufA, N, 1, 0, 1, 0, npairs * P,
-                                          &m3, lists, dev_slot_of_rs, nullptr, /*xq_even=*/P % 2 == 0, 0, stream)))
-        return rc;
+    QsQuarterStore s3;
+    s3.out = bufA;
+    s3.x_inner = N;
+    s3.sx0 = 1;
+    s3.sw1 = npairs * P;
+    s3.xq_table = dev_slot_of_rs;
+    s3.xq_even = P % 2 == 0;
+    s3.mask = &m3;
+    s3.list_ws = lists;
+    if ((rc = qs_quarter_launch(bufB, td, M * M * N, N, P, img3, c_dtype, M, s3, stream))) return rc;
     // step 4: dense over rows (q, pair);  out[p, q, r, s] at p M^3 + q M^2 + (r M + s)(pair)
-    if ((rc = qs_quarter_transform_masked(bufA, td, M * npairs, N, P, img3, c_dtype, M, out, npairs, 0, M * M, 1, 0,
-                                          M * M * M, nullptr, nullptr, nullptr, dev_rs_of_pair, 0, /*xr_paired=*/paired,
-                                          stream)))
-        return rc;
+    QsQuarterStore s4;
+    s4.out = out;
+    s4.x_inner = npairs;
+    s4.sx1 = M * M;
+    s4.sw1 = M * M * M;
+    s4.xr_table = dev_rs_of_pair;
+    s4.xr_paired = paired;
+    if ((rc = qs_quarter_launch(bufA, td, M * npairs, N, P, img3, c_dtype, M, s4, stream))) return rc;
     return qs_mirror_fill(out, td, M, symmetry, stream);
 }
 

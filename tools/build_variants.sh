@@ -15,14 +15,5 @@ build noload_nostore -DQS_DBG_NOLOAD -DQS_DBG_NOSTORE
 build nolds -DQS_DBG_NOLDS -DQS_DBG_NOSTORE
 build nowait -DQS_DBG_NOWAIT -DQS_DBG_NOLOAD -DQS_DBG_NOSTORE
 build nolds_nowait -DQS_DBG_NOLDS -DQS_DBG_NOWAIT -DQS_DBG_NOLOAD -DQS_DBG_NOSTORE
-build sigend -DQS_SIGNAL_END
-build sig1 -DQS_SIGNAL_NUM=1
-build sig2 -DQS_SIGNAL_NUM=2
-build sig3 -DQS_SIGNAL_NUM=3
-build sig5 -DQS_SIGNAL_NUM=5
-build sig6 -DQS_SIGNAL_NUM=6
-build stages6 -DQS_STAGES=6
-build l2none -DQS_L2_PROMOTION=CU_TENSOR_MAP_L2_PROMOTION_NONE
-build l2_128 -DQS_L2_PROMOTION=CU_TENSOR_MAP_L2_PROMOTION_L2_128B
 wait
 ls -la tools/variants

@@ -1,6 +1,6 @@
 // Stand-alone timing of the quarter GEMM (development aid): build variants with -D switches and
 // compare them in one gpurun call.
-//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 [-DQS_STAGES=3 ...] -o qgemm_bench \
+//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 [-DQS_DBG_NOSTORE ...] -o qgemm_bench \
 //        tools/qgemm_bench.cu quantum_systems_b200/csrc/quarter_gemm.cu quantum_systems_b200/csrc/core.cu
 #include <cuda_runtime.h>
 #include <stdio.h>
