@@ -123,6 +123,14 @@ int qs_mirror_fill(void* out, int dtype, int64_t m, int mode, void* stream);
 // Internal (not part of the C ABI): coefficient image of the ODQD shielded-Coulomb matrix.
 int qs_build_coulomb_image(const double* grid, double alpha, double a, int64_t Gp, void* image, void* stream);
 
+// Internal (not part of the C ABI): planes p in [p_begin, p_end) of qs_transform_two_body_diagonal (structured.cu),
+// written to `out`, which points at plane p_begin; the arguments are checked by the exported entries.  A null w2d
+// means that the caller has already written the coefficient image of W (w_dtype, as qs_build_coeff_image lays it out
+// for A = D) at the start of the workspace: the ODQD build generates it there with qs_build_coulomb_image.
+int qs_transform_diagonal_planes(const void* w2d, int w_dtype, const void* C, const void* Ct, int c_dtype, int64_t n,
+                                 int64_t m, int64_t p_begin, int64_t p_end, int anti_symmetrize, void* out,
+                                 void* workspace, void* stream);
+
 #ifdef __CUDACC__
 // ---------------------------------------------------------------------------------------------
 // PTX wrappers: mbarrier, TMA (tensor and 1-D bulk), FP64 tensor-core MMA

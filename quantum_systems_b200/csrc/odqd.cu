@@ -1,64 +1,18 @@
 // ODQD grid Coulomb build:  u_abcd = sum_pq C_pa C_qb C_pc C_qd W_pq,  W_pq = alpha / sqrt((x_p-x_q)^2 + a^2)
 //
 // Replaces the 5-operand einsum of ODQD.setup_basis (reference quantum_dots/one_dim/one_dim_qd.py:275-280),
-// which numpy contracts as two chained GEMMs.  Here:
-//   D[(a,c), p] = C[p,a] C[p,c]                      (Khatri-Rao rows, memory-bound kernel below)
-//   Tt[q, (a,c)] = sum_p D[(a,c), p] W[p, q]         (quarter GEMM, plain rotated store; W image generated from the grid)
-//   u[a,b,c,d]  = sum_q D[(b,d), q] Tt[q, (a,c)]     (quarter GEMM; the acbd -> abcd permutation is the store stride)
+// which numpy contracts as two chained GEMMs.  It is the transform of the diagonal two-body operator W with the grid
+// eigenvectors C and Ct = C^T (structured.cu): D[(a,c), p] = C[p,a] C[p,c], Tt = (D W)^T, u = T D^T with the
+// acbd -> abcd permutation in the store stride.  W is generated from the grid straight into its coefficient image.
 //
 // Multi-GPU (SURVEY.md section 8e): the build shards on the leading index a.  A rank computes only the rows
 // (a_loc, c) of T and the planes u[a_begin:a_end] -- C and the grid are replicated, D is built whole (it is the
 // A operand of the second GEMM for every (b, d)), and there is no communication.
 #include "common.cuh"
 
-namespace {
-
-struct OdqdPlan {
-    int64_t pitch, d_bytes, tt_bytes, img1_bytes, img2_bytes, total;
-};
-
-int make_odqd_plan(int64_t l, int64_t Gp, OdqdPlan* plan) {
-    plan->pitch = Gp + (Gp & 1);
-    plan->d_bytes = qs_round_up(l * l * plan->pitch * 8, 1024);
-    plan->tt_bytes = qs_round_up(Gp * l * l * 8, 1024);
-    int rc = qs_coeff_image_bytes(Gp, Gp, QS_F64, QS_F64, &plan->img1_bytes);
-    if (rc) return rc;
-    rc = qs_coeff_image_bytes(Gp, l * l, QS_F64, QS_F64, &plan->img2_bytes);
-    if (rc) return rc;
-    plan->img1_bytes = qs_round_up(plan->img1_bytes, 1024);
-    plan->img2_bytes = qs_round_up(plan->img2_bytes, 1024);
-    plan->total = plan->d_bytes + plan->tt_bytes + plan->img1_bytes + plan->img2_bytes;
-    return QS_OK;
-}
-
-// D[(a*l + c) * pitch + p] = C[p*l + a] * C[p*l + c]; block handles 32 grid points x all (a, c)
-__global__ void __launch_bounds__(256) khatri_rao_kernel(const double* __restrict__ C, double* __restrict__ D, int l,
-                                                         int Gp, int pitch) {
-    extern __shared__ double cs[];  // [32][l + 1]
-    const int p0 = blockIdx.x * 32;
-    const int ld = l + 1;
-    for (int i = threadIdx.x; i < 32 * l; i += blockDim.x) {
-        const int pp = i / l, a = i - pp * l;
-        cs[pp * ld + a] = (p0 + pp < Gp) ? C[(long long)(p0 + pp) * l + a] : 0.0;
-    }
-    __syncthreads();
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-    const int p = p0 + lane;
-    for (int ac = warp; ac < l * l; ac += nwarps) {
-        const int a = ac / l, c = ac - a * l;
-        if (p < pitch) D[(long long)ac * pitch + p] = cs[lane * ld + a] * cs[lane * ld + c];
-    }
-}
-
-}  // namespace
-
 extern "C" int qs_odqd_coulomb_workspace_bytes(int64_t l, int64_t Gp, int64_t* bytes) {
     QS_REQUIRE(l > 0 && Gp > 0 && bytes, "qs_odqd_coulomb_workspace_bytes: bad arguments");
-    OdqdPlan plan;
-    int rc = make_odqd_plan(l, Gp, &plan);
-    if (rc) return rc;
-    *bytes = plan.total;
-    return QS_OK;
+    return qs_transform_two_body_diagonal_workspace_bytes(Gp, l, QS_F64, QS_F64, 0, bytes);
 }
 
 extern "C" int qs_odqd_coulomb(const double* Cmat, const double* grid, double alpha, double a, int64_t l, int64_t Gp,
@@ -73,37 +27,13 @@ extern "C" int qs_odqd_coulomb_planes(const double* Cmat, const double* grid, do
     QS_REQUIRE(0 <= a_begin && a_begin <= a_end && a_end <= l, "qs_odqd_coulomb: bad plane range");
     if (a_begin == a_end) return QS_OK;  // an empty shard
     QS_REQUIRE(Cmat && grid && u_out && workspace, "qs_odqd_coulomb: null pointer");
-    OdqdPlan plan;
-    int rc = make_odqd_plan(l, Gp, &plan);
+    int64_t need;
+    int rc = qs_odqd_coulomb_workspace_bytes(l, Gp, &need);
     if (rc) return rc;
-    QS_REQUIRE(workspace_bytes >= plan.total, "qs_odqd_coulomb: workspace too small (%lld < %lld)",
-               (long long)workspace_bytes, (long long)plan.total);
+    QS_REQUIRE(workspace_bytes >= need, "qs_odqd_coulomb: workspace too small (%lld < %lld)",
+               (long long)workspace_bytes, (long long)need);
     QS_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0, "qs_odqd_coulomb: workspace must be 1 KiB aligned");
-    char* ws = static_cast<char*>(workspace);
-    double* D = reinterpret_cast<double*>(ws);
-    double* Tt = reinterpret_cast<double*>(ws + plan.d_bytes);
-    void* img1 = ws + plan.d_bytes + plan.tt_bytes;
-    void* img2 = static_cast<char*>(img1) + plan.img1_bytes;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-
-    const int smem = 32 * (int)(l + 1) * 8;
-    QS_REQUIRE(smem <= 200 * 1024, "qs_odqd_coulomb: l too large for the Khatri-Rao tile");
-    if (smem > 48 * 1024) QS_CUDA(cudaFuncSetAttribute(khatri_rao_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    khatri_rao_kernel<<<(unsigned)qs_ceil_div(plan.pitch, 32), 256, smem, st>>>(Cmat, D, (int)l, (int)Gp, (int)plan.pitch);
-    QS_LAUNCH_CHECK();
-
-    const int64_t L2 = l * l;
-    const int64_t rows = (a_end - a_begin) * l;  // the (a_loc, c) rows of T this call needs
-    if ((rc = qs_build_coulomb_image(grid, alpha, a, Gp, img1, stream))) return rc;
-    // Tt[q, (a_loc c)]: rows x = (a_loc, c) of D, new index w = q stored slowest
-    if ((rc = qs_quarter_transform(D + a_begin * l * plan.pitch, QS_F64, rows, Gp, plan.pitch, img1, QS_F64, Gp, Tt,
-                                   rows, 1, 0, 1, 0, rows, stream)))
-        return rc;
-    // M[k = q, w = (a_loc c)] = Tt[q * rows + (a_loc c)]
-    if ((rc = qs_build_coeff_image(Tt, QS_F64, rows, 1, 0, Gp, rows, QS_F64, img2, stream))) return rc;
-    // u[a_loc,b,c,d]: x = (b,d) -> b*l^2 + d ; w = (a_loc,c) -> a_loc*l^3 + c*l
-    if ((rc = qs_quarter_transform(D, QS_F64, L2, Gp, plan.pitch, img2, QS_F64, rows, u_out, l, 1, L2, l, l, L2 * l,
-                                   stream)))
-        return rc;
-    return QS_OK;
+    if ((rc = qs_build_coulomb_image(grid, alpha, a, Gp, workspace, stream))) return rc;
+    return qs_transform_diagonal_planes(nullptr, QS_F64, Cmat, nullptr, QS_F64, Gp, l, a_begin, a_end, 0, u_out,
+                                        workspace, stream);
 }

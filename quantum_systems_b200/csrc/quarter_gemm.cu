@@ -1113,7 +1113,8 @@ extern "C" int qs_build_coeff_image(const void* m, int m_dtype, int64_t m_sk, in
 }
 
 // Coefficient image of the shielded-Coulomb matrix W[p, q] on `grid` (real, Gp x Gp), never
-// materialised as a dense matrix.  Internal entry used by qs_odqd_coulomb.
+// materialised as a dense matrix.  Internal entry used by qs_odqd_coulomb_planes, which hands the image to the
+// diagonal two-body transform as its W.
 int qs_build_coulomb_image(const double* grid, double alpha, double a, int64_t Gp, void* image, void* stream) {
     QS_REQUIRE(grid && image && Gp > 0, "qs_build_coulomb_image: bad arguments");
     const Tiling tl = make_tiling(Gp, Gp, QS_F64, QS_F64);

@@ -3,17 +3,21 @@
 //   u'[p,q,r,s] = sum_ab Ct[p,a] C[a,r] Ct[q,b] C[b,s] W[a,b]      ( - the r <-> s exchange if anti-symmetrised )
 // replaces the 5-operand einsum of ODSincDVR.transform_two_body_elements (reference
 // sinc_dvr/one_dim/sinc_dvr.py:217-252).  O(m^2 n^2 + m^4 n) instead of the O(n^5) of the dense transform,
-// and the same two chained DMMA GEMMs as the ODQD grid build (csrc/odqd.cu):
-//   D[(p,r), a]   = Ct[p,a] C[a,r]                   (Khatri-Rao rows, memory-bound kernel below)
+// as two chained DMMA GEMMs:
+//   D[(p,r), a]   = Ct[p,a] C[a,r]                   (pair products, memory-bound kernel below)
 //   Tt[b, (p,r)]  = sum_a D[(p,r), a] W[a,b]         (quarter GEMM, rotated store)
 //   u'[p,q,r,s]   = sum_b D[(q,s), b] Tt[b, (p,r)]   (quarter GEMM; the prqs -> pqrs permutation is the store stride)
+// The ODQD grid Coulomb build (odqd.cu) is the same transform with W generated from the grid and Ct = C^T, on a
+// range of planes p.
 #include "common.cuh"
 
 namespace {
 
+// Workspace: the image of W, D, Tt, the image of Tt and the temporary of the anti-symmetrised result, in this order.
+// The image of W comes first so that a caller that generates W (the ODQD build) knows where to write it.
 struct DiagPlan {
     int d_dtype, t_dtype;
-    int64_t pitch, d_bytes, tt_bytes, img1_bytes, img2_bytes, tmp_bytes, total;
+    int64_t pitch, img1_bytes, d_bytes, tt_bytes, img2_bytes, tmp_bytes, total;
 };
 
 int make_diag_plan(int64_t n, int64_t m, int w_dtype, int c_dtype, int anti_symmetrize, DiagPlan* plan) {
@@ -88,6 +92,52 @@ __global__ void __launch_bounds__(256) pair_product_kernel(const double* __restr
 
 }  // namespace
 
+int qs_transform_diagonal_planes(const void* w2d, int w_dtype, const void* C, const void* Ct, int c_dtype, int64_t n,
+                                 int64_t m, int64_t p_begin, int64_t p_end, int anti_symmetrize, void* out,
+                                 void* workspace, void* stream) {
+    DiagPlan plan;
+    int rc = make_diag_plan(n, m, w_dtype, c_dtype, anti_symmetrize, &plan);
+    if (rc) return rc;
+    char* ws = static_cast<char*>(workspace);
+    void* img1 = ws;
+    double* D = reinterpret_cast<double*>(ws + plan.img1_bytes);
+    void* Tt = ws + plan.img1_bytes + plan.d_bytes;
+    void* img2 = static_cast<char*>(Tt) + plan.tt_bytes;
+    void* tmp = static_cast<char*>(img2) + plan.img2_bytes;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+
+    // D[(p,r), a] = Ct[p,a] C[a,r];  Ct = conj(C)^T when absent (reference sinc_dvr.py:225-226).  D is built whole: it
+    // is the A operand of the second GEMM for every (q,s).
+    const double* lmat = static_cast<const double*>(Ct ? Ct : C);
+    const long long lsx = Ct ? n : 1, lsk = Ct ? 1 : m;
+    const int l_conj = Ct ? 0 : 1;
+    dim3 grid((unsigned)qs_ceil_div(plan.pitch, 32), (unsigned)qs_ceil_div(m, kXT), (unsigned)qs_ceil_div(m, kYT));
+    if (c_dtype == QS_C128)
+        pair_product_kernel<true><<<grid, 256, 0, st>>>(lmat, lsx, lsk, l_conj, static_cast<const double*>(C), D, (int)n,
+                                                        (int)m, (int)plan.pitch);
+    else
+        pair_product_kernel<false><<<grid, 256, 0, st>>>(lmat, lsx, lsk, l_conj, static_cast<const double*>(C), D,
+                                                         (int)n, (int)m, (int)plan.pitch);
+    QS_LAUNCH_CHECK();
+
+    const int64_t m2 = m * m;
+    const int64_t rows = (p_end - p_begin) * m;  // the rows (p_loc, r) of T these planes need
+    // Tt[b, (p_loc,r)]: rows x = (p_loc,r), K = a, new index w = b stored slowest
+    if (w2d && (rc = qs_build_coeff_image(w2d, w_dtype, n, 1, 0, n, n, plan.d_dtype, img1, stream))) return rc;
+    if ((rc = qs_quarter_transform(D + p_begin * m * plan.pitch * qs_elem_doubles(plan.d_dtype), plan.d_dtype, rows,
+                                   n, plan.pitch, img1, w_dtype, n, Tt, rows, 1, 0, 1, 0, rows, stream)))
+        return rc;
+    // M[k = b, w = (p_loc,r)] = Tt[b * rows + (p_loc,r)]
+    if ((rc = qs_build_coeff_image(Tt, plan.t_dtype, rows, 1, 0, n, rows, plan.d_dtype, img2, stream))) return rc;
+    // u'[p_loc,q,r,s]: x = (q,s) -> q m^2 + s ; w = (p_loc,r) -> p_loc m^3 + r m
+    void* dst = anti_symmetrize ? tmp : out;
+    if ((rc = qs_quarter_transform(D, plan.d_dtype, m2, n, plan.pitch, img2, plan.t_dtype, rows, dst, m, 1, m2, m, m,
+                                   m2 * m, stream)))
+        return rc;
+    if (anti_symmetrize) return qs_anti_symmetrize(tmp, plan.t_dtype, m, out, 0, p_end - p_begin, stream);
+    return QS_OK;
+}
+
 extern "C" int qs_transform_two_body_diagonal_workspace_bytes(int64_t n, int64_t m, int w_dtype, int c_dtype,
                                                               int anti_symmetrize, int64_t* bytes) {
     QS_REQUIRE(n > 0 && m > 0 && bytes, "qs_transform_two_body_diagonal_workspace_bytes: bad arguments");
@@ -112,39 +162,6 @@ extern "C" int qs_transform_two_body_diagonal(const void* w2d, int w_dtype, cons
                (long long)workspace_bytes, (long long)plan.total);
     QS_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0,
                "qs_transform_two_body_diagonal: workspace must be 1 KiB aligned");
-    char* ws = static_cast<char*>(workspace);
-    double* D = reinterpret_cast<double*>(ws);
-    void* Tt = ws + plan.d_bytes;
-    void* img1 = ws + plan.d_bytes + plan.tt_bytes;
-    void* img2 = static_cast<char*>(img1) + plan.img1_bytes;
-    void* tmp = static_cast<char*>(img2) + plan.img2_bytes;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-
-    // D[(p,r), a] = Ct[p,a] C[a,r];  Ct = conj(C)^T when absent (reference sinc_dvr.py:225-226)
-    const double* lmat = static_cast<const double*>(Ct ? Ct : C);
-    const long long lsx = Ct ? n : 1, lsk = Ct ? 1 : m;
-    const int l_conj = Ct ? 0 : 1;
-    dim3 grid((unsigned)qs_ceil_div(plan.pitch, 32), (unsigned)qs_ceil_div(m, kXT), (unsigned)qs_ceil_div(m, kYT));
-    if (c_dtype == QS_C128)
-        pair_product_kernel<true><<<grid, 256, 0, st>>>(lmat, lsx, lsk, l_conj, static_cast<const double*>(C), D, (int)n,
-                                                        (int)m, (int)plan.pitch);
-    else
-        pair_product_kernel<false><<<grid, 256, 0, st>>>(lmat, lsx, lsk, l_conj, static_cast<const double*>(C), D,
-                                                         (int)n, (int)m, (int)plan.pitch);
-    QS_LAUNCH_CHECK();
-
-    const int64_t m2 = m * m;
-    // Tt[b, (p,r)]: rows x = (p,r), K = a, new index w = b stored slowest
-    if ((rc = qs_build_coeff_image(w2d, w_dtype, n, 1, 0, n, n, plan.d_dtype, img1, stream))) return rc;
-    if ((rc = qs_quarter_transform(D, plan.d_dtype, m2, n, plan.pitch, img1, w_dtype, n, Tt, m2, 1, 0, 1, 0, m2, stream)))
-        return rc;
-    // M[k = b, w = (p,r)] = Tt[b * m^2 + (p,r)]
-    if ((rc = qs_build_coeff_image(Tt, plan.t_dtype, m2, 1, 0, n, m2, plan.d_dtype, img2, stream))) return rc;
-    // u'[p,q,r,s]: x = (q,s) -> q m^2 + s ; w = (p,r) -> p m^3 + r m
-    void* dst = anti_symmetrize ? tmp : out;
-    if ((rc = qs_quarter_transform(D, plan.d_dtype, m2, n, plan.pitch, img2, plan.t_dtype, m2, dst, m, 1, m2, m, m,
-                                   m2 * m, stream)))
-        return rc;
-    if (anti_symmetrize) return qs_anti_symmetrize(tmp, plan.t_dtype, m, out, 0, m, stream);
-    return QS_OK;
+    return qs_transform_diagonal_planes(w2d, w_dtype, C, Ct, c_dtype, n, m, 0, m, anti_symmetrize, out, workspace,
+                                        stream);
 }
