@@ -13,6 +13,16 @@
 // partial row a_d D + a_x X goes to the caller's workspace.
 // Pass 2: f[p,q] = h[p,q] + sum over chunks in chunk order.
 //
+// Unrestricted (two spin densities, qs_fock_density_unrestricted):
+//
+//   f_s[p,q] = h[p,q] + sum_{r,s} u[p,r,q,s] (rho_a + rho_b)[s,r] - sum_{r,s} u[p,r,s,q] rho_s[s,r],   s in {a, b}
+//
+// Pass 1 with SPLIT writes a chunk's direct row D and exchange row X as two rows instead of a_d D + a_x X.  Real u
+// and real densities: rho_c = rho_a + i rho_b goes through the real-u x complex-rho pass once, so D = J[rho_a] +
+// i J[rho_b] and X = K[rho_a] + i K[rho_b], and u is read once for both spins.  Complex u or complex densities:
+// the split pass runs once per density and u is read twice.  The unrestricted sum kernel forms both matrices from
+// those rows in chunk order.
+//
 // No floating-point atomics.  The chunking depends on n only (fd_chunk), never on the plane range, so a row computed
 // on a shard is bit-identical to the same row computed on the whole tensor.
 #include "common.cuh"
@@ -86,7 +96,8 @@ __device__ __forceinline__ Piece<UC, V> load_piece(const double* __restrict__ p)
 // complex rho and 16-byte pieces holds twice the exchange accumulators: two CTAs per SM give it the registers.
 // (Unrolling the r loop of real u four times instead of two needs that register budget for every real kernel and
 // was measured slower at n = 128: 0.508 against 0.412 ms on a B200.)
-template <bool UC, bool RC, int V>
+// SPLIT: write the chunk's D and X as two rows of the workspace (a_d, a_x unused).
+template <bool UC, bool RC, int V, bool SPLIT>
 __global__ void __launch_bounds__(kFdThreads, (!UC && RC && V == 2) ? 2 : 3)
     fock_density_kernel(const double* __restrict__ u, const double* __restrict__ rho, int n, int chunk, int n_chunks,
                         double a_d, double a_x, double* __restrict__ ws) {
@@ -161,8 +172,16 @@ __global__ void __launch_bounds__(kFdThreads, (!UC && RC && V == 2) ? 2 : 3)
         }
         __syncthreads();
     }
-    A* out = reinterpret_cast<A*>(ws) + ((size_t)pl * n_chunks + c_idx) * n;
-    for (int q = threadIdx.x; q < n; q += kFdThreads) out[q] = add(mul(dacc[q], a_d), mul(xcol[q], a_x));
+    if constexpr (SPLIT) {
+        A* out = reinterpret_cast<A*>(ws) + ((size_t)pl * n_chunks + c_idx) * 2 * n;
+        for (int q = threadIdx.x; q < n; q += kFdThreads) {
+            out[q] = dacc[q];
+            out[n + q] = xcol[q];
+        }
+    } else {
+        A* out = reinterpret_cast<A*>(ws) + ((size_t)pl * n_chunks + c_idx) * n;
+        for (int q = threadIdx.x; q < n; q += kFdThreads) out[q] = add(mul(dacc[q], a_d), mul(xcol[q], a_x));
+    }
 }
 
 // f[p,q] = h[p,q] + sum_c ws[p][c][q] in chunk order.
@@ -192,6 +211,54 @@ __global__ void fock_density_sum_kernel(const double* __restrict__ h, bool h_c, 
     }
 }
 
+// f_a, f_b from the split rows of pass 1 (complex: ws[p][c] = [D, X]), summed in chunk order.  packed: one pass on
+// rho_a + i rho_b, D = J_a + i J_b and X = K_a + i K_b (u, rho real).  Else two passes, the second (rho_b) at
+// element offset `second`; both D rows are added.
+__global__ void fock_density_unrestricted_sum_kernel(const double* __restrict__ h, bool h_c,
+                                                     const cplx* __restrict__ ws, bool packed, long long second,
+                                                     double* __restrict__ fa, double* __restrict__ fb, bool f_c,
+                                                     int n, int n_chunks, long long p_begin, long long rows) {
+    const long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (e >= rows * n) return;
+    const long long pl = e / n, q = e - pl * n;
+    const long long o = (p_begin + pl) * n + q;
+    double ar = h_c ? h[2 * o] : h[o];
+    double ai = h_c ? h[2 * o + 1] : 0.0;
+    double br = ar, bi = ai;
+    for (int c = 0; c < n_chunks; ++c) {
+        const long long w = (pl * n_chunks + c) * 2 * n + q;
+        const cplx d = ws[w], x = ws[w + n];
+        if (packed) {
+            const double j = d.x + d.y;
+            ar += j - x.x;
+            br += j - x.y;
+        } else {
+            const cplx d2 = ws[second + w], x2 = ws[second + w + n];
+            const double jr = d.x + d2.x, ji = d.y + d2.y;
+            ar += jr - x.x;
+            ai += ji - x.y;
+            br += jr - x2.x;
+            bi += ji - x2.y;
+        }
+    }
+    if (f_c) {
+        fa[2 * o] = ar;
+        fa[2 * o + 1] = ai;
+        fb[2 * o] = br;
+        fb[2 * o + 1] = bi;
+    } else {
+        fa[o] = ar;
+        fb[o] = br;
+    }
+}
+
+// rho_c = rho_a + i rho_b for two real (n, n) densities
+__global__ void pack_densities_kernel(const double* __restrict__ ra, const double* __restrict__ rb,
+                                      cplx* __restrict__ rc, long long n2) {
+    const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (i < n2) rc[i] = {ra[i], rb[i]};
+}
+
 size_t fd_smem_bytes(int64_t n, int u_dtype, int rho_dtype) {
     const bool acc_c = u_dtype == QS_C128 || rho_dtype == QS_C128;
     const int v = (u_dtype == QS_F64 && n % 2 == 0) ? 2 : 1;
@@ -200,10 +267,10 @@ size_t fd_smem_bytes(int64_t n, int u_dtype, int rho_dtype) {
            (size_t)kFdWarps * 32 * v * kFdTiles * a;
 }
 
-template <bool UC, bool RC, int V>
+template <bool UC, bool RC, int V, bool SPLIT = false>
 int launch_pass1(const void* u, const void* rho, int n, int chunk, int n_chunks, double a_d, double a_x, void* ws,
                  long long rows, size_t smem, cudaStream_t st) {
-    auto kern = fock_density_kernel<UC, RC, V>;
+    auto kern = fock_density_kernel<UC, RC, V, SPLIT>;
     QS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<(unsigned)(rows * n_chunks), kFdThreads, smem, st>>>(static_cast<const double*>(u),
                                                                  static_cast<const double*>(rho), n, chunk, n_chunks,
@@ -211,6 +278,20 @@ int launch_pass1(const void* u, const void* rho, int n, int chunk, int n_chunks,
     QS_LAUNCH_CHECK();
     return QS_OK;
 }
+
+// Split pass 1 over one density.  Real u is only ever split against a complex density (the packed pair or a
+// complex rho_s), so four instantiations cover every case.
+int launch_split_pass1(const void* u, bool u_c, const void* rho, bool rho_c, bool vec, int n, int chunk, int n_chunks,
+                       void* ws, long long rows, size_t smem, cudaStream_t st) {
+    if (u_c)
+        return rho_c ? launch_pass1<true, true, 1, true>(u, rho, n, chunk, n_chunks, 0.0, 0.0, ws, rows, smem, st)
+                     : launch_pass1<true, false, 1, true>(u, rho, n, chunk, n_chunks, 0.0, 0.0, ws, rows, smem, st);
+    return vec ? launch_pass1<false, true, 2, true>(u, rho, n, chunk, n_chunks, 0.0, 0.0, ws, rows, smem, st)
+               : launch_pass1<false, true, 1, true>(u, rho, n, chunk, n_chunks, 0.0, 0.0, ws, rows, smem, st);
+}
+
+// Bytes of the split rows of one pass: [rows][chunks][D, X][n] complex.
+int64_t split_rows_bytes(int64_t n, int64_t rows) { return rows * qs_ceil_div(n, fd_chunk(n)) * 2 * n * 16; }
 
 }  // namespace
 
@@ -267,6 +348,73 @@ extern "C" int qs_fock_density(const void* h, int h_dtype, const void* u, int u_
         static_cast<const double*>(h), h_dtype == QS_C128, static_cast<const double*>(workspace),
         u_dtype == QS_C128 || rho_dtype == QS_C128, static_cast<double*>(f), f_dtype == QS_C128, N, n_chunks, p_begin,
         rows);
+    QS_LAUNCH_CHECK();
+    return QS_OK;
+}
+
+extern "C" int qs_fock_density_unrestricted_workspace_bytes(int64_t n, int64_t p_begin, int64_t p_end, int u_dtype,
+                                                            int rho_dtype, int64_t* bytes) {
+    QS_REQUIRE(bytes && n >= 1 && 0 <= p_begin && p_begin <= p_end && p_end <= n,
+               "qs_fock_density_unrestricted_workspace_bytes: bad arguments");
+    QS_REQUIRE((u_dtype == QS_F64 || u_dtype == QS_C128) && (rho_dtype == QS_F64 || rho_dtype == QS_C128),
+               "qs_fock_density_unrestricted_workspace_bytes: bad dtype");
+    const int64_t rows = split_rows_bytes(n, p_end - p_begin);
+    // real u and real densities: one pass plus the packed density rho_a + i rho_b; else one pass per density
+    *bytes = (u_dtype == QS_F64 && rho_dtype == QS_F64) ? rows + n * n * 16 : 2 * rows;
+    return QS_OK;
+}
+
+extern "C" int qs_fock_density_unrestricted(const void* h, int h_dtype, const void* u, int u_dtype,
+                                            const void* rho_alpha, const void* rho_beta, int rho_dtype, int64_t n,
+                                            void* f_alpha, void* f_beta, int f_dtype, int64_t p_begin, int64_t p_end,
+                                            void* workspace, int64_t workspace_bytes, void* stream) {
+    QS_REQUIRE(h && rho_alpha && rho_beta && f_alpha && f_beta && n >= 1 && n <= (1 << 20),
+               "qs_fock_density_unrestricted: bad arguments");
+    QS_REQUIRE(0 <= p_begin && p_begin <= p_end && p_end <= n, "qs_fock_density_unrestricted: bad row range");
+    for (int d : {h_dtype, u_dtype, rho_dtype, f_dtype})
+        QS_REQUIRE(d == QS_F64 || d == QS_C128, "qs_fock_density_unrestricted: bad dtype");
+    QS_REQUIRE(!(f_dtype == QS_F64 && (h_dtype == QS_C128 || u_dtype == QS_C128 || rho_dtype == QS_C128)),
+               "qs_fock_density_unrestricted: complex u cannot be accumulated into a real Fock matrix");
+    if (p_begin == p_end) return QS_OK;
+    int64_t need = 0;
+    qs_fock_density_unrestricted_workspace_bytes(n, p_begin, p_end, u_dtype, rho_dtype, &need);
+    QS_REQUIRE(u && workspace && workspace_bytes >= need,
+               "qs_fock_density_unrestricted: workspace too small (%lld < %lld bytes)", (long long)workspace_bytes,
+               (long long)need);
+    const int N = (int)n;
+    const int chunk = (int)fd_chunk(n);
+    const int n_chunks = (int)qs_ceil_div(n, chunk);
+    const long long rows = p_end - p_begin;
+    QS_REQUIRE(rows * n_chunks < (1LL << 31), "qs_fock_density_unrestricted: too many planes for one launch");
+    const bool u_c = u_dtype == QS_C128;
+    const bool packed = !u_c && rho_dtype == QS_F64;
+    const size_t smem = fd_smem_bytes(n, u_dtype, packed ? QS_C128 : rho_dtype);
+    QS_REQUIRE(smem <= 227 * 1024, "qs_fock_density_unrestricted: n = %lld needs %zu bytes of shared memory",
+               (long long)n, smem);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const bool vec = !u_c && n % 2 == 0 && (reinterpret_cast<uintptr_t>(u) & 15) == 0;
+    const int64_t split_bytes = split_rows_bytes(n, rows);
+    char* ws = static_cast<char*>(workspace);
+    int status;
+    if (packed) {
+        cplx* rho_c = reinterpret_cast<cplx*>(ws + split_bytes);
+        pack_densities_kernel<<<(unsigned)qs_ceil_div(n * n, 256), 256, 0, st>>>(
+            static_cast<const double*>(rho_alpha), static_cast<const double*>(rho_beta), rho_c, n * n);
+        QS_LAUNCH_CHECK();
+        status = launch_split_pass1(u, false, rho_c, true, vec, N, chunk, n_chunks, ws, rows, smem, st);
+    } else {
+        const bool rho_c = rho_dtype == QS_C128;
+        status = launch_split_pass1(u, u_c, rho_alpha, rho_c, vec, N, chunk, n_chunks, ws, rows, smem, st);
+        if (status == QS_OK)
+            status = launch_split_pass1(u, u_c, rho_beta, rho_c, vec, N, chunk, n_chunks, ws + split_bytes, rows,
+                                        smem, st);
+    }
+    if (status != QS_OK) return status;
+    const long long total = rows * n;
+    fock_density_unrestricted_sum_kernel<<<(unsigned)qs_ceil_div(total, 256), 256, 0, st>>>(
+        static_cast<const double*>(h), h_dtype == QS_C128, reinterpret_cast<const cplx*>(ws), packed,
+        split_bytes / 16, static_cast<double*>(f_alpha), static_cast<double*>(f_beta), f_dtype == QS_C128, N,
+        n_chunks, p_begin, rows);
     QS_LAUNCH_CHECK();
     return QS_OK;
 }

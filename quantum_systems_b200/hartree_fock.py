@@ -14,11 +14,21 @@ The only O(n^4) step of an iteration, the Fock build from the density matrix, is
 Aufbau filling of the lowest orbitals (in ``eigh`` order).  When ``h``, ``s``, ``u`` and a given initial ``C`` have no
 imaginary part the iteration runs in float64 and ``C`` is real, so that ``change_basis(state.C)`` takes the real
 quarter GEMM; otherwise it runs in complex128.
+
+``ground_state_unrestricted(system, n_alpha, n_beta)`` solves unrestricted HF (UHF) on the spatial ``u``: one
+coefficient matrix per spin, for open shells and spin-polarised or broken-symmetry states.  Its Fock build,
+``ops.fock_from_density_unrestricted``, reads a real ``u`` once for both spins.  ``spin_orbital_coefficients``
+turns the result into the ``(2l, 2l)`` coefficients of the spin-doubled basis::
+
+    state = hartree_fock.ground_state_unrestricted(basis, n_alpha=2, n_beta=1)
+    C, epsilon = hartree_fock.spin_orbital_coefficients(state)
+    GeneralOrbitalSystem(3, basis).change_basis(C)
 """
 
 import dataclasses
 import warnings
 
+import numpy as np
 import torch
 
 from . import _arrays, ops
@@ -41,6 +51,27 @@ class HartreeFockState:
     density_matrix: object
     converged: bool
     iterations: int
+
+
+@dataclasses.dataclass
+class UnrestrictedHartreeFockState:
+    """``C_alpha``, ``C_beta`` (l, l): orbitals of each spin as columns in ascending orbital energy
+    ``epsilon_alpha``, ``epsilon_beta``, ``C^dagger S C = I``; the first ``n_alpha`` (``n_beta``) are occupied.
+    ``density_alpha`` / ``density_beta`` are ``C_o C_o^dagger``; ``energy`` includes the nuclear repulsion;
+    ``spin_squared`` is ``<S^2>`` of the UHF determinant.  ``converged`` is False when ``max_iterations`` ran out."""
+
+    C_alpha: object
+    C_beta: object
+    epsilon_alpha: object
+    epsilon_beta: object
+    density_alpha: object
+    density_beta: object
+    energy: float
+    spin_squared: float
+    converged: bool
+    iterations: int
+    n_alpha: int
+    n_beta: int
 
 
 def ground_state(system, tol=1e-9, max_iterations=100, C=None):
@@ -92,10 +123,25 @@ def ground_state_sharded(basis, n_occ, tol=1e-9, max_iterations=100, C=None, nuc
     all ranks.  A real-valued complex128 ``u`` is NOT copied to float64 here: the slabs of a tensor that needs several
     GPUs are sized to fill them, so the Fock build reads the complex slabs and keeps the real part of ``f`` (its
     imaginary part is exactly zero for a real density)."""
+    restricted = not basis.includes_spin
+    h, s, (C,), agree = _sharded_inputs(basis, (C,))
+    dtype = h.dtype
+    scales = _scales(restricted, basis.anti_symmetrized_u)
+
+    def fock(rho):
+        f = basis.fock_from_density(h, rho, *scales)
+        # real working dtype: u has no imaginary part, so with a real density the imaginary part of f is exactly zero
+        return f.real.contiguous() if dtype == torch.float64 and f.is_complex() else f
+
+    return _scf(h, s, fock, n_occ, restricted, tol, max_iterations, C, nuclear_repulsion_energy, agree)
+
+
+def _sharded_inputs(basis, guesses):
+    """``h``, ``s`` and the initial guesses (rank 0's everywhere) of a ``ShardedBasisSet`` on the device in the working
+    dtype, and the callback that broadcasts rank 0's tensors (None on one process)."""
     from .sharded import ProcessContext
 
     ctx = basis.ctx
-    restricted = not basis.includes_spin
     h = _arrays.to_device(basis.h)
     s = _arrays.to_device(basis.s) if basis.s is not None else None
     collective = isinstance(ctx, ProcessContext) and ctx.world > 1
@@ -104,27 +150,116 @@ def ground_state_sharded(basis, n_occ, tol=1e-9, max_iterations=100, C=None, nuc
         for t in tensors:
             ctx.dist.broadcast(torch.view_as_real(t) if t.is_complex() else t, src=0, group=ctx.group)
 
-    if C is not None:
-        C = _arrays.to_device(C).contiguous()
-        if collective:
-            agree(C)
+    guesses = [_arrays.to_device(C).contiguous() if C is not None else None for C in guesses]
+    if collective:
+        agree(*(C for C in guesses if C is not None))
     u_imag = any(_has_imag(basis.u.local(r)) for r in ctx.local_ranks)
     if collective:
         flag = torch.tensor([float(u_imag)], dtype=torch.float64, device=h.device)
         ctx.dist.all_reduce(flag, op=ctx.dist.ReduceOp.MAX, group=ctx.group)
         u_imag = bool(flag.item())
-    dtype = _working_dtype(_has_imag(h), _has_imag(s), u_imag, _has_imag(C))
-    h, s, C = (_as_dtype(t, dtype) for t in (h, s, C))
-    scales = _scales(restricted, basis.anti_symmetrized_u)
+    dtype = _working_dtype(_has_imag(h), _has_imag(s), u_imag, *(_has_imag(C) for C in guesses))
+    h, s = _as_dtype(h, dtype), _as_dtype(s, dtype)
+    guesses = [_as_dtype(C, dtype) for C in guesses]
+    return h, s, guesses, agree if collective else None
 
-    def fock(rho):
-        f = basis.fock_from_density(h, rho, *scales)
-        # real working dtype: u has no imaginary part, so with a real density the imaginary part of f is exactly zero
-        return f.real.contiguous() if dtype == torch.float64 and f.is_complex() else f
 
-    return _scf(h, s, fock, n_occ, restricted, tol, max_iterations, C, nuclear_repulsion_energy,
-                agree if collective else None)
+def ground_state_unrestricted(system, n_alpha=None, n_beta=None, tol=1e-9, max_iterations=100, C=None):
+    """UHF ground state with ``n_alpha`` spin-up and ``n_beta`` spin-down electrons on the spatial ``u`` of
+    ``system``: a ``SpatialOrbitalSystem`` (both default to ``system.n``, its number of doubly occupied orbitals)
+    or a spatial ``BasisSet`` (both required).  ``C = (C_alpha, C_beta)`` is the initial guess (default: the core
+    Hamiltonian for both spins; a spin-symmetric guess stays spin-symmetric, so a broken-symmetry solution needs a
+    guess that breaks it).  Fock matrices ``f_s = h + J[rho_a + rho_b] - K[rho_s]`` from
+    ``ops.fock_from_density_unrestricted``, one Pulay DIIS over the errors of both spins with one coefficient set,
+    converged when the larger error of the two is at most ``tol``.  Working dtype and the float64 copy of a
+    real-valued complex ``u`` as in ``ground_state``.  Host (numpy) systems get ndarrays back."""
+    basis = getattr(system, "_basis_set", system)
+    if basis.includes_spin:
+        raise ValueError("UHF needs the spatial two-body tensor; a spin-doubled basis is solved by "
+                         "hartree_fock.ground_state (GHF)")
+    if getattr(basis, "u_repr", "4d") == "2d":
+        raise ValueError("Hartree-Fock needs the 4-d two-body tensor; call set_u_repr('4d') on a sinc-DVR basis first")
+    if basis.anti_symmetrized_u:
+        raise ValueError("UHF needs the plain spatial u, not an anti-symmetrised one")
+    if system is not basis:
+        n_alpha = system.n if n_alpha is None else n_alpha
+        n_beta = system.n if n_beta is None else n_beta
+    n_alpha, n_beta = _occupations(n_alpha, n_beta, basis.l)
+    h = _arrays.to_device(basis.h)
+    s = _arrays.to_device(basis.s) if basis.s is not None else None
+    u = _arrays.to_device(basis.u)  # uploaded once for a host basis, resident for the iterations
+    C = (None, None) if C is None else tuple(_arrays.to_device(c) for c in C)
+    dtype = _working_dtype(_has_imag(h), _has_imag(s), _has_imag(u), *(_has_imag(c) for c in C))
+    h, s = _as_dtype(h, dtype), _as_dtype(s, dtype)
+    C = None if C[0] is None else tuple(_as_dtype(c, dtype) for c in C)
+    if dtype == torch.float64:
+        u = _as_dtype(u, dtype)
 
+    def fock(rho_alpha, rho_beta):
+        return ops.fock_from_density_unrestricted(h, u, rho_alpha, rho_beta)
+
+    state = _uscf(h, s, fock, n_alpha, n_beta, tol, max_iterations, C, basis.nuclear_repulsion_energy, None)
+    if _arrays.is_host_module(basis.np):
+        for name in ("C_alpha", "C_beta", "epsilon_alpha", "epsilon_beta", "density_alpha", "density_beta"):
+            setattr(state, name, _arrays.to_host(getattr(state, name)))
+    return state
+
+
+def ground_state_unrestricted_sharded(basis, n_alpha, n_beta, tol=1e-9, max_iterations=100, C=None,
+                                      nuclear_repulsion_energy=0.0):
+    """The UHF iteration of ``ground_state_unrestricted`` on a ``ShardedBasisSet`` with ``includes_spin=False``:
+    only the Fock build is distributed (``ShardedBasisSet.fock_from_density_unrestricted``); rank 0's coefficients,
+    orbital energies, energy and convergence decision are broadcast, the working dtype and the given guesses are
+    handled as in ``ground_state_sharded`` (a real-valued complex ``u`` is not copied to float64)."""
+    if basis.includes_spin:
+        raise ValueError("UHF needs the spatial two-body tensor; a spin-doubled basis is solved by "
+                         "hartree_fock.ground_state_sharded (GHF)")
+    if basis.anti_symmetrized_u:
+        raise ValueError("UHF needs the plain spatial u, not an anti-symmetrised one")
+    n_alpha, n_beta = _occupations(n_alpha, n_beta, basis.u.n)
+    h, s, C, agree = _sharded_inputs(basis, (None, None) if C is None else C)
+    C = None if C[0] is None else tuple(C)
+    dtype = h.dtype
+
+    def fock(rho_alpha, rho_beta):
+        fs = basis.fock_from_density_unrestricted(h, rho_alpha, rho_beta)
+        # real working dtype: u has no imaginary part, so with real densities the imaginary parts are exactly zero
+        return tuple(f.real.contiguous() if dtype == torch.float64 and f.is_complex() else f for f in fs)
+
+    return _uscf(h, s, fock, n_alpha, n_beta, tol, max_iterations, C, nuclear_repulsion_energy, agree)
+
+
+def spin_orbital_coefficients(state):
+    """The UHF state as ``(C, epsilon)`` of the spin-doubled basis: ``C`` is ``(2l, 2l)`` for
+    ``GeneralOrbitalSystem(n_alpha + n_beta, basis).change_basis(C)``.  Rows follow ``add_spin`` (row ``2a + s``,
+    ``s = 0`` the spin-up component); the columns are the occupied spin-orbitals, then the virtual ones, each block
+    ordered by (orbital index, spin) with alpha before beta.  A closed shell with ``C_alpha = C_beta`` gives
+    ``kron(C, I_2)``.  Returns tensors or ndarrays, as the state holds."""
+    Ca, Cb = state.C_alpha, state.C_beta
+    xp = torch if isinstance(Ca, torch.Tensor) else np
+    l = Ca.shape[0]
+    occupied = [(j, spin) for j in range(l) for spin, n_occ in ((0, state.n_alpha), (1, state.n_beta)) if j < n_occ]
+    virtual = [(j, spin) for j in range(l) for spin, n_occ in ((0, state.n_alpha), (1, state.n_beta)) if j >= n_occ]
+    order = occupied + virtual
+    dtype = Ca.dtype if Ca.dtype == Cb.dtype else (torch.complex128 if xp is torch else np.complex128)
+    kw = {"device": Ca.device} if xp is torch else {}
+    C = xp.zeros((2 * l, 2 * l), dtype=dtype, **kw)
+    eps = xp.zeros(2 * l, dtype=state.epsilon_alpha.dtype, **kw)
+    for spin, (Cs, es) in enumerate(((Ca, state.epsilon_alpha), (Cb, state.epsilon_beta))):
+        cols = [k for k, (_, sp) in enumerate(order) if sp == spin]
+        orbs = [j for j, sp in order if sp == spin]
+        C[spin::2, cols] = Cs[:, orbs].to(dtype) if xp is torch else Cs[:, orbs]
+        eps[cols] = es[orbs]
+    return C, eps
+
+
+def _occupations(n_alpha, n_beta, l):
+    if n_alpha is None or n_beta is None:
+        raise ValueError("n_alpha and n_beta are required for a basis set")
+    n_alpha, n_beta = int(n_alpha), int(n_beta)
+    if not (0 <= n_alpha <= l and 0 <= n_beta <= l):
+        raise ValueError(f"n_alpha = {n_alpha} and n_beta = {n_beta} must lie in [0, {l}]")
+    return n_alpha, n_beta
 
 def _working_dtype(*has_imag):
     return torch.complex128 if any(has_imag) else torch.float64
@@ -227,3 +362,60 @@ def _scf(h, s, fock, n_occ, restricted, tol, max_iterations, C, e_nuc, agree):
     if not converged:
         warnings.warn(f"Hartree-Fock did not converge in {max_iterations} iterations", RuntimeWarning, stacklevel=3)
     return HartreeFockState(C=C, epsilon=eps, energy=energy, density_matrix=rho, converged=converged, iterations=it)
+
+
+def _uscf(h, s, fock, n_alpha, n_beta, tol, max_iterations, C, e_nuc, agree):
+    """The UHF sibling of ``_scf``: ``fock(rho_a, rho_b)`` returns ``(F_a, F_b)``; DIIS extrapolates the stacked pair
+    with one coefficient set from the stacked errors of both spins."""
+    n = h.shape[0]
+    dtype, device = h.dtype, h.device
+    X = _orthogonaliser(s, n, dtype, device)
+    S = s if s is not None else torch.eye(n, dtype=dtype, device=device)
+
+    def diagonalise(F):
+        eps, Cp = torch.linalg.eigh(X.mH @ F @ X)
+        C_new = X @ Cp
+        if agree is not None:
+            agree(C_new, eps)
+        return C_new, eps
+
+    if C is None:
+        Ca, ea = diagonalise(h)
+        Cb, eb = Ca.clone(), ea.clone()
+    else:
+        (Ca, Cb), ea, eb = C, None, None
+    rho_a, rho_b = _density(Ca, n_alpha, False), _density(Cb, n_beta, False)
+    fs, errs = [], []
+    converged, it, energy = False, 0, 0.0
+    for it in range(1, max_iterations + 1):
+        Fa, Fb = fock(rho_a, rho_b)
+        energy_t = 0.5 * (torch.sum(rho_a.transpose(0, 1) * (h + Fa)) + torch.sum(rho_b.transpose(0, 1) * (h + Fb))).real
+        energy_t = energy_t + e_nuc
+        err = torch.stack([X.mH @ (F @ rho @ S - S @ rho @ F) @ X for F, rho in ((Fa, rho_a), (Fb, rho_b))])
+        decision = torch.stack([energy_t.to(torch.float64), err.abs().max().to(torch.float64)])
+        if agree is not None:
+            agree(decision)
+        energy, err_max = (float(x) for x in decision.tolist())
+        converged = err_max <= tol
+        if not converged:
+            fs.append(torch.stack([Fa, Fb]))
+            errs.append(err)
+            if len(fs) > DIIS_VECTORS:
+                fs.pop(0)
+                errs.pop(0)
+            if len(fs) > 1:
+                Fa, Fb = _diis(fs, errs)
+        Ca, ea = diagonalise(Fa)
+        Cb, eb = diagonalise(Fb)
+        rho_a, rho_b = _density(Ca, n_alpha, False), _density(Cb, n_beta, False)
+        if converged:
+            break
+    if not converged:
+        warnings.warn(f"Hartree-Fock did not converge in {max_iterations} iterations", RuntimeWarning, stacklevel=3)
+    overlap = Ca[:, :n_alpha].mH @ S @ Cb[:, :n_beta]
+    s_z = 0.5 * (n_alpha - n_beta)
+    spin_squared = s_z * (s_z + 1) + n_beta - float((overlap.abs() ** 2).sum())
+    return UnrestrictedHartreeFockState(
+        C_alpha=Ca, C_beta=Cb, epsilon_alpha=ea, epsilon_beta=eb, density_alpha=rho_a, density_beta=rho_b,
+        energy=energy, spin_squared=spin_squared, converged=converged, iterations=it, n_alpha=n_alpha, n_beta=n_beta,
+    )

@@ -355,6 +355,58 @@ def fock_from_density(h, u, rho, scale_direct, scale_exchange, f=None, planes=No
     return f
 
 
+def fock_from_density_unrestricted(h, u, rho_alpha, rho_beta, f_alpha=None, f_beta=None, planes=None):
+    """Both unrestricted Fock matrices ``f_s[p,q] = h[p,q] + sum_rs u[p,r,q,s] (rho_a + rho_b)[s,r]
+    - sum_rs u[p,r,s,q] rho_s[s,r]`` of the spin densities ``rho_alpha`` and ``rho_beta`` on a spatial ``u``
+    (``qs_fock_density_unrestricted``).  Real ``u`` and real densities: ``u`` is read once for both spins; complex
+    ``u`` or a complex density: twice.  ``planes``, the in-place ``f_alpha`` / ``f_beta`` and the result dtype
+    follow ``fock_from_density``; a real density is promoted to complex when the other one is complex.
+    Returns ``(f_alpha, f_beta)``."""
+    h = _device_tensor(h, "h")
+    u = _device_tensor(u, "u")
+    rho_alpha = _device_tensor(rho_alpha, "rho_alpha")
+    rho_beta = _device_tensor(rho_beta, "rho_beta")
+    rho_dtype = _result_dtype(rho_alpha, rho_beta)
+    rho_alpha, rho_beta = rho_alpha.to(rho_dtype), rho_beta.to(rho_dtype)
+    n = h.shape[0]
+    p0, p1 = (0, n) if planes is None else (int(planes[0]), int(planes[1]))
+    if not 0 <= p0 <= p1 <= n:
+        raise ValueError(f"planes {planes} out of range for n = {n}")
+    if (tuple(h.shape) != (n, n) or tuple(rho_alpha.shape) != (n, n) or tuple(rho_beta.shape) != (n, n)
+            or tuple(u.shape) != (p1 - p0, n, n, n)):
+        raise ValueError(
+            f"h, rho_alpha and rho_beta must be (n,n) and u (planes,n,n,n), got {tuple(h.shape)}, "
+            f"{tuple(rho_alpha.shape)}, {tuple(rho_beta.shape)}, {tuple(u.shape)}"
+        )
+    fs = []
+    for name, f in (("f_alpha", f_alpha), ("f_beta", f_beta)):
+        if f is None:
+            alloc = torch.empty if (p0, p1) == (0, n) else torch.zeros
+            f = alloc((n, n), dtype=_result_dtype(h, u, rho_alpha), device=h.device)
+        else:
+            if not (isinstance(f, torch.Tensor) and f.is_cuda and f.is_contiguous()):
+                raise RuntimeError(f"{name} must be a contiguous CUDA tensor to be filled in place")
+            if tuple(f.shape) != (n, n):
+                raise ValueError(f"{name} must be {(n, n)}, got {tuple(f.shape)}")
+            _code(f)
+            _mark_written(f)
+        fs.append(f)
+    f_alpha, f_beta = fs
+    if f_alpha.dtype != f_beta.dtype:
+        raise ValueError(f"f_alpha and f_beta must have one dtype, got {f_alpha.dtype} and {f_beta.dtype}")
+    nbytes = ctypes.c_int64(0)
+    _native.call(
+        "qs_fock_density_unrestricted_workspace_bytes", n, p0, p1, _code(u), _code(rho_alpha), ctypes.byref(nbytes)
+    )
+    owner, ws = _workspace(nbytes.value, h.device)
+    _native.call(
+        "qs_fock_density_unrestricted", _ptr(h), _code(h), _ptr(u), _code(u), _ptr(rho_alpha), _ptr(rho_beta),
+        _code(rho_alpha), n, _ptr(f_alpha), _ptr(f_beta), _code(f_alpha), p0, p1, ws, nbytes.value, _stream(),
+    )
+    owner.record_stream(torch.cuda.current_stream())
+    return f_alpha, f_beta
+
+
 def odqd_coulomb(C, inner_grid, alpha, a, planes=None):
     """Grid Coulomb elements ``u_abcd`` of the 1-D quantum dot (reference one_dim_qd.py:275-280).
     ``C``: (G', l) eigenvectors on the interior grid; ``inner_grid``: (G',).  ``planes=(a0, a1)`` builds only the

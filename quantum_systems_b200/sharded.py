@@ -1079,19 +1079,40 @@ class ShardedBasisSet:
                 ops.fock_from_density(h, u.local(r), rho, scale_direct, scale_exchange, f=f, planes=(p0, p1))
         return _gather_rows(ctx, u, f)
 
+    def fock_from_density_unrestricted(self, h, rho_alpha, rho_beta):
+        """Both unrestricted Fock matrices ``(f_alpha, f_beta)`` of a spatial ``u``
+        (``ops.fock_from_density_unrestricted``): every rank computes the rows p it owns, then the rows of both
+        matrices are gathered in one all-reduce (2 n^2 elements).  ``h`` and the densities are replicated.  A row
+        is bit-identical to the same row of the single-tensor kernel."""
+        from . import _arrays, ops
 
-def _gather_rows(ctx, u, f):
-    """Every rank has written the rows of ``f`` that belong to its planes of ``u``; afterwards every rank holds all
-    rows.  One process per rank: an all-reduce of the disjoint rows (n^2 elements).  Emulated: nothing to do."""
+        ctx, u = self.ctx, self.u
+        h, rho_alpha, rho_beta = (_arrays.to_device(t) for t in (h, rho_alpha, rho_beta))
+        dtype = ops._result_dtype(h, rho_alpha, rho_beta, u.local(ctx.local_ranks[0]))
+        f_alpha, f_beta = (torch.zeros((u.n, u.n), dtype=dtype, device=h.device) for _ in range(2))
+        for r in ctx.local_ranks:
+            p0, p1 = u.planes(r)
+            if p1 > p0:
+                ops.fock_from_density_unrestricted(h, u.local(r), rho_alpha, rho_beta, f_alpha=f_alpha, f_beta=f_beta,
+                                                   planes=(p0, p1))
+        return _gather_rows(ctx, u, f_alpha, f_beta)
+
+
+def _gather_rows(ctx, u, *fs):
+    """Every rank has written the rows of each ``f`` (all of one dtype) that belong to its planes of ``u``;
+    afterwards every rank holds all rows.  One process per rank: one all-reduce of the disjoint rows of all the
+    matrices (n^2 elements each).  Emulated: nothing to do.  Returns the one matrix, or the tuple of them."""
     if isinstance(ctx, ProcessContext) and ctx.world > 1:
         n = u.n
         block, offsets = u.block, u.offsets
-        padded = torch.zeros((ctx.world, block, n), dtype=f.dtype, device=f.device)
+        padded = torch.zeros((len(fs), ctx.world, block, n), dtype=fs[0].dtype, device=fs[0].device)
         p0, p1 = u.planes(ctx.rank)
-        padded[ctx.rank, : p1 - p0] = f[p0:p1]
+        for i, f in enumerate(fs):
+            padded[i, ctx.rank, : p1 - p0] = f[p0:p1]
         flat = torch.view_as_real(padded) if padded.is_complex() else padded
         ctx.dist.all_reduce(flat, group=ctx.group)  # disjoint rows: sum == gather
-        for r in range(ctx.world):
-            q0, q1 = offsets[r], offsets[r + 1]
-            f[q0:q1] = padded[r, : q1 - q0]
-    return f
+        for i, f in enumerate(fs):
+            for r in range(ctx.world):
+                q0, q1 = offsets[r], offsets[r + 1]
+                f[q0:q1] = padded[i, r, : q1 - q0]
+    return fs[0] if len(fs) == 1 else fs
