@@ -268,7 +268,7 @@ int qs_fock_spatial(const void* h, int h_dtype, const void* u, int u_dtype, int6
                     int64_t n_occ, void* f, int64_t p_begin, int64_t p_end, void* stream);
 /* General Fock matrix from a tensor sharded on its THIRD index (what a sharded change_basis leaves):
  * u_cols = u[:, :, q_begin:q_end, :] stored dense as (n, n, q_end-q_begin, n); writes columns
- * [q_begin, q_end) of f (h, f full (n, n) matrices). */
+ * [q_begin, q_end) of f (h, f full (n, n) matrices); u_cols may be NULL when the range is empty. */
 int qs_fock_general_cols(const void* h, int h_dtype, const void* u_cols, int u_dtype, int64_t n,
                          int64_t n_occ, void* f, int64_t q_begin, int64_t q_end, void* stream);
 /* Same reductions on pre-gathered (n_occ, n, n) blocks direct[i,p,q] = u[p,i,q,i] and (optional,

@@ -75,7 +75,8 @@ int launch_fock(const void* h, int h_dtype, const void* ud, const void* ue, int 
                 int64_t q_begin = 0, int64_t q_count = -1) {
     if (q_count < 0) q_count = n;
     QS_REQUIRE(0 <= n_occ && n_occ <= n, "qs_fock: n_occ out of range");
-    QS_REQUIRE(h && f && n > 0 && (ud || n_occ == 0), "qs_fock: bad arguments");  // no occupied orbital: u is never read
+    // no occupied orbital or an empty row / column range: u is never read, and an empty block may be NULL
+    QS_REQUIRE(h && f && n > 0 && (ud || n_occ == 0 || p_begin == p_end || q_count == 0), "qs_fock: bad arguments");
     QS_REQUIRE(0 <= p_begin && p_begin <= p_end && p_end <= n, "qs_fock: bad row range");
     QS_REQUIRE(0 <= q_begin && q_begin + q_count <= n, "qs_fock: bad column range");
     QS_REQUIRE(!(h_dtype == QS_F64 && u_dtype == QS_C128),
