@@ -70,6 +70,17 @@ int qs_transform_two_body_symmetric(const void* u, int u_dtype, const void* C, c
                                     int c_dtype, int64_t n, int64_t n_new, int symmetry, void* out,
                                     void* workspace, int64_t workspace_bytes, void* stream);
 
+/* Four-coefficient transform   out[p,q,r,s] = sum_abcd Ct_p[p,a] Ct_q[q,b] u[a,b,c,d] C_r[c,r] C_s[d,s]
+ * the mixed-spin blocks of an unrestricted basis change (see qs_spin_orbital_two_body), whose two ket and two bra
+ * indices belong to two different spins.  The same four quarter steps in the order s, r, q, p as qs_transform_two_body, one coefficient image per step.
+ *   C_r, C_s   : (n, n_new) row-major     dtype c_dtype
+ *   Ct_p, Ct_q : (n_new, n) row-major     dtype c_dtype, or NULL for conj(C_r)^T, conj(C_s)^T respectively
+ * u, out and the workspace (qs_transform_two_body_workspace_bytes) as in qs_transform_two_body.  No symmetry is
+ * assumed: with two different matrices none survives; equal matrices take qs_transform_two_body_symmetric. */
+int qs_transform_two_body_mixed(const void* u, int u_dtype, const void* C_r, const void* C_s,
+                                const void* Ct_p, const void* Ct_q, int c_dtype, int64_t n, int64_t n_new,
+                                void* out, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* Building blocks of the SHARDED symmetry-aware transform (anti-symmetric u only: its mirror image stays inside a
  * (p, q) plane, i.e. on the rank that owns p).  Of each pair (r, s), (s, r) the rank that owns r computes the one
  * whose cyclic distance (s - r) mod m is the shorter (qs_cyclic_pair_wanted; ties go to r < s), so every r has the
@@ -245,6 +256,19 @@ int qs_anti_symmetrize(const void* u, int dtype, int64_t n, void* out, int64_t p
                        int64_t p_end, void* stream);
 int qs_add_spin_one_body(const void* h, int in_dtype, int64_t l, void* out, int out_dtype,
                          void* stream);
+
+/* Anti-symmetrised spin-orbital tensor of an unrestricted basis from the spin blocks of the spatial tensor
+ *   B_st[i,j,k,l] = sum_abcd conj(C_s[a,i]) conj(C_t[b,j]) u[a,b,c,d] C_s[c,k] C_t[d,l]   (s, t in {alpha, beta})
+ *   U[I,J,K,L] = [sI==sK][sJ==sL] B_{sI sJ}[oI,oJ,oK,oL] - [sI==sL][sJ==sK] B_{sI sJ}[oI,oJ,oL,oK]
+ * with spin-orbital I = (orbital[I], spin[I]); orbital, spin: int32 device tables of length 2l that together are a
+ * bijection onto {0..l-1} x {0, 1} (0 = alpha).  b_aa, b_ab, b_ba, b_bb: (l,l,l,l) of in_dtype; b_ba = NULL derives
+ * it from b_ab by particle exchange, B_ba[i,j,k,l] = B_ab[j,i,l,k] (exact when u[a,b,c,d] = u[b,a,d,c]).
+ * in_dtype -> out_dtype: F64 -> F64, F64 -> C128 or C128 -> C128.  Planes I in [p_begin, p_end) of the (2l)^4 result
+ * are written, to `out` pointing at plane p_begin.  Every output element, zeros included, is written once: reads
+ * 4 l^4 input and writes 16 l^4 output elements for the whole tensor. */
+int qs_spin_orbital_two_body(const void* b_aa, const void* b_ab, const void* b_ba, const void* b_bb,
+                             int in_dtype, int64_t l, const int32_t* orbital, const int32_t* spin,
+                             void* out, int out_dtype, int64_t p_begin, int64_t p_end, void* stream);
 
 /* Two-body part of S^2 from the three (n, n) complex128 spin matrices S_x, S_y, S_z:
  *   out[p,q,r,s] = sum_i S_i[p,r] S_i[q,s]  (- sum_i S_i[p,s] S_i[q,r] if anti_symmetrize)

@@ -28,6 +28,7 @@ SIGNATURES = {
     "qs_transform_two_body": [_ptr, _int, _ptr, _ptr, _int, _i64, _i64, _ptr, _ptr, _i64, _ptr],
     "qs_two_body_symmetry": [_ptr, _int, _i64, _int, ctypes.POINTER(_int), _ptr, _ptr],
     "qs_transform_two_body_symmetric": [_ptr, _int, _ptr, _ptr, _int, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr],
+    "qs_transform_two_body_mixed": [_ptr, _int, _ptr, _ptr, _ptr, _ptr, _int, _i64, _i64, _ptr, _ptr, _i64, _ptr],
     "qs_coeff_image_bytes": [_i64, _i64, _int, _int, ctypes.POINTER(_i64)],
     "qs_build_coeff_image": [_ptr, _int, _i64, _i64, _int, _i64, _i64, _int, _ptr, _ptr],
     "qs_quarter_transform": [_ptr, _int, _i64, _i64, _i64, _ptr, _int, _i64, _ptr, _i64, _i64, _i64, _i64, _i64, _i64, _ptr],
@@ -55,6 +56,7 @@ SIGNATURES = {
     "qs_add_spin_two_body": [_ptr, _int, _i64, _ptr, _int, _int, _i64, _i64, _ptr],
     "qs_anti_symmetrize": [_ptr, _int, _i64, _ptr, _i64, _i64, _ptr],
     "qs_add_spin_one_body": [_ptr, _int, _i64, _ptr, _int, _ptr],
+    "qs_spin_orbital_two_body": [_ptr, _ptr, _ptr, _ptr, _int, _i64, _ptr, _ptr, _ptr, _int, _i64, _i64, _ptr],
     "qs_spin_squared_two_body": [_ptr, _ptr, _ptr, _i64, _int, _ptr, _i64, _i64, _ptr],
     "qs_fock_gathered": [_ptr, _int, _ptr, _ptr, _int, _i64, _i64, _dbl, _dbl, _ptr, _ptr],
     "qs_fock_general": [_ptr, _int, _ptr, _int, _i64, _i64, _ptr, _i64, _i64, _ptr],

@@ -326,6 +326,9 @@ class BasisSet:
 
     def _change_basis_two_body_elements(self, C, C_tilde):
         self.u = self.transform_two_body_elements(self.u, C, np=self.np, C_tilde=C_tilde)
+        self._change_basis_spin_2_tb(C, C_tilde)
+
+    def _change_basis_spin_2_tb(self, C, C_tilde):
         if self._spin_tb_factors is not None:
             # transform of sum_i S_i (x) S_i == sum_i (C~ S_i C) (x) (C~ S_i C): O(n^3), exact
             self._spin_tb_factors = tuple(
@@ -360,6 +363,10 @@ class BasisSet:
         (basis_set.py:413-464): h, s, u, spin_2_tb, position, momentum, spf and bra_spf are replaced
         by new arrays; inputs are never modified in place.
         """
+        self._change_basis(C, C_tilde, two_body=True)
+
+    def _change_basis(self, C, C_tilde, two_body):
+        """``change_basis``; ``two_body=False`` leaves ``u`` alone (the caller stores the transformed one)."""
         C_dev = _arrays.to_device(C)
         self.l = C_dev.shape[1]
         if C_tilde is None:
@@ -367,7 +374,10 @@ class BasisSet:
         C_tilde_dev = _arrays.to_device(C_tilde)
 
         self._change_basis_one_body_elements(C_dev, C_tilde_dev)
-        self._change_basis_two_body_elements(C_dev, C_tilde_dev)
+        if two_body:
+            self._change_basis_two_body_elements(C_dev, C_tilde_dev)
+        else:
+            self._change_basis_spin_2_tb(C_dev, C_tilde_dev)
         if self.position is not None:
             self._change_basis_position_elements(C_dev, C_tilde_dev)
         if self.momentum is not None:
@@ -414,7 +424,11 @@ class BasisSet:
         if self._includes_spin:
             warnings.warn("The basis has already been spin-doubled. Avoiding a second doubling.")
             return
+        return self._spin_double(a, b, anti_symmetrize, two_body=True)
 
+    def _spin_double(self, a, b, anti_symmetrize, two_body):
+        """``change_to_general_orbital_basis``; ``two_body=False`` leaves ``u`` alone and records it as
+        anti-symmetrised when ``anti_symmetrize`` is set (the caller stores that tensor)."""
         self._includes_spin = True
         self.l = 2 * self.l
         widen = self.cast_to_complex_on_spin_doubling
@@ -424,15 +438,16 @@ class BasisSet:
         self.s = self.add_spin_one_body(self.s, np=self.np)
 
         # A subclass that overrides the static hooks (reference dispatch through `self`, basis_set.py:523, :576;
-        # e.g. the 2-D sinc-DVR storage) gets its own add_spin_two_body / anti_symmetrize_u, un-fused.
-        hooks_overridden = (
+        # e.g. the 2-D sinc-DVR storage) gets its own add_spin_two_body / anti_symmetrize_u, un-fused.  Without the
+        # u step the hooks do not run and the anti-symmetrisation is recorded as fused.
+        hooks_overridden = two_body and (
             type(self).add_spin_two_body is not BasisSet.add_spin_two_body
             or type(self).anti_symmetrize_u is not BasisSet.anti_symmetrize_u
         )
         fuse_as = bool(anti_symmetrize) and not self._anti_symmetrized_u and not hooks_overridden
         if hooks_overridden:
             self.u = self.add_spin_two_body(self._u, np=self.np)
-        else:
+        elif two_body:
             u_dev = _arrays.to_device(self._u)
             out_dtype = torch.complex128 if (widen or u_dev.is_complex()) else torch.float64
             self.u = _arrays.to_module(
@@ -560,7 +575,13 @@ class BasisSet:
     # ------------------------------------------------------------------ copies
     def copy_basis(self):
         """Deep copy (basis_set.py:784-805).  Array modules are shared, never copied."""
+        return self._copy_basis(with_u=True)
+
+    def _copy_basis(self, with_u):
+        """``copy_basis``; ``with_u=False`` gives a copy whose ``u`` is None instead of a copy of ``u``."""
         memo = {}
+        if not with_u and self._u is not None:
+            memo[id(self._u)] = None  # deepcopy takes a memo entry as the copy of that object
         for value in vars(self).values():
             if isinstance(value, types.ModuleType):
                 memo[id(value)] = value

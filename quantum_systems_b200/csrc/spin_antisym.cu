@@ -4,6 +4,8 @@
 //                          fused with BasisSet.anti_symmetrize_u (:776-778) and cast_to_complex (:298-319)
 //   qs_anti_symmetrize   : BasisSet.anti_symmetrize_u alone
 //   qs_add_spin_one_body : BasisSet.add_spin_one_body (:768-770)
+//   qs_spin_orbital_two_body : the anti-symmetrised spin-orbital tensor of an unrestricted basis from the spin
+//                          blocks of the spatial tensor (hartree_fock.general_orbital_system)
 //
 // Fused pass, per output plane (P = 2p+s1, Q = 2q+s2) and 32x32 tile of spatial (r, s):
 //   U[P,Q,2r+g,2s+d] = [s1==g][s2==d] A[r,s] - [s1==d][s2==g] A[s,r],   A = u[p,q,:,:]
@@ -198,6 +200,124 @@ __global__ void __launch_bounds__(256) antisym_kernel(const double* __restrict__
     }
 }
 
+// Spin-orbital tensor of an unrestricted basis from its spin blocks.  Output plane (I, J) needs one spatial plane,
+// A = B_{sI sJ}[oI, oJ], and its transpose:
+//   U[I,J,K,L] = [sK==sI][sL==sJ] A[oK,oL] - [sL==sI][sK==sJ] A[oL,oK]
+// A derived B_ba plane is B_ab[oJ, oI] transposed, so there the two tiles swap roles.  The tile scheme is
+// add_spin_kernel's: one block owns the direct tile D[i][j] = A[r0+i, s0+j] and its partner E[i][j] = A[s0+i, r0+j],
+// both read with coalesced rows, and writes the four spin-orbital elements (K(r, g), L(s, d)) of every spatial
+// (r, s) of the tile -- each output element, zeros included, exactly once.  K and L come from the inverse of the
+// index tables, built by each block for its 32 + 32 orbitals.  Unlike add_spin_kernel's fixed order, a spin pair
+// (s, 0), (s, 1) is one 16-byte store only where the tables put it on an aligned couple of real outputs.
+// grid: x = tile index over (r-tile, s-tile), y = J, z = I - p_begin ; block = (32, 8)
+template <bool IN_COMPLEX, bool OUT_COMPLEX>
+__global__ void __launch_bounds__(256) spin_orbital_kernel(const double* __restrict__ b_aa,
+                                                            const double* __restrict__ b_ab,
+                                                            const double* __restrict__ b_ba,
+                                                            const double* __restrict__ b_bb,
+                                                            const int* __restrict__ orbital,
+                                                            const int* __restrict__ spin, double* __restrict__ out,
+                                                            int l, int tiles, long long p_begin) {
+    __shared__ double dre[kTile][kTile + 1], ere[kTile][kTile + 1];
+    __shared__ double dim_[IN_COMPLEX ? kTile : 1][kTile + 1], eim[IN_COMPLEX ? kTile : 1][kTile + 1];
+    __shared__ int row_of[2][kTile], col_of[2][kTile];  // [spin][orbital - r0 (s0)] -> spin-orbital index
+
+    const int tr = blockIdx.x / tiles, ts = blockIdx.x % tiles;
+    const int J = blockIdx.y;
+    const long long I = p_begin + blockIdx.z;
+    const int r0 = tr * kTile, s0 = ts * kTile;
+    const long long n = 2LL * l;
+    const int oI = orbital[I], sI = spin[I], oJ = orbital[J], sJ = spin[J];
+    const bool derived = sI == 1 && sJ == 0 && b_ba == nullptr;
+    const double* blk = sI == 0 ? (sJ == 0 ? b_aa : b_ab) : (sJ == 0 ? (derived ? b_ab : b_ba) : b_bb);
+    const long long src_plane = derived ? (long long)oJ * l + oI : (long long)oI * l + oJ;
+    const double* A = blk + src_plane * l * l * (IN_COMPLEX ? 2 : 1);
+
+    const int tx = threadIdx.x, ty = threadIdx.y;
+    for (int t = ty * 32 + tx; t < n; t += 256) {
+        const int o = orbital[t], sp = spin[t];
+        if (o >= r0 && o < r0 + kTile) row_of[sp][o - r0] = t;
+        if (o >= s0 && o < s0 + kTile) col_of[sp][o - s0] = t;
+    }
+    for (int i = ty; i < kTile; i += 8) {
+        if (r0 + i < l && s0 + tx < l) {
+            const Elem<IN_COMPLEX> v = Elem<IN_COMPLEX>::load(A, (long long)(r0 + i) * l + s0 + tx);
+            dre[i][tx] = v.real();
+            if (IN_COMPLEX) dim_[i][tx] = v.imag();
+        }
+        if (s0 + i < l && r0 + tx < l) {
+            const Elem<IN_COMPLEX> v = Elem<IN_COMPLEX>::load(A, (long long)(s0 + i) * l + r0 + tx);
+            ere[i][tx] = v.real();
+            if (IN_COMPLEX) eim[i][tx] = v.imag();
+        }
+    }
+    __syncthreads();
+
+    constexpr int OD = OUT_COMPLEX ? 2 : 1;
+    double* plane = out + ((long long)blockIdx.z * n + J) * n * n * OD;
+    if (OUT_COMPLEX) {
+        // lane tx writes spin columns tx and tx + 32 of the tile, (s, d) = (s0 + c / 2, c % 2): in the usual orders
+        // (spin fastest within runs of orbitals) each store instruction of the warp covers 512 contiguous bytes
+#pragma unroll
+        for (int g = 0; g < 2; ++g) {
+            for (int i = ty; i < kTile; i += 8) {
+                if (r0 + i >= l) break;
+                double* row = plane + (long long)row_of[g][i] * n * OD;
+#pragma unroll
+                for (int half = 0; half < 2; ++half) {
+                    const int c = tx + 32 * half;
+                    const int sl = c >> 1, d = c & 1;
+                    if (s0 + sl < l) {
+                        const bool direct = (g == sI) && (d == sJ);
+                        const bool exch = (d == sI) && (g == sJ);
+                        double ar = dre[i][sl], br = ere[sl][i];
+                        double ai = IN_COMPLEX ? dim_[i][sl] : 0.0, bi = IN_COMPLEX ? eim[sl][i] : 0.0;
+                        if (derived) {
+                            const double cr = ar, ci = ai;
+                            ar = br, ai = bi, br = cr, bi = ci;
+                        }
+                        double vr = 0.0, vi = 0.0;
+                        if (direct) vr = ar, vi = ai;
+                        if (exch) vr -= br, vi -= bi;
+                        reinterpret_cast<double2*>(row)[col_of[d][sl]] = make_double2(vr, vi);
+                    }
+                }
+            }
+        }
+        return;
+    }
+    const int sl = tx;
+    if (s0 + sl >= l) return;
+    const int L0 = col_of[0][sl], L1 = col_of[1][sl];
+#pragma unroll
+    for (int g = 0; g < 2; ++g) {
+        for (int i = ty; i < kTile; i += 8) {
+            if (r0 + i >= l) break;
+            double a = dre[i][sl], b = ere[sl][i];
+            if (derived) {
+                const double t = a;
+                a = b, b = t;
+            }
+            double v[2];
+#pragma unroll
+            for (int d = 0; d < 2; ++d) {
+                v[d] = 0.0;
+                if ((g == sI) && (d == sJ)) v[d] = a;
+                if ((d == sI) && (g == sJ)) v[d] -= b;
+            }
+            double* row = plane + (long long)row_of[g][i] * n;
+            if (L1 == L0 + 1 && !(L0 & 1)) {
+                *reinterpret_cast<double2*>(row + L0) = make_double2(v[0], v[1]);
+            } else if (L0 == L1 + 1 && !(L1 & 1)) {
+                *reinterpret_cast<double2*>(row + L1) = make_double2(v[1], v[0]);
+            } else {
+                row[L0] = v[0];
+                row[L1] = v[1];
+            }
+        }
+    }
+}
+
 template <bool IN_COMPLEX, bool OUT_COMPLEX>
 __global__ void add_spin_one_body_kernel(const double* __restrict__ h, double* __restrict__ out, int l) {
     const long long n = 2LL * l;
@@ -300,6 +420,49 @@ extern "C" int qs_add_spin_two_body(const void* u, int in_dtype, int64_t l, void
         else
             QS_SPIN_LAUNCH(false, false);
 #undef QS_SPIN_LAUNCH
+        QS_LAUNCH_CHECK();
+    }
+    qs_timing_end(span, stream);
+    return QS_OK;
+}
+
+extern "C" int qs_spin_orbital_two_body(const void* b_aa, const void* b_ab, const void* b_ba, const void* b_bb,
+                                        int in_dtype, int64_t l, const int32_t* orbital, const int32_t* spin,
+                                        void* out, int out_dtype, int64_t p_begin, int64_t p_end, void* stream) {
+    QS_REQUIRE(l > 0 && 0 <= p_begin && p_begin <= p_end && p_end <= 2 * l,
+               "qs_spin_orbital_two_body: bad plane range");
+    QS_REQUIRE((in_dtype == QS_F64 || in_dtype == QS_C128) && (out_dtype == QS_F64 || out_dtype == QS_C128),
+               "qs_spin_orbital_two_body: unknown dtype");
+    QS_REQUIRE(!(in_dtype == QS_C128 && out_dtype == QS_F64),
+               "qs_spin_orbital_two_body: cannot narrow complex to real");
+    if (p_begin == p_end) return QS_OK;  // an empty shard
+    QS_REQUIRE(b_aa && b_ab && b_bb && orbital && spin && out, "qs_spin_orbital_two_body: bad arguments");
+    QS_REQUIRE(l <= 32767, "qs_spin_orbital_two_body: l too large");
+    const int tiles = (int)qs_ceil_div(l, kTile);
+    const int64_t planes = p_end - p_begin;
+    const int64_t n = 2 * l;
+    const dim3 block(32, 8);
+    const double *aa = static_cast<const double*>(b_aa), *ab = static_cast<const double*>(b_ab),
+                 *ba = static_cast<const double*>(b_ba), *bb = static_cast<const double*>(b_bb);
+    double* o = static_cast<double*>(out);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    int span = -1;
+    // algorithmic bytes: one spatial plane per output plane (I, J) + every output element written once
+    qs_timing_begin(QS_FAMILY_SPIN_PASS,
+                    (double)planes * n * l * l * 8.0 * qs_elem_doubles(in_dtype) +
+                        (double)planes * n * n * n * 8.0 * qs_elem_doubles(out_dtype),
+                    stream, &span);
+    for (int64_t z0 = 0; z0 < planes; z0 += 65535) {
+        const int64_t nz = planes - z0 < 65535 ? planes - z0 : 65535;
+        const dim3 grid((unsigned)(tiles * tiles), (unsigned)n, (unsigned)nz);
+        double* oz = o + z0 * n * n * n * qs_elem_doubles(out_dtype);
+        const long long pb = p_begin + z0;
+        if (in_dtype == QS_C128)
+            spin_orbital_kernel<true, true><<<grid, block, 0, st>>>(aa, ab, ba, bb, orbital, spin, oz, (int)l, tiles, pb);
+        else if (out_dtype == QS_C128)
+            spin_orbital_kernel<false, true><<<grid, block, 0, st>>>(aa, ab, ba, bb, orbital, spin, oz, (int)l, tiles, pb);
+        else
+            spin_orbital_kernel<false, false><<<grid, block, 0, st>>>(aa, ab, ba, bb, orbital, spin, oz, (int)l, tiles, pb);
         QS_LAUNCH_CHECK();
     }
     qs_timing_end(span, stream);

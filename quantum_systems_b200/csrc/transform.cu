@@ -211,21 +211,29 @@ extern "C" int qs_transform_two_body_workspace_bytes(int64_t n, int64_t n_new, i
     return QS_OK;
 }
 
-extern "C" int qs_transform_two_body(const void* u, int u_dtype, const void* C, const void* Ct, int c_dtype, int64_t n,
-                                     int64_t n_new, void* out, void* workspace, int64_t workspace_bytes,
-                                     void* stream) {
-    return qs_transform_two_body_symmetric(u, u_dtype, C, Ct, c_dtype, n, n_new, 0, out, workspace, workspace_bytes,
-                                           stream);
+namespace {
+
+// Coefficients of the four quarter steps s, r, q, p: steps 1 and 2 contract with the ket matrices C_s and C_r
+// (n x m), steps 3 and 4 with the bra matrices Ct_q and Ct_p (m x n); a null bra stands for conj(ket)^T of the
+// same index pair (Ct_q: conj(C_s)^T, Ct_p: conj(C_r)^T).
+struct StepCoeffs {
+    const void *C_s, *C_r, *Ct_q, *Ct_p;
+};
+
+// image M[k, w] = Ct[w, k] of a bra step from Ct (m x n row-major), or from conj(C)^T: conj(C[k, w])
+int build_bra_image(const void* Ct, const void* C, int c_dtype, int64_t N, int64_t M, int td, void* img, void* stream) {
+    if (Ct) return qs_build_coeff_image(Ct, c_dtype, 1, N, 0, N, M, td, img, stream);
+    return qs_build_coeff_image(C, c_dtype, M, 1, 1, N, M, td, img, stream);
 }
 
 // symmetry = 0: no assumption.  symmetry = 1: u[p,q,r,s] = -u[p,q,s,r]; symmetry = 2: u[p,q,r,s] = u[q,p,s,r] (the
 // caller has verified it with qs_two_body_symmetry).  After the two ket contractions T2[r,s,a,b] inherits the
 // symmetry in (r,s), so steps 2-4 visit only the tiles that hold a pair r < s (r <= s) and the other half of the
-// result is filled in by its mirror image (csrc/symmetry.cu).
-extern "C" int qs_transform_two_body_symmetric(const void* u, int u_dtype, const void* C, const void* Ct, int c_dtype,
-                                               int64_t n, int64_t n_new, int symmetry, void* out, void* workspace,
-                                               int64_t workspace_bytes, void* stream) {
-    QS_REQUIRE(u && C && out && workspace, "qs_transform_two_body: null pointer");
+// result is filled in by its mirror image (csrc/symmetry.cu).  That needs one coefficient pair for both kets and one
+// for both bras; four different matrices take symmetry = 0.
+int two_body_steps(const void* u, int u_dtype, const StepCoeffs& c, int c_dtype, int64_t n, int64_t n_new,
+                   int symmetry, void* out, void* workspace, int64_t workspace_bytes, void* stream) {
+    QS_REQUIRE(u && c.C_s && c.C_r && out && workspace, "qs_transform_two_body: null pointer");
     QS_REQUIRE(n > 0 && n_new > 0, "qs_transform_two_body: bad extents");
     QS_REQUIRE(symmetry >= 0 && symmetry <= 2, "qs_transform_two_body: unknown symmetry %d", symmetry);
     TwoBodyPlan plan;
@@ -247,15 +255,15 @@ extern "C" int qs_transform_two_body_symmetric(const void* u, int u_dtype, const
     long long* tables = reinterpret_cast<long long*>(static_cast<char*>(lists) + plan.list_bytes);
     const int td = plan.t_dtype;
 
+    // step 4 reads a bra image of its own only when its bra differs from step 3's
+    const bool bra_p_differs = c.Ct_p != c.Ct_q || (!c.Ct_p && c.C_r != c.C_s);
+    QS_REQUIRE(!(symmetry && (bra_p_differs || c.C_r != c.C_s)),
+               "qs_transform_two_body: the symmetry-aware steps need one ket and one bra matrix");
     // M[k, w] = C[k, w] (row-major n x m) for steps 1-2
-    if ((rc = qs_build_coeff_image(C, c_dtype, M, 1, 0, N, M, u_dtype, img1, stream))) return rc;
-    if ((rc = qs_build_coeff_image(C, c_dtype, M, 1, 0, N, M, td, img2, stream))) return rc;
-    // M[k, w] = Ct[w, k] for steps 3-4; Ct (m x n row-major), or conj(C)^T -> conj(C[k, w])
-    if (Ct) {
-        if ((rc = qs_build_coeff_image(Ct, c_dtype, 1, N, 0, N, M, td, img3, stream))) return rc;
-    } else {
-        if ((rc = qs_build_coeff_image(C, c_dtype, M, 1, 1, N, M, td, img3, stream))) return rc;
-    }
+    if ((rc = qs_build_coeff_image(c.C_s, c_dtype, M, 1, 0, N, M, u_dtype, img1, stream))) return rc;
+    if ((rc = qs_build_coeff_image(c.C_r, c_dtype, M, 1, 0, N, M, td, img2, stream))) return rc;
+    // M[k, w] = Ct[w, k] for step 3 (and step 4 when its bra is the same)
+    if ((rc = build_bra_image(c.Ct_q, c.C_s, c_dtype, N, M, td, img3, stream))) return rc;
     const void* a0 = u;
     if (plan.pad_bytes) {
         if ((rc = pad_rows(u, padded, N * N * N, N, plan.pitch_u, stream))) return rc;
@@ -266,6 +274,8 @@ extern "C" int qs_transform_two_body_symmetric(const void* u, int u_dtype, const
     if (!symmetry) {
         if ((rc = rotated_quarter(bufA, td, M * N * N, N, P, img2, c_dtype, M, bufB, N, P, stream))) return rc;
         if ((rc = rotated_quarter(bufB, td, M * M * N, N, P, img3, c_dtype, M, bufA, N, P, stream))) return rc;
+        // step 4's image replaces step 3's in the same slot: the stream orders the rebuild after step 3's reads
+        if (bra_p_differs && (rc = build_bra_image(c.Ct_p, c.C_r, c_dtype, N, M, td, img3, stream))) return rc;
         if ((rc = rotated_quarter(bufA, td, M * M * M, N, P, img3, c_dtype, M, out, M, M, stream))) return rc;
         return QS_OK;
     }
@@ -336,6 +346,32 @@ extern "C" int qs_transform_two_body_symmetric(const void* u, int u_dtype, const
     s4.xr_paired = paired;
     if ((rc = qs_quarter_launch(bufA, td, M * npairs, N, P, img3, c_dtype, M, s4, stream))) return rc;
     return qs_mirror_fill(out, td, M, symmetry, stream);
+}
+
+}  // namespace
+
+extern "C" int qs_transform_two_body(const void* u, int u_dtype, const void* C, const void* Ct, int c_dtype, int64_t n,
+                                     int64_t n_new, void* out, void* workspace, int64_t workspace_bytes,
+                                     void* stream) {
+    return qs_transform_two_body_symmetric(u, u_dtype, C, Ct, c_dtype, n, n_new, 0, out, workspace, workspace_bytes,
+                                           stream);
+}
+
+extern "C" int qs_transform_two_body_symmetric(const void* u, int u_dtype, const void* C, const void* Ct, int c_dtype,
+                                               int64_t n, int64_t n_new, int symmetry, void* out, void* workspace,
+                                               int64_t workspace_bytes, void* stream) {
+    const StepCoeffs c = {C, C, Ct, Ct};
+    return two_body_steps(u, u_dtype, c, c_dtype, n, n_new, symmetry, out, workspace, workspace_bytes, stream);
+}
+
+// The spin blocks of an unrestricted basis change pair two coefficient matrices: out[p,q,r,s] =
+// sum Ct_p[p,a] Ct_q[q,b] u[a,b,c,d] C_r[c,r] C_s[d,s].  Same steps, same workspace, one image per step.
+extern "C" int qs_transform_two_body_mixed(const void* u, int u_dtype, const void* C_r, const void* C_s,
+                                           const void* Ct_p, const void* Ct_q, int c_dtype, int64_t n, int64_t n_new,
+                                           void* out, void* workspace, int64_t workspace_bytes, void* stream) {
+    QS_REQUIRE(C_r && C_s, "qs_transform_two_body_mixed: null coefficient matrix");
+    const StepCoeffs c = {C_s, C_r, Ct_q, Ct_p};
+    return two_body_steps(u, u_dtype, c, c_dtype, n, n_new, 0, out, workspace, workspace_bytes, stream);
 }
 
 extern "C" int qs_transform_one_body_workspace_bytes(int64_t n, int64_t n_new, int h_dtype, int c_dtype,

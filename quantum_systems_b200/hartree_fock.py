@@ -17,12 +17,17 @@ quarter GEMM; otherwise it runs in complex128.
 
 ``ground_state_unrestricted(system, n_alpha, n_beta)`` solves unrestricted HF (UHF) on the spatial ``u``: one
 coefficient matrix per spin, for open shells and spin-polarised or broken-symmetry states.  Its Fock build,
-``ops.fock_from_density_unrestricted``, reads a real ``u`` once for both spins.  ``spin_orbital_coefficients``
-turns the result into the ``(2l, 2l)`` coefficients of the spin-doubled basis::
+``ops.fock_from_density_unrestricted``, reads a real ``u`` once for both spins.  ``general_orbital_system`` moves
+the spin-orbital system into the UHF basis, ready for CC or CI::
 
     state = hartree_fock.ground_state_unrestricted(basis, n_alpha=2, n_beta=1)
-    C, epsilon = hartree_fock.spin_orbital_coefficients(state)
-    GeneralOrbitalSystem(3, basis).change_basis(C)
+    system = hartree_fock.general_orbital_system(state, basis)    # GeneralOrbitalSystem(3, ...) in the UHF basis
+
+It transforms the spin blocks of the spatial ``u`` and assembles the anti-symmetrised ``(2l)^4`` tensor from them
+in one pass.  ``spin_orbital_coefficients`` gives the ``(2l, 2l)`` coefficients and orbital energies of the same
+basis; ``GeneralOrbitalSystem(3, basis).change_basis(C)`` with them computes the same system through the
+spin-doubled ``u``: eight to ten times the tensor-core flops (twice that on a complex128 ``u``) and four
+``(2l)^4`` buffers.
 """
 
 import dataclasses
@@ -229,28 +234,100 @@ def ground_state_unrestricted_sharded(basis, n_alpha, n_beta, tol=1e-9, max_iter
     return _uscf(h, s, fock, n_alpha, n_beta, tol, max_iterations, C, nuclear_repulsion_energy, agree)
 
 
+def spin_orbital_order(n_alpha, n_beta, l):
+    """The spin-orbital order of an unrestricted state: ``(orbital, spin)``, integer ndarrays of length ``2l`` with
+    spin-orbital ``I`` the spatial orbital ``orbital[I]`` of spin ``spin[I]`` (0 = alpha).  The occupied spin-orbitals
+    come first, then the virtual ones, each block ordered by (orbital index, spin) with alpha before beta.  The one
+    order of ``spin_orbital_coefficients`` and ``general_orbital_system``."""
+    occ = (n_alpha, n_beta)
+    pairs = ([(j, s) for j in range(l) for s in (0, 1) if j < occ[s]]
+             + [(j, s) for j in range(l) for s in (0, 1) if j >= occ[s]])
+    table = np.array(pairs, dtype=np.int64).reshape(2 * l, 2)
+    return table[:, 0].copy(), table[:, 1].copy()
+
+
 def spin_orbital_coefficients(state):
     """The UHF state as ``(C, epsilon)`` of the spin-doubled basis: ``C`` is ``(2l, 2l)`` for
     ``GeneralOrbitalSystem(n_alpha + n_beta, basis).change_basis(C)``.  Rows follow ``add_spin`` (row ``2a + s``,
-    ``s = 0`` the spin-up component); the columns are the occupied spin-orbitals, then the virtual ones, each block
-    ordered by (orbital index, spin) with alpha before beta.  A closed shell with ``C_alpha = C_beta`` gives
-    ``kron(C, I_2)``.  Returns tensors or ndarrays, as the state holds."""
+    ``s = 0`` the spin-up component); the columns follow ``spin_orbital_order``: the occupied spin-orbitals, then the
+    virtual ones, each block ordered by (orbital index, spin) with alpha before beta.  A closed shell with
+    ``C_alpha = C_beta`` gives ``kron(C, I_2)``.  Returns tensors or ndarrays, as the state holds."""
     Ca, Cb = state.C_alpha, state.C_beta
     xp = torch if isinstance(Ca, torch.Tensor) else np
     l = Ca.shape[0]
-    occupied = [(j, spin) for j in range(l) for spin, n_occ in ((0, state.n_alpha), (1, state.n_beta)) if j < n_occ]
-    virtual = [(j, spin) for j in range(l) for spin, n_occ in ((0, state.n_alpha), (1, state.n_beta)) if j >= n_occ]
-    order = occupied + virtual
+    orbital, spin_of = spin_orbital_order(state.n_alpha, state.n_beta, l)
     dtype = Ca.dtype if Ca.dtype == Cb.dtype else (torch.complex128 if xp is torch else np.complex128)
     kw = {"device": Ca.device} if xp is torch else {}
     C = xp.zeros((2 * l, 2 * l), dtype=dtype, **kw)
     eps = xp.zeros(2 * l, dtype=state.epsilon_alpha.dtype, **kw)
     for spin, (Cs, es) in enumerate(((Ca, state.epsilon_alpha), (Cb, state.epsilon_beta))):
-        cols = [k for k, (_, sp) in enumerate(order) if sp == spin]
-        orbs = [j for j, sp in order if sp == spin]
+        cols = [int(k) for k in np.flatnonzero(spin_of == spin)]
+        orbs = [int(j) for j in orbital[cols]]
         C[spin::2, cols] = Cs[:, orbs].to(dtype) if xp is torch else Cs[:, orbs]
         eps[cols] = es[orbs]
     return C, eps
+
+
+def general_orbital_system(state, basis):
+    """``GeneralOrbitalSystem(state.n_alpha + state.n_beta, ...)`` in the spin-orbital basis of the UHF ``state`` of
+    the spatial ``basis``, which is left unmodified: what ``GeneralOrbitalSystem(n, basis.copy_basis())
+    .change_basis(spin_orbital_coefficients(state)[0])`` computes, without the spin-doubled ``(2l)^4`` input and its
+    ``(2l)^4`` four-index transform.
+
+    ``u`` is built from the spin blocks ``B_st = C_s^dagger C_t^dagger u C_s C_t`` of the spatial tensor
+    (``ops.transform_two_body`` for the same-spin blocks, with the symmetry found by one exact test of ``u``, and
+    ``ops.transform_two_body_mixed`` for alpha-beta, and for beta-alpha only when ``u`` lacks particle-exchange
+    symmetry) and one assembly pass into the anti-symmetrised result (``ops.spin_orbital_two_body``), whose dtype
+    follows ``cast_to_complex_on_spin_doubling`` as on the spin-doubling route.  The one-body elements, the grid
+    orbitals and the spin operators take the code of ``change_to_general_orbital_basis`` and ``change_basis`` and are
+    bit-identical to that route.  A host (numpy) basis gets ndarrays."""
+    from .general_orbital_system import GeneralOrbitalSystem
+
+    if basis.includes_spin:
+        raise ValueError("the UHF spin-orbital system is built from a spatial basis; this one is spin-doubled already")
+    if getattr(basis, "u_repr", "4d") == "2d":
+        raise ValueError("the UHF spin-orbital system needs the 4-d two-body tensor; call set_u_repr('4d') first")
+    if basis.anti_symmetrized_u:
+        raise ValueError("the UHF spin-orbital system needs the plain spatial u, not an anti-symmetrised one")
+    l = basis.l
+    if tuple(state.C_alpha.shape) != (l, l) or tuple(state.C_beta.shape) != (l, l):
+        raise ValueError(f"the state has {tuple(state.C_alpha.shape)} coefficients, the basis l = {l}")
+    C, _ = spin_orbital_coefficients(state)
+    U = _spin_orbital_u(_arrays.to_device(basis.u), _arrays.to_device(state.C_alpha),
+                        _arrays.to_device(state.C_beta), state.n_alpha, state.n_beta,
+                        basis.cast_to_complex_on_spin_doubling)
+    # the one-body side of GeneralOrbitalSystem(n, basis.copy_basis()).change_basis(C): the same calls without u
+    gos_basis = basis._copy_basis(with_u=False)
+    gos_basis._spin_double(a=[1, 0], b=[0, 1], anti_symmetrize=True, two_body=False)
+    system = GeneralOrbitalSystem(state.n_alpha + state.n_beta, gos_basis)
+    gos_basis._change_basis(C, None, two_body=False)
+    gos_basis.u = _arrays.to_module(U, basis.np)
+    system.set_system_size(system.n, gos_basis.l)
+    return system
+
+
+def _spin_orbital_u(u, Ca, Cb, n_alpha, n_beta, widen):
+    """The anti-symmetrised ``(2l)^4`` tensor of ``general_orbital_system`` from the spin blocks of ``u``."""
+    l = u.shape[0]
+    flags = ops.proven_symmetry(u)
+    if flags != ops.PARTICLE_EXCHANGE:
+        flags = ops.two_body_symmetry(u)
+    exchange = bool(flags & ops.PARTICLE_EXCHANGE)
+    # the same-spin blocks keep both symmetries of u (one matrix for both kets and both bras); below
+    # ops.SYMMETRY_MIN_N the plain steps are cheaper, as in transform_two_body
+    same_spin = 0
+    if ops.EXPLOIT_SYMMETRY and l >= ops.SYMMETRY_MIN_N:
+        same_spin = (ops.ANTISYMMETRIC_LAST_PAIR if flags & ops.ANTISYMMETRIC_LAST_PAIR
+                     else ops.PARTICLE_EXCHANGE if exchange else 0)
+    b_aa = ops.transform_two_body(u, Ca, symmetry=same_spin)
+    b_bb = ops.transform_two_body(u, Cb, symmetry=same_spin)
+    b_ab = ops.transform_two_body_mixed(u, Ca, Cb)
+    b_ba = None if exchange else ops.transform_two_body_mixed(u, Cb, Ca)
+    out_dtype = torch.complex128 if (widen or b_aa.is_complex()) else torch.float64
+    orbital, spin = spin_orbital_order(n_alpha, n_beta, l)
+    U = ops.spin_orbital_two_body(b_aa, b_ab, b_ba, b_bb, orbital, spin, out_dtype=out_dtype)
+    del b_aa, b_ab, b_ba, b_bb  # consumed: back to the allocator before the caller goes on
+    return U
 
 
 def _occupations(n_alpha, n_beta, l):

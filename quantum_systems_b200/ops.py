@@ -180,6 +180,38 @@ def transform_two_body(u, C, C_tilde=None, symmetry=None):
     return out
 
 
+def transform_two_body_mixed(u, C_r, C_s, Ct_p=None, Ct_q=None):
+    """``u'_pqrs = sum Ct_p[p,a] Ct_q[q,b] u[a,b,c,d] C_r[c,r] C_s[d,s]`` (``qs_transform_two_body_mixed``): the
+    four-index transform with one coefficient matrix per index, ``Ct_p`` defaulting to ``C_r^dagger`` and ``Ct_q``
+    to ``C_s^dagger``.  The mixed-spin blocks of an unrestricted basis change; no symmetry of ``u`` is used.  The
+    matrices are brought to one dtype, and complex-typed ones without imaginary part are handed over as real ones
+    for a complex ``u`` (``real_coefficients_if_exact``)."""
+    u = _device_tensor(u, "u")
+    C_r, Ct_p = _coefficients(C_r, Ct_p)
+    C_s, Ct_q = _coefficients(C_s, Ct_q)
+    if C_r.shape != C_s.shape:
+        raise ValueError(f"C_r and C_s must have one shape, got {tuple(C_r.shape)} and {tuple(C_s.shape)}")
+    mats = [M for M in (C_r, C_s, Ct_p, Ct_q) if M is not None]
+    dt = _result_dtype(*mats)
+    C_r, C_s, Ct_p, Ct_q = (M.to(dt) if M is not None else None for M in (C_r, C_s, Ct_p, Ct_q))
+    # all four real or none: one exact test over every matrix, so that the kernels see a single dtype
+    if u.is_complex() and dt == torch.complex128 and not any(_has_imaginary_part(M) for M in mats):
+        C_r, C_s, Ct_p, Ct_q = (M.real.contiguous() if M is not None else None for M in (C_r, C_s, Ct_p, Ct_q))
+    n, m = C_r.shape
+    if tuple(u.shape) != (n, n, n, n):
+        raise ValueError(f"u must have shape {(n,) * 4} to be contracted with C {tuple(C_r.shape)}, got {tuple(u.shape)}")
+    out = torch.empty((m, m, m, m), dtype=_result_dtype(u, C_r), device=u.device)
+    nbytes = ctypes.c_int64(0)
+    _native.call("qs_transform_two_body_workspace_bytes", n, m, _code(u), _code(C_r), ctypes.byref(nbytes))
+    owner, ws = _workspace(nbytes.value, u.device)
+    _native.call(
+        "qs_transform_two_body_mixed", _ptr(u), _code(u), _ptr(C_r), _ptr(C_s), _ptr(Ct_p), _ptr(Ct_q), _code(C_r),
+        n, m, _ptr(out), ws, nbytes.value, _stream(),
+    )
+    owner.record_stream(torch.cuda.current_stream())
+    return out
+
+
 def transform_one_body(h, C, C_tilde=None):
     """``C~ (h C)`` (reference basis_set.py:329-334)."""
     h = _device_tensor(h, "h")
@@ -286,6 +318,55 @@ def add_spin_one_body(h, out_dtype=None):
     out_dtype = h.dtype if out_dtype is None else out_dtype
     out = torch.empty((2 * l, 2 * l), dtype=out_dtype, device=h.device)
     _native.call("qs_add_spin_one_body", _ptr(h), _code(h), l, _ptr(out), _DTYPES[out_dtype], _stream())
+    return out
+
+
+def spin_orbital_two_body(b_aa, b_ab, b_ba, b_bb, orbital, spin, out_dtype=None, planes=None):
+    """The anti-symmetrised spin-orbital tensor of an unrestricted basis from the spin blocks ``b_st`` (l,l,l,l) of
+    the spatial tensor (``qs_spin_orbital_two_body``)::
+
+        U[I,J,K,L] = [sI=sK][sJ=sL] b_{sI sJ}[oI,oJ,oK,oL] - [sI=sL][sJ=sK] b_{sI sJ}[oI,oJ,oL,oK]
+
+    Spin-orbital ``I`` is spatial orbital ``orbital[I]`` with spin ``spin[I]`` (0 = alpha, 1 = beta): host integer
+    sequences of length ``2l`` that must pair every orbital below ``l`` with both spins exactly once.  ``b_ba=None``
+    derives that block from ``b_ab`` by particle exchange, ``b_ba[i,j,k,l] = b_ab[j,i,l,k]``.  ``out_dtype`` (default:
+    the blocks' dtype) may widen float64 to complex128.  ``planes=(P0, P1)`` writes only the leading planes
+    ``[P0, P1)``; the whole result is tagged anti-symmetric in its last pair, which it is exactly."""
+    import numpy as _numpy
+
+    blocks = [_device_tensor(b, name) if b is not None else None
+              for b, name in ((b_aa, "b_aa"), (b_ab, "b_ab"), (b_ba, "b_ba"), (b_bb, "b_bb"))]
+    if blocks[0] is None or blocks[1] is None or blocks[3] is None:
+        raise ValueError("b_aa, b_ab and b_bb are required; only b_ba may be derived")
+    given = [b for b in blocks if b is not None]
+    l = given[0].shape[0]
+    for b in given:
+        if tuple(b.shape) != (l,) * 4 or b.dtype != given[0].dtype or b.device != given[0].device:
+            raise ValueError("the spin blocks must all be (l,l,l,l) of one dtype on one device")
+    orbital = _numpy.asarray(orbital.cpu() if isinstance(orbital, torch.Tensor) else orbital)
+    spin = _numpy.asarray(spin.cpu() if isinstance(spin, torch.Tensor) else spin)
+    if orbital.shape != (2 * l,) or spin.shape != (2 * l,):
+        raise ValueError(f"orbital and spin must be 1-d of length 2l = {2 * l}")
+    if not (_numpy.issubdtype(orbital.dtype, _numpy.integer) and _numpy.issubdtype(spin.dtype, _numpy.integer)):
+        raise TypeError("orbital and spin must be integer tables")
+    if ((orbital < 0) | (orbital >= l)).any() or ((spin != 0) & (spin != 1)).any():
+        raise ValueError(f"orbital must lie in [0, {l}) and spin in {{0, 1}}")
+    if _numpy.unique(spin.astype(_numpy.int64) * l + orbital).size != 2 * l:
+        raise ValueError("orbital and spin must pair every orbital with both spins exactly once")
+    device = given[0].device
+    orbital_d = torch.from_numpy(orbital.astype(_numpy.int32)).to(device)
+    spin_d = torch.from_numpy(spin.astype(_numpy.int32)).to(device)
+    out_dtype = given[0].dtype if out_dtype is None else out_dtype
+    p0, p1 = (0, 2 * l) if planes is None else (int(planes[0]), int(planes[1]))
+    if not 0 <= p0 <= p1 <= 2 * l:
+        raise ValueError(f"planes {planes} out of range for 2l = {2 * l}")
+    out = torch.empty((p1 - p0, 2 * l, 2 * l, 2 * l), dtype=out_dtype, device=device)
+    _native.call(
+        "qs_spin_orbital_two_body", *(_ptr(b) for b in blocks), _code(given[0]), l, _ptr(orbital_d), _ptr(spin_d),
+        _ptr(out), _DTYPES[out_dtype], p0, p1, _stream(),
+    )
+    if planes is None:
+        _tag_symmetry(out, ANTISYMMETRIC_LAST_PAIR)  # a - b and b - a are exact negatives
     return out
 
 
