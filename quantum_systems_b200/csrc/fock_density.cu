@@ -267,27 +267,76 @@ size_t fd_smem_bytes(int64_t n, int u_dtype, int rho_dtype) {
            (size_t)kFdWarps * 32 * v * kFdTiles * a;
 }
 
-template <bool UC, bool RC, int V, bool SPLIT = false>
-int launch_pass1(const void* u, const void* rho, int n, int chunk, int n_chunks, double a_d, double a_x, void* ws,
-                 long long rows, size_t smem, cudaStream_t st) {
+// Launch geometry of both entries, from fd_geometry.
+struct FdGeometry {
+    int n, chunk, n_chunks;
+    long long rows;  // p_end - p_begin; 0: nothing to launch
+    size_t smem;     // dynamic shared memory of pass 1
+    bool vec;        // 16-byte pieces of a real u
+};
+
+// The checks of both entries in order and their launch geometry.  `args` is the entry's null-pointer check.  A split
+// pass runs real u against a complex density only (the packed pair or a complex rho_s), so its shared memory is
+// sized for one.
+int fd_geometry(const char* entry, bool args, int64_t n, int64_t p_begin, int64_t p_end, int h_dtype, const void* u,
+                int u_dtype, int rho_dtype, int f_dtype, bool split, const void* workspace, int64_t workspace_bytes,
+                FdGeometry* g) {
+    QS_REQUIRE(args && n >= 1 && n <= (1 << 20), "%s: bad arguments", entry);
+    QS_REQUIRE(0 <= p_begin && p_begin <= p_end && p_end <= n, "%s: bad row range", entry);
+    for (int d : {h_dtype, u_dtype, rho_dtype, f_dtype})
+        QS_REQUIRE(d == QS_F64 || d == QS_C128, "%s: bad dtype", entry);
+    QS_REQUIRE(!(f_dtype == QS_F64 && (h_dtype == QS_C128 || u_dtype == QS_C128 || rho_dtype == QS_C128)),
+               "%s: complex u cannot be accumulated into a real Fock matrix", entry);
+    g->rows = p_end - p_begin;
+    if (g->rows == 0) return QS_OK;
+    int64_t need = 0;
+    if (split)
+        qs_fock_density_unrestricted_workspace_bytes(n, p_begin, p_end, u_dtype, rho_dtype, &need);
+    else
+        qs_fock_density_workspace_bytes(n, p_begin, p_end, u_dtype, rho_dtype, &need);
+    QS_REQUIRE(u && workspace && workspace_bytes >= need, "%s: workspace too small (%lld < %lld bytes)", entry,
+               (long long)workspace_bytes, (long long)need);
+    g->n = (int)n;
+    g->chunk = (int)fd_chunk(n);
+    g->n_chunks = (int)qs_ceil_div(n, g->chunk);
+    QS_REQUIRE(g->rows * g->n_chunks < (1LL << 31), "%s: too many planes for one launch", entry);
+    g->smem = fd_smem_bytes(n, u_dtype, split && u_dtype == QS_F64 ? QS_C128 : rho_dtype);
+    QS_REQUIRE(g->smem <= 227 * 1024, "%s: n = %lld needs %zu bytes of shared memory", entry, (long long)n, g->smem);
+    // 16-byte loads of a real row need an even row length and a 16-byte aligned plane
+    g->vec = u_dtype == QS_F64 && n % 2 == 0 && (reinterpret_cast<uintptr_t>(u) & 15) == 0;
+    return QS_OK;
+}
+
+template <bool UC, bool RC, int V, bool SPLIT>
+int launch_pass1(const void* u, const void* rho, const FdGeometry& g, double a_d, double a_x, void* ws,
+                 cudaStream_t st) {
     auto kern = fock_density_kernel<UC, RC, V, SPLIT>;
-    QS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<(unsigned)(rows * n_chunks), kFdThreads, smem, st>>>(static_cast<const double*>(u),
-                                                                 static_cast<const double*>(rho), n, chunk, n_chunks,
-                                                                 a_d, a_x, static_cast<double*>(ws));
+    QS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem));
+    kern<<<(unsigned)(g.rows * g.n_chunks), kFdThreads, g.smem, st>>>(static_cast<const double*>(u),
+                                                                       static_cast<const double*>(rho), g.n, g.chunk,
+                                                                       g.n_chunks, a_d, a_x, static_cast<double*>(ws));
     QS_LAUNCH_CHECK();
     return QS_OK;
 }
 
-// Split pass 1 over one density.  Real u is only ever split against a complex density (the packed pair or a
-// complex rho_s), so four instantiations cover every case.
-int launch_split_pass1(const void* u, bool u_c, const void* rho, bool rho_c, bool vec, int n, int chunk, int n_chunks,
-                       void* ws, long long rows, size_t smem, cudaStream_t st) {
+// Pass 1 for (u complex, rho complex, g.vec, SPLIT).  Real u is only ever split against a complex density, so real u
+// x real rho has no split instantiation.
+template <bool SPLIT>
+int pass1(const void* u, bool u_c, const void* rho, bool rho_c, const FdGeometry& g, double a_d, double a_x, void* ws,
+          cudaStream_t st) {
     if (u_c)
-        return rho_c ? launch_pass1<true, true, 1, true>(u, rho, n, chunk, n_chunks, 0.0, 0.0, ws, rows, smem, st)
-                     : launch_pass1<true, false, 1, true>(u, rho, n, chunk, n_chunks, 0.0, 0.0, ws, rows, smem, st);
-    return vec ? launch_pass1<false, true, 2, true>(u, rho, n, chunk, n_chunks, 0.0, 0.0, ws, rows, smem, st)
-               : launch_pass1<false, true, 1, true>(u, rho, n, chunk, n_chunks, 0.0, 0.0, ws, rows, smem, st);
+        return rho_c ? launch_pass1<true, true, 1, SPLIT>(u, rho, g, a_d, a_x, ws, st)
+                     : launch_pass1<true, false, 1, SPLIT>(u, rho, g, a_d, a_x, ws, st);
+    if (rho_c)
+        return g.vec ? launch_pass1<false, true, 2, SPLIT>(u, rho, g, a_d, a_x, ws, st)
+                     : launch_pass1<false, true, 1, SPLIT>(u, rho, g, a_d, a_x, ws, st);
+    if constexpr (SPLIT) {
+        qs_set_error("fock_density: no split pass for real u and a real density");
+        return QS_ERR_INVALID;
+    } else {
+        return g.vec ? launch_pass1<false, false, 2, false>(u, rho, g, a_d, a_x, ws, st)
+                     : launch_pass1<false, false, 1, false>(u, rho, g, a_d, a_x, ws, st);
+    }
 }
 
 // Bytes of the split rows of one pass: [rows][chunks][D, X][n] complex.
@@ -310,44 +359,18 @@ extern "C" int qs_fock_density(const void* h, int h_dtype, const void* u, int u_
                                int64_t n, double scale_direct, double scale_exchange, void* f, int f_dtype,
                                int64_t p_begin, int64_t p_end, void* workspace, int64_t workspace_bytes,
                                void* stream) {
-    QS_REQUIRE(h && rho && f && n >= 1 && n <= (1 << 20), "qs_fock_density: bad arguments");
-    QS_REQUIRE(0 <= p_begin && p_begin <= p_end && p_end <= n, "qs_fock_density: bad row range");
-    for (int d : {h_dtype, u_dtype, rho_dtype, f_dtype})
-        QS_REQUIRE(d == QS_F64 || d == QS_C128, "qs_fock_density: bad dtype");
-    QS_REQUIRE(!(f_dtype == QS_F64 && (h_dtype == QS_C128 || u_dtype == QS_C128 || rho_dtype == QS_C128)),
-               "qs_fock_density: complex u cannot be accumulated into a real Fock matrix");
-    if (p_begin == p_end) return QS_OK;
-    int64_t need = 0;
-    qs_fock_density_workspace_bytes(n, p_begin, p_end, u_dtype, rho_dtype, &need);
-    QS_REQUIRE(u && workspace && workspace_bytes >= need, "qs_fock_density: workspace too small (%lld < %lld bytes)",
-               (long long)workspace_bytes, (long long)need);
-    const int N = (int)n;
-    const int chunk = (int)fd_chunk(n);
-    const int n_chunks = (int)qs_ceil_div(n, chunk);
-    const long long rows = p_end - p_begin;
-    QS_REQUIRE(rows * n_chunks < (1LL << 31), "qs_fock_density: too many planes for one launch");
-    const size_t smem = fd_smem_bytes(n, u_dtype, rho_dtype);
-    QS_REQUIRE(smem <= 227 * 1024, "qs_fock_density: n = %lld needs %zu bytes of shared memory", (long long)n, smem);
+    FdGeometry g;
+    int status = fd_geometry("qs_fock_density", h && rho && f, n, p_begin, p_end, h_dtype, u, u_dtype, rho_dtype,
+                             f_dtype, false, workspace, workspace_bytes, &g);
+    if (status != QS_OK || g.rows == 0) return status;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    // 16-byte loads of a real row need an even row length and a 16-byte aligned plane
-    const bool vec = u_dtype == QS_F64 && n % 2 == 0 && (reinterpret_cast<uintptr_t>(u) & 15) == 0;
-    int status;
-    if (u_dtype == QS_C128)
-        status = rho_dtype == QS_C128
-                     ? launch_pass1<true, true, 1>(u, rho, N, chunk, n_chunks, scale_direct, scale_exchange, workspace, rows, smem, st)
-                     : launch_pass1<true, false, 1>(u, rho, N, chunk, n_chunks, scale_direct, scale_exchange, workspace, rows, smem, st);
-    else if (rho_dtype == QS_C128)
-        status = vec ? launch_pass1<false, true, 2>(u, rho, N, chunk, n_chunks, scale_direct, scale_exchange, workspace, rows, smem, st)
-                     : launch_pass1<false, true, 1>(u, rho, N, chunk, n_chunks, scale_direct, scale_exchange, workspace, rows, smem, st);
-    else
-        status = vec ? launch_pass1<false, false, 2>(u, rho, N, chunk, n_chunks, scale_direct, scale_exchange, workspace, rows, smem, st)
-                     : launch_pass1<false, false, 1>(u, rho, N, chunk, n_chunks, scale_direct, scale_exchange, workspace, rows, smem, st);
+    status = pass1<false>(u, u_dtype == QS_C128, rho, rho_dtype == QS_C128, g, scale_direct, scale_exchange, workspace,
+                          st);
     if (status != QS_OK) return status;
-    const long long total = rows * n;
-    fock_density_sum_kernel<<<(unsigned)qs_ceil_div(total, 256), 256, 0, st>>>(
+    fock_density_sum_kernel<<<(unsigned)qs_ceil_div(g.rows * n, 256), 256, 0, st>>>(
         static_cast<const double*>(h), h_dtype == QS_C128, static_cast<const double*>(workspace),
-        u_dtype == QS_C128 || rho_dtype == QS_C128, static_cast<double*>(f), f_dtype == QS_C128, N, n_chunks, p_begin,
-        rows);
+        u_dtype == QS_C128 || rho_dtype == QS_C128, static_cast<double*>(f), f_dtype == QS_C128, g.n, g.n_chunks,
+        p_begin, g.rows);
     QS_LAUNCH_CHECK();
     return QS_OK;
 }
@@ -368,53 +391,31 @@ extern "C" int qs_fock_density_unrestricted(const void* h, int h_dtype, const vo
                                             const void* rho_alpha, const void* rho_beta, int rho_dtype, int64_t n,
                                             void* f_alpha, void* f_beta, int f_dtype, int64_t p_begin, int64_t p_end,
                                             void* workspace, int64_t workspace_bytes, void* stream) {
-    QS_REQUIRE(h && rho_alpha && rho_beta && f_alpha && f_beta && n >= 1 && n <= (1 << 20),
-               "qs_fock_density_unrestricted: bad arguments");
-    QS_REQUIRE(0 <= p_begin && p_begin <= p_end && p_end <= n, "qs_fock_density_unrestricted: bad row range");
-    for (int d : {h_dtype, u_dtype, rho_dtype, f_dtype})
-        QS_REQUIRE(d == QS_F64 || d == QS_C128, "qs_fock_density_unrestricted: bad dtype");
-    QS_REQUIRE(!(f_dtype == QS_F64 && (h_dtype == QS_C128 || u_dtype == QS_C128 || rho_dtype == QS_C128)),
-               "qs_fock_density_unrestricted: complex u cannot be accumulated into a real Fock matrix");
-    if (p_begin == p_end) return QS_OK;
-    int64_t need = 0;
-    qs_fock_density_unrestricted_workspace_bytes(n, p_begin, p_end, u_dtype, rho_dtype, &need);
-    QS_REQUIRE(u && workspace && workspace_bytes >= need,
-               "qs_fock_density_unrestricted: workspace too small (%lld < %lld bytes)", (long long)workspace_bytes,
-               (long long)need);
-    const int N = (int)n;
-    const int chunk = (int)fd_chunk(n);
-    const int n_chunks = (int)qs_ceil_div(n, chunk);
-    const long long rows = p_end - p_begin;
-    QS_REQUIRE(rows * n_chunks < (1LL << 31), "qs_fock_density_unrestricted: too many planes for one launch");
-    const bool u_c = u_dtype == QS_C128;
-    const bool packed = !u_c && rho_dtype == QS_F64;
-    const size_t smem = fd_smem_bytes(n, u_dtype, packed ? QS_C128 : rho_dtype);
-    QS_REQUIRE(smem <= 227 * 1024, "qs_fock_density_unrestricted: n = %lld needs %zu bytes of shared memory",
-               (long long)n, smem);
+    FdGeometry g;
+    int status = fd_geometry("qs_fock_density_unrestricted", h && rho_alpha && rho_beta && f_alpha && f_beta, n,
+                             p_begin, p_end, h_dtype, u, u_dtype, rho_dtype, f_dtype, true, workspace,
+                             workspace_bytes, &g);
+    if (status != QS_OK || g.rows == 0) return status;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const bool vec = !u_c && n % 2 == 0 && (reinterpret_cast<uintptr_t>(u) & 15) == 0;
-    const int64_t split_bytes = split_rows_bytes(n, rows);
+    const bool u_c = u_dtype == QS_C128, rho_c = rho_dtype == QS_C128;
+    const bool packed = !u_c && !rho_c;
+    const int64_t split_bytes = split_rows_bytes(n, g.rows);
     char* ws = static_cast<char*>(workspace);
-    int status;
     if (packed) {
-        cplx* rho_c = reinterpret_cast<cplx*>(ws + split_bytes);
+        cplx* rho_p = reinterpret_cast<cplx*>(ws + split_bytes);
         pack_densities_kernel<<<(unsigned)qs_ceil_div(n * n, 256), 256, 0, st>>>(
-            static_cast<const double*>(rho_alpha), static_cast<const double*>(rho_beta), rho_c, n * n);
+            static_cast<const double*>(rho_alpha), static_cast<const double*>(rho_beta), rho_p, n * n);
         QS_LAUNCH_CHECK();
-        status = launch_split_pass1(u, false, rho_c, true, vec, N, chunk, n_chunks, ws, rows, smem, st);
+        status = pass1<true>(u, false, rho_p, true, g, 0.0, 0.0, ws, st);
     } else {
-        const bool rho_c = rho_dtype == QS_C128;
-        status = launch_split_pass1(u, u_c, rho_alpha, rho_c, vec, N, chunk, n_chunks, ws, rows, smem, st);
-        if (status == QS_OK)
-            status = launch_split_pass1(u, u_c, rho_beta, rho_c, vec, N, chunk, n_chunks, ws + split_bytes, rows,
-                                        smem, st);
+        status = pass1<true>(u, u_c, rho_alpha, rho_c, g, 0.0, 0.0, ws, st);
+        if (status == QS_OK) status = pass1<true>(u, u_c, rho_beta, rho_c, g, 0.0, 0.0, ws + split_bytes, st);
     }
     if (status != QS_OK) return status;
-    const long long total = rows * n;
-    fock_density_unrestricted_sum_kernel<<<(unsigned)qs_ceil_div(total, 256), 256, 0, st>>>(
+    fock_density_unrestricted_sum_kernel<<<(unsigned)qs_ceil_div(g.rows * n, 256), 256, 0, st>>>(
         static_cast<const double*>(h), h_dtype == QS_C128, reinterpret_cast<const cplx*>(ws), packed,
-        split_bytes / 16, static_cast<double*>(f_alpha), static_cast<double*>(f_beta), f_dtype == QS_C128, N,
-        n_chunks, p_begin, rows);
+        split_bytes / 16, static_cast<double*>(f_alpha), static_cast<double*>(f_beta), f_dtype == QS_C128, g.n,
+        g.n_chunks, p_begin, g.rows);
     QS_LAUNCH_CHECK();
     return QS_OK;
 }

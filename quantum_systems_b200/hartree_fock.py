@@ -13,7 +13,8 @@ The only O(n^4) step of an iteration, the Fock build from the density matrix, is
 ``X = S^(-1/2)``, Pulay DIIS on the error ``X^dagger (F rho S - S rho F) X`` with 8 vectors, ``torch.linalg.eigh`` and
 Aufbau filling of the lowest orbitals (in ``eigh`` order).  When ``h``, ``s``, ``u`` and a given initial ``C`` have no
 imaginary part the iteration runs in float64 and ``C`` is real, so that ``change_basis(state.C)`` takes the real
-quarter GEMM; otherwise it runs in complex128.
+quarter GEMM; otherwise it runs in complex128.  One SCF loop serves every solver of this module: it iterates over
+spin channels, one for RHF and GHF, two for UHF.
 
 ``ground_state_unrestricted(system, n_alpha, n_beta)`` solves unrestricted HF (UHF) on the spatial ``u``: one
 coefficient matrix per spin, for open shells and spin-polarised or broken-symmetry states.  Its Fock build,
@@ -93,27 +94,17 @@ def ground_state(system, tol=1e-9, max_iterations=100, C=None):
     from .spatial_orbital_system import SpatialOrbitalSystem
 
     basis = system._basis_set
-    if getattr(basis, "u_repr", "4d") == "2d":
-        raise ValueError("Hartree-Fock needs the 4-d two-body tensor; call set_u_repr('4d') on a sinc-DVR basis first")
+    _require_4d(basis)
     restricted = isinstance(system, SpatialOrbitalSystem)
-    h = _arrays.to_device(system.h)
-    s = _arrays.to_device(system.s) if system.s is not None else None
-    u = _arrays.to_device(system.u)  # uploaded once for a host system, resident for the iterations
-    C = _arrays.to_device(C) if C is not None else None
-    dtype = _working_dtype(_has_imag(h), _has_imag(s), _has_imag(u), _has_imag(C))
-    h, s, C = (_as_dtype(t, dtype) for t in (h, s, C))
-    if dtype == torch.float64:
-        u = _as_dtype(u, dtype)
+    h, s, u, C = _device_inputs(system, (C,))
     scales = _scales(restricted, basis.anti_symmetrized_u)
 
     def fock(rho):
-        return ops.fock_from_density(h, u, rho, *scales)
+        return (ops.fock_from_density(h, u, rho[0], *scales),)
 
-    state = _scf(h, s, fock, system.n, restricted, tol, max_iterations, C, system.nuclear_repulsion_energy, None)
-    if _arrays.is_host_module(system.np):
-        for name in ("C", "epsilon", "density_matrix"):
-            setattr(state, name, _arrays.to_host(getattr(state, name)))
-    return state
+    occupations = ((system.n, 2 if restricted else 1),)
+    result = _scf(h, s, fock, occupations, tol, max_iterations, C, system.nuclear_repulsion_energy, None)
+    return _host_results(system, _hf_state(result))
 
 
 def ground_state_sharded(basis, n_occ, tol=1e-9, max_iterations=100, C=None, nuclear_repulsion_energy=0.0):
@@ -129,16 +120,76 @@ def ground_state_sharded(basis, n_occ, tol=1e-9, max_iterations=100, C=None, nuc
     GPUs are sized to fill them, so the Fock build reads the complex slabs and keeps the real part of ``f`` (its
     imaginary part is exactly zero for a real density)."""
     restricted = not basis.includes_spin
-    h, s, (C,), agree = _sharded_inputs(basis, (C,))
-    dtype = h.dtype
+    h, s, C, agree = _sharded_inputs(basis, (C,))
     scales = _scales(restricted, basis.anti_symmetrized_u)
+    fock = _sharded_fock(lambda rho: (basis.fock_from_density(h, rho[0], *scales),), h.dtype)
+    occupations = ((n_occ, 2 if restricted else 1),)
+    return _hf_state(_scf(h, s, fock, occupations, tol, max_iterations, C, nuclear_repulsion_energy, agree))
+
+
+def ground_state_unrestricted(system, n_alpha=None, n_beta=None, tol=1e-9, max_iterations=100, C=None):
+    """UHF ground state with ``n_alpha`` spin-up and ``n_beta`` spin-down electrons on the spatial ``u`` of
+    ``system``: a ``SpatialOrbitalSystem`` (both default to ``system.n``, its number of doubly occupied orbitals)
+    or a spatial ``BasisSet`` (both required).  ``C = (C_alpha, C_beta)`` is the initial guess (default: the core
+    Hamiltonian for both spins; a spin-symmetric guess stays spin-symmetric, so a broken-symmetry solution needs a
+    guess that breaks it).  Fock matrices ``f_s = h + J[rho_a + rho_b] - K[rho_s]`` from
+    ``ops.fock_from_density_unrestricted``, one Pulay DIIS over the errors of both spins with one coefficient set,
+    converged when the larger error of the two is at most ``tol``.  Working dtype and the float64 copy of a
+    real-valued complex ``u`` as in ``ground_state``.  Host (numpy) systems get ndarrays back."""
+    basis = getattr(system, "_basis_set", system)
+    _require_plain_spatial_u(basis, "ground_state")
+    if system is not basis:
+        n_alpha = system.n if n_alpha is None else n_alpha
+        n_beta = system.n if n_beta is None else n_beta
+    n_alpha, n_beta = _occupations(n_alpha, n_beta, basis.l)
+    h, s, u, C = _device_inputs(basis, (None, None) if C is None else C)
 
     def fock(rho):
-        f = basis.fock_from_density(h, rho, *scales)
-        # real working dtype: u has no imaginary part, so with a real density the imaginary part of f is exactly zero
-        return f.real.contiguous() if dtype == torch.float64 and f.is_complex() else f
+        return ops.fock_from_density_unrestricted(h, u, *rho)
 
-    return _scf(h, s, fock, n_occ, restricted, tol, max_iterations, C, nuclear_repulsion_energy, agree)
+    occupations = ((n_alpha, 1), (n_beta, 1))
+    result = _scf(h, s, fock, occupations, tol, max_iterations, C, basis.nuclear_repulsion_energy, None)
+    return _host_results(basis, _uhf_state(result, h, s, n_alpha, n_beta))
+
+
+def ground_state_unrestricted_sharded(basis, n_alpha, n_beta, tol=1e-9, max_iterations=100, C=None,
+                                      nuclear_repulsion_energy=0.0):
+    """The UHF iteration of ``ground_state_unrestricted`` on a ``ShardedBasisSet`` with ``includes_spin=False``:
+    only the Fock build is distributed (``ShardedBasisSet.fock_from_density_unrestricted``); rank 0's coefficients,
+    orbital energies, energy and convergence decision are broadcast, the working dtype and the given guesses are
+    handled as in ``ground_state_sharded`` (a real-valued complex ``u`` is not copied to float64)."""
+    _require_plain_spatial_u(basis, "ground_state_sharded")
+    n_alpha, n_beta = _occupations(n_alpha, n_beta, basis.u.n)
+    h, s, C, agree = _sharded_inputs(basis, (None, None) if C is None else C)
+    fock = _sharded_fock(lambda rho: basis.fock_from_density_unrestricted(h, *rho), h.dtype)
+    occupations = ((n_alpha, 1), (n_beta, 1))
+    result = _scf(h, s, fock, occupations, tol, max_iterations, C, nuclear_repulsion_energy, agree)
+    return _uhf_state(result, h, s, n_alpha, n_beta)
+
+
+def _device_inputs(source, guesses):
+    """``h``, ``s``, ``u`` and the initial guesses of a system or basis on the device in the working dtype, with a
+    complex ``u`` without imaginary part copied to float64 (see ``ground_state``)."""
+    h = _arrays.to_device(source.h)
+    s = _arrays.to_device(source.s) if source.s is not None else None
+    u = _arrays.to_device(source.u)  # uploaded once for a host system, resident for the iterations
+    guesses = [_arrays.to_device(C) if C is not None else None for C in guesses]
+    dtype = _working_dtype(_has_imag(h), _has_imag(s), _has_imag(u), *(_has_imag(C) for C in guesses))
+    h, s = _as_dtype(h, dtype), _as_dtype(s, dtype)
+    guesses = tuple(_as_dtype(C, dtype) for C in guesses)
+    if dtype == torch.float64:
+        u = _as_dtype(u, dtype)
+    return h, s, u, guesses
+
+
+def _host_results(source, state):
+    """``state`` with its tensors as ndarrays when ``source`` keeps its arrays on the host."""
+    if _arrays.is_host_module(source.np):
+        for field in dataclasses.fields(state):
+            value = getattr(state, field.name)
+            if isinstance(value, torch.Tensor):
+                setattr(state, field.name, _arrays.to_host(value))
+    return state
 
 
 def _sharded_inputs(basis, guesses):
@@ -165,73 +216,34 @@ def _sharded_inputs(basis, guesses):
         u_imag = bool(flag.item())
     dtype = _working_dtype(_has_imag(h), _has_imag(s), u_imag, *(_has_imag(C) for C in guesses))
     h, s = _as_dtype(h, dtype), _as_dtype(s, dtype)
-    guesses = [_as_dtype(C, dtype) for C in guesses]
+    guesses = tuple(_as_dtype(C, dtype) for C in guesses)
     return h, s, guesses, agree if collective else None
 
 
-def ground_state_unrestricted(system, n_alpha=None, n_beta=None, tol=1e-9, max_iterations=100, C=None):
-    """UHF ground state with ``n_alpha`` spin-up and ``n_beta`` spin-down electrons on the spatial ``u`` of
-    ``system``: a ``SpatialOrbitalSystem`` (both default to ``system.n``, its number of doubly occupied orbitals)
-    or a spatial ``BasisSet`` (both required).  ``C = (C_alpha, C_beta)`` is the initial guess (default: the core
-    Hamiltonian for both spins; a spin-symmetric guess stays spin-symmetric, so a broken-symmetry solution needs a
-    guess that breaks it).  Fock matrices ``f_s = h + J[rho_a + rho_b] - K[rho_s]`` from
-    ``ops.fock_from_density_unrestricted``, one Pulay DIIS over the errors of both spins with one coefficient set,
-    converged when the larger error of the two is at most ``tol``.  Working dtype and the float64 copy of a
-    real-valued complex ``u`` as in ``ground_state``.  Host (numpy) systems get ndarrays back."""
-    basis = getattr(system, "_basis_set", system)
-    if basis.includes_spin:
-        raise ValueError("UHF needs the spatial two-body tensor; a spin-doubled basis is solved by "
-                         "hartree_fock.ground_state (GHF)")
+def _sharded_fock(build, dtype):
+    """The ``fock`` of the sharded solvers from ``build``, which maps the densities to the distributed Fock builds."""
+
+    def fock(rho):
+        # real working dtype: u has no imaginary part, so with real densities the imaginary parts are exactly zero
+        return tuple(f.real.contiguous() if dtype == torch.float64 and f.is_complex() else f for f in build(rho))
+
+    return fock
+
+
+def _require_4d(basis):
     if getattr(basis, "u_repr", "4d") == "2d":
         raise ValueError("Hartree-Fock needs the 4-d two-body tensor; call set_u_repr('4d') on a sinc-DVR basis first")
-    if basis.anti_symmetrized_u:
-        raise ValueError("UHF needs the plain spatial u, not an anti-symmetrised one")
-    if system is not basis:
-        n_alpha = system.n if n_alpha is None else n_alpha
-        n_beta = system.n if n_beta is None else n_beta
-    n_alpha, n_beta = _occupations(n_alpha, n_beta, basis.l)
-    h = _arrays.to_device(basis.h)
-    s = _arrays.to_device(basis.s) if basis.s is not None else None
-    u = _arrays.to_device(basis.u)  # uploaded once for a host basis, resident for the iterations
-    C = (None, None) if C is None else tuple(_arrays.to_device(c) for c in C)
-    dtype = _working_dtype(_has_imag(h), _has_imag(s), _has_imag(u), *(_has_imag(c) for c in C))
-    h, s = _as_dtype(h, dtype), _as_dtype(s, dtype)
-    C = None if C[0] is None else tuple(_as_dtype(c, dtype) for c in C)
-    if dtype == torch.float64:
-        u = _as_dtype(u, dtype)
-
-    def fock(rho_alpha, rho_beta):
-        return ops.fock_from_density_unrestricted(h, u, rho_alpha, rho_beta)
-
-    state = _uscf(h, s, fock, n_alpha, n_beta, tol, max_iterations, C, basis.nuclear_repulsion_energy, None)
-    if _arrays.is_host_module(basis.np):
-        for name in ("C_alpha", "C_beta", "epsilon_alpha", "epsilon_beta", "density_alpha", "density_beta"):
-            setattr(state, name, _arrays.to_host(getattr(state, name)))
-    return state
 
 
-def ground_state_unrestricted_sharded(basis, n_alpha, n_beta, tol=1e-9, max_iterations=100, C=None,
-                                      nuclear_repulsion_energy=0.0):
-    """The UHF iteration of ``ground_state_unrestricted`` on a ``ShardedBasisSet`` with ``includes_spin=False``:
-    only the Fock build is distributed (``ShardedBasisSet.fock_from_density_unrestricted``); rank 0's coefficients,
-    orbital energies, energy and convergence decision are broadcast, the working dtype and the given guesses are
-    handled as in ``ground_state_sharded`` (a real-valued complex ``u`` is not copied to float64)."""
+def _require_plain_spatial_u(basis, ghf_entry):
+    """Refuses a basis whose ``u`` is not the plain spatial 4-d tensor of UHF; a spin-doubled one is pointed to the
+    GHF solver ``ghf_entry``."""
     if basis.includes_spin:
         raise ValueError("UHF needs the spatial two-body tensor; a spin-doubled basis is solved by "
-                         "hartree_fock.ground_state_sharded (GHF)")
+                         f"hartree_fock.{ghf_entry} (GHF)")
+    _require_4d(basis)
     if basis.anti_symmetrized_u:
         raise ValueError("UHF needs the plain spatial u, not an anti-symmetrised one")
-    n_alpha, n_beta = _occupations(n_alpha, n_beta, basis.u.n)
-    h, s, C, agree = _sharded_inputs(basis, (None, None) if C is None else C)
-    C = None if C[0] is None else tuple(C)
-    dtype = h.dtype
-
-    def fock(rho_alpha, rho_beta):
-        fs = basis.fock_from_density_unrestricted(h, rho_alpha, rho_beta)
-        # real working dtype: u has no imaginary part, so with real densities the imaginary parts are exactly zero
-        return tuple(f.real.contiguous() if dtype == torch.float64 and f.is_complex() else f for f in fs)
-
-    return _uscf(h, s, fock, n_alpha, n_beta, tol, max_iterations, C, nuclear_repulsion_energy, agree)
 
 
 def spin_orbital_order(n_alpha, n_beta, l):
@@ -283,12 +295,7 @@ def general_orbital_system(state, basis):
     bit-identical to that route.  A host (numpy) basis gets ndarrays."""
     from .general_orbital_system import GeneralOrbitalSystem
 
-    if basis.includes_spin:
-        raise ValueError("the UHF spin-orbital system is built from a spatial basis; this one is spin-doubled already")
-    if getattr(basis, "u_repr", "4d") == "2d":
-        raise ValueError("the UHF spin-orbital system needs the 4-d two-body tensor; call set_u_repr('4d') first")
-    if basis.anti_symmetrized_u:
-        raise ValueError("the UHF spin-orbital system needs the plain spatial u, not an anti-symmetrised one")
+    _require_plain_spatial_u(basis, "ground_state")
     l = basis.l
     if tuple(state.C_alpha.shape) != (l, l) or tuple(state.C_beta.shape) != (l, l):
         raise ValueError(f"the state has {tuple(state.C_alpha.shape)} coefficients, the basis l = {l}")
@@ -374,10 +381,16 @@ def _orthogonaliser(s, n, dtype, device):
     return (V * w.rsqrt().to(dtype)) @ V.mH
 
 
-def _density(C, n_occ, restricted):
+def _density(C, n_occ, weight):
     C_o = C[:, :n_occ]
     rho = C_o @ C_o.mH
-    return 2 * rho if restricted else rho
+    return rho if weight == 1 else weight * rho
+
+
+def _stacked(ts):
+    """The matrices of all channels as one tensor for DIIS: one channel's matrix itself, without a copy, else the
+    (channels, n, n) stack."""
+    return ts[0] if len(ts) == 1 else torch.stack(ts)
 
 
 def _diis(fs, errs):
@@ -394,12 +407,18 @@ def _diis(fs, errs):
     return sum(ci.to(fs[0].dtype) * Fi for ci, Fi in zip(c, fs))
 
 
-def _scf(h, s, fock, n_occ, restricted, tol, max_iterations, C, e_nuc, agree):
-    """``h``, ``s``, ``C`` and what ``fock`` returns are all in the working dtype, the dtype of ``h``."""
+def _scf(h, s, fock, occupations, tol, max_iterations, C, e_nuc, agree):
+    """The SCF iteration over spin channels, ``(n_occ, weight)`` each in ``occupations``: RHF is one channel of weight
+    2, GHF one of weight 1, UHF two of weight 1.  ``fock`` maps the tuple of channel densities to the tuple of Fock
+    matrices; ``C`` holds one initial guess per channel, or None for the core Hamiltonian (one ``eigh`` of ``h``,
+    copied to every channel).  The energy is ``1/2 sum_s tr rho_s (h + F_s) + e_nuc``; DIIS extrapolates the
+    stacked Fock matrices of all channels with one coefficient set from their stacked errors, and the largest error
+    decides convergence.  ``h``, ``s``, ``C`` and what ``fock`` returns are all in the working dtype, the dtype of
+    ``h``.  Returns ``(C, epsilon, rho, energy, converged, iterations)``, the first three a tuple per channel."""
     n = h.shape[0]
     dtype, device = h.dtype, h.device
     X = _orthogonaliser(s, n, dtype, device)
-    S = s if s is not None else torch.eye(n, dtype=dtype, device=device)
+    S = _metric(s, h)
 
     def diagonalise(F):
         eps, Cp = torch.linalg.eigh(X.mH @ F @ X)
@@ -408,88 +427,58 @@ def _scf(h, s, fock, n_occ, restricted, tol, max_iterations, C, e_nuc, agree):
             agree(C_new, eps)
         return C_new, eps
 
-    if C is None:
-        C, eps = diagonalise(h)
+    if C[0] is None:
+        C0, eps0 = diagonalise(h)
+        C = (C0,) + tuple(C0.clone() for _ in occupations[1:])
+        eps = (eps0,) + tuple(eps0.clone() for _ in occupations[1:])
     else:
-        eps = None
-    rho = _density(C, n_occ, restricted)
+        eps = (None,) * len(occupations)
+    rho = tuple(_density(Cs, n_occ, weight) for Cs, (n_occ, weight) in zip(C, occupations))
     fs, errs = [], []
     converged, it, energy = False, 0, 0.0
     for it in range(1, max_iterations + 1):
         F = fock(rho)
-        energy_t = 0.5 * torch.sum(rho.transpose(0, 1) * (h + F)).real + e_nuc
-        err = X.mH @ (F @ rho @ S - S @ rho @ F) @ X
+        traces = [torch.sum(r.transpose(0, 1) * (h + f)) for r, f in zip(rho, F)]
+        energy_t = 0.5 * sum(traces[1:], traces[0]).real + e_nuc
+        err = _stacked([X.mH @ (f @ r @ S - S @ r @ f) @ X for f, r in zip(F, rho)])
         decision = torch.stack([energy_t.to(torch.float64), err.abs().max().to(torch.float64)])
         if agree is not None:
             agree(decision)
         energy, err_max = (float(x) for x in decision.tolist())
         converged = err_max <= tol
         if not converged:
-            fs.append(F)
+            fs.append(_stacked(F))
             errs.append(err)
             if len(fs) > DIIS_VECTORS:
                 fs.pop(0)
                 errs.pop(0)
             if len(fs) > 1:
                 F = _diis(fs, errs)
-        C, eps = diagonalise(F)
-        rho = _density(C, n_occ, restricted)
+                F = (F,) if len(occupations) == 1 else tuple(F)
+        C, eps = zip(*(diagonalise(f) for f in F))
+        rho = tuple(_density(Cs, n_occ, weight) for Cs, (n_occ, weight) in zip(C, occupations))
         if converged:
             break
     if not converged:
         warnings.warn(f"Hartree-Fock did not converge in {max_iterations} iterations", RuntimeWarning, stacklevel=3)
+    return C, eps, rho, energy, converged, it
+
+
+def _metric(s, h):
+    """The overlap matrix, the identity when ``s is None``, in the dtype of ``h``."""
+    return s if s is not None else torch.eye(h.shape[0], dtype=h.dtype, device=h.device)
+
+
+def _hf_state(result):
+    """The ``HartreeFockState`` of a one-channel ``_scf`` result."""
+    (C,), (eps,), (rho,), energy, converged, it = result
     return HartreeFockState(C=C, epsilon=eps, energy=energy, density_matrix=rho, converged=converged, iterations=it)
 
 
-def _uscf(h, s, fock, n_alpha, n_beta, tol, max_iterations, C, e_nuc, agree):
-    """The UHF sibling of ``_scf``: ``fock(rho_a, rho_b)`` returns ``(F_a, F_b)``; DIIS extrapolates the stacked pair
-    with one coefficient set from the stacked errors of both spins."""
-    n = h.shape[0]
-    dtype, device = h.dtype, h.device
-    X = _orthogonaliser(s, n, dtype, device)
-    S = s if s is not None else torch.eye(n, dtype=dtype, device=device)
-
-    def diagonalise(F):
-        eps, Cp = torch.linalg.eigh(X.mH @ F @ X)
-        C_new = X @ Cp
-        if agree is not None:
-            agree(C_new, eps)
-        return C_new, eps
-
-    if C is None:
-        Ca, ea = diagonalise(h)
-        Cb, eb = Ca.clone(), ea.clone()
-    else:
-        (Ca, Cb), ea, eb = C, None, None
-    rho_a, rho_b = _density(Ca, n_alpha, False), _density(Cb, n_beta, False)
-    fs, errs = [], []
-    converged, it, energy = False, 0, 0.0
-    for it in range(1, max_iterations + 1):
-        Fa, Fb = fock(rho_a, rho_b)
-        energy_t = 0.5 * (torch.sum(rho_a.transpose(0, 1) * (h + Fa)) + torch.sum(rho_b.transpose(0, 1) * (h + Fb))).real
-        energy_t = energy_t + e_nuc
-        err = torch.stack([X.mH @ (F @ rho @ S - S @ rho @ F) @ X for F, rho in ((Fa, rho_a), (Fb, rho_b))])
-        decision = torch.stack([energy_t.to(torch.float64), err.abs().max().to(torch.float64)])
-        if agree is not None:
-            agree(decision)
-        energy, err_max = (float(x) for x in decision.tolist())
-        converged = err_max <= tol
-        if not converged:
-            fs.append(torch.stack([Fa, Fb]))
-            errs.append(err)
-            if len(fs) > DIIS_VECTORS:
-                fs.pop(0)
-                errs.pop(0)
-            if len(fs) > 1:
-                Fa, Fb = _diis(fs, errs)
-        Ca, ea = diagonalise(Fa)
-        Cb, eb = diagonalise(Fb)
-        rho_a, rho_b = _density(Ca, n_alpha, False), _density(Cb, n_beta, False)
-        if converged:
-            break
-    if not converged:
-        warnings.warn(f"Hartree-Fock did not converge in {max_iterations} iterations", RuntimeWarning, stacklevel=3)
-    overlap = Ca[:, :n_alpha].mH @ S @ Cb[:, :n_beta]
+def _uhf_state(result, h, s, n_alpha, n_beta):
+    """The ``UnrestrictedHartreeFockState`` of a two-channel ``_scf`` result, with ``<S^2>``."""
+    (Ca, Cb), (ea, eb), (rho_a, rho_b), energy, converged, it = result
+    overlap = Ca[:, :n_alpha].mH @ _metric(s, h) @ Cb[:, :n_beta]
     s_z = 0.5 * (n_alpha - n_beta)
     spin_squared = s_z * (s_z + 1) + n_beta - float((overlap.abs() ** 2).sum())
     return UnrestrictedHartreeFockState(

@@ -404,35 +404,9 @@ def fock_from_density(h, u, rho, scale_direct, scale_exchange, f=None, planes=No
     ``u`` is the GHF Fock matrix, ``(1, -1/2)`` with ``rho = 2 C_o C_o^dagger`` the RHF one.  ``planes=(p0, p1)``:
     ``u`` is the leading-index shard ``(p1 - p0, n, n, n)`` and only rows ``[p0, p1)`` of ``f`` are written (a new
     ``f`` is zero elsewhere).  ``f`` is complex128 when any input is; a given ``f`` is filled in place."""
-    h = _device_tensor(h, "h")
-    u = _device_tensor(u, "u")
-    rho = _device_tensor(rho, "rho")
-    n = h.shape[0]
-    p0, p1 = (0, n) if planes is None else (int(planes[0]), int(planes[1]))
-    if not 0 <= p0 <= p1 <= n:
-        raise ValueError(f"planes {planes} out of range for n = {n}")
-    if tuple(h.shape) != (n, n) or tuple(rho.shape) != (n, n) or tuple(u.shape) != (p1 - p0, n, n, n):
-        raise ValueError(
-            f"h and rho must be (n,n) and u (planes,n,n,n), got {tuple(h.shape)}, {tuple(rho.shape)}, {tuple(u.shape)}"
-        )
-    if f is None:
-        alloc = torch.empty if (p0, p1) == (0, n) else torch.zeros
-        f = alloc((n, n), dtype=_result_dtype(h, u, rho), device=h.device)
-    else:
-        if not (isinstance(f, torch.Tensor) and f.is_cuda and f.is_contiguous()):
-            raise RuntimeError("f must be a contiguous CUDA tensor to be filled in place")
-        if tuple(f.shape) != (n, n):
-            raise ValueError(f"f must be {(n, n)}, got {tuple(f.shape)}")
-        _code(f)
-        _mark_written(f)
-    nbytes = ctypes.c_int64(0)
-    _native.call("qs_fock_density_workspace_bytes", n, p0, p1, _code(u), _code(rho), ctypes.byref(nbytes))
-    owner, ws = _workspace(nbytes.value, h.device)
-    _native.call(
-        "qs_fock_density", _ptr(h), _code(h), _ptr(u), _code(u), _ptr(rho), _code(rho), n, float(scale_direct),
-        float(scale_exchange), _ptr(f), _code(f), p0, p1, ws, nbytes.value, _stream(),
+    (f,) = _fock_density(
+        "qs_fock_density", h, u, {"rho": rho}, {"f": f}, (float(scale_direct), float(scale_exchange)), planes
     )
-    owner.record_stream(torch.cuda.current_stream())
     return f
 
 
@@ -443,27 +417,37 @@ def fock_from_density_unrestricted(h, u, rho_alpha, rho_beta, f_alpha=None, f_be
     ``u`` or a complex density: twice.  ``planes``, the in-place ``f_alpha`` / ``f_beta`` and the result dtype
     follow ``fock_from_density``; a real density is promoted to complex when the other one is complex.
     Returns ``(f_alpha, f_beta)``."""
+    return _fock_density(
+        "qs_fock_density_unrestricted", h, u, {"rho_alpha": rho_alpha, "rho_beta": rho_beta},
+        {"f_alpha": f_alpha, "f_beta": f_beta}, (), planes,
+    )
+
+
+def _fock_density(entry, h, u, densities, fs, scales, planes):
+    """The front end of the density Fock builds: checks ``h``, ``u`` and the ``densities`` (name -> tensor, a real
+    one promoted when the other is complex), allocates or validates the outputs ``fs`` (name -> tensor or None) and
+    calls ``entry`` with its workspace.  The C arguments are h, u, the densities, n, ``scales``, the outputs, the row
+    range, the workspace and the stream.  Returns the tuple of outputs."""
     h = _device_tensor(h, "h")
     u = _device_tensor(u, "u")
-    rho_alpha = _device_tensor(rho_alpha, "rho_alpha")
-    rho_beta = _device_tensor(rho_beta, "rho_beta")
-    rho_dtype = _result_dtype(rho_alpha, rho_beta)
-    rho_alpha, rho_beta = rho_alpha.to(rho_dtype), rho_beta.to(rho_dtype)
+    rhos = [_device_tensor(rho, name) for name, rho in densities.items()]
+    if len(rhos) > 1 and rhos[0].dtype != rhos[1].dtype:
+        rhos = [rho.to(torch.complex128) for rho in rhos]
     n = h.shape[0]
     p0, p1 = (0, n) if planes is None else (int(planes[0]), int(planes[1]))
     if not 0 <= p0 <= p1 <= n:
         raise ValueError(f"planes {planes} out of range for n = {n}")
-    if (tuple(h.shape) != (n, n) or tuple(rho_alpha.shape) != (n, n) or tuple(rho_beta.shape) != (n, n)
-            or tuple(u.shape) != (p1 - p0, n, n, n)):
-        raise ValueError(
-            f"h, rho_alpha and rho_beta must be (n,n) and u (planes,n,n,n), got {tuple(h.shape)}, "
-            f"{tuple(rho_alpha.shape)}, {tuple(rho_beta.shape)}, {tuple(u.shape)}"
-        )
-    fs = []
-    for name, f in (("f_alpha", f_alpha), ("f_beta", f_beta)):
+    if (tuple(h.shape) != (n, n) or tuple(u.shape) != (p1 - p0, n, n, n)
+            or [rho.shape for rho in rhos] != [h.shape] * len(rhos)):
+        names = list(densities)
+        shapes = ", ".join(str(tuple(t.shape)) for t in (h, *rhos, u))
+        raise ValueError(f"{', '.join(['h'] + names[:-1])} and {names[-1]} must be (n,n) and u (planes,n,n,n), "
+                         f"got {shapes}")
+    outs = []
+    for name, f in fs.items():
         if f is None:
             alloc = torch.empty if (p0, p1) == (0, n) else torch.zeros
-            f = alloc((n, n), dtype=_result_dtype(h, u, rho_alpha), device=h.device)
+            f = alloc((n, n), dtype=_result_dtype(h, u, *rhos), device=h.device)
         else:
             if not (isinstance(f, torch.Tensor) and f.is_cuda and f.is_contiguous()):
                 raise RuntimeError(f"{name} must be a contiguous CUDA tensor to be filled in place")
@@ -471,21 +455,18 @@ def fock_from_density_unrestricted(h, u, rho_alpha, rho_beta, f_alpha=None, f_be
                 raise ValueError(f"{name} must be {(n, n)}, got {tuple(f.shape)}")
             _code(f)
             _mark_written(f)
-        fs.append(f)
-    f_alpha, f_beta = fs
-    if f_alpha.dtype != f_beta.dtype:
-        raise ValueError(f"f_alpha and f_beta must have one dtype, got {f_alpha.dtype} and {f_beta.dtype}")
+        outs.append(f)
+    if len(outs) > 1 and outs[0].dtype != outs[1].dtype:
+        raise ValueError(f"{' and '.join(fs)} must have one dtype, got {outs[0].dtype} and {outs[1].dtype}")
     nbytes = ctypes.c_int64(0)
-    _native.call(
-        "qs_fock_density_unrestricted_workspace_bytes", n, p0, p1, _code(u), _code(rho_alpha), ctypes.byref(nbytes)
-    )
+    _native.call(entry + "_workspace_bytes", n, p0, p1, _code(u), _code(rhos[0]), ctypes.byref(nbytes))
     owner, ws = _workspace(nbytes.value, h.device)
     _native.call(
-        "qs_fock_density_unrestricted", _ptr(h), _code(h), _ptr(u), _code(u), _ptr(rho_alpha), _ptr(rho_beta),
-        _code(rho_alpha), n, _ptr(f_alpha), _ptr(f_beta), _code(f_alpha), p0, p1, ws, nbytes.value, _stream(),
+        entry, _ptr(h), _code(h), _ptr(u), _code(u), *[_ptr(r) for r in rhos], _code(rhos[0]), n, *scales,
+        *[_ptr(f) for f in outs], _code(outs[0]), p0, p1, ws, nbytes.value, _stream(),
     )
     owner.record_stream(torch.cuda.current_stream())
-    return f_alpha, f_beta
+    return tuple(outs)
 
 
 def odqd_coulomb(C, inner_grid, alpha, a, planes=None):

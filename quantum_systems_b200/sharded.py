@@ -1067,35 +1067,41 @@ class ShardedBasisSet:
         (``ops.fock_from_density``): every rank computes the rows p it owns from its own planes, then the rows are
         all-gathered (n^2 elements).  ``h`` and ``rho`` are replicated.  A row is bit-identical to the same row of
         the single-tensor kernel."""
-        from . import _arrays, ops
+        from . import ops
 
-        ctx, u = self.ctx, self.u
-        h, rho = _arrays.to_device(h), _arrays.to_device(rho)
-        if f is None:
-            f = torch.zeros((u.n, u.n), dtype=ops._result_dtype(h, rho, u.local(ctx.local_ranks[0])), device=h.device)
-        for r in ctx.local_ranks:
-            p0, p1 = u.planes(r)
-            if p1 > p0:
-                ops.fock_from_density(h, u.local(r), rho, scale_direct, scale_exchange, f=f, planes=(p0, p1))
-        return _gather_rows(ctx, u, f)
+        return self._density_fock_rows(
+            lambda h, u, rho, f, planes: ops.fock_from_density(h, u, rho, scale_direct, scale_exchange, f=f,
+                                                               planes=planes),
+            h, (rho,), (f,),
+        )
 
     def fock_from_density_unrestricted(self, h, rho_alpha, rho_beta):
         """Both unrestricted Fock matrices ``(f_alpha, f_beta)`` of a spatial ``u``
         (``ops.fock_from_density_unrestricted``): every rank computes the rows p it owns, then the rows of both
         matrices are gathered in one all-reduce (2 n^2 elements).  ``h`` and the densities are replicated.  A row
         is bit-identical to the same row of the single-tensor kernel."""
+        from . import ops
+
+        return self._density_fock_rows(
+            lambda h, u, ra, rb, fa, fb, planes: ops.fock_from_density_unrestricted(h, u, ra, rb, fa, fb, planes),
+            h, (rho_alpha, rho_beta), (None, None),
+        )
+
+    def _density_fock_rows(self, build, h, rhos, fs):
+        """The per-rank loop of the density Fock builds: ``build(h, u_r, *rhos, *fs, planes)`` writes the rows of
+        the outputs ``fs`` (new zero matrices where None) that rank r owns, then the rows are gathered."""
         from . import _arrays, ops
 
         ctx, u = self.ctx, self.u
-        h, rho_alpha, rho_beta = (_arrays.to_device(t) for t in (h, rho_alpha, rho_beta))
-        dtype = ops._result_dtype(h, rho_alpha, rho_beta, u.local(ctx.local_ranks[0]))
-        f_alpha, f_beta = (torch.zeros((u.n, u.n), dtype=dtype, device=h.device) for _ in range(2))
+        h = _arrays.to_device(h)
+        rhos = [_arrays.to_device(rho) for rho in rhos]
+        dtype = ops._result_dtype(h, *rhos, u.local(ctx.local_ranks[0]))
+        fs = [torch.zeros((u.n, u.n), dtype=dtype, device=h.device) if f is None else f for f in fs]
         for r in ctx.local_ranks:
             p0, p1 = u.planes(r)
             if p1 > p0:
-                ops.fock_from_density_unrestricted(h, u.local(r), rho_alpha, rho_beta, f_alpha=f_alpha, f_beta=f_beta,
-                                                   planes=(p0, p1))
-        return _gather_rows(ctx, u, f_alpha, f_beta)
+                build(h, u.local(r), *rhos, *fs, (p0, p1))
+        return _gather_rows(ctx, u, *fs)
 
 
 def _gather_rows(ctx, u, *fs):

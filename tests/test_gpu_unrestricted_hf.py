@@ -228,7 +228,8 @@ def test_sharded_processes_agree():
     world = min(torch.cuda.device_count(), 8)
     cmd = [
         sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={world}",
-        "--master-addr", "127.0.0.1", "--master-port", "29533", os.path.join(ROOT, "tests", "_multi_gpu_uhf_worker.py"),
+        "--master-addr", "127.0.0.1", "--master-port", "29533", os.path.join(ROOT, "tests", "_multi_gpu_hf_worker.py"),
+        "uhf",
     ]
     proc = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert proc.returncode == 0, proc.stdout[-3000:] + proc.stderr[-3000:]
