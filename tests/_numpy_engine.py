@@ -100,23 +100,11 @@ class NumpyEngine:
         """qs_quarter_transform_scatter_pairs: cyclic destinations, and ONLY the CTA tiles the library's own host-side
         planner (qs_quarter_plan_tiles, mask kind 3; no device involved) would launch are written -- everything else
         keeps the NaN the buffers were created with, so a later read of a tile that was never sent shows up."""
-        import ctypes
-
-        from quantum_systems_b200 import _native
-
         if X <= 0:
             return
-        lib = _native.load()
-        code = {torch.float64: 0, torch.complex128: 1}
-        args = (X, K, W, code[A.dtype], code[m_dtype], x_inner, 3, 0 if padded else 1, 1, 1, rows_per_s, W,
-                ctypes.c_void_p(0))
-        count = ctypes.c_int64(0)
-        assert lib.qs_quarter_plan_tiles(*args, ctypes.c_void_p(0), 0, ctypes.byref(count)) == 0
-        tiles = np.zeros((count.value, 4), dtype=np.int64)
-        assert lib.qs_quarter_plan_tiles(*args, ctypes.c_void_p(tiles.ctypes.data), count.value, ctypes.byref(count)) == 0
         res = self._product(A, X, K, lda, image)
         launched = np.zeros((X, W), dtype=bool)
-        for x0, x1, w0, w1 in tiles:
+        for x0, x1, w0, w1 in self._pair_tiles(X, K, W, A.dtype, m_dtype, x_inner, rows_per_s, padded):
             launched[x0 : x1 + 1, w0 : w1 + 1] = True
         x = np.arange(X)
         xq = x // x_inner
@@ -130,6 +118,23 @@ class NumpyEngine:
             flat = buf.flat()
             rows, cidx = np.nonzero(launched[:, cols])
             flat[off + ax[rows] + aw[cidx]] = res[rows, cols[cidx]]
+
+    @staticmethod
+    def _pair_tiles(X, K, W, a_dtype, m_dtype, x_inner, rows_per_s, padded):
+        """The tiles ``(x0, x1, w0, w1)`` (inclusive) that qs_quarter_transform_scatter_pairs launches."""
+        import ctypes
+
+        from quantum_systems_b200 import _native
+
+        lib = _native.load()
+        code = {torch.float64: 0, torch.complex128: 1}
+        args = (X, K, W, code[a_dtype], code[m_dtype], x_inner, 3, 0 if padded else 1, 1, 1, rows_per_s, W,
+                ctypes.c_void_p(0))
+        count = ctypes.c_int64(0)
+        assert lib.qs_quarter_plan_tiles(*args, ctypes.c_void_p(0), 0, ctypes.byref(count)) == 0
+        tiles = np.zeros((count.value, 4), dtype=np.int64)
+        assert lib.qs_quarter_plan_tiles(*args, ctypes.c_void_p(tiles.ctypes.data), count.value, ctypes.byref(count)) == 0
+        return tiles
 
     # consumers of a shard: documented semantics of qs_extract_block / qs_scale_add / qs_occupied_traces
     def extract_block(self, buf, planes, n, bounds):

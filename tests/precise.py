@@ -65,17 +65,43 @@ def one_body(h, C, Ct, dt, absolute=False):
     return Ct @ (h @ C)
 
 
-def kron_transform_planes(A, B, C, Ct, planes, dt, anti=False, absolute=False):
-    """Planes ``u'[p]`` (``p`` in ``planes``) of the four-index transform of ``u[a,b,c,d] = A[a,c] B[b,d]``
-    (minus ``A[a,d] B[b,c]`` when ``anti``): ``u'[p,q,r,s] = X[p,r] Y[q,s] (- X[p,s] Y[q,r])`` with ``X = C̃ A C``,
-    ``Y = C̃ B C``.  O(n³) per plane; the absolute-value companion of this form is the exact ``|terms|`` of the
-    dense transform when ``anti`` is off and an upper bound of it when on."""
-    X, Y = Ct @ (A @ C), Ct @ (B @ C)
-    Xp = X[list(planes)]
-    out = Xp[:, None, :, None] * Y[None, :, None, :]
+def mixed_steps(u, C_r, C_s, Ct_p, Ct_q, dt, absolute=False):
+    """The kernels' order with one matrix per step: s with ``C_s``, r with ``C_r``, q with ``Ct_qᵀ``, p with
+    ``Ct_pᵀ``, the new index first every time."""
+    t = u
+    for M in (C_s, C_r, Ct_q.T, Ct_p.T):
+        t = np.ascontiguousarray(np.moveaxis(np.tensordot(t, M, ([3], [0])), 3, 0))
+    return t
+
+
+def kron_factors(A, B, C, Ct, C_s=None, Ct_q=None, dt=None, absolute=False):
+    """The two-index factors of the transform of ``u[a,b,c,d] = A[a,c] B[b,d]`` with one matrix per index, in the
+    convention of ``mixed_steps`` (``C`` is ``C_r``, ``Ct`` is ``Ct_p``; ``C_s`` and ``Ct_q`` default to them):
+    ``X = C̃_p A C_r``, ``Y = C̃_q B C_s`` and, for the exchanged term of the anti-symmetric tensor,
+    ``X' = C̃_p A C_s``, ``Y' = C̃_q B C_r``.  Products of non-negative inputs stay so: the same form gives the
+    factors of the absolute-value companion."""
+    C_s = C if C_s is None else C_s
+    Ct_q = Ct if Ct_q is None else Ct_q
+    return Ct @ (A @ C), Ct_q @ (B @ C_s), Ct @ (A @ C_s), Ct_q @ (B @ C)
+
+
+def kron_planes(factors, planes, anti=False, absolute=False):
+    """Planes ``u'[p] = X[p,r] Y[q,s] (- X'[p,s] Y'[q,r])`` from the ``kron_factors`` ``(X, Y, X', Y')``."""
+    X, Y, Xx, Yx = factors
+    planes = list(planes)
+    out = X[planes][:, None, :, None] * Y[None, :, None, :]
     if anti:
-        out = _sub(out, Xp[:, None, None, :] * Y[None, :, :, None], absolute)
+        out = _sub(out, Xx[planes][:, None, None, :] * Yx[None, :, :, None], absolute)
     return out
+
+
+def kron_transform_planes(A, B, C, Ct, C_s=None, Ct_q=None, planes=(), dt=None, anti=False, absolute=False):
+    """Planes ``u'[p]`` (``p`` in ``planes``) of the four-index transform of ``u[a,b,c,d] = A[a,c] B[b,d]``
+    (minus ``A[a,d] B[b,c]`` when ``anti``): ``u'[p,q,r,s] = X[p,r] Y[q,s] (- X'[p,s] Y'[q,r])`` with the
+    ``kron_factors`` ``X = C̃ A C``, ``Y = C̃ B C`` (``C̃_q B C_s`` with one matrix per index).  O(n³) per plane;
+    the absolute-value companion of this form is the exact ``|terms|`` of the dense transform when ``anti`` is
+    off and an upper bound of it when on."""
+    return kron_planes(kron_factors(A, B, C, Ct, C_s, Ct_q), planes, anti, absolute)
 
 
 def diagonal_rows(W, C, Ct, dt, rows=None, anti=False, absolute=False):
@@ -129,6 +155,22 @@ def kron_fock_density(h, A, B, rho, a_d, a_x, dt, absolute=False):
     return h + a_d * A * np.sum(B * rho.T) + a_x * (A @ rho @ B)
 
 
+def kron_fock_unrestricted(h, A, B, rho_a, rho_b, dt, absolute=False):
+    """``fock_unrestricted`` of ``u[p,r,q,s] = A[p,q] B[r,s]``: ``h + A tr(B rho_a) + A tr(B rho_b) - A rho_s B``,
+    the direct term from both densities' separate sums.  The absolute-value companion is the exact ``|terms|``."""
+    j = A * np.sum(B * rho_a.T) + A * np.sum(B * rho_b.T)
+    return np.stack([_sub(h + j, A @ r @ B, absolute) for r in (rho_a, rho_b)])
+
+
+def kron_fock_occupied(h, A, B, n_occ, dt, anti=False, absolute=False):
+    """``fock_occupied`` (general form) of ``u[a,b,c,d] = A[a,c] B[b,d]`` (minus ``A[a,d] B[b,c]``):
+    ``h + A sum_i B[i,i] (- sum_i A[p,i] B[i,q])`` over ``i < n_occ``.  The absolute-value companion is the exact
+    ``|terms|`` without ``anti`` and an upper bound of it with."""
+    o = slice(0, n_occ)
+    f = h + A * np.sum(np.diagonal(B)[o])
+    return _sub(f, A[:, o] @ B[o, :], absolute) if anti else f
+
+
 def fock_occupied(h, u, n_occ, spatial, dt, absolute=False):
     """``h + sum_i u[p,i,q,i]`` over ``i < n_occ``, or ``h + 2 sum_i u[p,i,q,i] - sum_i u[p,i,i,q]`` (spatial)."""
     i = np.arange(n_occ)
@@ -149,6 +191,13 @@ def spin_2_tb(S, dt, p=None, q=None, anti=False, absolute=False):
     return out
 
 
+def kron_occupied_traces(h, A, B, n_occ, dt, absolute=False):
+    """``occupied_traces`` of ``u[a,b,c,d] = A[a,c] B[b,d]``: ``u[i,j,i,j] = A[i,i] B[j,j]`` and
+    ``u[i,j,j,i] = A[i,j] B[j,i]``, summed as the ``n_occ²`` products of the dense form."""
+    o = np.arange(n_occ)
+    return np.array([h[o, o].sum(), np.sum(np.outer(A[o, o], B[o, o])), np.sum(A[:n_occ, :n_occ] * B[:n_occ, :n_occ].T)])
+
+
 def occupied_traces(h, u, n_occ, dt, absolute=False):
     """``(tr h[o,o], sum_ij u[i,j,i,j], sum_ij u[i,j,j,i])`` over ``i, j < n_occ``."""
     o = np.arange(n_occ)
@@ -157,6 +206,15 @@ def occupied_traces(h, u, n_occ, dt, absolute=False):
 
 
 # ------------------------------------------------------------------------------------------- reference and bound
+
+
+def chop(x, bits):
+    """``x`` rounded to ``bits`` mantissa bits (a kernel that computes in fewer bits than FP64)."""
+    def one(v):
+        m, e = np.frexp(v)
+        return np.ldexp(np.round(m * 2.0**bits) / 2.0**bits, e)
+
+    return one(x.real) + 1j * one(x.imag) if np.iscomplexobj(x) else one(x)
 
 
 def companions(fn, *arrays, **kw):
@@ -235,6 +293,11 @@ def k_diagonal(n, complex_, generated_w=False, anti=False):
 def graded(n, lo=-4.0):
     """``logspace(0, lo, n)``: orbital weights whose products keep a ``10^(4 lo)`` dynamic range in ``u``."""
     return np.logspace(0.0, lo, n)
+
+
+def pow2_graded(n):
+    """``graded(n)`` rounded to powers of two, so that dyadic values scaled by it stay exact in products."""
+    return 2.0 ** np.round(np.log2(graded(n)))
 
 
 def graded_two_body(rng, n, complex_=False, lo=-4.0):

@@ -11,6 +11,12 @@ to n = 48 (and for small ``n`` with large ``m``); above that ``u = A ⊗ B`` (``
 an O(n³)-per-plane reference, and whole planes are compared at the leading indices where the kernels switch: 0, the
 64 and 128 boundaries, n - 1 and two random ones.
 
+Past n = 128 the same exact inputs reach the schedules whose machinery is idle at small n: the sharded peer schedule
+and the sharded anti-symmetric pair schedule on emulated ranks (tests/sharded_bounds.py: whole planes plus a sweep of
+every element of every rank), the single-GPU symmetry-aware path, the mixed four-matrix transform and the consumers of
+a sharded tensor.  Their buffers, outputs and workspaces start as NaN, so an element that was never written or was
+computed from memory nobody wrote fails the check; each case asserts the property it is there for.
+
 The module prints, per kernel family, the largest criterion-A ratio (|error| / bound) and the largest ratio of the
 kernel's RMS error to plain numpy FP64's (criterion B), and its wall time (``pytest -s``)."""
 
@@ -29,7 +35,10 @@ import precise as P
 torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
+import sharded_bounds as SB  # noqa: E402  (needs torch)
+
 _STATS = collections.defaultdict(list)
+_SWEEP = collections.defaultdict(list)  # family -> largest |got - X̂ Ŷ| / bound of each whole-tensor sweep
 
 
 @pytest.fixture(scope="module", autouse=True)
@@ -40,7 +49,10 @@ def report():
     for family, rows in sorted(_STATS.items()):
         a = max(r["a"] for r in rows)
         b = max(r["rms"] / max(r["rms_fp64"], 1e-300) for r in rows)
-        lines.append(f"  {family:28s} {len(rows):3d} checks  max A ratio {a:.3g}  max RMS(GPU)/RMS(FP64) {b:.3g}")
+        lines.append(f"  {family:34s} {len(rows):3d} checks  max A ratio {a:.3g}  max RMS(GPU)/RMS(FP64) {b:.3g}")
+    for family, ratios in sorted(_SWEEP.items()):
+        lines.append(f"  {family + ' (sweep)':34s} {len(ratios):3d} tensors max |error| / bound {max(ratios):.3g}")
+    lines.append(f"  peak device memory {torch.cuda.max_memory_allocated() / 2**30:.1f} GiB")
     print("\n" + "\n".join(lines))
 
 
@@ -60,14 +72,34 @@ def rand(rng, shape, complex_=False):
     return rng.standard_normal(shape) + (1j * rng.standard_normal(shape) if complex_ else 0)
 
 
-def plane_indices(n, rng):
-    fixed = {i for i in (0, 63, 64, 127, 128, n - 1) if i < n}
-    return sorted(fixed | {int(i) for i in rng.integers(0, n, 2)})
+plane_indices = SB.plane_indices
 
 
-def pow2_graded(n):
-    """``graded(n)`` rounded to powers of two, so that dyadic values scaled by it stay exact in products."""
-    return 2.0 ** np.round(np.log2(P.graded(n)))
+class _PoisonedTorch:
+    """Stands in for ``torch`` inside ``ops``: every floating-point ``empty`` (outputs, workspaces) comes back filled
+    with NaN, 0xFF bytes for the byte workspaces (NaN doubles); everything else is torch itself."""
+
+    def __getattr__(self, name):
+        return getattr(torch, name)
+
+    @staticmethod
+    def empty(*args, **kwargs):
+        t = torch.empty(*args, **kwargs)
+        if t.dtype == torch.uint8:
+            t.fill_(0xFF)
+        elif t.is_floating_point() or t.is_complex():
+            t.fill_(float("nan") if not t.is_complex() else complex(float("nan"), float("nan")))
+        return t
+
+
+@pytest.fixture
+def poisoned_ops(monkeypatch):
+    """``ops`` with NaN-filled outputs and workspaces: an element that no kernel writes, or one computed from
+    workspace that nobody wrote, is non-finite."""
+    from quantum_systems_b200 import ops
+
+    monkeypatch.setattr(ops, "torch", _PoisonedTorch())
+    return ops
 
 
 # ------------------------------------------------------------------------------------------- four-index transform
@@ -142,18 +174,82 @@ def test_transform_large_k_planes(case):
     check_kron_planes("quarter GEMM (planes)", label, out, A, B, C, Ct, plane_indices(m, rng), False, u_c or c_c)
 
 
-@pytest.mark.parametrize("n", [128, 130])
-@pytest.mark.parametrize("kind", [1, 2], ids=["antisymmetric", "exchange"])
-def test_symmetry_aware_default_path(n, kind):
-    from quantum_systems_b200 import ops
+# (id, n, m, u complex, C complex, bi-orthogonal C~, kind): kind 1 anti-symmetric in the last pair, 2 particle-exchange
+# symmetric (B = A), 3 both (anti-symmetric with B = A: the library picks 1).  Complex dyadic products and their
+# differences are exact (<= 46 bits), so every symmetry holds exactly.
+SYMMETRY = [(f"{name}-{n}", n, n, False, False, False, kind) for name, kind in (("antisymmetric", 1), ("exchange", 2))
+            for n in (128, 130)] + [
+    ("both-144", 144, 144, False, False, False, 3),
+    ("antisymmetric-129-unpaired", 129, 129, False, False, False, 1),
+    ("exchange-144", 144, 144, False, False, False, 2),
+    ("antisymmetric-complex-biorth-129", 129, 129, True, True, True, 1),
+    ("exchange-complex-biorth-144", 144, 144, True, True, True, 2),
+    ("both-complex-130", 130, 130, True, True, False, 3),
+    ("antisymmetric-split-144", 144, 144, True, False, False, 1),
+    ("exchange-split-129", 129, 129, True, False, False, 2),
+    ("antisymmetric-real-u-complex-C-144", 144, 144, False, True, False, 1),
+    ("exchange-real-u-complex-C-129", 129, 129, False, True, False, 2),
+    ("antisymmetric-144-to-129", 144, 129, False, False, False, 1),
+    ("exchange-129-to-144", 129, 144, False, False, False, 2),
+]
 
-    anti = kind == ops.ANTISYMMETRIC_LAST_PAIR
-    rng, A, B, C, Ct, u = kron_case(n, False, False, anti=anti, same=not anti, seed=kind)
-    out = ops.transform_two_body(u, dev(C))
-    assert ops.proven_symmetry(out) == kind, "the symmetry-aware path did not run"
+
+@pytest.mark.parametrize("case", SYMMETRY, ids=[c[0] for c in SYMMETRY])
+def test_symmetry_aware_default_path(case, poisoned_ops):
+    """The single-GPU symmetry-aware transform (``two_body_steps`` with symmetry 1/2: masked step 2, packed pair
+    steps 3-4, mirror fill) with NaN-filled output and workspace."""
+    ops = poisoned_ops
+    label, n, m, u_c, c_c, biorth, kind = case
+    anti = kind != ops.PARTICLE_EXCHANGE
+    rng, A, B, C, Ct, u = kron_case(n, u_c, c_c, anti=anti, same=kind != ops.ANTISYMMETRIC_LAST_PAIR, m=m,
+                                    seed=kind)
+    if biorth:
+        Ct = rand(rng, (m, n), c_c)
+    if kind == 3:
+        assert ops.two_body_symmetry(u) == ops.ANTISYMMETRIC_LAST_PAIR | ops.PARTICLE_EXCHANGE
+    want = ops.ANTISYMMETRIC_LAST_PAIR if anti else ops.PARTICLE_EXCHANGE
+    out = ops.transform_two_body(u, dev(C), dev(Ct) if biorth else None)
+    assert ops.proven_symmetry(out) == want, "the symmetry-aware path did not run"
+    # step 2 skips tiles: column tiles r right of every s of a row tile (r < s, or r <= s)
+    t_dtype = torch.complex128 if (u_c or c_c) else torch.float64
+    c_dtype = torch.complex128 if c_c else torch.float64
+    X = m * n * n
+    kept = SB.planned_tiles(X, n, m, t_dtype, c_dtype, n, 1, int(anti), 1, 1, n * n, m)
+    assert kept < SB.planned_tiles(X, n, m, t_dtype, c_dtype, n), "the step-2 mask keeps every tile"
     del u
-    check_kron_planes("symmetry-aware transform", f"n={n} symmetry {kind}", out, A, B, C, Ct,
-                      plane_indices(n, rng), anti, False)
+    check_kron_planes("symmetry-aware transform", f"{label} symmetry {want}", out, A, B, C, Ct,
+                      plane_indices(m, rng), anti, u_c or c_c)
+
+
+# (label, n, m, u complex, C complex, explicit bras): four different matrices, so step 4 rebuilds its bra image in the
+# slot step 3 read.  A ⊗ B inputs, whole planes, K > 128.
+MIXED = [
+    ("n=129 real", 129, 129, False, False, False),
+    ("n=144 real explicit bras", 144, 144, False, False, True),
+    ("n=144 complex", 144, 144, True, True, False),
+    ("n=129 complex explicit bras", 129, 129, True, True, True),
+    ("n=144 split explicit bras", 144, 144, True, False, True),
+    ("n=129 real u complex C", 129, 129, False, True, False),
+    ("144 -> 130 rectangular", 144, 130, False, False, False),
+    ("144 -> 130 complex rectangular explicit bras", 144, 130, True, True, True),
+]
+
+
+@pytest.mark.parametrize("case", MIXED, ids=[c[0] for c in MIXED])
+def test_mixed_transform_large_k_planes(case, poisoned_ops):
+    ops = poisoned_ops
+    label, n, m, u_c, c_c, explicit = case
+    assert n > 128  # the K > 128 chunk loop
+    rng, A, B, C_r, _, u = kron_case(n, u_c, c_c, m=m, seed=7)
+    C_s = rand(rng, (n, m), c_c)
+    Ct_p = rand(rng, (m, n), c_c) if explicit else C_r.conj().T
+    Ct_q = rand(rng, (m, n), c_c) if explicit else C_s.conj().T
+    out = ops.transform_two_body_mixed(u, dev(C_r), dev(C_s), *((dev(Ct_p), dev(Ct_q)) if explicit else ()))
+    del u
+    planes = plane_indices(m, rng)
+    ref, absval, fp64 = P.companions(P.kron_transform_planes, A, B, C_r, Ct_p, C_s, Ct_q, planes=planes)
+    check("mixed transform (planes)", host(out[planes]), ref, absval, P.k_transform([n] * 4, [u_c or c_c] * 4), fp64,
+          f"{label}, planes {planes}")
 
 
 @functools.lru_cache(maxsize=None)
@@ -221,6 +317,147 @@ def test_one_body_and_functions(n, m, h_c, c_c, biorth):
         ref, absval, fp64 = P.companions(fn, spf, M)
         got = host(ops.transform_functions(dev(spf), dev(M), bra))
         check("transform_functions", got, ref, absval, P.k_transform([n], [h_c or c_c]), fp64, f"bra={bra}")
+
+
+# ---------------------------------------------------------------------------- sharded transform on emulated ranks
+# EmulatedContext(W) runs every rank's kernels on this GPU, with the same scattering stores as one process per GPU;
+# only the destination pointers differ.  The input is an exact A ⊗ B tensor built slab by slab, every buffer the
+# schedule allocates starts as NaN, and tests/sharded_bounds.py checks whole planes under criteria A and B and every
+# element of every rank under criterion A.
+
+
+@functools.lru_cache(maxsize=None)
+def nan_engine():
+    """``sharded.CudaEngine`` whose ``empty`` returns NaN-filled memory (NaN + NaN j), so that slabs, spare, recv,
+    per-rank scratch, padded copies and outputs are poisoned; it counts the device-side anti-symmetry tests."""
+    from quantum_systems_b200 import sharded
+
+    class NaNEngine(sharded.CudaEngine):
+        symmetry_tests = 0
+
+        def empty(self, numel, dtype):
+            buf = super().empty(numel, dtype)
+            buf.tensor.fill_(complex(float("nan"), float("nan")) if dtype == torch.complex128 else float("nan"))
+            return buf
+
+        def is_antisymmetric(self, buf, n, planes):
+            self.symmetry_tests += 1
+            return super().is_antisymmetric(buf, n, planes)
+
+    return NaNEngine
+
+
+# (label, n, m, W, u complex, C complex, bi-orthogonal C~, graded family, chain, what the case reaches)
+SHARDED_FULL = [
+    ("128 W=8", 128, 128, 8, False, False, False, False, False, {"even", "K=128"}),
+    ("129 W=2 odd pitch", 129, 129, 2, False, False, False, False, False, {"uneven", "odd pitch"}),
+    ("129 W=3 complex biorth", 129, 129, 3, True, True, True, False, False, {"even", "A=43"}),
+    ("144 W=5 split", 144, 144, 5, True, False, False, False, False, {"uneven"}),
+    ("144 W=8 real u complex C", 144, 144, 8, False, True, False, False, False, {"even", "A=18", "own output"}),
+    ("144 W=3 graded", 144, 144, 3, False, False, False, True, False, {"even"}),
+    ("130 -> 144 W=4", 130, 144, 4, False, False, False, False, False, {"uneven"}),
+    ("144 -> 129 W=3 complex biorth", 144, 129, 3, True, True, True, False, False, {"even"}),
+    ("144 -> 5 W=8", 144, 5, 8, False, False, False, False, False, {"idle ranks"}),
+    ("129 W=3 twice", 129, 129, 3, False, False, False, False, True, {"even", "recycled"}),
+]
+SHARDED_PAIRS = [
+    ("130 W=2 couples", 130, 130, 2, False, False, False, False, False, {"even", "couples"}),
+    ("129 W=3 unpaired", 129, 129, 3, False, False, False, False, False, {"even", "unpaired"}),
+    ("144 W=5 complex biorth", 144, 144, 5, True, True, True, False, False, {"uneven"}),
+    ("144 W=8 split", 144, 144, 8, True, False, False, False, False, {"even"}),
+    ("144 -> 131 W=3", 144, 131, 3, False, False, False, False, False, {"even", "unpaired"}),
+    ("144 W=4 graded", 144, 144, 4, False, False, False, True, False, {"even", "couples"}),
+    ("130 W=2 twice", 130, 130, 2, False, False, False, False, True, {"even", "couples", "recycled"}),
+]
+
+
+def exact_case(n, m, u_c, c_c, biorth, graded, seed):
+    """Dyadic ``A``, ``B`` (family a), or scaled by power-of-two ``g_a g_c`` with a near-identity ``C`` (family b)."""
+    rng = np.random.default_rng(seed)
+    A, B = P.dyadic(rng, (n, n), u_c), P.dyadic(rng, (n, n), u_c)
+    if graded:
+        g = np.outer(P.pow2_graded(n), P.pow2_graded(n))
+        A, B, C = A * g, B * g, P.near_identity(rng, n, m, c_c)
+    else:
+        C = rand(rng, (n, m), c_c)
+    Ct = rand(rng, (m, n), c_c) if biorth else C.conj().T
+    return rng, A, B, C, Ct
+
+
+def assert_reaches(reach, out, n, m, W, u_dtype, t_dtype):
+    """The property each case is there for, so that a change of defaults cannot turn it into a duplicate."""
+    from quantum_systems_b200 import ops, sharded
+
+    _, off = sharded.block_partition(n, W)
+    sizes = {b - a for a, b in zip(off, off[1:])}
+    if "even" in reach:
+        assert len(sizes) == 1, f"sources {sizes} are not even"
+    if "uneven" in reach:
+        assert len(sizes) > 1, "every source holds equally many planes"
+    for A in (43, 18):
+        if f"A={A}" in reach:
+            assert sharded.block_partition(n, W)[0] == A
+    if "K=128" in reach:
+        assert n == 128 and t_dtype == torch.float64
+    if "odd pitch" in reach:
+        assert sharded.padded_pitch(n, u_dtype) != n
+    if "own output" in reach:
+        assert u_dtype != t_dtype and out.spare is None, "the output is the input's spare"
+    if "idle ranks" in reach:
+        assert m < W and any(out.planes(r)[0] == out.planes(r)[1] for r in range(W))
+    if "couples" in reach:
+        assert t_dtype == torch.float64 and m % 2 == 0
+    if "unpaired" in reach:
+        assert t_dtype == torch.float64 and m % 2 == 1
+    if W > 1 and m >= 16:
+        assert ops.scatter_deal(m) > 1, "step 4 deals no columns"
+    assert n > 128 or "K=128" in reach
+
+
+def run_sharded_case(case, pairs):
+    from quantum_systems_b200 import sharded
+
+    label, n, m, W, u_c, c_c, biorth, graded, chain, reach = case
+    family = "sharded pair schedule" if pairs else "sharded full steps"
+    rng, A, B, C, Ct = exact_case(n, m, u_c, c_c, biorth, graded, seed=n * 10 + W)
+    u_dtype = torch.complex128 if u_c else torch.float64
+    t_dtype = torch.complex128 if (u_c or c_c) else torch.float64
+    engine = nan_engine()()
+    ctx = sharded.EmulatedContext(W, engine=engine)
+    u = SB.exact_sharded(ctx, A, B, pairs, u_dtype, "cuda")
+    symmetry = None if pairs else 0
+    out = sharded.transform_two_body_sharded(u, dev(C), dev(Ct) if biorth else None, symmetry=symmetry)
+    assert out.proven_antisymmetric == pairs, "the case did not take the schedule it is there for"
+    if pairs:
+        assert engine.symmetry_tests > 0, "the anti-symmetry of the input was not tested on the device"
+        kept = SB.pair_step2_tiles(ctx, n, m, t_dtype, torch.complex128 if c_c else torch.float64)
+        assert any(k < planned for k, planned in kept), f"step 2 skipped no tile: {kept}"
+    assert_reaches(reach, out, n, m, W, u_dtype, t_dtype)
+    arrays, factors = (A, B, C, Ct), P.kron_factors
+    k = P.k_transform([n] * 4, [u_c or c_c] * 4)
+    if chain:
+        C2 = rand(rng, (m, m), c_c)
+        tests = engine.symmetry_tests
+        out = sharded.transform_two_body_sharded(out, dev(C2), symmetry=symmetry)
+        with pytest.raises(RuntimeError, match="recycled"):
+            u.buffers  # the second result went into the first input's buffers (ping-pong)
+        if pairs:
+            assert out.proven_antisymmetric and engine.symmetry_tests == tests, "the proof was not trusted"
+        arrays, factors = (A, B, C, Ct, C2, C2.conj().T), SB.chain_factors
+        k = P.k_transform([n] * 8, [u_c or c_c] * 8)
+    del u
+    ratio = SB.check_sharded(functools.partial(check, family), out, factors, arrays, k, pairs, rng, label)
+    _SWEEP[family].append(ratio)
+
+
+@pytest.mark.parametrize("case", SHARDED_FULL, ids=[c[0] for c in SHARDED_FULL])
+def test_sharded_full_steps(case):
+    run_sharded_case(case, pairs=False)
+
+
+@pytest.mark.parametrize("case", SHARDED_PAIRS, ids=[c[0] for c in SHARDED_PAIRS])
+def test_sharded_pair_schedule(case):
+    run_sharded_case(case, pairs=True)
 
 
 # ------------------------------------------------------------------------------------------ structured transforms
@@ -329,7 +566,7 @@ def test_fock_density_kron(n, u_c, rho_c, h_c):
     from quantum_systems_b200 import ops
 
     rng = np.random.default_rng(n)
-    g = pow2_graded(n)
+    g = P.pow2_graded(n)
     A = P.dyadic(rng, (n, n), u_c) * np.outer(g, g)
     B = P.dyadic(rng, (n, n), u_c) * np.outer(g, g)
     rho, h = graded_density(rng, n, rho_c), rand(rng, (n, n), h_c) * 1e-6
@@ -372,6 +609,50 @@ def test_fock_density_unrestricted(n, u_c, rho_c):
     ref, absval, fp64 = P.companions(P.fock_unrestricted, h, u, ra, rb)
     got = np.stack([host(f) for f in ops.fock_from_density_unrestricted(dev(h), dev(u), dev(ra), dev(rb))])
     check("fock_from_density_unrestricted", got, ref, absval, k_density(n, u_c, rho_c, 3), fp64, f"n={n}")
+
+
+# (n, W, complex): consumers of a sharded tensor at n > 128, each rank reading its own planes
+CONSUMERS = [(129, 3, False), (129, 5, True), (144, 3, True), (144, 5, False)]
+
+
+@pytest.mark.parametrize("n,W,cplx", CONSUMERS, ids=[f"n={n} W={W} {'complex' if c else 'real'}" for n, W, c in CONSUMERS])
+def test_sharded_consumers(n, W, cplx):
+    from quantum_systems_b200 import sharded
+
+    rng, A, B, _, _ = exact_case(n, n, cplx, False, False, True, seed=n + W)
+    dtype = torch.complex128 if cplx else torch.float64
+    ctx = sharded.EmulatedContext(W, engine=nan_engine()())
+    h = rand(rng, (n, n), cplx) * 1e-6
+    hd = dev(h)
+    _, off = sharded.block_partition(n, W)
+    assert off[1] < n - 1
+    for anti in (False, True):
+        u = SB.exact_sharded(ctx, A, B, anti, dtype, "cuda")
+        basis = sharded.ShardedBasisSet(ctx, n, hd, None, u)
+        for n_occ in (1, 33, off[1] - 1, off[1] + 1, n):
+            f = torch.full((n, n), float("nan"), dtype=dtype, device="cuda")
+            got = host(basis.construct_fock_matrix(hd, u, n_occ, f=f))  # qs_fock_general on rows p0..p1 per rank
+            ref, absval, fp64 = P.companions(P.kron_fock_occupied, h, A, B, n_occ=n_occ, anti=anti)
+            check("sharded consumers", got, ref, absval, n_occ + 1, fp64, f"construct_fock_matrix n_occ={n_occ}")
+        if anti:
+            break
+        for n_occ in (1, off[1] + 1, n):
+            traces = np.array(u.occupied_traces(hd, n_occ))
+            ref, absval, fp64 = P.companions(P.kron_occupied_traces, h, A, B, n_occ=n_occ)
+            check("sharded consumers", traces if cplx else traces.real, ref, absval, n_occ * n_occ, fp64,
+                  f"occupied_traces n_occ={n_occ}")
+            tr_h, direct, exchange = u.occupied_traces(hd, n_occ)
+            energy = 2 * tr_h + 2 * direct - exchange
+            assert basis.compute_reference_energy(n_occ) == (energy if cplx else energy.real)
+        rho, rho_b = graded_density(rng, n, cplx), graded_density(rng, n, cplx, scale=1e-6)
+        got = host(basis.fock_from_density(hd, dev(rho), 1.0, -0.5))
+        ref, absval, fp64 = P.companions(P.kron_fock_density, h, A, B, rho, a_d=1.0, a_x=-0.5)
+        check("sharded consumers", got, ref, absval, k_density(n, cplx, cplx, 2), fp64, "fock_from_density")
+        got = np.stack([host(f) for f in basis.fock_from_density_unrestricted(hd, dev(rho), dev(rho_b))])
+        ref, absval, fp64 = P.companions(P.kron_fock_unrestricted, h, A, B, rho, rho_b)
+        check("sharded consumers", got, ref, absval, k_density(n, cplx, cplx, 3), fp64,
+              "fock_from_density_unrestricted")
+        del u, basis
 
 
 # ---------------------------------------------------------------------------------------------- S² and the traces

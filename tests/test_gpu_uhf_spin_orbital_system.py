@@ -28,15 +28,6 @@ def rand(rng, shape, complex_=False):
 # ------------------------------------------------------------------------------------ four-coefficient transform
 
 
-def mixed_steps(u, C_r, C_s, Ct_p, Ct_q, dt, absolute=False):
-    """The kernels' order with one matrix per step: s with ``C_s``, r with ``C_r``, q with ``Ct_qᵀ``, p with
-    ``Ct_pᵀ``, the new index first every time."""
-    t = u
-    for M in (C_s, C_r, Ct_q.T, Ct_p.T):
-        t = np.ascontiguousarray(np.moveaxis(np.tensordot(t, M, ([3], [0])), 3, 0))
-    return t
-
-
 # (label, n, m, u complex, C complex, explicit bras)
 MIXED = [
     ("real odd pitch", 13, 13, False, False, False),
@@ -60,7 +51,7 @@ def test_mixed_transform_rounding_bound(case):
     C_r, C_s = rand(rng, (n, m), c_c), rand(rng, (n, m), c_c)
     Ct_p = rand(rng, (m, n), c_c) if explicit else C_r.conj().T
     Ct_q = rand(rng, (m, n), c_c) if explicit else C_s.conj().T
-    ref, absval, fp64 = P.companions(mixed_steps, u, C_r, C_s, Ct_p, Ct_q)
+    ref, absval, fp64 = P.companions(P.mixed_steps, u, C_r, C_s, Ct_p, Ct_q)
     got = ops.transform_two_body_mixed(dev(u), dev(C_r), dev(C_s), *((dev(Ct_p), dev(Ct_q)) if explicit else ()))
     assert got.dtype == (torch.complex128 if (u_c or c_c) else torch.float64)
     P.assert_rounding_bound(host(got), ref, absval, P.k_transform([n] * 4, [u_c or c_c] * 4), fp64, label)

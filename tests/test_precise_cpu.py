@@ -88,10 +88,65 @@ def test_kron_forms_match_the_dense_contractions():
     h, rho = rng.standard_normal((n, n)), rng.standard_normal((n, n))
     A = P.dyadic(rng, (n, n))
     u = np.einsum("pq,rs->prqs", A, B)
+    n_occ = 3
+    for anti in (False, True):
+        dense, dense_abs, _ = P.companions(P.fock_occupied, h, P.kron_two_body(A, B, anti), n_occ=n_occ, spatial=False)
+        ref, absval, _ = P.companions(P.kron_fock_occupied, h, A, B, n_occ=n_occ, anti=anti)
+        assert np.max(np.abs(ref - dense)) <= 1e-17 * np.max(dense_abs)
+        assert np.all(absval >= dense_abs * (1 - 1e-12))
+    dense, dense_abs, _ = P.companions(P.occupied_traces, h, P.kron_two_body(A, B), n_occ=n_occ)
+    ref, absval, _ = P.companions(P.kron_occupied_traces, h, A, B, n_occ=n_occ)
+    assert np.max(np.abs(ref - dense)) <= 1e-17 * np.max(dense_abs)
+    np.testing.assert_allclose(absval, dense_abs, rtol=1e-13)
+    rb = rng.standard_normal((n, n))
+    dense, dense_abs, _ = P.companions(P.fock_unrestricted, h, u, rho, rb)
+    ref, absval, _ = P.companions(P.kron_fock_unrestricted, h, A, B, rho, rb)
+    assert np.max(np.abs(ref - dense)) <= 1e-17 * np.max(dense_abs)
+    np.testing.assert_allclose(absval, dense_abs, rtol=1e-13)
     dense, dense_abs, _ = P.companions(P.fock_density, h, u, rho, a_d=1.0, a_x=-0.5)
     ref, absval, _ = P.companions(P.kron_fock_density, h, A, B, rho, a_d=1.0, a_x=-0.5)
     assert np.max(np.abs(ref - dense)) <= 1e-17 * np.max(dense_abs)
     np.testing.assert_allclose(absval, dense_abs, rtol=1e-13)
+
+
+def test_kron_forms_with_one_matrix_per_index_and_chained_match_the_dense_contractions():
+    from sharded_bounds import chain_factors, kron_planes_of
+
+    rng = np.random.default_rng(6)
+    n, m = 5, 4
+    A, B = P.dyadic(rng, (n, n), True), P.dyadic(rng, (n, n))
+    C_r, C_s = rng.standard_normal((n, m)), rng.standard_normal((n, m)) + 1j * rng.standard_normal((n, m))
+    Ct_p, Ct_q = rng.standard_normal((m, n)) + 1j * rng.standard_normal((m, n)), rng.standard_normal((m, n))
+    planes = [0, m - 1]
+    for anti in (False, True):
+        dense, dense_abs, _ = P.companions(P.mixed_steps, P.kron_two_body(A, B, anti), C_r, C_s, Ct_p, Ct_q)
+        ref, absval, _ = P.companions(P.kron_transform_planes, A, B, C_r, Ct_p, C_s, Ct_q, planes=planes, anti=anti)
+        assert np.max(np.abs(ref - dense[planes])) <= 1e-17 * np.max(dense_abs)
+        if anti:
+            assert np.all(absval >= dense_abs[planes] * (1 - 1e-12))
+        else:
+            np.testing.assert_allclose(absval, dense_abs[planes], rtol=1e-13)
+    # with the defaults it is the one-matrix form
+    one = P.companions(P.kron_transform_planes, A, B, C_r, Ct_p, planes=planes, anti=True)
+    both = P.companions(P.kron_transform_planes, A, B, C_r, Ct_p, C_r, Ct_p, planes=planes, anti=True)
+    for x, y in zip(one, both):
+        np.testing.assert_array_equal(x, y)
+    # two transforms in a row: the eight-step composite, its absolute-value companion built from |C1| and |C2|
+    C1, Ct1 = rng.standard_normal((n, n)), rng.standard_normal((n, n))
+    C2 = rng.standard_normal((n, m)) + 1j * rng.standard_normal((n, m))
+    Ct2 = C2.conj().T
+
+    def eight_steps(u, C1, Ct1, C2, Ct2, dt, absolute=False):
+        return P.quarter_steps(P.quarter_steps(u, C1, Ct1, dt), C2, Ct2, dt)
+
+    for anti in (False, True):
+        dense, dense_abs, _ = P.companions(eight_steps, P.kron_two_body(A, B, anti), C1, Ct1, C2, Ct2)
+        ref, absval, _ = P.companions(kron_planes_of(chain_factors), A, B, C1, Ct1, C2, Ct2, planes=planes, anti=anti)
+        assert np.max(np.abs(ref - dense[planes])) <= 1e-16 * np.max(dense_abs)
+        if anti:
+            assert np.all(absval >= dense_abs[planes] * (1 - 1e-12))
+        else:
+            np.testing.assert_allclose(absval, dense_abs[planes], rtol=1e-13)
 
 
 # ------------------------------------------------------------------ a correct FP64 evaluation passes on every family
@@ -167,15 +222,6 @@ def test_fp64_passes_the_round_trip_and_the_other_families():
 # ------------------------------------------------------------------------------------------- mutants are rejected
 
 
-def chop(x, bits):
-    """``x`` rounded to ``bits`` mantissa bits (a kernel that computes in fewer bits than FP64)."""
-    def one(v):
-        m, e = np.frexp(v)
-        return np.ldexp(np.round(m * 2.0**bits) / 2.0**bits, e)
-
-    return one(x.real) + 1j * one(x.imag) if np.iscomplexobj(x) else one(x)
-
-
 def steps_dropping_last_chunk(u, C, Ct, rows=128, chunk=16):
     """FP64 quarter steps in which step 1 skips the last k-chunk of the first row tile (a stale or skipped stage)."""
     n = u.shape[0]
@@ -203,7 +249,7 @@ def test_mutants_fail_the_check_and_the_first_two_pass_the_scaled_one():
     want = np.asarray(ref, dtype=np.float64)
 
     # 1. operands rounded to 46-bit mantissas
-    m46 = P.quarter_steps(chop(u, 46), chop(C, 46), chop(C.T, 46), np.float64)
+    m46 = P.quarter_steps(P.chop(u, 46), P.chop(C, 46), P.chop(C.T, 46), np.float64)
     assert_close_scaled(m46, want)
     rejected(m46, ref, absval, k, fp64)
     # 2. one input term dropped

@@ -299,3 +299,118 @@ def test_collective_schedule_world2_gloo(n, m, complex_):
     results = manager.dict()
     mp.spawn(_gloo_worker, args=(world, port, n, m, complex_, results), nprocs=world, join=True)
     assert dict(results) == {0: "ok", 1: "ok"}
+
+
+# ------------------------------------------------------- the rounding-bound check of the sharded schedule, on the host
+# tests/sharded_bounds.py holds the sharded transform of an exact A ⊗ B tensor to the rounding-error bound on whole
+# planes and on every element (tests/test_gpu_rounding_bounds.py runs it on the device).  Here it runs unchanged on
+# the numpy engine, whose buffers start as NaN: a correct schedule passes, and three broken engines fail it.
+
+
+class DroppedPairTile(NumpyEngine):
+    """Step 2 of the anti-symmetric pair schedule leaves out one of the tiles its planner keeps."""
+
+    @staticmethod
+    def _pair_tiles(*args):
+        tiles = NumpyEngine._pair_tiles(*args)
+        return np.delete(tiles, len(tiles) // 2, axis=0)
+
+
+class SwappedDealtColumns(NumpyEngine):
+    """The dealt store of step 4 (deal > 1) exchanges two output columns."""
+
+    def quarter_scatter(self, A, X, K, lda, image, m_dtype, W, dests, *args, deal=1, cyclic=False):
+        if deal > 1:
+            image = image.copy()
+            image[:, [0, 1]] = image[:, [1, 0]]
+        super().quarter_scatter(A, X, K, lda, image, m_dtype, W, dests, *args, deal=deal, cyclic=cyclic)
+
+
+class Step1In46Bits(NumpyEngine):
+    """Step 1 rounds its operands to 46-bit mantissas (with every source holding equally many planes, step 1 is the
+    only plain ``quarter`` launch of the peer schedule)."""
+
+    def quarter(self, A, X, K, lda, image, *args):
+        import precise as P
+        from _numpy_engine import HostBuffer
+
+        chopped = HostBuffer(torch.from_numpy(P.chop(A.flat()[: X * lda], 46)))
+        super().quarter(chopped, X, K, lda, P.chop(image, 46), *args)
+
+
+def graded_kron_case(n, seed):
+    """Graded family on an exact tensor: dyadic ``A``, ``B`` scaled by power-of-two ``g_a g_c`` and a near-identity
+    ``C``, so that the result spans 16 decades and small elements carry the rounding of every step."""
+    import precise as P
+
+    rng = np.random.default_rng(seed)
+    g = P.pow2_graded(n)
+    A, B = (P.dyadic(rng, (n, n)) * np.outer(g, g) for _ in range(2))
+    C = P.near_identity(rng, n)
+    return rng, A, B, C
+
+
+def run_sharded_bound(engine, n, anti, world=3):
+    """The sharded transform of the graded exact tensor through ``engine``, checked by tests/sharded_bounds.py.
+    Returns the result and its reference arrays."""
+    import precise as P
+    import sharded_bounds as SB
+    from quantum_systems_b200 import sharded
+
+    rng, A, B, C = graded_kron_case(n, seed=n + anti)
+    ctx = sharded.EmulatedContext(world, engine=engine)
+    u = SB.exact_sharded(ctx, A, B, anti, torch.float64, "cpu")
+    out = sharded.transform_two_body_sharded(u, torch.from_numpy(C))
+    assert out.proven_antisymmetric == anti, "the case did not take the schedule it is there for"
+    SB.check_sharded(P.assert_rounding_bound, out, P.kron_factors, (A, B, C, C.T), P.k_transform([n] * 4, [False] * 4),
+                     anti, rng, f"n={n} W={world} anti={anti}")
+    return out, (A, B, C, C.T)
+
+
+@pytest.fixture
+def pair_schedule_below_48(monkeypatch):
+    from quantum_systems_b200 import sharded
+    from quantum_systems_b200.build import build
+
+    build()  # the numpy pair step asks the library's planner for its tiles
+    monkeypatch.setattr(sharded, "SYMMETRY_MIN_N", 4)
+
+
+# n = 21 over 3 ranks: equal sources (7 planes each), an odd real pitch and 21 >= 16 dealt columns in step 4.
+# n = 20 anti-symmetric: uneven sources (7, 7, 6, per-source pair tables) and pair lists padded to couples.
+@pytest.mark.parametrize("n,anti", [(21, False), (20, True)], ids=["full steps", "pair schedule"])
+def test_sharded_bound_harness_passes_the_numpy_schedule(n, anti, pair_schedule_below_48):
+    from quantum_systems_b200 import sharded
+
+    assert np.isnan(NumpyEngine().empty(4, torch.float64).flat()).all(), "the stand-in's buffers must start as NaN"
+    _, off = sharded.block_partition(n, 3)
+    assert len({b - a for a, b in zip(off, off[1:])}) == (2 if anti else 1)
+    assert NumpyEngine().scatter_deal(n) > 1
+    run_sharded_bound(NumpyEngine(), n, anti)
+
+
+def test_sharded_bound_harness_rejects_a_dropped_pair_tile(pair_schedule_below_48):
+    with pytest.raises(AssertionError, match="non-finite|sweep"):
+        run_sharded_bound(DroppedPairTile(), 20, True)
+
+
+def test_sharded_bound_harness_rejects_swapped_dealt_columns(pair_schedule_below_48):
+    with pytest.raises(AssertionError, match="criterion"):
+        run_sharded_bound(SwappedDealtColumns(), 21, False)
+
+
+def test_sharded_bound_harness_rejects_a_46_bit_step_the_scaled_check_accepts(pair_schedule_below_48):
+    import precise as P
+    from conftest import assert_close_scaled
+
+    with pytest.raises(AssertionError, match="criterion B"):
+        run_sharded_bound(Step1In46Bits(), 21, False)
+    # the same mutant, end to end, is well inside the 1e-12 max-scaled tolerance
+    from quantum_systems_b200 import sharded
+    import sharded_bounds as SB
+
+    _, A, B, C = graded_kron_case(21, seed=21)
+    ctx = sharded.EmulatedContext(3, engine=Step1In46Bits())
+    out = sharded.transform_two_body_sharded(SB.exact_sharded(ctx, A, B, False, torch.float64, "cpu"),
+                                             torch.from_numpy(C))
+    assert_close_scaled(out.gather().numpy(), P.kron_transform_planes(A, B, C, C.T, planes=range(21), dt=np.float64))
