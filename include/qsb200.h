@@ -158,6 +158,20 @@ int qs_quarter_transform_scatter_pairs(const void* A, int a_dtype, int64_t X, in
                                        int64_t rows_per_s, int padded, void* list_ws, int64_t list_ws_bytes,
                                        void* stream);
 
+/* The scattering store with COLUMN TABLES: the physical column w (after dealing) goes to the destination
+ * host_out_table[col_dest[w]] (< n_dest <= 16) at element offset col_off[w] inside it; rows are placed as in
+ * qs_quarter_transform_scatter (x_inner, x_mid, sx0, sx1, sx2).  col_dest (int32) and col_off (int64) hold W entries
+ * each in device memory.  Unlike the blocks of w_inner columns, the tables give every destination any set of
+ * columns: the spin-orbital planes of an unrestricted basis, whose owners hold uneven -- possibly empty -- orbital
+ * ranges per spin.  `offsets_even` != 0 is the caller's promise that every col_off entry is even (real output then
+ * leaves in 16-byte row pairs when the row strides allow it).  Always the register-store epilogue. */
+int qs_quarter_transform_scatter_columns(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda,
+                                         const void* image, int m_dtype, int64_t W,
+                                         void* const* host_out_table, int64_t n_dest, const int32_t* col_dest,
+                                         const int64_t* col_off, int offsets_even, int64_t x_inner,
+                                         int64_t x_mid, int64_t sx0, int64_t sx1, int64_t sx2, int64_t w_deal,
+                                         void* stream);
+
 /* Epilogue of the quarter GEMM.  Besides storing from registers, a launch can stage each warp's accumulator tile
  * in shared memory ([column][row], 16 real columns at a time, two 4 KiB buffers per warp) and hand every run of rows
  * that is contiguous in the output to the copy engine (cp.async.bulk shared -> global, SASS UBLKCP.G.S), going on

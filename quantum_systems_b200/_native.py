@@ -36,6 +36,7 @@ SIGNATURES = {
     "qs_build_coeff_image_dealt": [_ptr, _int, _i64, _i64, _int, _i64, _i64, _int, _i64, _ptr, _ptr],
     "qs_quarter_transform_scatter": [_ptr, _int, _i64, _i64, _i64, _ptr, _int, _i64, ctypes.POINTER(_ptr), _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _int, _ptr],
     "qs_quarter_transform_scatter_pairs": [_ptr, _int, _i64, _i64, _i64, _ptr, _int, _i64, ctypes.POINTER(_ptr), _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _int, _ptr, _i64, _ptr],
+    "qs_quarter_transform_scatter_columns": [_ptr, _int, _i64, _i64, _i64, _ptr, _int, _i64, ctypes.POINTER(_ptr), _i64, _ptr, _ptr, _int, _i64, _i64, _i64, _i64, _i64, _i64, _ptr],
     "qs_transform_two_body_diagonal_workspace_bytes": [_i64, _i64, _int, _int, _int, ctypes.POINTER(_i64)],
     "qs_transform_two_body_diagonal": [_ptr, _int, _ptr, _ptr, _int, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr],
     "qs_is_antisymmetric_last_pair": [_ptr, _int, _i64, _i64, ctypes.POINTER(_int), _ptr, _ptr],

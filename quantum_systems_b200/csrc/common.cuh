@@ -109,6 +109,11 @@ struct QsQuarterStore {
     const long long* xr_table = nullptr;
     int xq_even = 0;                      // promise: every kept xq_table entry is even
     int xr_paired = 0;                    // promise: xr_table places rows 2k, 2k + 1 adjacently at an even offset
+    // Column tables (device memory, W entries each, indexed by the physical column): column w goes to destination
+    // out_table[col_dest[w]] at element offset col_off[w], in place of the w / w_inner, w_cyclic and sw0 rules.
+    const int32_t* col_dest = nullptr;
+    const long long* col_off = nullptr;
+    int col_off_even = 0;                 // promise: every col_off entry is even
     // Masked launch: only the tiles the mask, or the host copy of the block table, wants.  list_ws holds
     // qs_tile_list_bytes() bytes of device memory.
     const QsTileMask* mask = nullptr;

@@ -92,6 +92,10 @@ struct QuarterParams {
     // xr_table[xr] instead of xr * sx0.  Element offsets.
     const long long* xq_table;
     const long long* xr_table;
+    // Column tables (kernels instantiated with COLS only): physical column w goes to outs[col_dest[w]] at element
+    // offset col_off[w] -- uneven, caller-defined column ranges per destination.  Rows are placed as above.
+    const int* col_dest;
+    const long long* col_off;
 };
 
 __device__ __forceinline__ uint32_t dealt_column(uint32_t w, uint32_t mul, uint32_t mod) {
@@ -101,10 +105,12 @@ __device__ __forceinline__ uint32_t dealt_column(uint32_t w, uint32_t mul, uint3
 // Store addressing of the strided, staged and split epilogues (the rotated one has its own, see quarter_gemm_kernel).
 // Base of output column wl (before dealing) for output elements of ES bytes: the dealt column w goes to destination
 // w % ndest as its column w / ndest (cyclic) or to block w / w_inner as its column w % w_inner.  `plain`
-// (w_inner == 1 and no destination table, evaluated once per tile) stores column w at w * sw1.
-template <int ES>
+// (w_inner == 1 and no destination table, evaluated once per tile) stores column w at w * sw1.  COLS: the column
+// tables place the dealt column instead.
+template <int ES, bool COLS = false>
 __device__ __forceinline__ double* column_base(const QuarterParams& p, bool plain, uint32_t wl) {
     const uint32_t w = dealt_column(wl, p.deal_mul, p.deal_mod);
+    if constexpr (COLS) return p.outs[p.col_dest[w]] + (ES / 8) * p.col_off[w];
     if (plain) return p.out + (ES / 8) * ((long long)w * p.sw1);
     const uint32_t wq = p.w_cyclic ? w % (uint32_t)p.ndest : w / p.w_inner;
     const uint32_t wr = p.w_cyclic ? w / (uint32_t)p.ndest : w - wq * p.w_inner;
@@ -288,7 +294,9 @@ __device__ __forceinline__ bool cta_frame(const CUtensorMap& map_a, const Quarte
 // Cross-tile pipelining: after its main loop a warp waits for the first chunk of its NEXT tile and loads that chunk's
 // first A and B fragments (registers that are dead in the epilogue) before it stores the current tile, so its DMMA
 // stream restarts right behind the stores.
-enum Epilogue { kEpiStrided = 0, kEpiBulk = 1, kEpiRotated = 2 };
+// COLUMNS: the strided register epilogue with the column tables (col_dest, col_off) choosing each column's
+// destination and offset; a kernel of its own, so the other epilogues keep no table branch.
+enum Epilogue { kEpiStrided = 0, kEpiBulk = 1, kEpiRotated = 2, kEpiColumns = 3 };
 
 template <int NT, bool COMPLEX_OUT, int EPI>
 __global__ void __launch_bounds__(kThreads, 1)
@@ -590,7 +598,7 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             const uint32_t wp = wbase + 8 * nt + 2 * t;  // real column of acc[..][nt][0]; wp + 1 for [1]
             if (COMPLEX_OUT) {
                 if (wp < p.Wp) {
-                    double* col = column_base<16>(p, plain_w, wp >> 1);
+                    double* col = column_base<16, EPI == kEpiColumns>(p, plain_w, wp >> 1);
 #pragma unroll
                     for (int mt = 0; mt < 4; ++mt)
                         if (xok[mt])
@@ -600,7 +608,7 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 #pragma unroll
                 for (int e = 0; e < 2; ++e) {
                     if (wp + e < p.Wp) {
-                        double* col = column_base<8>(p, plain_w, wp + e);
+                        double* col = column_base<8, EPI == kEpiColumns>(p, plain_w, wp + e);
                         if (p.vec2) {
                             // rows (mt = 0, 1) and (mt = 2, 3) are adjacent and 16-byte aligned in the output
                             if (xok[0]) *reinterpret_cast<double2*>(col + xoff[0]) = make_double2(acc[0][nt][e], acc[1][nt][e]);
@@ -638,7 +646,7 @@ quarter_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 template <int NTC>
 using SplitRing = RingConfig<NTC * 512>;  // B tile: 8 complex k x 8*NTC columns, one double each
 
-template <int NTC>
+template <int NTC, bool COLS = false>
 __global__ void __launch_bounds__(kThreads, 1)
 quarter_gemm_split_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ QuarterParams p) {
     using Ring = SplitRing<NTC>;
@@ -765,7 +773,7 @@ quarter_gemm_split_kernel(const __grid_constant__ CUtensorMap map_a, const __gri
             for (int e = 0; e < 2; ++e) {
                 const uint32_t wl = wbase + 8 * ntc + 2 * t + e;
                 if (wl >= p.Wp) continue;  // Wp = number of complex columns in this mode
-                double* col = column_base<16>(p, plain_w, wl);
+                double* col = column_base<16, COLS>(p, plain_w, wl);
 #pragma unroll
                 for (int mt = 0; mt < 4; ++mt)
                     if (xok[mt])
@@ -977,6 +985,7 @@ int launch_epilogue(int epi, int NT, const CUtensorMap& map, const QuarterParams
     switch (epi) {
         case kEpiStrided: return launch_nt<CO, kEpiStrided>(NT, map, p, st);
         case kEpiBulk: return launch_nt<CO, kEpiBulk>(NT, map, p, st);
+        case kEpiColumns: return launch_nt<CO, kEpiColumns>(NT, map, p, st);
         default: return launch_nt<CO, kEpiRotated>(NT, map, p, st);
     }
 }
@@ -989,15 +998,20 @@ Divisor make_divisor(uint64_t d) {
     return {(uint32_t)(((1ull << shift) + d - 1) / d), shift};
 }
 
-int launch_split(int NTC, const CUtensorMap& map, const QuarterParams& p, cudaStream_t st) {
+template <bool COLS>
+int launch_split_ntc(int NTC, const CUtensorMap& map, const QuarterParams& p, cudaStream_t st) {
     switch (NTC) {
-        case 1: return launch_variant<quarter_gemm_split_kernel<1>, SplitRing<1>::kSmemBytes>(map, p, st);
-        case 2: return launch_variant<quarter_gemm_split_kernel<2>, SplitRing<2>::kSmemBytes>(map, p, st);
-        case 3: return launch_variant<quarter_gemm_split_kernel<3>, SplitRing<3>::kSmemBytes>(map, p, st);
-        case 4: return launch_variant<quarter_gemm_split_kernel<4>, SplitRing<4>::kSmemBytes>(map, p, st);
+        case 1: return launch_variant<quarter_gemm_split_kernel<1, COLS>, SplitRing<1>::kSmemBytes>(map, p, st);
+        case 2: return launch_variant<quarter_gemm_split_kernel<2, COLS>, SplitRing<2>::kSmemBytes>(map, p, st);
+        case 3: return launch_variant<quarter_gemm_split_kernel<3, COLS>, SplitRing<3>::kSmemBytes>(map, p, st);
+        case 4: return launch_variant<quarter_gemm_split_kernel<4, COLS>, SplitRing<4>::kSmemBytes>(map, p, st);
     }
     qs_set_error("internal: NTC=%d out of range", NTC);
     return QS_ERR_INVALID;
+}
+
+int launch_split(bool cols, int NTC, const CUtensorMap& map, const QuarterParams& p, cudaStream_t st) {
+    return cols ? launch_split_ntc<true>(NTC, map, p, st) : launch_split_ntc<false>(NTC, map, p, st);
 }
 
 int build_image(ImageParams q, const Tiling& tl, void* image, void* stream) {
@@ -1289,10 +1303,14 @@ int qs_quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t 
                "qs_quarter_transform: bad inner extents");
     const int64_t n_dest = s.n_dest;
     QS_REQUIRE(n_dest >= 0 && n_dest <= kMaxDest, "qs_quarter_transform_scatter: at most %d destinations", kMaxDest);
-    QS_REQUIRE(n_dest == 0 || s.w_cyclic || qs_ceil_div(W, s.w_inner) <= n_dest,
+    const bool columns = s.col_off != nullptr;
+    QS_REQUIRE(n_dest == 0 || s.w_cyclic || columns || qs_ceil_div(W, s.w_inner) <= n_dest,
                "qs_quarter_transform_scatter: W=%lld needs more than %lld destinations of %lld", (long long)W,
                (long long)n_dest, (long long)s.w_inner);
     QS_REQUIRE(!s.w_cyclic || n_dest > 0, "qs_quarter_transform_scatter: cyclic columns need a destination table");
+    QS_REQUIRE(!columns || (s.col_dest && n_dest > 0 && !s.w_cyclic && !s.xq_table && !s.xr_table && !s.mask &&
+                            !s.host_xq_table),
+               "qs_quarter_transform_scatter_columns: column tables need a destination table and no row tables");
     const Tiling tl = make_tiling(K, W, a_dtype, m_dtype);
     const bool out_complex = a_dtype == QS_C128 || m_dtype == QS_C128;
     const int64_t pitch_bytes = lda * 8 * qs_elem_doubles(a_dtype);
@@ -1332,7 +1350,9 @@ int qs_quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t 
     // Real rows leave in 16-byte pieces (row pairs of the register epilogue, runs of the staged one) when all extents,
     // strides and bases are even and every destination is 16-byte aligned.  With tabulated offsets that is the
     // table's business: block offsets (xq_table) must be even.
-    bool even16 = s.x_inner % 2 == 0 && X % 2 == 0 && s.sx1 % 2 == 0 && s.sx2 % 2 == 0 && s.sw0 % 2 == 0 &&
+    // Column tables: the caller's promise that every column offset is even stands in for an even sw0.
+    bool even16 = s.x_inner % 2 == 0 && X % 2 == 0 && s.sx1 % 2 == 0 && s.sx2 % 2 == 0 &&
+                  (columns ? s.col_off_even != 0 : s.sw0 % 2 == 0) &&
                   (n_dest > 0 || s.sw1 % 2 == 0) && (reinterpret_cast<uintptr_t>(s.out) & 15) == 0 &&
                   (!s.xq_table || xq_even);
     for (int64_t d = 0; d < n_dest; ++d) even16 = even16 && (reinterpret_cast<uintptr_t>(s.out_table[d]) & 15) == 0;
@@ -1342,14 +1362,15 @@ int qs_quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t 
     const int vec2 = !out_complex && rows_adjacent && even16;
     // Staged asynchronous epilogue: consecutive rows of a block are adjacent in the output (sx0 = 1) and every run of
     // rows handed to cp.async.bulk starts 16-byte aligned: always for complex output (16-byte elements), for real
-    // output under the conditions above.  Rows placed one by one (xr_table) keep the register stores.
+    // output under the conditions above.  Rows placed one by one (xr_table) and columns placed by the column tables
+    // keep the register stores.
     const bool bulk = (bulk_mode() == 2 || (bulk_mode() == 1 && n_dest > 1)) && s.sx0 == 1 && !s.xr_table &&
-                      !tl.split && (out_complex || even16);
+                      !columns && !tl.split && (out_complex || even16);
     // The rotated epilogue: one local destination, undealt columns, no row tables, the two-level row split with
     // adjacent rows, and 16-byte row pairs for real output.
     const bool rotated = n_dest == 0 && s.w_deal == 1 && !s.xq_table && !s.xr_table && s.x_mid == 0xFFFFFFFFLL &&
                          s.w_inner == 1 && s.sx0 == 1 && (out_complex || vec2);
-    const int epi = bulk ? kEpiBulk : rotated ? kEpiRotated : kEpiStrided;
+    const int epi = columns ? kEpiColumns : bulk ? kEpiBulk : rotated ? kEpiRotated : kEpiStrided;
 
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     // symmetry mask: per tile group, the ascending list of wanted linear tile ids, staged into list_ws
@@ -1416,8 +1437,10 @@ int qs_quarter_launch(const void* A, int a_dtype, int64_t X, int64_t K, int64_t 
         p.w_cyclic = s.w_cyclic;
         p.xq_table = s.xq_table;
         p.xr_table = s.xr_table;
+        p.col_dest = s.col_dest;
+        p.col_off = s.col_off;
         QS_REQUIRE((int64_t)p.tiles_x * p.tiles_w < (1LL << 31), "qs_quarter_transform: too many tiles");
-        const int rc = tl.split      ? launch_split(gr.NT, map, p, st)
+        const int rc = tl.split      ? launch_split(columns, gr.NT, map, p, st)
                        : out_complex ? launch_epilogue<true>(epi, gr.NT, map, p, st)
                                      : launch_epilogue<false>(epi, gr.NT, map, p, st);
         if (rc) return rc;
@@ -1578,5 +1601,30 @@ extern "C" int qs_quarter_transform_scatter(const void* A, int a_dtype, int64_t 
     s.sx2 = sx2;
     s.w_inner = w_inner;
     s.sw0 = sw0;
+    return qs_quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, s, stream);
+}
+
+// The scattering store with column tables: physical column w goes to host_out_table[col_dest[w]] at element offset
+// col_off[w] (device tables of W entries).  Rows as in qs_quarter_transform_scatter.
+extern "C" int qs_quarter_transform_scatter_columns(const void* A, int a_dtype, int64_t X, int64_t K, int64_t lda,
+                                                    const void* image, int m_dtype, int64_t W,
+                                                    void* const* host_out_table, int64_t n_dest,
+                                                    const int32_t* col_dest, const int64_t* col_off,
+                                                    int offsets_even, int64_t x_inner, int64_t x_mid, int64_t sx0,
+                                                    int64_t sx1, int64_t sx2, int64_t w_deal, void* stream) {
+    QS_REQUIRE(host_out_table && n_dest > 0 && col_dest && col_off,
+               "qs_quarter_transform_scatter_columns: null pointer or empty destination table");
+    QsQuarterStore s;
+    s.out_table = host_out_table;
+    s.n_dest = n_dest;
+    s.col_dest = col_dest;
+    s.col_off = reinterpret_cast<const long long*>(col_off);
+    s.col_off_even = offsets_even;
+    s.w_deal = w_deal;
+    s.x_inner = x_inner;
+    s.x_mid = x_mid;
+    s.sx0 = sx0;
+    s.sx1 = sx1;
+    s.sx2 = sx2;
     return qs_quarter_launch(A, a_dtype, X, K, lda, image, m_dtype, W, s, stream);
 }

@@ -313,6 +313,51 @@ def general_orbital_system(state, basis):
     return system
 
 
+def general_orbital_system_sharded(state, basis, out_dtype=torch.complex128, into=None):
+    """The spin-orbital system in the basis of the UHF ``state`` of the spatial ``ShardedBasisSet`` ``basis``, as a
+    ``ShardedBasisSet`` of extent 2l (``includes_spin=True``, ``anti_symmetrized_u=True``): what
+    ``ShardedBasisSet.from_spatial_planes(...)`` followed by ``change_basis(spin_orbital_coefficients(state)[0])``
+    computes, without the spin-doubled input and its ``(2l)^4`` transform.
+
+    ``u`` comes from the four spin blocks of the spatial tensor (``sharded.spin_orbital_two_body_sharded``): each rank
+    receives only the spatial planes its own spin-orbital planes are assembled from.  The result carries the proof of
+    its exact anti-symmetry and a spare buffer set (peer schedule), so a following ``change_basis`` takes the
+    symmetry-aware path without testing.  ``h`` and ``s`` are ``transform_one_body(add_spin_one_body(., out_dtype), C)``
+    with the ``C`` of ``spin_orbital_coefficients``, the calls of the spin-doubling route.  ``state`` may come from
+    ``ground_state_unrestricted_sharded`` or from the single-GPU solver; rank 0's coefficients are used on every rank.
+    ``out_dtype=torch.float64`` needs real spin blocks.  ``basis`` and its ``u`` are left untouched.
+
+    Each call allocates the result and its spare set as new peer-visible buffers, which live until ``ctx.close()``;
+    ``into`` (a ``ShardedTwoBody`` of extent 2l and dtype ``out_dtype``, e.g. the ``u`` of an earlier result that is
+    no longer needed) receives ``u`` instead, see ``sharded.spin_orbital_two_body_sharded``."""
+    from .sharded import ProcessContext, ShardedBasisSet, spin_orbital_two_body_sharded
+
+    _require_plain_spatial_u(basis, "ground_state_sharded")
+    ctx, l = basis.ctx, basis.u.n
+    if tuple(state.C_alpha.shape) != (l, l) or tuple(state.C_beta.shape) != (l, l):
+        raise ValueError(f"the state has {tuple(state.C_alpha.shape)} coefficients, the basis l = {l}")
+    if out_dtype not in (torch.float64, torch.complex128):
+        raise TypeError(f"out_dtype must be float64 or complex128, got {out_dtype}")
+    fields = {name: _arrays.to_device(getattr(state, name)).contiguous()
+              for name in ("C_alpha", "C_beta", "epsilon_alpha", "epsilon_beta")}
+    if isinstance(ctx, ProcessContext) and ctx.world > 1:
+        fields = {name: t.clone() for name, t in fields.items()}  # the caller's state keeps its own tensors
+        for t in fields.values():
+            ctx.dist.broadcast(torch.view_as_real(t) if t.is_complex() else t, src=0, group=ctx.group)
+    state = dataclasses.replace(state, **fields)
+    n_alpha, n_beta = _occupations(state.n_alpha, state.n_beta, l)
+    u = spin_orbital_two_body_sharded(basis.u, state.C_alpha, state.C_beta, n_alpha, n_beta, out_dtype=out_dtype,
+                                      into=into)
+    # the one-body side of from_spatial_planes + change_basis, call for call
+    C, _ = spin_orbital_coefficients(state)
+    C, _ = ops.real_coefficients_if_exact(out_dtype == torch.complex128, C, None)
+    h = ops.transform_one_body(ops.add_spin_one_body(_arrays.to_device(basis.h), out_dtype=out_dtype), C)
+    s = None
+    if basis.s is not None:
+        s = ops.transform_one_body(ops.add_spin_one_body(_arrays.to_device(basis.s), out_dtype=out_dtype), C)
+    return ShardedBasisSet(ctx, 2 * l, h, s, u, includes_spin=True, anti_symmetrized_u=True)
+
+
 def _spin_orbital_u(u, Ca, Cb, n_alpha, n_beta, widen):
     """The anti-symmetrised ``(2l)^4`` tensor of ``general_orbital_system`` from the spin blocks of ``u``."""
     l = u.shape[0]

@@ -52,13 +52,13 @@ def _result_dtype(*tensors):
     return torch.complex128 if any(t.dtype == torch.complex128 for t in tensors) else torch.float64
 
 
-def _coefficients(C, C_tilde):
-    """Bring C (n, n_new) and the optional C_tilde (n_new, n) to one dtype."""
-    C = _device_tensor(C, "C")
+def _coefficients(C, C_tilde, tensor=_device_tensor):
+    """Bring C (n, n_new) and the optional C_tilde (n_new, n) to one dtype (``tensor`` checks and converts each)."""
+    C = tensor(C, "C")
     if C.dim() != 2:
         raise ValueError("C must be a matrix (n, n_new)")
     if C_tilde is not None:
-        C_tilde = _device_tensor(C_tilde, "C_tilde")
+        C_tilde = tensor(C_tilde, "C_tilde")
         if tuple(C_tilde.shape) != (C.shape[1], C.shape[0]):
             raise ValueError(f"C_tilde must have shape {(C.shape[1], C.shape[0])}, got {tuple(C_tilde.shape)}")
         dt = _result_dtype(C, C_tilde)
@@ -187,16 +187,7 @@ def transform_two_body_mixed(u, C_r, C_s, Ct_p=None, Ct_q=None):
     matrices are brought to one dtype, and complex-typed ones without imaginary part are handed over as real ones
     for a complex ``u`` (``real_coefficients_if_exact``)."""
     u = _device_tensor(u, "u")
-    C_r, Ct_p = _coefficients(C_r, Ct_p)
-    C_s, Ct_q = _coefficients(C_s, Ct_q)
-    if C_r.shape != C_s.shape:
-        raise ValueError(f"C_r and C_s must have one shape, got {tuple(C_r.shape)} and {tuple(C_s.shape)}")
-    mats = [M for M in (C_r, C_s, Ct_p, Ct_q) if M is not None]
-    dt = _result_dtype(*mats)
-    C_r, C_s, Ct_p, Ct_q = (M.to(dt) if M is not None else None for M in (C_r, C_s, Ct_p, Ct_q))
-    # all four real or none: one exact test over every matrix, so that the kernels see a single dtype
-    if u.is_complex() and dt == torch.complex128 and not any(_has_imaginary_part(M) for M in mats):
-        C_r, C_s, Ct_p, Ct_q = (M.real.contiguous() if M is not None else None for M in (C_r, C_s, Ct_p, Ct_q))
+    C_r, C_s, Ct_p, Ct_q = mixed_coefficients(u.is_complex(), C_r, C_s, Ct_p, Ct_q)
     n, m = C_r.shape
     if tuple(u.shape) != (n, n, n, n):
         raise ValueError(f"u must have shape {(n,) * 4} to be contracted with C {tuple(C_r.shape)}, got {tuple(u.shape)}")
@@ -210,6 +201,23 @@ def transform_two_body_mixed(u, C_r, C_s, Ct_p=None, Ct_q=None):
     )
     owner.record_stream(torch.cuda.current_stream())
     return out
+
+
+def mixed_coefficients(u_is_complex, C_r, C_s, Ct_p, Ct_q, tensor=_device_tensor):
+    """The four matrices of a mixed transform in one dtype (``tensor`` checks and converts each: device tensors by
+    default); for a complex ``u`` complex-typed ones without imaginary part become real ones
+    (``real_coefficients_if_exact``), all four or none."""
+    C_r, Ct_p = _coefficients(C_r, Ct_p, tensor)
+    C_s, Ct_q = _coefficients(C_s, Ct_q, tensor)
+    if C_r.shape != C_s.shape:
+        raise ValueError(f"C_r and C_s must have one shape, got {tuple(C_r.shape)} and {tuple(C_s.shape)}")
+    mats = [M for M in (C_r, C_s, Ct_p, Ct_q) if M is not None]
+    dt = _result_dtype(*mats)
+    C_r, C_s, Ct_p, Ct_q = (M.to(dt) if M is not None else None for M in (C_r, C_s, Ct_p, Ct_q))
+    # all four real or none: one exact test over every matrix, so that the kernels see a single dtype
+    if u_is_complex and dt == torch.complex128 and not any(_has_imaginary_part(M) for M in mats):
+        C_r, C_s, Ct_p, Ct_q = (M.real.contiguous() if M is not None else None for M in (C_r, C_s, Ct_p, Ct_q))
+    return C_r, C_s, Ct_p, Ct_q
 
 
 def transform_one_body(h, C, C_tilde=None):

@@ -35,6 +35,7 @@ check the schedule under gloo without a GPU.
 import ctypes
 import weakref
 
+import numpy as np
 import torch
 
 from . import _native
@@ -249,6 +250,33 @@ class CudaEngine:
             "qs_quarter_transform_scatter", ctypes.c_void_p(A.at(0)), _CODES[A.dtype], X, K, lda,
             ctypes.c_void_p(image.data_ptr()), _CODES[m_dtype], W, self._dest_table(dests), len(dests), x_inner,
             max(x_mid, 1), sx0, sx1, sx2, max(w_inner, 1), sw0, int(deal), int(bool(cyclic)), self._stream(),
+        )
+
+    def quarter_scatter_columns(self, A, X, K, lda, image, m_dtype, W, dests, col_dest, col_off, offsets_even,
+                                x_inner, x_mid, sx0, sx1, sx2, deal=1):
+        """The scattering store with column tables (``qs_quarter_transform_scatter_columns``): physical column w goes to
+        ``dests[col_dest[w]]`` at element offset ``col_off[w]``; ``col_dest`` (int32) and ``col_off`` (int64) are
+        ``index_table`` device tables."""
+        if X <= 0:
+            return
+        _native.call(
+            "qs_quarter_transform_scatter_columns", ctypes.c_void_p(A.at(0)), _CODES[A.dtype], X, K, lda,
+            ctypes.c_void_p(image.data_ptr()), _CODES[m_dtype], W, self._dest_table(dests), len(dests),
+            ctypes.c_void_p(col_dest.data_ptr()), ctypes.c_void_p(col_off.data_ptr()), int(bool(offsets_even)),
+            x_inner, max(x_mid, 1), sx0, sx1, sx2, int(deal), self._stream(),
+        )
+
+    def spin_orbital_planes(self, blocks, l, orbital, spin, out, p0, p1):
+        """Planes ``[p0, p1)`` of the anti-symmetrised spin-orbital tensor into ``out`` (``qs_spin_orbital_two_body``).
+        ``blocks`` holds ``(buffer, offset)`` for B_aa, B_ab, B_ba, B_bb: spatial plane o of a block is at element
+        ``offset + o l^3`` of its buffer (a negative offset is the virtual base of a buffer that holds only the planes
+        these spin-orbital planes read).  ``orbital`` and ``spin`` are int32 ``index_table`` device tables."""
+        if p1 <= p0:
+            return
+        bases = [ctypes.c_void_p(buf.at(off)) for buf, off in blocks]
+        _native.call(
+            "qs_spin_orbital_two_body", *bases, _CODES[blocks[0][0].dtype], l, ctypes.c_void_p(orbital.data_ptr()),
+            ctypes.c_void_p(spin.data_ptr()), ctypes.c_void_p(out.at(0)), _CODES[out.dtype], p0, p1, self._stream(),
         )
 
 
@@ -616,26 +644,32 @@ class _RankTransform:
     def scratch_numel(self):
         return max(self.m * self.A * self.n * self.P, self.m * self.R * self.m * self.P, 1)
 
-    def prepare(self, C, C_tilde):
+    def prepare(self, C_r, C_s, Ct_p=None, Ct_q=None):
+        """Coefficient images of the four steps, one matrix each as in ``ops.transform_two_body_mixed``: step 1 (d -> s)
+        ``C_s``, step 2 (c -> r) ``C_r``, step 3 (b -> q) ``Ct_q``, step 4 (a -> p) ``Ct_p``; ``Ct_q`` defaults to
+        ``C_s^dagger`` and ``Ct_p`` to ``C_r^dagger``.  May be called again for the next transform of this rank; the
+        scratch buffer is kept."""
         eng, n, m = self.engine, self.n, self.m
-        self.img1 = eng.image(C, n, m, self.u_dtype, m, 1)
-        self.img2 = eng.image(C, n, m, self.t_dtype, m, 1)
-        if C_tilde is not None:
-            self.img3 = eng.image(C_tilde, n, m, self.t_dtype, 1, n)
-        else:
-            self.img3 = eng.image(C, n, m, self.t_dtype, m, 1, conj=True)  # C~ = C^dagger, basis_set.py:338-339
+        self.img1 = eng.image(C_s, n, m, self.u_dtype, m, 1)
+        self.img2 = eng.image(C_r, n, m, self.t_dtype, m, 1)
+        self.img3 = self._bra_image(C_s, Ct_q)
         # The last step scatters BLOCKS of the new leading index p (the result is block-partitioned), so it deals
         # its output columns over all destinations (uniform NVLink traffic): its image holds the columns of C~ in
         # dealt order.  The first exchange sends cyclic columns and needs no dealing.
         self.deal = eng.scatter_deal(m) if self.ctx.exchange == "peer" and self.ctx.world > 1 else 1
-        if self.deal > 1:
-            if C_tilde is not None:
-                self.img4_scatter = eng.image(C_tilde, n, m, self.t_dtype, 1, n, deal=self.deal)
-            else:
-                self.img4_scatter = eng.image(C, n, m, self.t_dtype, m, 1, conj=True, deal=self.deal)
+        if self.deal == 1 and C_r is C_s and Ct_p is Ct_q:
+            self.img4 = self.img3  # one matrix for both bras (the plain transform)
         else:
-            self.img4_scatter = self.img3
-        self.scratch = eng.empty(self.scratch_numel(), self.t_dtype)
+            self.img4 = self._bra_image(C_r, Ct_p, self.deal)
+        if getattr(self, "scratch", None) is None:
+            self.scratch = eng.empty(self.scratch_numel(), self.t_dtype)
+
+    def _bra_image(self, C, C_tilde, deal=1):
+        """Image of a bra step: ``C_tilde`` (m, n), or ``C^dagger`` when it is None (basis_set.py:338-339)."""
+        n, m = self.n, self.m
+        if C_tilde is not None:
+            return self.engine.image(C_tilde, n, m, self.t_dtype, 1, n, deal=deal)
+        return self.engine.image(C, n, m, self.t_dtype, m, 1, conj=True, deal=deal)
 
     def step1(self, u_in):
         """T1[s, a_loc, b, c] = sum_d u[a_loc, b, c, d] C[d, s]  (new index slowest, c at pitch P)."""
@@ -705,8 +739,25 @@ class _RankTransform:
         of every (r, s) block interleave with the other ranks' rows."""
         eng, n, m, R, P, W = self.engine, self.n, self.m, self.R, self.P, self.ctx.world
         dests = [(out[j], self.rank * m) for j in range(W)]
-        eng.quarter_scatter(self.scratch, m * R * m, n, P, self.img4_scatter, self.c_dtype, m, dests, m, R, 1, W * m,
+        eng.quarter_scatter(self.scratch, m * R * m, n, P, self.img4, self.c_dtype, m, dests, m, R, 1, W * m,
                             m * m, self.r_block, m**3, deal=self.deal)
+
+    def step4_scatter_columns(self, dests, col_dest, col_off):
+        """Step 4 with the plane of every p chosen by the column tables: u'[p, q, r, s] goes to
+        ``dests[col_dest[p]]`` at plane offset ``col_off[p]``, rows placed as in ``step4_scatter``.  ``dests`` are
+        ``(buffer, offset)`` pairs; this rank's offset ``rank * m`` (its first r) is added here."""
+        eng, n, m, R, P, W = self.engine, self.n, self.m, self.R, self.P, self.ctx.world
+        dests = [(buf, off + self.rank * m) for buf, off in dests]
+        eng.quarter_scatter_columns(self.scratch, m * R * m, n, P, self.img4, self.c_dtype, m, dests, col_dest,
+                                    col_off, m % 2 == 0, m, R, 1, W * m, m * m, deal=self.deal)
+
+    def step4_local_columns(self, send, col_off):
+        """Collective schedule: u'[p, q, r_loc, s] with plane p at ``col_off[p]`` of the local ``send`` buffer (dense
+        (q, r_loc, s) planes); the tables order the planes by their destination rank."""
+        eng, n, m, R, P = self.engine, self.n, self.m, self.R, self.P
+        dest = self.engine.index_table(np.zeros(m, dtype=np.int32))
+        eng.quarter_scatter_columns(self.scratch, m * R * m, n, P, self.img4, self.c_dtype, m, [(send, 0)], dest,
+                                    col_off, (m * R * m) % 2 == 0, m * R * m, 1, 1, 0, 0)
 
     # ---- anti-symmetric u: steps 3 and 4 on half of the (r, s) pairs (cyclic rule), packed by pair -------------
     def pairs_padded(self):
@@ -776,14 +827,14 @@ class _RankTransform:
         if self.npairs == 0:
             return
         dests = [(out[j], 0) for j in range(self.ctx.world)]
-        eng.quarter_scatter_rows(self.scratch, m * self.npairs, n, P, self.img4_scatter, self.c_dtype, m, dests,
+        eng.quarter_scatter_rows(self.scratch, m * self.npairs, n, P, self.img4, self.c_dtype, m, dests,
                                  self.npairs, m * m, self.rs_of_pair_dev, self.r_block, m**3, deal=self.deal,
                                  rows_paired=self.rows_paired)
 
     def step4_local(self, out_local):
         """Collective schedule: u'[p, q, r_loc, s] dense on this rank (sharded on the third index)."""
         eng, n, m, R, P = self.engine, self.n, self.m, self.R, self.P
-        eng.quarter(self.scratch, m * R * m, n, P, self.img3, self.c_dtype, m, out_local, 0, m * R * m, 1, 0, 1, 0,
+        eng.quarter(self.scratch, m * R * m, n, P, self.img4, self.c_dtype, m, out_local, 0, m * R * m, 1, 0, 1, 0,
                     m * R * m)
 
 
@@ -833,10 +884,7 @@ def transform_two_body_sharded(u, C, C_tilde=None, symmetry=None):
                          and is_antisymmetric_last_pair(u, trust_proof=True)) else 0
     if symmetry and ctx.exchange != "peer":
         raise ValueError("the symmetry-aware sharded transform needs the peer exchange")
-    work = {r: _RankTransform(ctx, r, n, m, u.dtype, C.dtype) for r in ctx.local_ranks}
-    t_dtype = next(iter(work.values())).t_dtype
-    for w in work.values():
-        w.prepare(C, C_tilde)
+    work, t_dtype = _rank_transforms(ctx, n, m, u.dtype, C.dtype, (C, C, C_tilde, C_tilde))
     any_w = next(iter(work.values()))
 
     if ctx.exchange == "peer":
@@ -847,40 +895,105 @@ def transform_two_body_sharded(u, C, C_tilde=None, symmetry=None):
             _recycle(ctx, out, keep=u)  # a caller still holding that older tensor gets an error, not new data
         else:
             out = ctx.shared_empty(out_numels, t_dtype)
-        ctx.barrier()  # every rank is done with whatever it last read from these buffers
-        for r, w in work.items():
-            w.step1(u.buffers[r][r])
-            w.step2_scatter(recv[r], pairs_only=bool(symmetry))
-        ctx.barrier()  # all tiles of T2 have landed
-        for r, w in work.items():
-            if symmetry:
-                w.prepare_pairs()
-                w.step3_pairs(recv[r][r])
-                w.step4_scatter_pairs(out[r])
-            else:
-                w.step3(recv[r][r])
-                w.step4_scatter(out[r])
-        ctx.barrier()  # all tiles of u' have landed
         if symmetry:
+            _peer_steps(u, work, recv, lambda r, w: w.step4_scatter_pairs(out[r]), pairs_only=True)
             for r, w in work.items():
                 # the other half of every local plane p: -u'[p,q,s,r]
                 ctx.engine.cyclic_fill(out[r][r], m, w.r_off[r + 1] - w.r_off[r])
+        else:
+            _peer_steps(u, work, recv, lambda r, w: w.step4_scatter(out[r]))
         spare = u.buffers if (u.dtype == t_dtype and m == n) else None
         result = ShardedTwoBody(ctx, m, t_dtype, out, spare)
         result.proven_antisymmetric = bool(symmetry)  # the cyclic fill wrote exact negatives and a zero diagonal
         return result
+    return _collective_transform(u, work, m, t_dtype)
 
-    # collective schedule (one rank per process)
-    (r, w), = work.items()
-    eng, P = ctx.engine, w.P
-    send = eng.empty(m * m * w.A * P, t_dtype)
-    recv = eng.empty(w.R * m * n * P, t_dtype)
+
+def transform_two_body_sharded_mixed(u, C_r, C_s, Ct_p=None, Ct_q=None):
+    """``u'_pqrs = sum Ct_p[p,a] Ct_q[q,b] u[a,b,c,d] C_r[c,r] C_s[d,s]`` of a ``ShardedTwoBody``: the sharded
+    counterpart of ``ops.transform_two_body_mixed``, with one coefficient matrix per index (``Ct_p`` defaults to
+    ``C_r^dagger``, ``Ct_q`` to ``C_s^dagger``; the matrices are brought to one dtype, and complex-typed ones without
+    imaginary part are handed over as real ones for a complex ``u``).  The same steps and exchanges as
+    ``transform_two_body_sharded``, in either schedule, without symmetry.  The result lives in NEW buffers: ``u``
+    and its spare set are left alone, so the handle of an earlier result stays valid."""
+    from . import ops
+
+    ctx = u.ctx
+    C_r, C_s, Ct_p, Ct_q = ops.mixed_coefficients(u.dtype == torch.complex128, C_r, C_s, Ct_p, Ct_q,
+                                                  tensor=_matrix_converter(ctx))
+    n, m = C_r.shape
+    if n != u.n:
+        raise ValueError(f"C_r has {n} rows but u has {u.n} orbitals")
+    work, t_dtype = _rank_transforms(ctx, n, m, u.dtype, C_r.dtype, (C_r, C_s, Ct_p, Ct_q))
+    any_w = next(iter(work.values()))
+    if ctx.exchange == "peer":
+        recv = ctx.shared_cached("recv", [any_w.recv_numel(r) for r in range(ctx.world)], t_dtype)
+        out = ctx.shared_empty([any_w.out_numel(r) for r in range(ctx.world)], t_dtype)
+        _peer_steps(u, work, recv, lambda r, w: w.step4_scatter(out[r]))
+        return ShardedTwoBody(ctx, m, t_dtype, out)
+    return _collective_transform(u, work, m, t_dtype)
+
+
+def _matrix_converter(ctx):
+    """``tensor(M, name)`` of ``ops.mixed_coefficients`` for this context's engine."""
+
+    def tensor(M, name):
+        M = ctx.engine.asarray(M)
+        if M.dtype not in _CODES:
+            raise TypeError(f"{name} must be float64 or complex128, got {M.dtype}")
+        return M.contiguous()
+
+    return tensor
+
+
+def _rank_transforms(ctx, n, m, u_dtype, c_dtype, mats):
+    """One prepared ``_RankTransform`` per local rank (``mats`` = (C_r, C_s, Ct_p, Ct_q)), and the dtype of T2."""
+    work = {r: _RankTransform(ctx, r, n, m, u_dtype, c_dtype) for r in ctx.local_ranks}
+    for w in work.values():
+        w.prepare(*mats)
+    return work, next(iter(work.values())).t_dtype
+
+
+def _peer_steps(u, work, recv, step4, pairs_only=False, lead=True):
+    """The four steps of the peer schedule: steps 1-2 scatter T2 into ``recv``, steps 3 and ``step4(rank, work)``
+    store the result.  The barriers order the exchanges; ``lead=False`` skips the first one when the caller's last
+    barrier already follows every read of ``recv`` and of the destination buffers."""
+    ctx = u.ctx
+    if lead:
+        ctx.barrier()  # every rank is done with whatever it last read from these buffers
+    for r, w in work.items():
+        w.step1(u.buffers[r][r])
+        w.step2_scatter(recv[r], pairs_only=pairs_only)
+    ctx.barrier()  # all tiles of T2 have landed
+    for r, w in work.items():
+        if pairs_only:
+            w.prepare_pairs()
+            w.step3_pairs(recv[r][r])
+        else:
+            w.step3(recv[r][r])
+        step4(r, w)
+    ctx.barrier()  # all tiles of u' have landed
+
+
+def _collective_steps_1_to_3(u, w):
+    """Steps 1-3 of the collective schedule (one rank per process): T3 in the scratch of ``w``."""
+    ctx, eng, n, m, P, r = u.ctx, u.ctx.engine, w.n, w.m, w.P, w.rank
+    send = eng.empty(m * m * w.A * P, w.t_dtype)
+    recv = eng.empty(w.R * m * n * P, w.t_dtype)
     w.step1(u.buffers[r][r])
     w.step2_local(send)
     send_splits = [(w.r_off[j + 1] - w.r_off[j]) * m * w.A * P for j in range(ctx.world)]
     recv_splits = [w.R * m * (w.a_off[k + 1] - w.a_off[k]) * P for k in range(ctx.world)]
     ctx.all_to_all(send, send_splits, recv, recv_splits)
     w.step3_blocked(recv)
+
+
+def _collective_transform(u, work, m, t_dtype):
+    """The collective schedule of a full transform (one rank per process)."""
+    ctx = u.ctx
+    (r, w), = work.items()
+    eng = ctx.engine
+    _collective_steps_1_to_3(u, w)
     out_local = eng.empty(m * w.R * m * m, t_dtype)  # u'[p, q, r_loc, s]
     w.step4_local(out_local)
     # r -> p re-partition: send [p in P_j][q][r_loc][s], receive [p_loc][q][r_loc(k)][s] from every k
@@ -896,6 +1009,151 @@ def transform_two_body_sharded(u, C, C_tilde=None, symmetry=None):
         block = staged.as_tensor()[offset : offset + recv_splits[k]].view(w.R, m, Rk, m)
         dense[:, :, w.r_off[k] : w.r_off[k + 1], :] = block  # data movement only
         offset += recv_splits[k]
+    return result
+
+
+# ------------------------------------------------------------------------------------------------
+# the spin-orbital tensor of an unrestricted basis, sharded
+# ------------------------------------------------------------------------------------------------
+SPIN_BLOCKS = ((0, 0), (0, 1), (1, 0), (1, 1))  # (sigma, tau) of B_aa, B_ab, B_ba, B_bb
+
+
+def spin_plane_routing(n_alpha, n_beta, l, world):
+    """Where the planes of the spin-orbital tensor of an unrestricted basis live when it is block-partitioned on its
+    leading index (``block_partition(2 l, world)``), in the order of ``hartree_fock.spin_orbital_order``.
+
+    Returns ``(owner, ranges)``: ``owner[s, o]`` is the rank holding the plane of orbital o with spin s, and
+    ``ranges[j, s] = (q0, q1)`` the orbitals of spin s whose planes rank j holds.  For each spin the plane index grows
+    with the orbital index (occupied orbitals first, then virtual ones, each in orbital order), so these are ONE
+    contiguous range per rank and spin, and over the ranks they tile ``[0, l)`` in rank order: rank j needs exactly
+    the planes ``[q0, q1)`` of the blocks ``B_s,alpha`` and ``B_s,beta``."""
+    from .hartree_fock import spin_orbital_order
+
+    orbital, spin = spin_orbital_order(n_alpha, n_beta, l)
+    plane = np.empty((2, l), dtype=np.int64)
+    plane[spin, orbital] = np.arange(2 * l)
+    _, offsets = block_partition(2 * l, world)
+    owner = np.searchsorted(np.asarray(offsets[1:]), plane, side="right")  # offsets[j] <= plane < offsets[j + 1]
+    if l > 1 and np.any(np.diff(owner, axis=1) < 0):
+        raise RuntimeError("internal: spin-orbital planes of one spin are not in orbital order")
+    ranks = np.arange(world)
+    ranges = np.empty((world, 2, 2), dtype=np.int64)
+    for s in (0, 1):
+        ranges[:, s, 0] = np.searchsorted(owner[s], ranks, side="left")
+        ranges[:, s, 1] = np.searchsorted(owner[s], ranks, side="right")
+    return owner, ranges
+
+
+def _staging_layout(ranges, j, plane_numel, base=0):
+    """Offsets (from ``base``) of the four blocks' planes that rank j assembles from, packed B_aa, B_ab (planes of the
+    alpha range), B_ba, B_bb (beta range), ``plane_numel`` elements a plane, and their size.  The staging buffer of
+    rank j in the peer schedule (whole ``l^3`` planes) and rank j's part of a send buffer in the collective one
+    (this rank's ``(q, r_loc, s)`` part of a plane) share this layout."""
+    offsets, size = {}, 0
+    for sigma, tau in SPIN_BLOCKS:
+        offsets[(sigma, tau)] = base + size
+        size += int(ranges[j, sigma, 1] - ranges[j, sigma, 0]) * plane_numel
+    return offsets, size
+
+
+def spin_orbital_two_body_sharded(u, C_alpha, C_beta, n_alpha, n_beta, out_dtype=torch.complex128, into=None):
+    """The anti-symmetrised ``(2l)^4`` spin-orbital tensor of an unrestricted basis (``ops.spin_orbital_two_body``)
+    from the spatial ``ShardedTwoBody`` ``u``, as a new ``ShardedTwoBody`` block-partitioned on its leading index.
+
+    The four spin blocks ``B_st = C_s^dagger C_t^dagger u C_s C_t`` are transformed explicitly (a derived B_ba would
+    need every plane of B_ab on every rank).  Only the planes a rank assembles from ever exist (``spin_plane_routing``):
+    in the peer schedule step 4 of every block stores plane p through the column tables straight into a peer-visible
+    staging buffer on the rank that owns spin-orbital plane P(p, s); in the collective one step 4 writes the planes
+    grouped by destination and one ``all_to_all`` with the uneven splits delivers them.  Every rank then assembles its
+    own planes with the fused kernel of ``ops.spin_orbital_two_body``.  ``u`` and its buffers are left untouched.
+
+    Memory: the result is a new ``ShardedTwoBody`` with a spare buffer set (peer schedule: two sets of peer-visible
+    IPC buffers, which live until ``ctx.close()``, like every ``shared_empty`` allocation), unless ``into`` -- a
+    ``ShardedTwoBody`` of extent ``2 l`` and dtype ``out_dtype`` -- is given: then the result is written into its
+    buffers and ``into`` itself is returned, so repeated calls (or a following ``from_spatial_planes(..., into=...)``
+    of the same size) reuse one allocation.  The staging buffers are cached in the context."""
+    from . import ops
+    from .hartree_fock import spin_orbital_order
+
+    ctx, l, eng = u.ctx, u.n, u.ctx.engine
+    C_alpha, C_beta, _, _ = ops.mixed_coefficients(u.dtype == torch.complex128, C_alpha, C_beta, None, None,
+                                                   tensor=_matrix_converter(ctx))
+    if tuple(C_alpha.shape) != (l, l):
+        raise ValueError(f"the coefficients are {tuple(C_alpha.shape)}, u has l = {l}")
+    t_dtype = torch.complex128 if torch.complex128 in (u.dtype, C_alpha.dtype) else torch.float64
+    if t_dtype == torch.complex128 and out_dtype != torch.complex128:
+        raise TypeError("complex spin blocks need a complex128 result")
+    owner, ranges = spin_plane_routing(n_alpha, n_beta, l, ctx.world)
+    mats = (C_alpha, C_beta)
+    work = {r: _RankTransform(ctx, r, l, l, u.dtype, C_alpha.dtype) for r in ctx.local_ranks}
+    if into is not None and (into.ctx is not ctx or into.n != 2 * l or into.dtype != out_dtype):
+        raise ValueError("`into` must be a ShardedTwoBody of this context, extent 2 l and the requested dtype")
+    result = into if into is not None else ShardedTwoBody.empty(ctx, 2 * l, out_dtype)
+    layouts = [_staging_layout(ranges, j, l**3) for j in range(ctx.world)]
+
+    if ctx.exchange == "peer":
+        any_w = next(iter(work.values()))
+        recv = ctx.shared_cached("recv", [any_w.recv_numel(r) for r in range(ctx.world)], t_dtype)
+        staging = ctx.shared_cached("spin_blocks", [total for _, total in layouts], t_dtype)
+        # per spin of p: the destination rank of plane p and its offset inside that rank's range of the block
+        tables = {s: (eng.index_table(owner[s].astype(np.int32)),
+                      eng.index_table((np.arange(l) - ranges[owner[s], s, 0]) * l**3)) for s in (0, 1)}
+        for b, (sigma, tau) in enumerate(SPIN_BLOCKS):
+            for w in work.values():
+                w.prepare(mats[sigma], mats[tau])
+
+            def step4(r, w, sigma=sigma, tau=tau):
+                dests = [(staging[r][j], layouts[j][0][(sigma, tau)]) for j in range(ctx.world)]
+                w.step4_scatter_columns(dests, *tables[sigma])
+
+            _peer_steps(u, work, recv, step4, lead=b == 0)
+        local_blocks = {r: staging[r][r] for r in ctx.local_ranks}
+    else:
+        (r, w), = work.items()
+        m, numel = l, l * w.R * l  # a sent plane: (q, r_loc, s) over this rank's block of r
+        # send buffer grouped by destination j, then block, then plane: the staging layout of every j, one after the
+        # other
+        send_offsets, total = [], 0
+        for j in range(ctx.world):
+            offsets, size = _staging_layout(ranges, j, numel, base=total)
+            send_offsets.append(offsets)
+            total += size
+        send = eng.empty(total, t_dtype)
+        for sigma, tau in SPIN_BLOCKS:
+            w.prepare(mats[sigma], mats[tau])
+            _collective_steps_1_to_3(u, w)
+            col_off = (np.array([send_offsets[j][(sigma, tau)] for j in owner[sigma]], dtype=np.int64)
+                       + (np.arange(l) - ranges[owner[sigma], sigma, 0]) * numel)
+            w.step4_local_columns(send, eng.index_table(col_off))
+        count = ranges[:, :, 1] - ranges[:, :, 0]  # (rank, spin)
+        send_splits = [int(2 * (count[j, 0] + count[j, 1])) * numel for j in range(ctx.world)]
+        r_counts = [w.r_off[k + 1] - w.r_off[k] for k in range(ctx.world)]
+        recv_splits = [int(2 * (count[r, 0] + count[r, 1])) * m * r_counts[k] * m for k in range(ctx.world)]
+        staged = eng.empty(sum(recv_splits), t_dtype)
+        ctx.all_to_all(send, send_splits, staged, recv_splits)
+        block_offsets, block_total = layouts[r]
+        local = eng.empty(block_total, t_dtype)
+        flat, offset = staged.as_tensor(), 0
+        for k in range(ctx.world):
+            for sigma, tau in SPIN_BLOCKS:
+                c, Rk = int(count[r, sigma]), r_counts[k]
+                piece = flat[offset : offset + c * m * Rk * m].view(c, m, Rk, m)
+                base = block_offsets[(sigma, tau)]
+                dense = local.as_tensor()[base : base + c * l**3].view(c, l, l, l)
+                dense[:, :, w.r_off[k] : w.r_off[k + 1], :] = piece  # data movement only
+                offset += c * m * Rk * m
+        local_blocks = {r: local}
+
+    orbital, spin = spin_orbital_order(n_alpha, n_beta, l)
+    orbital_d, spin_d = eng.index_table(orbital.astype(np.int32)), eng.index_table(spin.astype(np.int32))
+    for r in ctx.local_ranks:
+        p0, p1 = result.planes(r)
+        offsets, _ = layouts[r]
+        # virtual bases: spatial plane o of block (s, t) at offset + (o - q0_s) l^3 of the staged planes
+        blocks = [(local_blocks[r], offsets[(sigma, tau)] - int(ranges[r, sigma, 0]) * l**3)
+                  for sigma, tau in SPIN_BLOCKS]
+        eng.spin_orbital_planes(blocks, l, orbital_d, spin_d, result.buffers[r][r], p0, p1)
+    result.proven_antisymmetric = True  # every plane holds exact negatives a - b, b - a
     return result
 
 

@@ -21,7 +21,7 @@ def main():
     u.local().normal_()
     C = torch.from_numpy(np.linalg.qr(np.random.default_rng(0).standard_normal((n, n)))[0]).cuda()
     w = sharded._RankTransform(ctx, rank, n, n, torch.float64, torch.float64)
-    w.prepare(C, None)
+    w.prepare(C, C)
     recv = ctx.shared_cached("recv", [w.recv_numel(r) for r in range(world)], torch.float64)
     out = u.spare
     names = ["step1", "step2_scatter", "barrier", "step3", "step4_scatter", "barrier2"]
