@@ -121,6 +121,15 @@ def diagonal_rows(W, C, Ct, dt, rows=None, anti=False, absolute=False):
     return np.ascontiguousarray(out)
 
 
+def diagonal_plane(W, C, Ct, dt, p, anti=False, absolute=False):
+    """Plane ``u'[p]`` of ``diagonal_rows`` (minus its ``r <-> s`` exchange when ``anti``) from the ``m`` rows
+    ``(p, r)``: O(m n² + m³) instead of the whole result."""
+    m = C.shape[1]
+    R = diagonal_rows(W, C, Ct, dt, rows=[(p, r) for r in range(m)])  # [r, q, s] = u'[p, q, r, s]
+    plane = R.transpose(1, 0, 2)
+    return _sub(plane, R.transpose(1, 2, 0), absolute) if anti else np.ascontiguousarray(plane)
+
+
 def shielded_coulomb(grid, alpha, a, dt):
     """``W[p,q] = alpha / sqrt((x_p - x_q)^2 + a^2)`` (reference one_dim_qd.py:29-32) in precision ``dt``."""
     grid = cast(grid, dt)
@@ -162,13 +171,14 @@ def kron_fock_unrestricted(h, A, B, rho_a, rho_b, dt, absolute=False):
     return np.stack([_sub(h + j, A @ r @ B, absolute) for r in (rho_a, rho_b)])
 
 
-def kron_fock_occupied(h, A, B, n_occ, dt, anti=False, absolute=False):
+def kron_fock_occupied(h, A, B, n_occ, dt, anti=False, spatial=False, absolute=False):
     """``fock_occupied`` (general form) of ``u[a,b,c,d] = A[a,c] B[b,d]`` (minus ``A[a,d] B[b,c]``):
-    ``h + A sum_i B[i,i] (- sum_i A[p,i] B[i,q])`` over ``i < n_occ``.  The absolute-value companion is the exact
-    ``|terms|`` without ``anti`` and an upper bound of it with."""
+    ``h + A sum_i B[i,i] (- sum_i A[p,i] B[i,q])`` over ``i < n_occ``.  ``spatial``: the spatial form of the plain
+    ``A ⊗ B``, ``h + 2 A sum_i B[i,i] - sum_i A[p,i] B[i,q]``.  The absolute-value companion is the exact ``|terms|``
+    of the general form without ``anti`` and an upper bound of it otherwise."""
     o = slice(0, n_occ)
-    f = h + A * np.sum(np.diagonal(B)[o])
-    return _sub(f, A[:, o] @ B[o, :], absolute) if anti else f
+    f = h + (2 if spatial else 1) * A * np.sum(np.diagonal(B)[o])
+    return _sub(f, A[:, o] @ B[o, :], absolute) if anti or spatial else f
 
 
 def fock_occupied(h, u, n_occ, spatial, dt, absolute=False):

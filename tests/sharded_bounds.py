@@ -18,6 +18,7 @@ a row nobody wrote or an output element never stored is non-finite, and both che
 
 import bisect
 import ctypes
+import functools
 
 import numpy as np
 import torch
@@ -26,12 +27,14 @@ import precise as P
 
 # (b)'s extra slack in units of u, beyond the kernel's own 2 gamma(k) |terms| (sqrt 2 larger for complex values):
 # the device compares with fl(X̂ Ŷ) - fl(X̂' Ŷ') instead of the exact value.  X̂ = fl64(X_ld) is off by at most
-# u |X| for the rounding to FP64 plus the longdouble error of X_ld, gamma_ld(4n) |X|abs < 0.2 u for n <= 144 even
-# for complex factors: 1.2 u for each of the two factors.  The FP64 product adds u (real) or sqrt 2 gamma(2) < 2.9 u
-# (complex), the subtraction of the anti-symmetric form u: 2 x 1.2 + 2.9 + 1 = 6.3 u of (|X||Y| + |X'||Y'|).  The
-# bound itself is evaluated in FP64 from the rounded |X|, |Y|, which costs a relative few u of 2 gamma(k), far less
-# than the remaining 1.7 u.
+# u |X| for the rounding to FP64 plus the longdouble error of X_ld, gamma_ld(4n) |X|abs <= 4n 2^-64 |X|abs, at most
+# 0.5 u for n <= 256 even for complex factors (x86 extended; far less in IEEE quad): 1.5 u for each of the two
+# factors.  The FP64 product adds u (real) or sqrt 2 gamma(2) < 2.9 u (complex), the subtraction of the anti-symmetric
+# form u: 2 x 1.5 + 2.9 + 1 = 6.9 u of (|X||Y| + |X'||Y'|).  The bound itself is evaluated in FP64 from the rounded
+# |X|, |Y|, which costs a relative few u of 2 gamma(k), far less than the remaining 1.1 u.  ``n`` is the contraction
+# length of the factors (the extent of ``A``); ``sweep_slabs`` refuses a larger one.
 SWEEP_SLACK = 8.0
+SWEEP_MAX_N = 256
 
 
 def plane_indices(m, rng, extra=()):
@@ -64,7 +67,10 @@ def exact_sharded(ctx, A, B, anti, dtype, device):
 
 
 def planes_of(u, planes):
-    """Planes ``u[p]`` of a sharded tensor, copied to the host (only these planes, not the whole tensor)."""
+    """Planes ``u[p]`` of a sharded tensor or of a plain torch tensor, copied to the host (only these planes, not
+    the whole tensor)."""
+    if isinstance(u, torch.Tensor):
+        return u[list(planes)].cpu().numpy()
     rows = []
     for p in planes:
         r = bisect.bisect_right(u.offsets, p) - 1
@@ -102,10 +108,23 @@ def check_planes(check, u, factors_fn, arrays, planes, k, anti, what, batch=4):
 
 def sweep(u, factors_fn, arrays, k, anti, what, chunk=8):
     """(b): every element of every rank against ``fl(X̂ Ŷ) (- fl(X̂' Ŷ'))`` under criterion A plus ``SWEEP_SLACK``
-    (criterion A only: the aggregate B needs the longdouble reference).  Streams over each rank's planes in chunks
-    of ``chunk`` on the ranks' device.  Returns the largest ``|got - X̂ Ŷ| / bound``."""
-    dev = u.local(u.ctx.local_ranks[0]).device
-    out_dtype = u.dtype
+    (criterion A only: the aggregate B needs the longdouble reference), rank by rank (``sweep_slabs``).  Returns
+    the largest ``|got - X̂ Ŷ| / bound``."""
+    slabs = [(f"rank {r}", u.planes(r)[0], u.local(r)) for r in u.ctx.local_ranks]
+    return sweep_slabs(slabs, factors_fn, arrays, k, anti, what, chunk)
+
+
+def sweep_slabs(slabs, factors_fn, arrays, k, anti, what, chunk=8, boundary=None):
+    """(b) over ``slabs``, a list of ``(label, first plane, tensor of leading planes)`` of one dtype on one device
+    (a rank's shard, or a whole single-GPU result as ``("", 0, out)``), streamed in chunks of ``chunk`` planes on
+    that device.  ``boundary``: an element offset the sweep must reach within one slab (2**31 for the checks of
+    64-bit addressing); a violation reports where it lies relative to it.  Returns the largest
+    ``|got - X̂ Ŷ| / bound``."""
+    assert np.shape(arrays[0])[0] <= SWEEP_MAX_N, f"{what}: SWEEP_SLACK is derived for n <= {SWEEP_MAX_N}"
+    dev = slabs[0][2].device
+    out_dtype = slabs[0][2].dtype
+    if boundary is not None:
+        assert max(s.numel() for _, _, s in slabs) > boundary, f"{what}: no slab reaches element offset {boundary}"
 
     def to_dev(x):
         x = np.asarray(x)
@@ -120,9 +139,9 @@ def sweep(u, factors_fn, arrays, k, anti, what, chunk=8):
     cplx = out_dtype == torch.complex128
     coef = 2.0 * P.gamma(k) * (np.sqrt(2.0) if cplx else 1.0) + SWEEP_SLACK * P.U
     worst = 0.0
-    for r in u.ctx.local_ranks:
-        p0, p1 = u.planes(r)
-        slab = u.local(r)
+    for label, p0, slab in slabs:
+        p1 = p0 + slab.shape[0]
+        plane = slab[0].numel() if slab.shape[0] else 0
         for c0 in range(p0, p1, chunk):
             c1 = min(c0 + chunk, p1)
             X, Y, Xx, Yx = fac
@@ -139,8 +158,10 @@ def sweep(u, factors_fn, arrays, k, anti, what, chunk=8):
             if bool(bad.any()):
                 idx = tuple(int(i) for i in torch.nonzero(bad)[0])
                 g = (c0 + idx[0],) + idx[1:]
+                offset = (c0 - p0 + idx[0]) * plane + int(np.ravel_multi_index(idx[1:], tuple(got.shape[1:])))
+                where = "" if boundary is None else f", element offset {offset} ({offset / boundary:.3f} x {boundary})"
                 raise AssertionError(
-                    f"{what}: sweep (criterion A) fails at element {g} (rank {r}): got {complex(got[idx])!r}, "
+                    f"{what}: sweep (criterion A) fails at element {g} ({label}{where}): got {complex(got[idx])!r}, "
                     f"X Y = {complex(want[idx])!r}, |error| {float(err[idx]):.3g} > bound {float(bound[idx]):.3g}; "
                     f"{int(bad.sum())} such elements in planes [{c0}, {c1})")
             live = bound > 0
@@ -153,6 +174,54 @@ def check_sharded(check, u, factors_fn, arrays, k, anti, rng, what, batch=4):
     """(a) on ``rank_planes`` and (b) on the whole tensor; returns (b)'s largest ratio."""
     check_planes(check, u, factors_fn, arrays, rank_planes(u, rng), k, anti, what, batch)
     return sweep(u, factors_fn, arrays, k, anti, what)
+
+
+# -------------------------------------------------------------------------------------------- poisoned memory
+
+
+class PoisonedTorch:
+    """Stands in for ``torch`` inside ``ops``: every floating-point ``empty`` / ``empty_like`` (outputs, workspaces)
+    comes back filled with NaN, 0xFF bytes for the byte workspaces (NaN doubles); everything else is torch itself."""
+
+    def __getattr__(self, name):
+        return getattr(torch, name)
+
+    @staticmethod
+    def empty(*args, **kwargs):
+        return PoisonedTorch.poison(torch.empty(*args, **kwargs))
+
+    @staticmethod
+    def empty_like(*args, **kwargs):
+        return PoisonedTorch.poison(torch.empty_like(*args, **kwargs))
+
+    @staticmethod
+    def poison(t):
+        if t.dtype == torch.uint8:
+            t.fill_(0xFF)
+        elif t.is_floating_point() or t.is_complex():
+            t.fill_(float("nan") if not t.is_complex() else complex(float("nan"), float("nan")))
+        return t
+
+
+@functools.lru_cache(maxsize=None)
+def nan_engine():
+    """``sharded.CudaEngine`` whose ``empty`` returns NaN-filled memory (NaN + NaN j), so that slabs, spare, recv,
+    per-rank scratch, padded copies and outputs are poisoned; it counts the device-side anti-symmetry tests."""
+    from quantum_systems_b200 import sharded
+
+    class NaNEngine(sharded.CudaEngine):
+        symmetry_tests = 0
+
+        def empty(self, numel, dtype):
+            buf = super().empty(numel, dtype)
+            buf.tensor.fill_(complex(float("nan"), float("nan")) if dtype == torch.complex128 else float("nan"))
+            return buf
+
+        def is_antisymmetric(self, buf, n, planes):
+            self.symmetry_tests += 1
+            return super().is_antisymmetric(buf, n, planes)
+
+    return NaNEngine
 
 
 # ------------------------------------------------------------------------------------- what a case reaches

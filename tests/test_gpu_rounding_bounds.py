@@ -75,21 +75,7 @@ def rand(rng, shape, complex_=False):
 plane_indices = SB.plane_indices
 
 
-class _PoisonedTorch:
-    """Stands in for ``torch`` inside ``ops``: every floating-point ``empty`` (outputs, workspaces) comes back filled
-    with NaN, 0xFF bytes for the byte workspaces (NaN doubles); everything else is torch itself."""
-
-    def __getattr__(self, name):
-        return getattr(torch, name)
-
-    @staticmethod
-    def empty(*args, **kwargs):
-        t = torch.empty(*args, **kwargs)
-        if t.dtype == torch.uint8:
-            t.fill_(0xFF)
-        elif t.is_floating_point() or t.is_complex():
-            t.fill_(float("nan") if not t.is_complex() else complex(float("nan"), float("nan")))
-        return t
+_PoisonedTorch = SB.PoisonedTorch
 
 
 @pytest.fixture
@@ -326,25 +312,7 @@ def test_one_body_and_functions(n, m, h_c, c_c, biorth):
 # element of every rank under criterion A.
 
 
-@functools.lru_cache(maxsize=None)
-def nan_engine():
-    """``sharded.CudaEngine`` whose ``empty`` returns NaN-filled memory (NaN + NaN j), so that slabs, spare, recv,
-    per-rank scratch, padded copies and outputs are poisoned; it counts the device-side anti-symmetry tests."""
-    from quantum_systems_b200 import sharded
-
-    class NaNEngine(sharded.CudaEngine):
-        symmetry_tests = 0
-
-        def empty(self, numel, dtype):
-            buf = super().empty(numel, dtype)
-            buf.tensor.fill_(complex(float("nan"), float("nan")) if dtype == torch.complex128 else float("nan"))
-            return buf
-
-        def is_antisymmetric(self, buf, n, planes):
-            self.symmetry_tests += 1
-            return super().is_antisymmetric(buf, n, planes)
-
-    return NaNEngine
+nan_engine = SB.nan_engine
 
 
 # (label, n, m, W, u complex, C complex, bi-orthogonal C~, graded family, chain, what the case reaches)

@@ -68,6 +68,13 @@ def test_diagonal_reference_is_exact_to_longdouble(n, m):
     got = P.odqd_rows(P.cast(C, P.LD), P.LD, grid=grid, alpha=1.0, a=0.25)
     W_ld = P.shielded_coulomb(grid, 1.0, 0.25, P.LD)
     np.testing.assert_array_equal(got, P.diagonal_rows(W_ld, P.cast(C, P.LD), P.cast(C, P.LD).T, P.LD))
+    # one plane at a time, plain and anti-symmetrised, with its absolute-value companion
+    for anti in (False, True):
+        whole, whole_abs, _ = P.companions(P.diagonal_rows, W, C, Ct, anti=anti)
+        for p in range(m):
+            plane, plane_abs, _ = P.companions(P.diagonal_plane, W, C, Ct, p=p, anti=anti)
+            np.testing.assert_array_equal(plane, whole[p])
+            np.testing.assert_array_equal(plane_abs, whole_abs[p])
 
 
 def test_kron_forms_match_the_dense_contractions():
@@ -94,6 +101,10 @@ def test_kron_forms_match_the_dense_contractions():
         ref, absval, _ = P.companions(P.kron_fock_occupied, h, A, B, n_occ=n_occ, anti=anti)
         assert np.max(np.abs(ref - dense)) <= 1e-17 * np.max(dense_abs)
         assert np.all(absval >= dense_abs * (1 - 1e-12))
+    dense, dense_abs, _ = P.companions(P.fock_occupied, h, P.kron_two_body(A, B), n_occ=n_occ, spatial=True)
+    ref, absval, _ = P.companions(P.kron_fock_occupied, h, A, B, n_occ=n_occ, spatial=True)
+    assert np.max(np.abs(ref - dense)) <= 1e-17 * np.max(dense_abs)
+    assert np.all(absval >= dense_abs * (1 - 1e-12))
     dense, dense_abs, _ = P.companions(P.occupied_traces, h, P.kron_two_body(A, B), n_occ=n_occ)
     ref, absval, _ = P.companions(P.kron_occupied_traces, h, A, B, n_occ=n_occ)
     assert np.max(np.abs(ref - dense)) <= 1e-17 * np.max(dense_abs)
