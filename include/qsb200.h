@@ -331,9 +331,10 @@ int qs_fock_density(const void* h, int h_dtype, const void* u, int u_dtype, cons
 /* Unrestricted (UHF) Fock matrices of two spin densities rho_alpha, rho_beta (n, n) of one dtype rho_dtype:
  *   f_s[p,q] = h[p,q] + sum_{r,s} u[p,r,q,s] (rho_alpha + rho_beta)[s,r] - sum_{r,s} u[p,r,s,q] rho_s[s,r]
  * for s in {alpha, beta} and p in [p_begin, p_end); u, h, f_alpha, f_beta and the row range as in qs_fock_density
- * (f_dtype is the dtype of both f).  Real u and real densities: u is read once for both spins (the packed density
- * rho_alpha + i rho_beta).  Complex u or complex densities: u is read once per density, i.e. twice.  Deterministic,
- * and a row is bit-identical whatever plane range it is computed in. */
+ * (f_dtype is the dtype of both f).  Real u: u is read once for both spins (real densities through the packed
+ * density rho_alpha + i rho_beta, complex ones in one pass over rho_alpha + rho_beta, rho_alpha and rho_beta).
+ * Complex u: u is read once per density, i.e. twice.  Deterministic, and a row is bit-identical whatever plane range
+ * it is computed in. */
 int qs_fock_density_unrestricted_workspace_bytes(int64_t n, int64_t p_begin, int64_t p_end, int u_dtype,
                                                  int rho_dtype, int64_t* bytes);
 int qs_fock_density_unrestricted(const void* h, int h_dtype, const void* u, int u_dtype, const void* rho_alpha,

@@ -29,6 +29,15 @@ in one pass.  ``spin_orbital_coefficients`` gives the ``(2l, 2l)`` coefficients 
 basis; ``GeneralOrbitalSystem(3, basis).change_basis(C)`` with them computes the same system through the
 spin-doubled ``u``: eight to ten times the tensor-core flops (twice that on a complex128 ``u``) and four
 ``(2l)^4`` buffers.
+
+``propagate(system, state, t_final, dt)`` is time-dependent Hartree-Fock: it moves the occupied orbitals of an RHF,
+GHF or UHF state under ``system.h_t(t)`` and the two-body weight of the system's time-evolution operators with
+classical RK4, one Fock build of the same kernels per stage, and records the energy and the dipole moment::
+
+    system.set_time_evolution_operator(DipoleFieldInteraction(pulse))
+    run = hartree_fock.propagate(system, state, t_final=5.0, dt=1e-2)
+    run.times, run.energy, run.dipole                     # (k,), (k,), (k, dim)
+    run = hartree_fock.propagate(system, run, t_final=10.0, dt=1e-2)    # continues from run.t
 """
 
 import dataclasses
@@ -57,6 +66,24 @@ class HartreeFockState:
     density_matrix: object
     converged: bool
     iterations: int
+
+
+@dataclasses.dataclass
+class TimeDependentHartreeFockRun:
+    """One ``propagate`` call.  ``times`` (k,), ``energy`` (k,) and ``dipole`` (k, dim) are the observables at the
+    start of every ``observe_every``-th step: ``energy`` is ``1/2 sum_s tr rho_s (h(t) + F_s(t))`` plus the nuclear
+    repulsion, ``dipole`` is ``sum_s tr rho_s d`` for each axis of ``system.dipole_moment``.  ``t`` is the time the
+    run ended at and ``C`` / ``density_matrix`` the state there, one entry per spin channel (one for RHF and GHF,
+    alpha and beta for UHF): the occupied columns ``C_o`` (l, n_occ) in complex128 and ``C_o C_o^dagger`` (times 2 for
+    RHF).  Passing the run back to ``propagate`` continues from ``t``; the observables of ``t`` itself are the first
+    ones of that next call."""
+
+    times: object
+    energy: object
+    dipole: object
+    t: float
+    C: tuple
+    density_matrix: tuple
 
 
 @dataclasses.dataclass
@@ -97,13 +124,10 @@ def ground_state(system, tol=1e-9, max_iterations=100, C=None):
     _require_4d(basis)
     restricted = isinstance(system, SpatialOrbitalSystem)
     h, s, u, C = _device_inputs(system, (C,))
-    scales = _scales(restricted, basis.anti_symmetrized_u)
-
-    def fock(rho):
-        return (ops.fock_from_density(h, u, rho[0], *scales),)
-
+    fock = _density_fock(u, _scales(restricted, basis.anti_symmetrized_u))
     occupations = ((system.n, 2 if restricted else 1),)
-    result = _scf(h, s, fock, occupations, tol, max_iterations, C, system.nuclear_repulsion_energy, None)
+    result = _scf(h, s, lambda rho: fock(h, rho), occupations, tol, max_iterations, C, system.nuclear_repulsion_energy,
+                  None)
     return _host_results(system, _hf_state(result))
 
 
@@ -143,12 +167,10 @@ def ground_state_unrestricted(system, n_alpha=None, n_beta=None, tol=1e-9, max_i
         n_beta = system.n if n_beta is None else n_beta
     n_alpha, n_beta = _occupations(n_alpha, n_beta, basis.l)
     h, s, u, C = _device_inputs(basis, (None, None) if C is None else C)
-
-    def fock(rho):
-        return ops.fock_from_density_unrestricted(h, u, *rho)
-
+    fock = _density_fock(u, None)
     occupations = ((n_alpha, 1), (n_beta, 1))
-    result = _scf(h, s, fock, occupations, tol, max_iterations, C, basis.nuclear_repulsion_energy, None)
+    result = _scf(h, s, lambda rho: fock(h, rho), occupations, tol, max_iterations, C, basis.nuclear_repulsion_energy,
+                  None)
     return _host_results(basis, _uhf_state(result, h, s, n_alpha, n_beta))
 
 
@@ -165,6 +187,189 @@ def ground_state_unrestricted_sharded(basis, n_alpha, n_beta, tol=1e-9, max_iter
     occupations = ((n_alpha, 1), (n_beta, 1))
     result = _scf(h, s, fock, occupations, tol, max_iterations, C, nuclear_repulsion_energy, agree)
     return _uhf_state(result, h, s, n_alpha, n_beta)
+
+
+def propagate(system, state, t_final, dt, observe_every=1):
+    """Time-dependent Hartree-Fock from ``state`` to ``t_final`` in fixed steps ``dt``: a ``HartreeFockState`` of
+    ``ground_state(system)`` (RHF on a ``SpatialOrbitalSystem``, GHF on a ``GeneralOrbitalSystem``), an
+    ``UnrestrictedHartreeFockState`` of ``ground_state_unrestricted(system, ...)`` on a ``SpatialOrbitalSystem``, or
+    a ``TimeDependentHartreeFockRun`` of an earlier call, which continues from its ``t`` (a state starts at t = 0).
+    Returns a ``TimeDependentHartreeFockRun``; a chain of calls computes bit for bit what one call over the whole
+    interval computes.
+
+    The occupied columns ``C_o`` of each spin channel are propagated in complex128 in the Loewdin basis
+    ``X = S^(-1/2)``: ``i dC'/dt = X^dagger F(t) X C'`` with ``C = X C'``, classical RK4, one Fock build per stage.
+    ``F(t) = h(t) + w(t) G[rho]``: ``h(t)`` is ``system.h_t(t)``; the two-body operators enter as the weight
+    ``w(t) = [add_u_0] + sum_k w_k(t)`` of their ``u_t_scaled`` pairs, whose operand must be the system's own ``u``,
+    so the n^4 tensor is never scaled or copied.  The Fock builds and channels are those of the ground-state solvers
+    (``ops.fock_from_density`` with the RHF or GHF scales, ``ops.fock_from_density_unrestricted`` for UHF).  The
+    first stage of a step gives the observables at its start without another build.  ``round((t_final - t) / dt)``
+    steps are taken; time advances by repeated addition of ``dt``.
+
+    On a device-resident system no step synchronises with the host and the observables stay in device buffers; only
+    the set-up reads the host (the overlap check of ``S``, the imaginary-part test of a complex ``u``).  Host
+    (numpy) systems upload ``u`` once and get ndarrays, read once at the end.  A complex128 ``u`` without imaginary
+    part is copied to float64 for the call, as in ``ground_state``.  2-D sinc-DVR storage, a ``ShardedBasisSet`` and
+    two-body operators on any other tensor than ``system.u`` are refused."""
+    from .sharded import ShardedBasisSet
+    from .spatial_orbital_system import SpatialOrbitalSystem
+
+    if isinstance(system, ShardedBasisSet) or isinstance(getattr(system, "_basis_set", None), ShardedBasisSet):
+        raise TypeError("propagate runs on one GPU: a ShardedBasisSet has no dipole matrices or time-evolution "
+                        "operators")
+    basis = system._basis_set
+    _require_4d(basis)
+    restricted = isinstance(system, SpatialOrbitalSystem)
+    dt, t_final, observe_every = float(dt), float(t_final), int(observe_every)
+    if not dt > 0:
+        raise ValueError(f"dt must be positive, got {dt}")
+    if observe_every < 1:
+        raise ValueError(f"observe_every must be at least 1, got {observe_every}")
+    C_occ, t, unrestricted = _propagation_start(system, basis, state, restricted)
+    if not t_final >= t:
+        raise ValueError(f"t_final = {t_final} lies before the start time {t}")
+    n_steps = int(round((t_final - t) / dt))
+
+    s = _arrays.to_device(basis.s) if basis.s is not None else None
+    u = _arrays.to_device(basis.u)
+    if _has_imag(s):
+        s = s.to(torch.complex128)
+    elif s is not None:
+        s = _as_dtype(s, torch.float64)
+    if u.is_complex() and not _has_imag(u):
+        u = _as_dtype(u, torch.float64)
+    device, cdt = u.device, torch.complex128
+    l = basis.l
+    X = _orthogonaliser(s, l, s.dtype if s is not None else torch.float64, device).to(cdt)
+    X_inv = X @ (s.to(cdt) if s is not None else torch.eye(l, dtype=cdt, device=device))  # S^(1/2)
+    Xh = X.mH.contiguous()
+    weight = 2 if restricted and not unrestricted else 1
+    fock = _density_fock(u, None if unrestricted else _scales(restricted, basis.anti_symmetrized_u))
+    d = system.dipole_moment
+    d = _arrays.to_device(d).to(cdt) if d is not None else None
+    dim = 0 if d is None else d.shape[0]
+    e_nuc = float(system.nuclear_repulsion_energy)
+
+    # the two-body weight and its checks, before any step
+    _two_body_weight(system, t)
+
+    def h_at(time):
+        return _arrays.to_device(system.h_t(time))
+
+    def derivative(time, h, Cp):
+        """``-i X^dagger F X C'`` of every channel, the densities and the Fock matrices."""
+        Cs = [X @ c for c in Cp]
+        rho = tuple(_density(c, c.shape[1], weight) for c in Cs)
+        F = fock(h, rho, _two_body_weight(system, time))
+        return [-1j * (Xh @ (f @ c)) for f, c in zip(F, Cs)], rho, F
+
+    n_obs = (n_steps + observe_every - 1) // observe_every
+    energy = torch.empty(n_obs, dtype=torch.float64, device=device)
+    dipole = torch.empty((n_obs, dim), dtype=torch.float64, device=device)
+    times = []
+    Cp = [X_inv @ _arrays.to_device(c).to(cdt) for c in C_occ]
+    h = h_at(t)
+    for step in range(n_steps):
+        k1, rho, F = derivative(t, h, Cp)
+        if step % observe_every == 0:
+            j = len(times)
+            times.append(t)
+            energy[j] = 0.5 * sum(torch.sum(r.transpose(0, 1) * (h + f)) for r, f in zip(rho, F)).real + e_nuc
+            if d is not None:
+                rho_total = sum(rho[1:], rho[0])
+                dipole[j] = torch.einsum("rs,isr->i", rho_total, d).real
+        t_mid, t_end = t + 0.5 * dt, t + dt
+        h_mid = h_at(t_mid)
+        k2 = derivative(t_mid, h_mid, [c + (0.5 * dt) * k for c, k in zip(Cp, k1)])[0]
+        k3 = derivative(t_mid, h_mid, [c + (0.5 * dt) * k for c, k in zip(Cp, k2)])[0]
+        h = h_at(t_end)
+        k4 = derivative(t_end, h, [c + dt * k for c, k in zip(Cp, k3)])[0]
+        Cp = [c + (dt / 6.0) * (a + 2.0 * b + 2.0 * e + g) for c, a, b, e, g in zip(Cp, k1, k2, k3, k4)]
+        t = t_end
+    C = tuple(X @ c for c in Cp)
+    rho = tuple(_density(c, c.shape[1], weight) for c in C)
+    times = torch.tensor(times, dtype=torch.float64).to(device, non_blocking=True)
+    return _read_run(system, TimeDependentHartreeFockRun(times, energy, dipole, t, C, rho))
+
+
+def _propagation_start(system, basis, state, restricted):
+    """The occupied columns of each channel, the start time and whether the state is unrestricted, after checking
+    that ``state`` fits ``system``."""
+    l = basis.l
+
+    def shaped(C, n_occ, what):
+        if tuple(C.shape) != (l, n_occ):
+            raise ValueError(f"{what} has shape {tuple(C.shape)}, the system needs {(l, n_occ)}")
+        return C
+
+    if isinstance(state, UnrestrictedHartreeFockState):
+        if not restricted:
+            raise ValueError("an unrestricted state propagates on the SpatialOrbitalSystem it was solved on")
+        _require_plain_spatial_u(basis, "propagate")
+        shaped(state.C_alpha, l, "C_alpha")
+        shaped(state.C_beta, l, "C_beta")
+        return (state.C_alpha[:, :state.n_alpha], state.C_beta[:, :state.n_beta]), 0.0, True
+    if isinstance(state, HartreeFockState):
+        return (shaped(state.C, l, "C")[:, :system.n],), 0.0, False
+    if isinstance(state, TimeDependentHartreeFockRun):
+        if len(state.C) == 2:
+            if not restricted:
+                raise ValueError("an unrestricted run propagates on a SpatialOrbitalSystem")
+            _require_plain_spatial_u(basis, "propagate")
+            return tuple(shaped(c, c.shape[1], f"C[{k}]") for k, c in enumerate(state.C)), float(state.t), True
+        if len(state.C) != 1:
+            raise ValueError(f"a run has one or two spin channels, got {len(state.C)}")
+        return (shaped(state.C[0], system.n, "C[0]"),), float(state.t), False
+    raise TypeError("state must be a HartreeFockState, an UnrestrictedHartreeFockState or a "
+                    f"TimeDependentHartreeFockRun, got {type(state).__name__}")
+
+
+def _two_body_weight(system, t):
+    """``w(t) = [add_u_0] + sum_k w_k(t)`` over the two-body operators of ``system``, from their ``u_t_scaled`` pairs;
+    an operator without one, or whose operand is not ``system.u``, is refused."""
+    w = 1.0 if system._add_u_0 else 0.0
+    for op in system._time_evolution_operator:
+        if not op.is_two_body_operator:
+            continue
+        scaled = getattr(op, "u_t_scaled", None)
+        weight, operand = scaled(t) if scaled is not None else (None, None)
+        if operand is not system.u:
+            raise ValueError(f"propagate folds two-body operators into the Fock build as a weight on system.u; "
+                             f"{type(op).__name__} does not scale system.u")
+        w = w + weight
+    return w
+
+
+def _read_run(system, run):
+    """``run`` with its tensors as ndarrays when ``system`` keeps its arrays on the host: the one read of the call."""
+    if not _arrays.is_host_module(system.np):
+        return run
+    host = _arrays.to_host
+    return dataclasses.replace(run, times=host(run.times), energy=host(run.energy), dipole=host(run.dipole),
+                               C=tuple(host(c) for c in run.C),
+                               density_matrix=tuple(host(r) for r in run.density_matrix))
+
+
+def _density_fock(u, scales):
+    """The Fock build of the single-GPU solvers and the propagator: ``fock(h, rho, w=1)`` maps the tuple of channel
+    densities to the tuple of Fock matrices ``h + w G[rho]``.  ``scales`` (direct, exchange) give one channel through
+    ``ops.fock_from_density`` (``w`` multiplies the scales); None gives the two UHF channels through
+    ``ops.fock_from_density_unrestricted``, which takes no scales, so ``w != 1`` builds ``G`` on a zero ``h`` and adds
+    ``h + w G`` on the n^2 side."""
+    if scales is not None:
+        a_d, a_x = scales
+
+        def fock(h, rho, w=1.0):
+            return (ops.fock_from_density(h, u, rho[0], w * a_d, w * a_x),)
+
+        return fock
+
+    def fock(h, rho, w=1.0):
+        if w == 1.0:
+            return ops.fock_from_density_unrestricted(h, u, *rho)
+        return tuple(h + w * g for g in ops.fock_from_density_unrestricted(torch.zeros_like(h), u, *rho))
+
+    return fock
 
 
 def _device_inputs(source, guesses):

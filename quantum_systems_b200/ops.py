@@ -421,8 +421,8 @@ def fock_from_density(h, u, rho, scale_direct, scale_exchange, f=None, planes=No
 def fock_from_density_unrestricted(h, u, rho_alpha, rho_beta, f_alpha=None, f_beta=None, planes=None):
     """Both unrestricted Fock matrices ``f_s[p,q] = h[p,q] + sum_rs u[p,r,q,s] (rho_a + rho_b)[s,r]
     - sum_rs u[p,r,s,q] rho_s[s,r]`` of the spin densities ``rho_alpha`` and ``rho_beta`` on a spatial ``u``
-    (``qs_fock_density_unrestricted``).  Real ``u`` and real densities: ``u`` is read once for both spins; complex
-    ``u`` or a complex density: twice.  ``planes``, the in-place ``f_alpha`` / ``f_beta`` and the result dtype
+    (``qs_fock_density_unrestricted``).  Real ``u``: ``u`` is read once for both spins, with real or complex
+    densities; complex ``u``: twice.  ``planes``, the in-place ``f_alpha`` / ``f_beta`` and the result dtype
     follow ``fock_from_density``; a real density is promoted to complex when the other one is complex.
     Returns ``(f_alpha, f_beta)``."""
     return _fock_density(
