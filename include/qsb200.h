@@ -341,6 +341,20 @@ int qs_fock_density_unrestricted(const void* h, int h_dtype, const void* u, int 
                                  const void* rho_beta, int rho_dtype, int64_t n, void* f_alpha, void* f_beta,
                                  int f_dtype, int64_t p_begin, int64_t p_end, void* workspace,
                                  int64_t workspace_bytes, void* stream);
+/* Coulomb and exchange matrices of a batch of k real densities rho (k, n, n) in one read of a real u:
+ *   J[d,p,q] = sum_{r,s} u[p,r,q,s] rho[d,s,r]        K[d,p,q] = sum_{r,s} u[p,r,s,q] rho[d,s,r]
+ * for d < k <= QS_COULOMB_EXCHANGE_MAX_BATCH and p in [p_begin, p_end), on the FP64 tensor pipe.  `u` points at plane
+ * p_begin as in qs_fock_density; J and K are whole (k, n, n) arrays and rows outside [p_begin, p_end) are not
+ * touched.  u and rho must be F64 (complex ones are refused); n <= 384.  Deterministic (no atomics), with per-(plane,
+ * r-chunk) partial rows in the workspace (qs_coulomb_exchange_batch_workspace_bytes) summed in a fixed order that
+ * depends on n only: a density's J and K are bit-identical whatever the other densities of the batch, its position
+ * and k, and a row is bit-identical whatever plane range it is computed in. */
+#define QS_COULOMB_EXCHANGE_MAX_BATCH 16
+int qs_coulomb_exchange_batch_workspace_bytes(int64_t n, int64_t k, int64_t p_begin, int64_t p_end, int u_dtype,
+                                              int rho_dtype, int64_t* bytes);
+int qs_coulomb_exchange_batch(const void* u, int u_dtype, const void* rho, int rho_dtype, int64_t n, int64_t k,
+                              void* J, void* K, int64_t p_begin, int64_t p_end, void* workspace,
+                              int64_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * ODQD grid Coulomb build  u_abcd = sum_pq C_pa C_qb C_pc C_qd alpha/sqrt((x_p-x_q)^2 + a^2)

@@ -67,6 +67,8 @@ SIGNATURES = {
     "qs_fock_density": [_ptr, _int, _ptr, _int, _ptr, _int, _i64, _dbl, _dbl, _ptr, _int, _i64, _i64, _ptr, _i64, _ptr],
     "qs_fock_density_unrestricted_workspace_bytes": [_i64, _i64, _i64, _int, _int, ctypes.POINTER(_i64)],
     "qs_fock_density_unrestricted": [_ptr, _int, _ptr, _int, _ptr, _ptr, _int, _i64, _ptr, _ptr, _int, _i64, _i64, _ptr, _i64, _ptr],
+    "qs_coulomb_exchange_batch_workspace_bytes": [_i64, _i64, _i64, _i64, _int, _int, ctypes.POINTER(_i64)],
+    "qs_coulomb_exchange_batch": [_ptr, _int, _ptr, _int, _i64, _i64, _ptr, _ptr, _i64, _i64, _ptr, _i64, _ptr],
     "qs_odqd_coulomb_workspace_bytes": [_i64, _i64, ctypes.POINTER(_i64)],
     "qs_odqd_coulomb": [_ptr, _ptr, _dbl, _dbl, _i64, _i64, _ptr, _ptr, _i64, _ptr],
     "qs_odqd_coulomb_planes": [_ptr, _ptr, _dbl, _dbl, _i64, _i64, _ptr, _i64, _i64, _ptr, _i64, _ptr],

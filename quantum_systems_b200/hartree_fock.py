@@ -292,6 +292,302 @@ def propagate(system, state, t_final, dt, observe_every=1):
     return _read_run(system, TimeDependentHartreeFockRun(times, energy, dipole, t, C, rho))
 
 
+@dataclasses.dataclass
+class ExcitedStates:
+    """Linear-response excited states of one ``excited_states`` call, roots in ascending ``energies`` (n_states,).
+    ``X`` and ``Y`` hold one ``(n_states, n_occ, n_virt)`` array per spin channel (one for RHF and GHF, alpha and
+    beta for UHF), normalised to ``sum X^2 - sum Y^2 = 1`` over all channels; ``Y`` is zero for TDA.
+    ``transition_dipole`` (n_states, dim) is ``<0|d|n>`` for each axis of ``system.dipole_moment`` (sqrt 2 times the
+    spatial sum for RHF singlets, zero for RHF triplets) and ``oscillator_strength`` is ``2 omega |mu_a|^2`` per
+    axis.  ``residual_norms`` are the final residuals of the roots, ``converged`` says whether all are at most
+    ``tol``, ``iterations`` counts subspace iterations and ``densities_built`` the AO densities contracted with u."""
+
+    energies: object
+    X: tuple
+    Y: tuple
+    transition_dipole: object
+    oscillator_strength: object
+    residual_norms: object
+    converged: bool
+    iterations: int
+    densities_built: int
+
+
+def excited_states(system, state, n_states=5, tda=False, spin="singlet", tol=1e-6, max_iterations=100):
+    """Linear-response TDHF (RPA, or the Tamm-Dancoff approximation with ``tda=True``) excitation energies of a
+    converged reference: a ``HartreeFockState`` on a ``SpatialOrbitalSystem`` (RHF, ``spin="singlet"`` or
+    ``"triplet"``) or a ``GeneralOrbitalSystem`` (GHF), or an ``UnrestrictedHartreeFockState`` on a
+    ``SpatialOrbitalSystem`` (UHF, spin-conserving).  Returns ``ExcitedStates``; host (numpy) systems get ndarrays.
+
+    With ``F`` the Fock matrix of the state's density and ``(pq|rs) = u[p,r,q,s]``, ``A = dF + <aj||ib>`` and
+    ``B = <ab||ij>`` (GHF; RHF and UHF in their spin-adapted forms), ``dF = delta_ij F_ab - delta_ab F_ij``.  ``A +- B``
+    act on a trial vector ``Z`` of each channel through the AO density ``T = C_o Z C_v^T``: the two-electron part of
+    ``(A +- B) Z`` is ``C_v^T G[T^T +- T] C_o`` and that of ``A Z`` is ``C_v^T G[T^T] C_o``, with ``G`` the Coulomb and
+    exchange combination of the channel (RHF singlet ``2J - K``, triplet ``-K``, GHF the ground-state scales, UHF
+    ``J[D_alpha] + J[D_beta] - K[D_sigma]``).  All densities of an iteration go through one
+    ``ops.coulomb_exchange`` call, the only O(n^4) step; the rest is torch on the device.  TDA is a Davidson
+    iteration on ``A``; RPA the real symmetric subspace method of Stratmann, Scuseria and Frisch (J. Chem. Phys. 109,
+    8218 (1998)): ``A + B`` and ``A - B`` projected onto one expansion space, ``(A-B)^(1/2) (A+B) (A-B)^(1/2) z =
+    omega^2 z``, residuals preconditioned with ``(dF_diag - omega)^-1``.  The space starts from the unit vectors of
+    the lowest ``dF`` diagonal and is capped at the dimension ``n_occ n_virt``, where Rayleigh-Ritz is exact.  A
+    projected ``A - B`` or ``A + B`` that is not positive definite means an unstable reference: RPA raises
+    ``ValueError``; TDA returns the negative root.
+
+    Refused: a ``ShardedBasisSet`` and 2-D sinc-DVR storage, a complex working dtype (complex orbitals), an
+    unconverged state or one that does not fit ``system``, ``spin`` other than singlet or triplet or a triplet of
+    GHF or UHF, ``n_states`` outside ``[1, n_occ n_virt]`` and a reference without virtual orbitals.  A complex128
+    ``u`` without imaginary part is copied to float64 for the call, as in ``ground_state``."""
+    from .sharded import ShardedBasisSet
+    from .spatial_orbital_system import SpatialOrbitalSystem
+
+    if isinstance(system, ShardedBasisSet) or isinstance(getattr(system, "_basis_set", None), ShardedBasisSet):
+        raise TypeError("excited_states runs on one GPU: a ShardedBasisSet is not supported")
+    basis = system._basis_set
+    _require_4d(basis)
+    restricted = isinstance(system, SpatialOrbitalSystem)
+    if spin not in ("singlet", "triplet"):
+        raise ValueError(f"spin must be 'singlet' or 'triplet', got {spin!r}")
+    l = basis.l
+    if isinstance(state, UnrestrictedHartreeFockState):
+        if not restricted:
+            raise ValueError("an unrestricted state is solved on the SpatialOrbitalSystem it came from")
+        _require_plain_spatial_u(basis, "excited_states")
+        kind = "uhf"
+        coefficients = (state.C_alpha, state.C_beta)
+        occupied = (state.n_alpha, state.n_beta)
+    elif isinstance(state, HartreeFockState):
+        kind = "rhf" if restricted else "ghf"
+        coefficients, occupied = (state.C,), (system.n,)
+    else:
+        raise TypeError("state must be a HartreeFockState or an UnrestrictedHartreeFockState, "
+                        f"got {type(state).__name__}")
+    if spin == "triplet" and kind != "rhf":
+        raise ValueError(f"spin='triplet' is an RHF option; a {kind.upper()} reference has no spin adaptation")
+    if not state.converged:
+        raise ValueError("the reference state is not converged")
+    for C in coefficients:
+        if tuple(C.shape) != (l, l):
+            raise ValueError(f"the state has {tuple(C.shape)} coefficients, the system needs {(l, l)}")
+    if not all(0 <= n_occ <= l for n_occ in occupied):
+        raise ValueError(f"occupations {occupied} do not fit l = {l}")
+    sizes = [n_occ * (l - n_occ) for n_occ in occupied]
+    dim = sum(sizes)
+    if dim == 0:
+        raise ValueError("the reference has no virtual orbitals (or no occupied ones): nothing to excite")
+    n_states = int(n_states)
+    if not 1 <= n_states <= dim:
+        raise ValueError(f"n_states = {n_states} must lie in [1, {dim}] (n_occ * n_virt)")
+
+    h = _arrays.to_device(basis.h)
+    u = _arrays.to_device(basis.u)
+    Cs = [_arrays.to_device(C) for C in coefficients]
+    if any(_has_imag(t) for t in (h, u, *Cs)):
+        raise NotImplementedError("excited_states needs real orbitals and a real u: complex orbitals are not "
+                                  "supported")
+    h, u = _as_dtype(h, torch.float64), _as_dtype(u, torch.float64)
+    Cs = [_as_dtype(C, torch.float64) for C in Cs]
+
+    # the Fock matrices of the reference from one existing build, and the response scales (J, K) of each channel
+    if kind == "uhf":
+        F = _density_fock(u, None)(h, tuple(_density(C, n_occ, 1) for C, n_occ in zip(Cs, occupied)))
+        scales = (1.0, -1.0)
+    else:
+        F = _density_fock(u, _scales(restricted, basis.anti_symmetrized_u))(
+            h, (_density(Cs[0], occupied[0], 2 if restricted else 1),))
+        if kind == "rhf":
+            scales = (2.0, -1.0) if spin == "singlet" else (0.0, -1.0)
+        else:
+            scales = _scales(False, basis.anti_symmetrized_u)
+    channels = []
+    for C, f, n_occ in zip(Cs, F, occupied):
+        C_o, C_v = C[:, :n_occ].contiguous(), C[:, n_occ:].contiguous()
+        channels.append((C_o, C_v, C_o.T @ f @ C_o, C_v.T @ f @ C_v))
+    diagonal = torch.cat([(torch.diagonal(F_vv)[None, :] - torch.diagonal(F_oo)[:, None]).reshape(-1)
+                          for _, _, F_oo, F_vv in channels])
+    counter = [0]
+
+    def products(V, signs):
+        """``(A + s B) V`` for each ``s`` in ``signs`` (None: ``A`` alone) on the rows of ``V`` (m, dim)."""
+        m = V.shape[0]
+        Zs, Ts, offset = [], [], 0
+        for (C_o, C_v, _, _), size in zip(channels, sizes):
+            Z = V[:, offset:offset + size].reshape(m, C_o.shape[1], C_v.shape[1])
+            offset += size
+            Zs.append(Z)
+            Ts.append(C_o @ Z @ C_v.T)
+        densities = [T.transpose(1, 2) + (0.0 if s is None else s) * T for s in signs for T in Ts]
+        J, K = ops.coulomb_exchange(u, torch.cat(densities).contiguous())
+        counter[0] += J.shape[0]
+        J = J.reshape(len(signs), len(Ts), m, l, l)
+        K = K.reshape(len(signs), len(Ts), m, l, l)
+        out = []
+        for a in range(len(signs)):
+            J_total = J[a].sum(dim=0) if kind == "uhf" else J[a, 0]
+            parts = []
+            for c, ((C_o, C_v, F_oo, F_vv), Z) in enumerate(zip(channels, Zs)):
+                G = scales[0] * J_total + scales[1] * K[a, c]
+                parts.append((Z @ F_vv - F_oo @ Z + C_o.T @ G.transpose(1, 2) @ C_v).reshape(m, -1))
+            out.append(torch.cat(parts, dim=1))
+        return out
+
+    solve = _davidson_tda if tda else _davidson_rpa
+    omega, XpY, XmY, residuals, converged, iterations = solve(products, diagonal, n_states, tol, max_iterations)
+    X, Y = 0.5 * (XpY + XmY), 0.5 * (XpY - XmY)
+    # one sign per root: the largest component of X positive
+    pick = torch.argmax(X.abs(), dim=1)
+    sign = torch.sign(X.gather(1, pick[:, None]))
+    sign[sign == 0] = 1.0
+    X, Y, XpY = X * sign, Y * sign, XpY * sign
+
+    d = system.dipole_moment
+    n_axes = 0 if d is None else d.shape[0]
+    mu = torch.zeros((n_states, n_axes), dtype=torch.float64, device=u.device)
+    if d is not None and not (kind == "rhf" and spin == "triplet"):
+        d = _arrays.to_device(d)
+        if _has_imag(d):
+            raise NotImplementedError("excited_states needs a real dipole moment")
+        d = _as_dtype(d, torch.float64)
+        offset = 0
+        for (C_o, C_v, _, _), size in zip(channels, sizes):
+            d_ov = (C_o.T @ d @ C_v).reshape(n_axes, -1)
+            mu += XpY[:, offset:offset + size] @ d_ov.T
+            offset += size
+        if kind == "rhf":
+            mu *= 2.0 ** 0.5
+    strength = 2.0 * omega[:, None] * mu ** 2
+
+    def split(M):
+        out, offset = [], 0
+        for (C_o, C_v, _, _), size in zip(channels, sizes):
+            out.append(M[:, offset:offset + size].reshape(n_states, C_o.shape[1], C_v.shape[1]).contiguous())
+            offset += size
+        return tuple(out)
+
+    result = ExcitedStates(energies=omega, X=split(X), Y=split(Y), transition_dipole=mu, oscillator_strength=strength,
+                           residual_norms=residuals, converged=converged, iterations=iterations,
+                           densities_built=counter[0])
+    if _arrays.is_host_module(system.np):
+        host = _arrays.to_host
+        result = dataclasses.replace(result, energies=host(result.energies), X=tuple(host(x) for x in result.X),
+                                     Y=tuple(host(y) for y in result.Y),
+                                     transition_dipole=host(result.transition_dipole),
+                                     oscillator_strength=host(result.oscillator_strength),
+                                     residual_norms=host(result.residual_norms))
+    return result
+
+
+# a correction whose norm falls below this fraction of its length before projection adds nothing new to the space
+_DEPENDENT = 1e-8
+
+
+def _expand(basis, vectors, dim):
+    """``basis`` (m, dim), orthonormal rows, extended by the parts of ``vectors`` orthogonal to it and to each other
+    (two Gram-Schmidt passes), at most to ``dim`` rows.  Returns ``(basis, new rows)``."""
+    new = []
+    for v in vectors:
+        if basis.shape[0] + len(new) >= dim:
+            break
+        length = torch.linalg.vector_norm(v)
+        if not length > 0:
+            continue
+        v = v / length
+        Q = torch.cat([basis, *[w[None] for w in new]]) if new else basis
+        for _ in range(2):
+            v = v - (Q @ v) @ Q
+        norm = float(torch.linalg.vector_norm(v))
+        if norm > _DEPENDENT:
+            new.append(v / norm)
+    if not new:
+        return basis, basis[:0]
+    added = torch.stack(new)
+    return torch.cat([basis, added]), added
+
+
+def _start(diagonal, n_states):
+    """Unit vectors at the lowest entries of the orbital-energy diagonal: ``2 n_states`` of them, at most all."""
+    dim = diagonal.shape[0]
+    count = min(dim, 2 * n_states)
+    order = torch.argsort(diagonal, stable=True)[:count]
+    return torch.eye(dim, dtype=torch.float64, device=diagonal.device)[order]
+
+
+def _precondition(R, diagonal, omega):
+    den = diagonal[None, :] - omega[:, None]
+    den = torch.where(den.abs() < 1e-8, torch.copysign(torch.full_like(den, 1e-8), den), den)
+    return R / den
+
+
+def _davidson_tda(products, diagonal, n_states, tol, max_iterations):
+    """Davidson on ``A``; returns ``(omega, X, X, residual norms, converged, iterations)``."""
+    dim = diagonal.shape[0]
+    basis = diagonal.new_zeros((0, dim))
+    AV = diagonal.new_zeros((0, dim))
+    basis, new = _expand(basis, _start(diagonal, n_states), dim)
+    it = 0
+    for it in range(1, max_iterations + 1):
+        AV = torch.cat([AV, products(new, (None,))[0]])
+        a = basis @ AV.T
+        w, z = torch.linalg.eigh(0.5 * (a + a.T))
+        omega, z = w[:n_states], z[:, :n_states]
+        x = z.T @ basis
+        R = z.T @ AV - omega[:, None] * x
+        norms = torch.linalg.vector_norm(R, dim=1)
+        done = norms <= tol
+        if bool(done.all()) or it == max_iterations:
+            break
+        basis, new = _expand(basis, _precondition(R[~done], diagonal, omega[~done]), dim)
+        if new.shape[0] == 0:
+            break
+    return omega, x, x, norms, bool(done.all()), it
+
+
+def _davidson_rpa(products, diagonal, n_states, tol, max_iterations):
+    """Stratmann-Scuseria-Frisch on ``A + B`` and ``A - B``; returns ``(omega, X + Y, X - Y, residual norms,
+    converged, iterations)`` with ``(X + Y) . (X - Y) = 1``."""
+    dim = diagonal.shape[0]
+    basis = diagonal.new_zeros((0, dim))
+    PV = diagonal.new_zeros((0, dim))
+    MV = diagonal.new_zeros((0, dim))
+    basis, new = _expand(basis, _start(diagonal, n_states), dim)
+    it = 0
+    for it in range(1, max_iterations + 1):
+        plus, minus = products(new, (1.0, -1.0))
+        PV, MV = torch.cat([PV, plus]), torch.cat([MV, minus])
+        mp, mm = basis @ PV.T, basis @ MV.T
+        mp, mm = 0.5 * (mp + mp.T), 0.5 * (mm + mm.T)
+        em, Vm = torch.linalg.eigh(mm)
+        ep = torch.linalg.eigvalsh(mp)
+        if not float(em.min()) > 0:
+            raise ValueError(f"A - B is not positive definite in the subspace (eigenvalue {float(em.min()):.3e}): "
+                             "the reference is unstable, RPA has no real excitation energies")
+        if not float(ep.min()) > 0:
+            raise ValueError(f"A + B is not positive definite in the subspace (eigenvalue {float(ep.min()):.3e}): "
+                             "the reference is unstable, RPA has no real excitation energies")
+        root = (Vm * em.sqrt()) @ Vm.T
+        root_inv = (Vm * em.rsqrt()) @ Vm.T
+        H = root @ mp @ root
+        w2, z = torch.linalg.eigh(0.5 * (H + H.T))
+        omega = w2[:n_states].sqrt()
+        z = z[:, :n_states]
+        xp = (root @ z) / omega.sqrt()
+        xm = (root_inv @ z) * omega.sqrt()
+        XpY, XmY = xp.T @ basis, xm.T @ basis
+        R_plus = xp.T @ PV - omega[:, None] * XmY
+        R_minus = xm.T @ MV - omega[:, None] * XpY
+        norms = torch.sqrt(torch.linalg.vector_norm(R_plus, dim=1) ** 2
+                           + torch.linalg.vector_norm(R_minus, dim=1) ** 2)
+        done = norms <= tol
+        if bool(done.all()) or it == max_iterations:
+            break
+        open_ = ~done
+        corrections = torch.cat([_precondition(R_plus[open_], diagonal, omega[open_]),
+                                 _precondition(R_minus[open_], diagonal, omega[open_])])
+        basis, new = _expand(basis, corrections, dim)
+        if new.shape[0] == 0:
+            break
+    return omega, XpY, XmY, norms, bool(done.all()), it
+
+
 def _propagation_start(system, basis, state, restricted):
     """The occupied columns of each channel, the start time and whether the state is unrestricted, after checking
     that ``state`` fits ``system``."""

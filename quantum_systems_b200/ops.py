@@ -451,30 +451,77 @@ def _fock_density(entry, h, u, densities, fs, scales, planes):
         shapes = ", ".join(str(tuple(t.shape)) for t in (h, *rhos, u))
         raise ValueError(f"{', '.join(['h'] + names[:-1])} and {names[-1]} must be (n,n) and u (planes,n,n,n), "
                          f"got {shapes}")
-    outs = []
-    for name, f in fs.items():
-        if f is None:
-            alloc = torch.empty if (p0, p1) == (0, n) else torch.zeros
-            f = alloc((n, n), dtype=_result_dtype(h, u, *rhos), device=h.device)
-        else:
-            if not (isinstance(f, torch.Tensor) and f.is_cuda and f.is_contiguous()):
-                raise RuntimeError(f"{name} must be a contiguous CUDA tensor to be filled in place")
-            if tuple(f.shape) != (n, n):
-                raise ValueError(f"{name} must be {(n, n)}, got {tuple(f.shape)}")
-            _code(f)
-            _mark_written(f)
-        outs.append(f)
+    dtype = _result_dtype(h, u, *rhos)
+    outs = [_plane_output(name, f, (n, n), dtype, h.device, (p0, p1) == (0, n)) for name, f in fs.items()]
     if len(outs) > 1 and outs[0].dtype != outs[1].dtype:
         raise ValueError(f"{' and '.join(fs)} must have one dtype, got {outs[0].dtype} and {outs[1].dtype}")
-    nbytes = ctypes.c_int64(0)
-    _native.call(entry + "_workspace_bytes", n, p0, p1, _code(u), _code(rhos[0]), ctypes.byref(nbytes))
-    owner, ws = _workspace(nbytes.value, h.device)
+    owner, ws, nbytes = _entry_workspace(entry, h.device, n, p0, p1, _code(u), _code(rhos[0]))
     _native.call(
         entry, _ptr(h), _code(h), _ptr(u), _code(u), *[_ptr(r) for r in rhos], _code(rhos[0]), n, *scales,
-        *[_ptr(f) for f in outs], _code(outs[0]), p0, p1, ws, nbytes.value, _stream(),
+        *[_ptr(f) for f in outs], _code(outs[0]), p0, p1, ws, nbytes, _stream(),
     )
     owner.record_stream(torch.cuda.current_stream())
     return tuple(outs)
+
+
+def _plane_output(name, out, shape, dtype, device, whole):
+    """An output of a plane-range front end: a new tensor (``torch.empty`` when the call writes it ``whole``, else
+    zeros, so rows outside the plane range read zero), or the caller's ``out``, checked and marked written."""
+    if out is None:
+        return (torch.empty if whole else torch.zeros)(shape, dtype=dtype, device=device)
+    if not (isinstance(out, torch.Tensor) and out.is_cuda and out.is_contiguous()):
+        raise RuntimeError(f"{name} must be a contiguous CUDA tensor to be filled in place")
+    if tuple(out.shape) != shape:
+        raise ValueError(f"{name} must be {shape}, got {tuple(out.shape)}")
+    _code(out)
+    return _mark_written(out)
+
+
+def _entry_workspace(entry, device, *args):
+    """The scratch ``entry + "_workspace_bytes"`` asks for with ``args``: ``(owner, pointer, bytes)``."""
+    nbytes = ctypes.c_int64(0)
+    _native.call(entry + "_workspace_bytes", *args, ctypes.byref(nbytes))
+    owner, ws = _workspace(nbytes.value, device)
+    return owner, ws, nbytes.value
+
+
+# densities per launch of qs_coulomb_exchange_batch (QS_COULOMB_EXCHANGE_MAX_BATCH in include/qsb200.h)
+COULOMB_EXCHANGE_MAX_BATCH = 16
+
+
+def coulomb_exchange(u, rho, planes=None, J=None, K=None):
+    """Coulomb and exchange matrices ``J[d,p,q] = sum_rs u[p,r,q,s] rho[d,s,r]`` and ``K[d,p,q] = sum_rs u[p,r,s,q]
+    rho[d,s,r]`` of a batch of real densities ``rho`` (k, n, n) on a real ``u`` (``qs_coulomb_exchange_batch``, on the
+    FP64 tensor pipe).  Each launch reads ``u`` once for up to ``COULOMB_EXCHANGE_MAX_BATCH`` densities; a larger
+    batch takes ``ceil(k / COULOMB_EXCHANGE_MAX_BATCH)`` launches.  A density's ``J`` and ``K`` are bit-identical
+    whatever else is in the batch.  ``planes``, the in-place ``J`` / ``K`` and the zero rows of new outputs outside
+    the plane range follow ``fock_from_density``.  Complex ``u`` or densities are refused.  Returns ``(J, K)``."""
+    u = _device_tensor(u, "u")
+    rho = _device_tensor(rho, "rho")
+    if rho.dim() != 3 or rho.shape[0] < 1 or rho.shape[1] != rho.shape[2]:
+        raise ValueError(f"rho must be a batch (k, n, n) of k >= 1 densities, got {tuple(rho.shape)}")
+    k, n = rho.shape[0], rho.shape[1]
+    p0, p1 = (0, n) if planes is None else (int(planes[0]), int(planes[1]))
+    if not 0 <= p0 <= p1 <= n:
+        raise ValueError(f"planes {planes} out of range for n = {n}")
+    if tuple(u.shape) != (p1 - p0, n, n, n):
+        raise ValueError(f"u must be (planes, n, n, n) = {(p1 - p0, n, n, n)}, got {tuple(u.shape)}")
+    for name, t in (("rho", rho), ("J", J), ("K", K)):
+        if t is not None and isinstance(t, torch.Tensor) and t.device != u.device:
+            raise ValueError(f"{name} lives on {t.device}, u on {u.device}")
+    whole = (p0, p1) == (0, n)
+    J, K = (_plane_output(name, out, (k, n, n), torch.float64, u.device, whole) for name, out in (("J", J), ("K", K)))
+    if J.dtype != torch.float64 or K.dtype != torch.float64:
+        raise ValueError(f"J and K must be float64, got {J.dtype} and {K.dtype}")
+    entry = "qs_coulomb_exchange_batch"
+    owner, ws, nbytes = _entry_workspace(entry, u.device, n, min(k, COULOMB_EXCHANGE_MAX_BATCH), p0, p1, _code(u),
+                                         _code(rho))
+    for d0 in range(0, k, COULOMB_EXCHANGE_MAX_BATCH):
+        d1 = min(k, d0 + COULOMB_EXCHANGE_MAX_BATCH)
+        _native.call(entry, _ptr(u), _code(u), _ptr(rho[d0:d1]), _code(rho), n, d1 - d0, _ptr(J[d0:d1]),
+                     _ptr(K[d0:d1]), p0, p1, ws, nbytes, _stream())
+    owner.record_stream(torch.cuda.current_stream())
+    return J, K
 
 
 def odqd_coulomb(C, inner_grid, alpha, a, planes=None):
